@@ -12,9 +12,10 @@ region.  The single-stream latency (one sequence, p50 / p95 per frame, C2 / C3 /
 `next_rows` times the callers either side of the path (SURVEY 8f: YUV input stage, FAST, reprojector, pose and structure
 optimisers, seed initialisation) on the device next to the reference's code on one host core.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--seqs TOTAL]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--seqs TOTAL] [--dump-outputs DIR]
 """
 import argparse
+import atexit
 import json
 import os
 import subprocess
@@ -27,6 +28,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True           # the benchmark writes nothing into the tree it runs from (it may be read-only)
 
 from android_svo_b200 import synth, frontend, sharding  # noqa: E402
 
@@ -66,7 +68,13 @@ def parse_args():
                     help="insert a keyframe every K frames INSIDE the timed region, in both arms (svob200_tracker_add_keyframe / "
                          "DepthFilter::addKeyframe: occupancy, FAST + Shi-Tomasi + grid, seed initialisation; seeds of up to 4 keyframes, "
                          "ageing by max_n_kfs = 3, finished seeds leave the pool): FAST shows up in a step time")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (the per-sequence step records and a fixed, "
+                         "seeded sample of the seed states; rank 0's sequences) as DIR/<name>.npy, to compare two builds output for output")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
+    return args
 
 
 def ping_pong(n_pool, n_steps):
@@ -158,6 +166,8 @@ class ClockSampler:
                                       stdout=self.f, stderr=subprocess.DEVNULL)
         except Exception:
             self.p = None
+        if self.p is not None:
+            atexit.register(self.p.kill)     # a run that fails inside the load window must not leave the poller behind
 
     def stop(self, t0=None, t1=None):
         import datetime
@@ -456,6 +466,21 @@ def seed_workload_of(obs, capi, regime):
             "note": "direct = epipolar segment shorter than 2 px (align2D at the midpoint, matcher.cpp:257-278); walk = ZMSSD over the segment"}
 
 
+DUMP_MAX_SEEDS = 1 << 20      # 20 MB of float32 seed states: the dump stays well under 64 MB at any batch size
+
+
+def dump_outputs(out_dir, stats, seeds):
+    """The last timed step's results as float64 / float32 .npy files: every field of the step records of every sequence, and
+    the seed states (a, b, mu, z_range, sigma2) of all pool slots, or of a fixed seeded sample of DUMP_MAX_SEEDS slots."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name in stats.dtype.names:
+        np.save(os.path.join(out_dir, "step_%s.npy" % name), stats[name].astype(np.float64))
+    idx = np.arange(len(seeds))
+    if len(idx) > DUMP_MAX_SEEDS:
+        idx = np.sort(np.random.RandomState(0).choice(len(seeds), DUMP_MAX_SEEDS, replace=False))
+    np.save(os.path.join(out_dir, "seeds.npy"), np.stack([seeds[k][idx] for k in seeds.dtype.names], 1).astype(np.float32))
+
+
 def run_b200(args, rank, world, local_rank):
     import torch
     import torch.distributed as dist
@@ -508,6 +533,8 @@ def run_b200(args, rank, world, local_rank):
     value = total * K / (ms * 1e-3)
     stats_dev_copy = np.zeros(wl.B, capi.step_stats_dt)
     ctx.dev_download(stats_dev_copy, wl.stats_dev)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, stats_dev_copy, wl.trk.seeds())
 
     # ---------------- stage breakdown (separate, untimed-for-the-headline pass)
     wl.trk.enable_profiling(True)
