@@ -457,6 +457,7 @@ int svob200_match_direct(svob200_ctx* ctx, int64_t cur_frame_id, const svob200_c
   FrameRec* cur = find_frame(ctx, cur_frame_id);
   if (!cur) return fail(ctx, SVOB200_ERR_NOFRAME, "match_direct: current frame not resident");
   if (opts->max_search_level >= cur->f.n_levels) return fail(ctx, SVOB200_ERR_ARG, "match_direct: max_search_level outside the pyramid");
+  if (opts->max_epi_search_steps < 0) return fail(ctx, SVOB200_ERR_ARG, "match_direct: negative max_epi_search_steps");
   if (n == 0) return SVOB200_OK;
   Stage st(ctx, mem);
   const int i_f = st.add(ftrs, nullptr, sizeof(svob200_feature_ref) * n, 0);
@@ -481,6 +482,7 @@ int svob200_epipolar_match(svob200_ctx* ctx, int64_t cur_frame_id, const svob200
   FrameRec* cur = find_frame(ctx, cur_frame_id);
   if (!cur) return fail(ctx, SVOB200_ERR_NOFRAME, "epipolar_match: current frame not resident");
   if (opts->max_search_level >= cur->f.n_levels) return fail(ctx, SVOB200_ERR_ARG, "epipolar_match: max_search_level outside the pyramid");
+  if (opts->max_epi_search_steps < 0) return fail(ctx, SVOB200_ERR_ARG, "epipolar_match: negative max_epi_search_steps");
   if (n == 0) return SVOB200_OK;
   Stage st(ctx, mem);
   const int i_f = st.add(ftrs, nullptr, sizeof(svob200_feature_ref) * n, 0);
@@ -506,6 +508,7 @@ int svob200_seeds_update(svob200_ctx* ctx, int64_t cur_frame_id, const svob200_c
   FrameRec* cur = find_frame(ctx, cur_frame_id);
   if (!cur) return fail(ctx, SVOB200_ERR_NOFRAME, "seeds_update: current frame not resident");
   if (opts->max_search_level >= cur->f.n_levels) return fail(ctx, SVOB200_ERR_ARG, "seeds_update: max_search_level outside the pyramid");
+  if (opts->max_epi_search_steps < 0) return fail(ctx, SVOB200_ERR_ARG, "seeds_update: negative max_epi_search_steps");
   if (n == 0) return SVOB200_OK;
   Stage st(ctx, mem);
   const int i_f = st.add(ftrs, nullptr, sizeof(svob200_feature_ref) * n, 0);
@@ -806,6 +809,7 @@ int svob200_reproject_map(svob200_ctx* ctx, int64_t cur_frame_id, const svob200_
   if (!cur) return fail(ctx, SVOB200_ERR_NOFRAME, "reproject_map: current frame not resident");
   if (batch != cur->f.batch) return fail(ctx, SVOB200_ERR_ARG, "reproject_map: batch differs from the frame's");
   if (opts->max_search_level >= cur->f.n_levels) return fail(ctx, SVOB200_ERR_ARG, "reproject_map: max_search_level outside the pyramid");
+  if (opts->max_epi_search_steps < 0) return fail(ctx, SVOB200_ERR_ARG, "reproject_map: negative max_epi_search_steps");
   const int gc = (cam->width + cell_size - 1) / cell_size, gr = (cam->height + cell_size - 1) / cell_size;
   const size_t n_cells = (size_t)gc * gr;
   Stage st(ctx, mem);

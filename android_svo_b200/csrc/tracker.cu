@@ -450,6 +450,7 @@ int svob200_tracker_create(svob200_ctx* ctx, const svob200_camera* cam, int batc
     return fail(ctx, SVOB200_ERR_ARG, "tracker_create: alignment level range [%d,%d] outside the %d-level pyramid", aopts->min_level, aopts->max_level, n_levels);
   if (mopts->max_search_level < 0 || mopts->max_search_level >= n_levels)
     return fail(ctx, SVOB200_ERR_ARG, "tracker_create: max_search_level %d outside the %d-level pyramid", mopts->max_search_level, n_levels);
+  if (mopts->max_epi_search_steps < 0) return fail(ctx, SVOB200_ERR_ARG, "tracker_create: negative max_epi_search_steps %d", mopts->max_epi_search_steps);
   if (cam->width <= 0 || cam->height <= 0) return fail(ctx, SVOB200_ERR_ARG, "tracker_create: bad camera size");
   static std::atomic<int64_t> uid_counter{0};
   const int64_t uid = ++uid_counter;

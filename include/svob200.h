@@ -157,6 +157,8 @@ typedef struct {
   double epi_search_edgelet_max_angle;
   int max_search_level;            /* Config::nPyrLevels()-1 */
 } svob200_matcher_opts;
+/* max_epi_search_steps: 0 .. INT_MAX (the reference's size_t, clamped); a walk of up to that many steps is searched,
+ * whatever its length.  Every entry point that takes these options returns SVOB200_ERR_ARG for a negative value. */
 void svob200_matcher_opts_default(svob200_matcher_opts* o, int n_pyr_levels);
 
 /* reference-side description of one feature (Feature{px,f,level,type,grad}, feature.h:24-76) */

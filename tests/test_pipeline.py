@@ -89,10 +89,14 @@ class SeedParity:
       free     runs on its own aligned pose -> value tolerance 1e-5 relative; seeds outside it are COUNTED, and each one must be
                reproduced bit for bit by the pinned oracle (i.e. the deviation is the 1e-10 pose difference moving a float
                rounding of 1/z or tau^2, amplified by the cancellation in sigma2 = C1(s2+m^2) + C2(sigma2+mu^2) - mu_new^2)
-      pinned   gets the device's pose injected -> discrete decisions and seed bits must be IDENTICAL (count asserted 0)"""
+      pinned   gets the device's pose injected -> discrete decisions and seed bits must be IDENTICAL (count asserted 0)
+    Under the pinned pose the observations themselves are compared too: epi_length bit-exact wherever the matcher ran, the
+    triangulated depth z within 1e-12 relative wherever a seed was updated.  In the young-seed regime (every seed reset to its
+    prior after each frame) equal seed states prove little; the observations carry the information."""
 
     def __init__(self):
         self.n_seeds = self.n_outside_tol = self.n_pinned_bit_diff = self.n_discrete_diff = self.n_free_discrete_diff = 0
+        self.n_evals = self.n_long_walks = 0
 
     def check(self, seeds_gpu, obs_gpu, free, pinned):
         sg = seed_matrix(seeds_gpu)
@@ -105,6 +109,12 @@ class SeedParity:
             self.n_free_discrete_diff += int((obs_gpu[key] != of[key]).sum())
         upd = obs_gpu["status"] >= 3
         assert np.array_equal(obs_gpu["px_cur"][upd], op["px_cur"][upd]), "matched pixel differs under the same pose"
+        assert np.array_equal(obs_gpu["epi_length"][upd].view(np.uint64), op["epi_length"][upd].view(np.uint64)), \
+            "epipolar segment length differs under the same pose"
+        tri = (obs_gpu["status"] >= 4) & (op["status"] >= 4)
+        assert np.all(np.abs(obs_gpu["z"][tri] - op["z"][tri]) <= 1e-12 * np.abs(op["z"][tri])), "triangulated depth differs under the same pose"
+        self.n_evals += int(obs_gpu["n_evals"].sum())
+        self.n_long_walks += int((upd & (obs_gpu["epi_length"] / 0.7 > 64)).sum())
         bit_diff = (sg.view(np.uint32) != sp.view(np.uint32)).any(axis=1)
         self.n_pinned_bit_diff += int(bit_diff.sum())
         # own pose: 1e-5 relative, deviations counted and each explained by the pinned oracle
@@ -113,27 +123,47 @@ class SeedParity:
         assert not (outside & bit_diff).any(), "a seed deviates from the oracle beyond 1e-5 and the pose difference does not explain it"
         assert np.allclose(sg, sf, rtol=2e-2, atol=0), "a seed deviates grossly from the free-running oracle"
 
+    def mean_evals(self):
+        return self.n_evals / max(self.n_seeds, 1)
+
     def finish(self, max_outside_frac=0.01):
         print("seed parity: %d seed-frames, %d outside 1e-5 vs the free-running oracle (all reproduced bit-exactly under the device's pose), "
-              "%d bit differences / %d discrete differences under the same pose, %d discrete differences vs the free-running oracle"
-              % (self.n_seeds, self.n_outside_tol, self.n_pinned_bit_diff, self.n_discrete_diff, self.n_free_discrete_diff))
+              "%d bit differences / %d discrete differences under the same pose, %d discrete differences vs the free-running oracle; "
+              "mean n_evals %.2f, %d walks longer than 64 samples"
+              % (self.n_seeds, self.n_outside_tol, self.n_pinned_bit_diff, self.n_discrete_diff, self.n_free_discrete_diff,
+                 self.mean_evals(), self.n_long_walks))
         assert self.n_discrete_diff == 0, "%d discrete seed decisions differ under the same pose" % self.n_discrete_diff
         assert self.n_pinned_bit_diff == 0, "%d seeds differ in bits under the same pose" % self.n_pinned_bit_diff
         assert self.n_outside_tol <= max_outside_frac * self.n_seeds
 
+    def assert_young(self):
+        """the regime really is young: far more ZMSSD evaluations per seed than the steady regime's 2.6, and long walks"""
+        assert self.mean_evals() > 2 * 2.6 and self.n_long_walks > 0, (self.mean_evals(), self.n_long_walks)
+
+
+# bench.py --seed-regime: steady re-initialises finished seeds (the defaults), young re-initialises every seed after every frame
+# to a wide prior (reseed = 2, depth_min = 0.3)
+REGIMES = {"steady": (100.0, 2.4, 1.2, 1), "young": (100.0, 2.4, 0.3, 2)}
+
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("mode", ["host", "device"])
-@pytest.mark.parametrize("name,batch,n_frames", [("C2", 3, 10), ("C3", 2, 4), ("C2", 1, 6)])
-def test_tracker_step_matches_oracle(ctx, oracle, name, batch, n_frames, mode):
+@pytest.mark.parametrize("regime", ["steady", "young"])
+@pytest.mark.parametrize("name,batch,n_frames", [("C2", 3, 10), ("C3", 2, 4), ("C2", 1, 6), ("C2", 70, 4)])
+def test_tracker_step_matches_oracle(ctx, oracle, name, batch, n_frames, mode, regime):
+    """svob200_tracker_step against the oracle, in both seed regimes of bench.py.  A batch above 64 runs direct launches, the
+    asynchronous depth filter and a two-wave search grid; it replicates 3 distinct sequences, and every replica must return
+    the bit-identical step record, refined pixels, seed state and seed observations of its first copy."""
     from android_svo_b200 import capi
-    seqs = [make_sequence(oracle, name, 0x00C0FFEE + i, n_frames + 1) for i in range(batch)]
+    n_distinct = min(batch, 3)
+    seqs = [make_sequence(oracle, name, 0x00C0FFEE + i, n_frames + 1) for i in range(n_distinct)]
+    which = np.arange(batch) % n_distinct
     cfg = seqs[0][0]
     cam_o, cam_g = scenes.cam_of(cfg, Cam), scenes.cam_of(cfg, capi.Camera)
     args = (cfg["n_levels"], cfg["max_level"], cfg["min_level"], cfg["n_pyr"])
-    free = [OracleSeq(oracle, cam_o, *args) for _ in range(batch)]
-    pinned = [OracleSeq(oracle, cam_o, *args) for _ in range(batch)]
-    trk = capi.Tracker(ctx, cam_g, batch, *args)
+    free = [OracleSeq(oracle, cam_o, *args, *REGIMES[regime]) for _ in range(n_distinct)]
+    pinned = [OracleSeq(oracle, cam_o, *args, *REGIMES[regime]) for _ in range(n_distinct)]
+    trk = capi.Tracker(ctx, cam_g, batch, *args, *REGIMES[regime])
     par = SeedParity()
     try:
         N, S = cfg["n_features"], cfg["n_seeds"]
@@ -141,18 +171,24 @@ def test_tracker_step_matches_oracle(ctx, oracle, name, batch, n_frames, mode):
             for s, (_, poses, imgs, kf, _) in zip(grp, seqs):
                 s.set_keyframe(imgs[0], poses[0], kf["kf_px"], kf["kf_level"], kf["pt_world"], kf["seed_px"], kf["seed_level"])
                 s.set_last(imgs[0])
-        cat = lambda key: np.concatenate([q[3][key] for q in seqs])
-        trk.set_keyframe(np.stack([q[2][0] for q in seqs]), np.stack([q[1][0] for q in seqs]), np.arange(batch + 1) * N,
+        cat = lambda key: np.concatenate([seqs[w][3][key] for w in which])
+        trk.set_keyframe(np.stack([seqs[w][2][0] for w in which]), np.stack([seqs[w][1][0] for w in which]), np.arange(batch + 1) * N,
                          cat("kf_px"), cat("kf_level"), cat("pt_world"), np.arange(batch + 1) * S, cat("seed_px"), cat("seed_level"))
         if mode == "host":
-            trk.set_last(np.stack([q[2][0] for q in seqs]))
+            trk.set_last(np.stack([seqs[w][2][0] for w in which]))
         else:
-            trk.set_last_device(np.stack([q[2][0] for q in seqs]))
+            trk.set_last_device(np.stack([seqs[w][2][0] for w in which]))
         for k in range(1, n_frames + 1):
-            stats, px, ok = gpu_step(trk, mode, np.stack([q[2][k] for q in seqs]), np.stack([q[1][k - 1] for q in seqs]),
-                                     np.concatenate([q[4][k - 1] for q in seqs]), want_px=True)
+            stats, px, ok = gpu_step(trk, mode, np.stack([seqs[w][2][k] for w in which]), np.stack([seqs[w][1][k - 1] for w in which]),
+                                     np.concatenate([seqs[w][4][k - 1] for w in which]), want_px=True)
             seeds_g, obs_g = trk.seeds(), trk.seed_obs()
-            for b in range(batch):
+            for b in range(n_distinct, batch):
+                d = which[b]
+                assert stats[b].tobytes() == stats[d].tobytes(), "replica %d of sequence %d: step record differs" % (b, d)
+                assert np.array_equal(px[b * N:(b + 1) * N], px[d * N:(d + 1) * N]) and np.array_equal(ok[b * N:(b + 1) * N], ok[d * N:(d + 1) * N])
+                assert seeds_g[b * S:(b + 1) * S].tobytes() == seeds_g[d * S:(d + 1) * S].tobytes()
+                assert obs_g[b * S:(b + 1) * S].tobytes() == obs_g[d * S:(d + 1) * S].tobytes()
+            for b in range(n_distinct):
                 g = stats[b]
                 e, pxe, oke = free[b].step(seqs[b][2][k], seqs[b][1][k - 1], seqs[b][4][k - 1], want_px=True)
                 pinned[b].set_pose_override(g["T_cur_w"])
@@ -171,6 +207,8 @@ def test_tracker_step_matches_oracle(ctx, oracle, name, batch, n_frames, mode):
                     assert g[key] == getattr(p, key), key
                 par.check(seeds_g[b * S:(b + 1) * S], obs_g[b * S:(b + 1) * S], free[b], pinned[b])
         par.finish()
+        if regime == "young":
+            par.assert_young()
     finally:
         trk.close()
         for s in free + pinned:
@@ -256,58 +294,74 @@ def test_tracker_step_full_size_c4(ctx, oracle):
 def test_tracker_c5_size_replicas(ctx, oracle):
     """BASELINE.json configs[4] at its full size (4,096 sequences in one batch) through a size-independent property:
     the batch holds 32 distinct sequences, each replicated 128 times at scattered batch positions; every replica must
-    return the bit-identical step record, refined pixels and seed state (no cross-talk, no dependence on the position
-    in the batch or on which SM / group processed it), and replica 0 of each sequence must match the oracle.
+    return the bit-identical step record, refined pixels, seed state and seed observations (no cross-talk, no dependence
+    on the position in the batch or on which SM / group processed it), and replica 0 of each sequence must match the oracle.
     Runs the EXACT path bench.py's `value` times — SVOB200_MEM_DEVICE: svob200_frame_bind_only aliasing + ONE 4,096-wide
     range (491 k candidates, 3.1 M seeds per launch) — and the SVOB200_MEM_HOST path (16 chunks of 256 on a copy stream):
-    the two must agree bit for bit."""
+    the two must agree bit for bit.  Four steps, so that the frame slot the asynchronous depth filter searches is reused while
+    that filter runs; in both seed regimes of bench.py."""
     from android_svo_b200 import capi
-    n_distinct, B = 32, 4096
-    seqs = [make_sequence(oracle, "C2", 0x00C0FFEE + 100 + i, 3) for i in range(n_distinct)]
+    n_distinct, B, n_steps = 32, 4096, 4
+    seqs = [make_sequence(oracle, "C2", 0x00C0FFEE + 100 + i, n_steps + 1) for i in range(n_distinct)]
     cfg = seqs[0][0]
     cam_o, cam_g = scenes.cam_of(cfg, Cam), scenes.cam_of(cfg, capi.Camera)
     args = (cfg["n_levels"], cfg["max_level"], cfg["min_level"], cfg["n_pyr"])
     N, S = cfg["n_features"], cfg["n_seeds"]
     which = (np.arange(B) * 13) % n_distinct                      # scattered assignment of sequences to batch slots
     take = lambda key: np.concatenate([seqs[w][3][key] for w in which])
-    frames = [np.stack([seqs[w][2][k] for w in which]) for k in range(3)]
-    res = {}
-    for mode in ("device", "host"):
-        trk = capi.Tracker(ctx, cam_g, B, *args)
-        try:
-            trk.set_keyframe(frames[0], np.stack([seqs[w][1][0] for w in which]), np.arange(B + 1) * N,
-                             take("kf_px"), take("kf_level"), take("pt_world"), np.arange(B + 1) * S, take("seed_px"), take("seed_level"))
-            (trk.set_last if mode == "host" else trk.set_last_device)(frames[0])
-            for k in (1, 2):
-                stats, px, ok = gpu_step(trk, mode, frames[k], np.stack([seqs[w][1][k - 1] for w in which]),
-                                         np.concatenate([seqs[w][4][k - 1] for w in which]), want_px=True)
-            res[mode] = (stats, px, ok, trk.seeds(), trk.seed_obs())
-        finally:
-            trk.close()
-    for name, x, y in zip(("stats", "px", "ok", "seeds", "seed_obs"), res["device"], res["host"]):
-        assert x.tobytes() == y.tobytes(), "%s differs between the one-range device path and the chunked host path" % name
-    stats, px, ok, seeds, obs = res["device"]
-    px = px.reshape(B, N, 2); ok = ok.reshape(B, N)
-    seeds = seed_matrix(seeds).reshape(B, S, 5)
-    for d in range(n_distinct):
-        idx = np.nonzero(which == d)[0]
-        first = idx[0]
-        for name in stats.dtype.names:
-            assert (stats[name][idx] == stats[name][first]).all(), "replicas of sequence %d differ in %s" % (d, name)
-        assert (px[idx] == px[first]).all() and (ok[idx] == ok[first]).all()
-        assert (seeds[idx].view(np.uint32) == seeds[first].view(np.uint32)).all()
-    for d in range(0, n_distinct, 8):                          # a few against the oracle
-        so = OracleSeq(oracle, cam_o, *args)
-        _, poses, imgs, kf, last_px = seqs[d]
-        so.set_keyframe(imgs[0], poses[0], kf["kf_px"], kf["kf_level"], kf["pt_world"], kf["seed_px"], kf["seed_level"]); so.set_last(imgs[0])
-        for k in (1, 2):
-            e, pxe, oke = so.step(imgs[k], poses[k - 1], last_px[k - 1], want_px=True)
-        first = np.nonzero(which == d)[0][0]
-        g = stats[first]
-        rot, trans = synth.pose_error(g["T_cur_w"], np.array(e.T_cur_w[:]))
-        assert rot < 1e-9 and trans < 1e-9 and g["n_matched"] == e.n_matched and g["n_seeds_updated"] == e.n_seeds_updated
-        assert np.array_equal(ok[first], oke) and np.abs(px[first] - pxe).max() <= 1e-3
-        so.close()
+    frames = [np.stack([seqs[w][2][k] for w in which]) for k in range(n_steps + 1)]
+    for regime in ("steady", "young"):
+        res, device_poses = {}, []
+        for mode in ("device", "host"):
+            trk = capi.Tracker(ctx, cam_g, B, *args, *REGIMES[regime])
+            try:
+                trk.set_keyframe(frames[0], np.stack([seqs[w][1][0] for w in which]), np.arange(B + 1) * N,
+                                 take("kf_px"), take("kf_level"), take("pt_world"), np.arange(B + 1) * S, take("seed_px"), take("seed_level"))
+                (trk.set_last if mode == "host" else trk.set_last_device)(frames[0])
+                for k in range(1, n_steps + 1):
+                    stats, px, ok = gpu_step(trk, mode, frames[k], np.stack([seqs[w][1][k - 1] for w in which]),
+                                             np.concatenate([seqs[w][4][k - 1] for w in which]), want_px=True)
+                    if mode == "device":
+                        device_poses.append(stats["T_cur_w"].copy())
+                res[mode] = (stats, px, ok, trk.seeds(), trk.seed_obs())
+            finally:
+                trk.close()
+        for name, x, y in zip(("stats", "px", "ok", "seeds", "seed_obs"), res["device"], res["host"]):
+            assert x.tobytes() == y.tobytes(), "%s: %s differs between the one-range device path and the chunked host path" % (regime, name)
+        stats, px, ok, seeds_flat, obs_flat = res["device"]
+        px = px.reshape(B, N, 2); ok = ok.reshape(B, N)
+        seeds, obs = seed_matrix(seeds_flat).reshape(B, S, 5), obs_flat.reshape(B, S)
+        for d in range(n_distinct):
+            idx = np.nonzero(which == d)[0]
+            first = idx[0]
+            for name in stats.dtype.names:
+                assert (stats[name][idx] == stats[name][first]).all(), "%s: replicas of sequence %d differ in %s" % (regime, d, name)
+            assert (px[idx] == px[first]).all() and (ok[idx] == ok[first]).all()
+            assert (seeds[idx].view(np.uint32) == seeds[first].view(np.uint32)).all()
+            assert all(obs[i].tobytes() == obs[first].tobytes() for i in idx)
+        par = SeedParity()
+        for d in range(0, n_distinct, 8):                      # a few against the oracle: free-running, and pinned to the device's poses
+            so, sp = OracleSeq(oracle, cam_o, *args, *REGIMES[regime]), OracleSeq(oracle, cam_o, *args, *REGIMES[regime])
+            try:
+                _, poses, imgs, kf, last_px = seqs[d]
+                first = np.nonzero(which == d)[0][0]
+                for s in (so, sp):
+                    s.set_keyframe(imgs[0], poses[0], kf["kf_px"], kf["kf_level"], kf["pt_world"], kf["seed_px"], kf["seed_level"]); s.set_last(imgs[0])
+                for k in range(1, n_steps + 1):
+                    e, pxe, oke = so.step(imgs[k], poses[k - 1], last_px[k - 1], want_px=True)
+                    sp.set_pose_override(device_poses[k - 1][first])
+                    p = sp.step(imgs[k], poses[k - 1], last_px[k - 1])
+                g = stats[first]
+                rot, trans = synth.pose_error(g["T_cur_w"], np.array(e.T_cur_w[:]))
+                assert rot < 1e-9 and trans < 1e-9 and g["n_matched"] == e.n_matched and g["n_seeds_updated"] == p.n_seeds_updated, regime
+                assert np.array_equal(ok[first], oke) and np.abs(px[first] - pxe).max() <= 1e-3, regime
+                par.check(seeds_flat[first * S:(first + 1) * S], obs_flat[first * S:(first + 1) * S], so, sp)
+            finally:
+                so.close(); sp.close()
+        par.finish()
+        if regime == "young":
+            # (the tracker-step test asserts the long walks; these four sequences need not have one in four steps)
+            assert par.mean_evals() > 2 * 2.6, par.mean_evals()
 
 
 def test_oracle_chain_matches_reference(oracle, ref):
