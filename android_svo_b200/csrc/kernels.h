@@ -72,7 +72,6 @@ struct __align__(16) SeedRef {
   int pad2[3];
 };
 static_assert(sizeof(SeedRef) == 64, "SeedRef must be two 32-byte sectors");
-constexpr int SEED_RANGES = 8;
 // per (keyframe, image): T_ref_cur = ref.T_f_w * cur.T_f_w^-1 (depth_filter.cpp:263), its inverse (:264), the matcher's
 // T_cur_ref = cur.T_f_w * ref.T_f_w^-1 (matcher.cpp:216) and px_error_angle (depth_filter.cpp:245-247)
 struct __align__(16) SeedPoseRec { double T_ref_cur[7], T_cur_ref[7], T_cur_ref_m[7]; double px_error_angle; };
@@ -85,7 +84,6 @@ int launch_seeds_update_compact(const DevFrame* d_frames, int cur_slot, const De
                                 const int* d_kf_slot, int batch, const SeedPoseRec* d_pose_table, int batch_counter, int max_n_kfs,
                                 svob200_matcher_opts opts, double conv_thresh,
                                 svob200_seed* d_seeds, svob200_seed_obs* d_obs, void* d_scratch, int scratch_total, int first,
-                                int range /* < SEED_RANGES: sub-ranges in flight together use distinct job regions / counters */,
                                 cudaStream_t s, long long* launches, cudaEvent_t* marks = nullptr);
 int launch_update_seed(int n, const float* d_x, const float* d_tau2, svob200_seed* d_seeds, cudaStream_t s, long long* launches);
 int launch_compute_tau(int n, const double* d_T, const double* d_f, const double* d_z, double angle, double* d_out,

@@ -20,7 +20,6 @@
 // own problem.  The epipolar sample positions come from the reference's running sum `uv += step`, replayed by two lanes of the
 // group (x and y are independent chains).  Only libm calls (acos/sin/atan/exp) are tolerance-matched — and fed the same pose they
 // reproduce the oracle's seeds bit for bit (DESIGN.md section 3).
-#include <cstdlib>
 #include <cuda_fp16.h>
 #include "common.cuh"
 #include "kernels.h"
@@ -1424,16 +1423,11 @@ static int search_sms()
 }
 // Grid of the search kernel = SEARCH_CTAS resident CTAs per SM times `waves`: 1 = persistent (every CTA lives for the whole kernel);
 // more = CTAs that retire during the kernel, so that CTAs of a higher-priority stream (the tracking chain running beside an
-// asynchronous depth filter) find free slots.  SVOB200_SEARCH_WAVES overrides (A/B runs).
+// asynchronous depth filter) find free slots.  The LK job list (job_capacity) is sized for grids of up to SEARCH_MAX_WAVES waves:
+// 4 leaves headroom over the 2 waves seeds_update_impl launches.
 constexpr int SEARCH_MAX_WAVES = 4;
-static int search_waves_override()
-{
-  static const int v = [] { const char* e = getenv("SVOB200_SEARCH_WAVES"); const int w = e ? atoi(e) : 0; return (w < 0 || w > SEARCH_MAX_WAVES) ? 0 : w; }();
-  return v;
-}
 static int search_grid(int n, int waves = 1)
 {
-  if (search_waves_override()) waves = search_waves_override();
   const int want = (n + 4 * GPW - 1) / (4 * GPW), cap = search_sms() * SEARCH_CTAS * waves;
   return want < cap ? want : cap;
 }
@@ -1468,13 +1462,10 @@ int launch_epipolar(const DevFrame* d_frames, int cur_slot, const DevCam& cam, i
   return cudaGetLastError() == cudaSuccess ? 0 : -1;
 }
 
-// The seed list may be processed as up to SEED_RANGES sub-ranges IN FLIGHT TOGETHER (the tracker pipelines sub-batches over two
-// streams): range r compacts its LK jobs into its own region [first_r + r * slack, ...) behind its own counter.
-static size_t job_slack() { return job_capacity(0); }
 size_t seeds_scratch_bytes(int n)
 {
   const size_t m = (size_t)(n > 0 ? n : 1);
-  return up256(m * sizeof(SearchTask)) + up256(m * sizeof(SeedMatch)) + up256((m + SEED_RANGES * job_slack()) * sizeof(LkJob)) + 512;
+  return up256(m * sizeof(SearchTask)) + up256(m * sizeof(SeedMatch)) + up256(job_capacity(m) * sizeof(LkJob)) + 512;
 }
 
 // DepthFilter::updateSeeds for n seeds: geometry (thread) -> search (group, persistent) -> LK (thread per job) -> update (thread).
@@ -1483,16 +1474,15 @@ size_t seeds_scratch_bytes(int n)
 template <class SRC>
 static int seeds_update_impl(const DevFrame* d_frames, int cur_slot, const DevCam& cam, int n, const SRC& src,
                              svob200_matcher_opts opts, double conv_thresh, svob200_seed* d_seeds, svob200_seed_obs* d_obs, void* d_scratch,
-                             int scratch_total, int first, int range, cudaStream_t s, long long* launches, cudaEvent_t* marks)
+                             int scratch_total, int first, cudaStream_t s, long long* launches, cudaEvent_t* marks)
 {
   if (n <= 0) return 0;
-  if (range < 0 || range >= SEED_RANGES) return -1;
   const size_t m = (size_t)(scratch_total > 0 ? scratch_total : 1);
   char* p = static_cast<char*>(d_scratch);
   SearchTask* tasks = reinterpret_cast<SearchTask*>(p) + first; p += up256(m * sizeof(SearchTask));
   SeedMatch* match = reinterpret_cast<SeedMatch*>(p) + first; p += up256(m * sizeof(SeedMatch));
-  LkJob* jobs = reinterpret_cast<LkJob*>(p) + first + (size_t)range * job_slack(); p += up256((m + SEED_RANGES * job_slack()) * sizeof(LkJob));
-  int* count = reinterpret_cast<int*>(p) + range;
+  LkJob* jobs = reinterpret_cast<LkJob*>(p) + first; p += up256(job_capacity(m) * sizeof(LkJob));
+  int* count = reinterpret_cast<int*>(p);
   seeds_geom_kernel<SRC><<<(n + 127) / 128, 128, 0, s>>>(cam, n, src, opts, d_seeds, tasks, count);
   if (marks) cudaEventRecord(marks[0], s);
   // small seed lists (the shard of an 8-GPU run): two waves of CTAs instead of a persistent grid, so that the tracking chain of the next
@@ -1517,7 +1507,7 @@ int launch_seeds_update(const DevFrame* d_frames, int cur_slot, const DevCam& ca
                         cudaStream_t s, long long* launches, cudaEvent_t* marks)
 {
   SeedSrcApi src{d_ftrs, d_T_ref_w, d_T_cur_w};
-  return seeds_update_impl(d_frames, cur_slot, cam, n, src, opts, conv_thresh, d_seeds, d_obs, d_scratch, scratch_total, first, 0, s, launches, marks);
+  return seeds_update_impl(d_frames, cur_slot, cam, n, src, opts, conv_thresh, d_seeds, d_obs, d_scratch, scratch_total, first, s, launches, marks);
 }
 
 // rows (keyframe k, image b), b in [image0, image0 + n_images), of the pose table the compact seed kernels read
@@ -1534,11 +1524,11 @@ int launch_seed_pose_table(const DevCam& cam, int batch, int n_kfs, int image0, 
 int launch_seeds_update_compact(const DevFrame* d_frames, int cur_slot, const DevCam& cam, int n, SeedRef* d_refs,
                                 const int* d_kf_slot, int batch, const SeedPoseRec* d_pose_table, int batch_counter, int max_n_kfs,
                                 svob200_matcher_opts opts, double conv_thresh,
-                                svob200_seed* d_seeds, svob200_seed_obs* d_obs, void* d_scratch, int scratch_total, int first, int range,
+                                svob200_seed* d_seeds, svob200_seed_obs* d_obs, void* d_scratch, int scratch_total, int first,
                                 cudaStream_t s, long long* launches, cudaEvent_t* marks)
 {
   SeedSrcCompact src{d_refs, d_pose_table, d_kf_slot, batch, batch_counter, max_n_kfs};
-  return seeds_update_impl(d_frames, cur_slot, cam, n, src, opts, conv_thresh, d_seeds, d_obs, d_scratch, scratch_total, first, range, s, launches, marks);
+  return seeds_update_impl(d_frames, cur_slot, cam, n, src, opts, conv_thresh, d_seeds, d_obs, d_scratch, scratch_total, first, s, launches, marks);
 }
 
 int launch_update_seed(int n, const float* d_x, const float* d_tau2, svob200_seed* d_seeds, cudaStream_t s, long long* launches)

@@ -9,9 +9,6 @@
 // ever re-read from HBM.  Both reference roundings are implemented bit-exactly:
 //   SSE2  : avg_epu8 of the row pair then avg_epu16 of neighbours (round-half-up twice)
 //   TRUNC : (a+b+c+d)>>2  (scalar and NEON paths)
-#include <cuda.h>
-#include <cstdlib>
-#include <algorithm>
 #include "common.cuh"
 #include "kernels.h"
 
@@ -161,7 +158,8 @@ __device__ __forceinline__ void tile_level(const uint8_t* src, uint8_t* dst, int
 // (Measured alone, tools/pyr_probe.py, 4,096 VGA frames x 4 levels: 0.292 ms = 5.73 TB/s algorithmic = 0.876 of the copy peak.
 // PERSISTENT CTAs walking the tiles with a grid stride, 8 or 6 per SM, measured 0.362 / 0.394 ms: a CTA that loops has a block
 // barrier between tiles and nothing in flight across it, where the hardware scheduler starts the next short-lived CTA while the
-// previous one's last warps drain.)
+// previous one's last warps drain.  A persistent TMA-load version reached the same bandwidth, lost inside the tracker step and
+// was removed: DESIGN §8.)
 // Thread t: 16-pixel segment (t&7) of row pair (t>>3).
 // YUV = true: level 0 is PRODUCED here from the camera's YUV planes (and written once) instead of being read,
 // so the input stage costs no extra pass over the frame.
@@ -236,109 +234,6 @@ __global__ void __launch_bounds__(PNT) pyramid_fused_kernel(DevFrame f, int mode
 #undef PYR_LEVEL
 }
 
-// ---------------------------------------------------------------- the same pyramid with TMA loads (large batches)
-// A persistent CTA per resident slot walks the level-0 tiles with a grid stride; one thread keeps TMA_STAGES tiles in flight with
-// cp.async.bulk.tensor (a 3-D tensor map over x, y, image: box 128 x 64 x 1, rows and columns past the image arrive as zeros),
-// each landing on its own mbarrier; the 256 threads take their two 16-byte segments from shared memory instead of global memory
-// and run the unchanged reduction.  A stage is re-armed right after the block barrier that follows its last read.
-constexpr int TMA_STAGES = 3;
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity)
-{
-  uint32_t done = 0;
-  for (int spin = 0; !done; ++spin) {
-    asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                 : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-    if (spin > (1 << 24)) __trap();                      // a tile that never lands is a bug, not a reason to hang the GPU
-  }
-}
-
-template <int NL, int TW_, int TH_>
-__global__ void __launch_bounds__(PNT) pyramid_tma_kernel(const __grid_constant__ CUtensorMap map0, DevFrame f, int modes_mask, int tiles_x, int tiles_y)
-{
-  __shared__ __align__(128) uint8_t s_tile[TMA_STAGES][TH_ * TW_];  // level-0 tiles in flight (8 KB each)
-  __shared__ __align__(16) uint8_t s_a[(TH_ / 2) * (TW_ / 2)];      // level-1 tile 64 x 32
-  __shared__ __align__(16) uint8_t s_b[(TH_ / 4) * (TW_ / 4)];      // level-2 tile 32 x 16
-  __shared__ __align__(8) unsigned long long s_bar[TMA_STAGES];
-  __shared__ int4 s_coord[TMA_STAGES];                              // (image, tile x0, tile y0) of the tile in flight in a stage
-  const int t = threadIdx.x;
-  const int per_image = tiles_x * tiles_y;
-  const int total = per_image * f.batch;                            // (the launcher keeps this below 2^31)
-  const int G = gridDim.x;
-  // thread 0 does all the index arithmetic of a tile, once, when it puts the tile in flight
-  auto issue = [&](int tile, int stage) {
-    const int b = tile / per_image;
-    const int rem = tile - b * per_image;
-    const int tyi = rem / tiles_x;
-    const int x = (rem - tyi * tiles_x) * TW_, y = tyi * TH_;
-    s_coord[stage] = make_int4(b, x, y, 0);
-    const uint32_t bar = smem_u32(&s_bar[stage]);
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(bar), "r"(TH_ * TW_) : "memory");
-    asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
-                 :: "r"(smem_u32(s_tile[stage])), "l"(reinterpret_cast<uint64_t>(&map0)), "r"(x), "r"(y), "r"(b), "r"(bar) : "memory");
-  };
-  if (t == 0) {
-#pragma unroll
-    for (int k = 0; k < TMA_STAGES; ++k) asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" :: "r"(smem_u32(&s_bar[k])) : "memory");
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-#pragma unroll
-    for (int k = 0; k < TMA_STAGES; ++k) { const int tile = (int)blockIdx.x + k * G; if (tile < total) issue(tile, k); }
-  }
-  __syncthreads();
-  int stage = 0;
-  uint32_t parity = 0;
-  for (int tile = blockIdx.x; tile < total; tile += G) {
-    const int4 co = s_coord[stage];
-    const int b = co.x, tx0 = co.y, ty0 = co.z;
-    mbar_wait(smem_u32(&s_bar[stage]), parity);
-    // ---- level 0 -> 1 (registers)
-    {
-      constexpr int SEGS = TW_ / 16;                      // 16-byte segments per tile row; PNT / SEGS row pairs = TH_ / 2
-      static_assert(SEGS * (TH_ / 2) == PNT, "one 16-byte segment of one row pair per thread");
-      const int seg = t % SEGS, rp = t / SEGS;
-      const int x0 = tx0 + seg * 16, y0 = ty0 + rp * 2;
-      const int w1 = f.w[1], h1 = f.h[1];
-      const int x1 = x0 >> 1, y1 = y0 >> 1;
-      uint32_t o0 = 0, o1 = 0;
-      if ((y1 < h1) && (x1 < w1)) {
-        const uint4 r0 = *reinterpret_cast<const uint4*>(&s_tile[stage][(2 * rp) * TW_ + seg * 16]);
-        const uint4 r1 = *reinterpret_cast<const uint4*>(&s_tile[stage][(2 * rp + 1) * TW_ + seg * 16]);
-        if (modes_mask & 1) {
-          o0 = half4_sse2(r0.x, r0.y, r1.x, r1.y);
-          o1 = half4_sse2(r0.z, r0.w, r1.z, r1.w);
-        } else {
-          o0 = half4_trunc(r0.x, r0.y, r1.x, r1.y);
-          o1 = half4_trunc(r0.z, r0.w, r1.z, r1.w);
-        }
-        uint8_t* out = f.lvl[1] + (size_t)b * f.img_stride[1] + (size_t)y1 * f.pitch[1] + x1;
-        if (x1 + 8 <= f.pitch[1]) {
-          *reinterpret_cast<uint2*>(out) = make_uint2(o0, o1);     // pitch padding absorbs the tail
-        } else {
-          for (int k = 0; k < 8 && x1 + k < w1; ++k) out[k] = (uint8_t)(((k < 4 ? o0 : o1) >> (8 * (k & 3))) & 0xff);
-        }
-      }
-      if (NL > 2) *reinterpret_cast<uint2*>(&s_a[rp * (TW_ / 2) + seg * 8]) = make_uint2(o0, o1);
-    }
-    __syncthreads();                                       // the stage's tile has been read by everyone; s_a is complete
-    if (t == 0) { const int next = tile + TMA_STAGES * G; if (next < total) issue(next, stage); }
-#define PYR_LEVEL(L, SW_, SH_, SRC, DST)                                                                                         \
-    if (NL > (L)) {                                                                                                              \
-      tile_level<SW_, SH_, PNT>(SRC, DST, (modes_mask >> ((L) - 1)) & 1, f.lvl[L] + (size_t)b * f.img_stride[L], f.pitch[L], f.w[L], \
-                                f.h[L], tx0 >> (L), ty0 >> (L), t);                                                              \
-      __syncthreads();                                                                                                           \
-    }
-    PYR_LEVEL(2, TW_ / 2, TH_ / 2, s_a, s_b)
-    PYR_LEVEL(3, TW_ / 4, TH_ / 4, s_b, s_a)
-    PYR_LEVEL(4, TW_ / 8, TH_ / 8, s_a, s_b)
-    PYR_LEVEL(5, TW_ / 16, TH_ / 16, s_b, s_a)
-    if (TH_ >= 64) { PYR_LEVEL(6, TW_ / 32, TH_ / 32, s_a, s_b) }
-#undef PYR_LEVEL
-    if (++stage == TMA_STAGES) { stage = 0; parity ^= 1u; }
-  }
-}
-
 // Generic single-level kernel: any size, both roundings, and the reference's scalar pointer
 // walk for ODD input widths (vision.cpp:92-109: `top` advances 2*out_w per row, then += stride,
 // so each output row starts one pixel early — reproduced through dense flat offsets).
@@ -400,64 +295,6 @@ static void launch_fused(const DevFrame& f, int mask, const YuvPlanes& yuv, cuda
   }
 }
 
-// SVOB200_PYRAMID_TMA=R: R persistent CTAs per SM of the TMA kernel for batches of at least 64 frames.  Unset / 0: the plain kernel.
-// Measured on one B200 (tools/pyr_probe.py, tools/r2_tma_ab.sh; 4,096 VGA frames x 4 levels, bit-identical output):
-//   kernel alone      plain 0.2915 ms (5.73 TB/s algorithmic, 0.877 of the copy peak) | TMA R=6 0.2882, R=5 0.2894, R=4 0.2985, R=7 0.321
-//   (256 x 32 tiles, rows read in 256-byte runs: 0.298 - 0.340 ms: 640 is not a multiple of 256)
-//   whole tracker step  4,096 sequences: 3.742 ms plain, 3.744 R=6, 3.68 R=5 | 2,048: 1.855 vs 1.921 (R=5) | 1,024: 0.981 vs 1.004 | 512: 0.537 vs 0.555
-// Both kernels sit at the same ~5.8 TB/s: the bound is the DRAM access pattern of the tiles (3 : 1 read : write, 128-byte row
-// segments), not the load instructions TMA removes; inside the step the persistent grid competes with the depth-filter stream
-// of the previous frame and loses at every batch size but one.  So it stays opt-in.
-static int pyramid_tma_ctas()
-{
-  static const int v = [] { const char* e = getenv("SVOB200_PYRAMID_TMA"); const int r = e ? atoi(e) : 0; return (r < 0 || r > 8) ? 0 : r; }();
-  return v;
-}
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
-                                  const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static EncodeTiledFn encode_tiled_fn()
-{
-  static const EncodeTiledFn fn = [] {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess) return (EncodeTiledFn)p;
-    return (EncodeTiledFn) nullptr;
-  }();
-  return fn;
-}
-
-// true: launched.  false: the frame does not qualify (alignment / pitch), the caller uses the plain kernel.
-static bool launch_fused_tma(const DevFrame& f, int mask, cudaStream_t s)
-{
-  const int R = pyramid_tma_ctas();
-  if (R <= 0 || f.batch < 64 || f.n_levels < 2 || f.n_levels > 7) return false;
-  if ((reinterpret_cast<uintptr_t>(f.lvl[0]) & 15) || (f.pitch[0] & 15) || (f.img_stride[0] & 15)) return false;
-  EncodeTiledFn enc = encode_tiled_fn();
-  if (!enc) return false;
-  CUtensorMap map;
-  const cuuint64_t dims[3] = {(cuuint64_t)f.w[0], (cuuint64_t)f.h[0], (cuuint64_t)f.batch};
-  const cuuint64_t strides[2] = {(cuuint64_t)f.pitch[0], (cuuint64_t)f.img_stride[0]};
-  constexpr int TW = PTW, TH = PTH;
-  const cuuint32_t box[3] = {(cuuint32_t)TW, (cuuint32_t)TH, 1}, es[3] = {1, 1, 1};
-  if (enc(&map, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, f.lvl[0], dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-          CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS) return false;
-  static const int sms = [] { int dev = 0, n = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev); return n > 0 ? n : 148; }();
-  const int tiles_x = (f.w[0] + TW - 1) / TW, tiles_y = (f.h[0] + TH - 1) / TH;
-  const long long total = (long long)tiles_x * tiles_y * f.batch;
-  if (total >= (1ll << 30)) return false;
-  const unsigned grid = (unsigned)std::min<long long>(total, (long long)sms * R);
-  switch (f.n_levels) {
-    case 2: pyramid_tma_kernel<2, PTW, PTH><<<grid, PNT, 0, s>>>(map, f, mask, tiles_x, tiles_y); break;
-    case 3: pyramid_tma_kernel<3, PTW, PTH><<<grid, PNT, 0, s>>>(map, f, mask, tiles_x, tiles_y); break;
-    case 4: pyramid_tma_kernel<4, PTW, PTH><<<grid, PNT, 0, s>>>(map, f, mask, tiles_x, tiles_y); break;
-    case 5: pyramid_tma_kernel<5, PTW, PTH><<<grid, PNT, 0, s>>>(map, f, mask, tiles_x, tiles_y); break;
-    case 6: pyramid_tma_kernel<6, PTW, PTH><<<grid, PNT, 0, s>>>(map, f, mask, tiles_x, tiles_y); break;
-    default: pyramid_tma_kernel<7, PTW, PTH><<<grid, PNT, 0, s>>>(map, f, mask, tiles_x, tiles_y); break;
-  }
-  return true;
-}
-
 static bool fused_ok(const DevFrame& f)
 {
   bool odd = false;
@@ -488,7 +325,7 @@ int launch_pyramid(const DevFrame& f, const int* modes, cudaStream_t s, long lon
   if (fused_ok(f)) {
     int mask = 0;
     for (int l = 0; l + 1 < f.n_levels; ++l) if (modes[l] == SVOB200_ROUND_SSE2) mask |= 1 << l;
-    if (!launch_fused_tma(f, mask, s)) launch_fused<false>(f, mask, YuvPlanes{}, s);
+    launch_fused<false>(f, mask, YuvPlanes{}, s);
     ++*launches;
   } else {
     for (int l = 0; l + 1 < f.n_levels; ++l) {

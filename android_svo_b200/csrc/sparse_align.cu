@@ -21,7 +21,6 @@
 // values are closer than the worst-case rounding error of the float chain, in which case the CTA
 // replays the exact sequential float chain in parallel (counted in n_exact_chi2).
 #include <cooperative_groups.h>
-#include <cstdlib>
 #include "common.cuh"
 #include "kernels.h"
 #include "ldlt.cuh"
@@ -766,13 +765,6 @@ int launch_chi2_chain_test(int block, const float* d_res, const uint8_t* d_visib
   return cudaGetLastError() == cudaSuccess ? 0 : -1;
 }
 
-// SVOB200_ALIGN_CLUSTER=1|2|4|8 forces the cluster size (tests / A-B runs); unset or 0 = automatic
-static int sparse_align_cluster_override()
-{
-  static const int v = [] { const char* e = getenv("SVOB200_ALIGN_CLUSTER"); const int c = e ? atoi(e) : 0; return (c == 1 || c == 2 || c == 4 || c == 8) ? c : 0; }();
-  return v;
-}
-
 // per feature: 16 floats x (ref_patch, gdx, gdy, res0, res1) + 15 doubles (a, b, patch gradient sums) + 3 flag bytes
 size_t sparse_align_scratch_bytes(int total_features)
 {
@@ -806,12 +798,10 @@ int launch_sparse_align(const DevFrame& ref, const DevFrame& cur, const DevCam& 
   // few problems (single-stream latency): spread each problem over a thread-block cluster, one SM per CTA, so the
   // per-iteration work of a 1,000-feature frame is shared by 8 SMs instead of serialising on one;
   // small problems / few problems: more threads per problem (latency); big batches: more CTAs per SM (throughput)
-  const int force = sparse_align_cluster_override();
   int cluster = 1;
   if (batch <= 16 && max_per_problem >= 64) cluster = 8;
   else if (batch <= 32 && max_per_problem >= 64) cluster = 4;
   else if (batch <= 64 && max_per_problem >= 128) cluster = 2;
-  if (force > 0) cluster = force;
   if (cluster > 1) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)batch * cluster, 1, 1); cfg.blockDim = dim3(256, 1, 1); cfg.dynamicSmemBytes = 0; cfg.stream = s;

@@ -8,7 +8,6 @@
 // reference does in host code is done by the glue kernels, so a step is 14 launches (15 when the depth
 // filter runs on its own stream and the step records are written in two halves) with no host round trip; in SVOB200_MEM_HOST mode it is bracketed by one H2D of the frame(s), one
 // H2D of the small per-step inputs and one D2H of the per-sequence results.
-#include <cstdlib>
 #include <atomic>
 #include "ctx_internal.h"
 
@@ -349,23 +348,15 @@ struct svob200_tracker {
   uint8_t* h_pinned = nullptr; size_t h_cap = 0;
   std::vector<void*> owned;
   std::vector<int> h_ftr_off, h_seed_off;
-  int chunk = 256;                     // sequences per H2D/compute pipeline chunk (host mode)
-  // Big batches run as sub-ranges of sequences alternating between the context's stream and `range_stream`: the kernels of
-  // one sub-range fill the SMs while the other sits in a latency-bound stage (the sparse-alignment wave, whose length is its
-  // slowest problem's Gauss-Newton chain) or in a kernel's tail; results are bit-identical (same kernels, same per-sequence work).
-  int ranges = 1;                      // sub-ranges per step in device mode (direct launches); 1 = one range on one stream (measured with the asynchronous depth filter: 1 range 0.601 ms per 512 sequences, 2 ranges 0.619; equal at 4,096)
-  int min_range = 128;                 // ... but never fewer sequences than this per sub-range
-  cudaStream_t range_stream = nullptr;
-  cudaEvent_t range_ev[2] = {};
+  static constexpr int CHUNK = 256;    // sequences per H2D/compute pipeline chunk (host mode)
   // Asynchronous depth filter (device-memory steps of big batches): like the reference, whose DepthFilter runs in its own
   // thread behind a frame queue (depth_filter.cpp:63-103, :191-229), the seed update of frame k runs on its own stream while
   // the tracking chain (pyramid -> alignment -> matching) of frame k+1 is already in flight: the latency-bound alignment wave
   // overlaps the issue-bound epipolar search.  Everything a chain reads that the next steps overwrite is double-buffered by
   // step parity (pose table, step records) or guarded by an event (the frame slot it searches in is reused two steps later).
   // Every synchronising entry point joins the stream (ctx_join_aux).
-  int async_df = 1;                    // SVOB200_TRACKER_ASYNC_DF=0 switches it off (A/B runs)
   cudaStream_t df_stream = nullptr;
-  cudaEvent_t df_done[2] = {}, ev_pose[4] = {}, ev_track[4] = {};
+  cudaEvent_t df_done[2] = {}, ev_pose = nullptr, ev_track = nullptr;
   bool df_pending[2] = {false, false};
   long long step_no = 0;
   SeedPoseRec* d_seed_poses2 = nullptr;      // second pose table (odd steps)
@@ -392,13 +383,12 @@ struct svob200_tracker {
   // per-launch driver cost and most of the inter-kernel gaps
   struct StepGraph { std::vector<uintptr_t> key; cudaGraphExec_t exec; long long launches; };
   std::vector<StepGraph> graphs;
-  int graph_max_batch = 64;
+  static constexpr int GRAPH_MAX_BATCH = 64;
   // inside a captured step the independent stages fork onto a second stream (see run_range): the graph then has parallel
   // branches and its critical path is 7 kernels instead of 13
   cudaStream_t fork_stream = nullptr;
   cudaEvent_t fork_ev[4] = {};
   bool forking = false;
-  int graph_fork = 1;
   // optional per-stage CUDA-event timing (bench.py's stage breakdown / roofline)
   bool profiling = false;
   cudaEvent_t ev[kNumStages + 1] = {};
@@ -460,11 +450,6 @@ int svob200_tracker_create(svob200_ctx* ctx, const svob200_camera* cam, int batc
   // Seed ctor depth_filter.cpp:36-45
   t->seed_init.a = 10; t->seed_init.b = 10; t->seed_init.mu = (float)(1.0 / depth_mean); t->seed_init.z_range = (float)(1.0 / depth_min);
   t->seed_init.sigma2 = t->seed_init.z_range * t->seed_init.z_range / 36;
-  if (const char* e = getenv("SVOB200_TRACKER_CHUNK")) { if (atoi(e) > 0) t->chunk = atoi(e); }   // sequences per H2D/compute pipeline chunk (A/B runs)
-  if (const char* e = getenv("SVOB200_TRACKER_RANGES")) { if (atoi(e) > 0) t->ranges = std::min(atoi(e), (int)SEED_RANGES); }   // A/B runs
-  if (const char* e = getenv("SVOB200_TRACKER_ASYNC_DF")) t->async_df = atoi(e) != 0;
-  if (const char* e = getenv("SVOB200_TRACKER_FORK")) t->graph_fork = atoi(e) != 0;   // 0: captured steps stay one chain of kernels (A/B runs)
-  if (const char* e = getenv("SVOB200_TRACKER_GRAPH")) t->graph_max_batch = atoi(e) > 0 ? atoi(e) : 0;   // 0 disables graph replay; N = largest batch replayed as a graph
   // frame ids of this tracker: -(uid << 8 | n); three to start with (keyframe 0, last, cur), more as keyframes are inserted
   t->next_fid = 1;
   auto new_frame = [&](int64_t* out_id) -> int {
@@ -491,12 +476,10 @@ void svob200_tracker_destroy(svob200_tracker* t)
   for (auto e : t->chunk_ev) cudaEventDestroy(e);
   for (auto& g : t->graphs) cudaGraphExecDestroy(g.exec);
   if (t->copy_stream) cudaStreamDestroy(t->copy_stream);
-  if (t->range_stream) cudaStreamDestroy(t->range_stream);
-  for (auto e : t->range_ev) if (e) cudaEventDestroy(e);
   if (t->df_stream) { cudaStreamSynchronize(t->df_stream); ctx_remove_aux(ctx, t->df_stream); cudaStreamDestroy(t->df_stream); }
   for (auto e : t->df_done) if (e) cudaEventDestroy(e);
-  for (auto e : t->ev_pose) if (e) cudaEventDestroy(e);
-  for (auto e : t->ev_track) if (e) cudaEventDestroy(e);
+  if (t->ev_pose) cudaEventDestroy(t->ev_pose);
+  if (t->ev_track) cudaEventDestroy(t->ev_track);
   if (t->fork_stream) cudaStreamDestroy(t->fork_stream);
   for (auto e : t->fork_ev) if (e) cudaEventDestroy(e);
   for (int k = 0; k <= kNumStages; ++k) if (t->ev[k]) cudaEventDestroy(t->ev[k]);
@@ -802,12 +785,11 @@ static DevFrame frame_view(const DevFrame& f, int c0, int cnt)
 // all stages of one step for the sequences [c0, c1) on the compute stream (level 0 of cur is in place)
 // out_px / out_ok: optional device destinations of the refined pixels / match flags (device-mode callers): copied as soon as
 // the matching stage is done, beside the depth filter in a forked step
-// s: the stream this range runs on; range: its index among the ranges of the step that may be in flight together
 static int run_range(svob200_tracker* t, int c0, int c1, const double* d_T_last, const double* d_last_px, bool marks,
-                     double* out_px = nullptr, int* out_ok = nullptr, cudaStream_t s = nullptr, int range = 0)
+                     double* out_px = nullptr, int* out_ok = nullptr)
 {
   svob200_ctx* ctx = t->ctx;
-  if (!s) s = ctx->stream;
+  cudaStream_t s = ctx->stream;
   const DevCam cam = to_cam(&t->cam);
   FrameRec* last = find_frame(ctx, t->fid_last);
   FrameRec* cur = find_frame(ctx, t->fid_cur);
@@ -891,11 +873,11 @@ static int run_range(svob200_tracker* t, int c0, int c1, const double* d_T_last,
     // the step's final T_cur) — and writes the tracking half of the step records; the events tell the df stream when
     if (launch_seed_pose_table(cam, t->batch, t->n_kfs, c0, cnt, t->d_T_kf, t->d_T_cur, table, s, &ctx->launches))
       return fail(ctx, SVOB200_ERR_CUDA, "tracker_step: seed pose table failed");
-    CU(cudaEventRecord(t->ev_pose[range], s));
+    CU(cudaEventRecord(t->ev_pose, s));
     step_stats_kernel<<<cnt, 128, 0, s>>>(t->d_ftr_off + c0, t->d_seed_off + c0, t->d_align + c0, t->d_T_cur + 7 * (size_t)c0, t->d_match_ok, t->d_obs,
                                           t->d_seeds, t->seed_init, t->reseed, d_stats + c0, 1, t->d_seed_refs);
     ++ctx->launches;
-    CU(cudaEventRecord(t->ev_track[range], s));
+    CU(cudaEventRecord(t->ev_track, s));
     if (cudaGetLastError() != cudaSuccess) return fail(ctx, SVOB200_ERR_CUDA, "tracker_step: launch error");
     return 0;
   }
@@ -903,7 +885,7 @@ static int run_range(svob200_tracker* t, int c0, int c1, const double* d_T_last,
   if (launch_seed_pose_table(cam, t->batch, t->n_kfs, c0, cnt, t->d_T_kf, t->d_T_cur, table, s_seeds, &ctx->launches))
     return fail(ctx, SVOB200_ERR_CUDA, "tracker_step: seed pose table failed");
   if (launch_seeds_update_compact(ctx->d_table, cur->slot, cam, ns, t->d_seed_refs + s0, t->d_kf_slot, t->batch, table, t->batch_counter, t->max_n_kfs, t->mopts,
-                                  t->conv_thresh, t->d_seeds + s0, t->d_obs + s0, t->d_seed_scratch, t->S, s0, range, s_seeds, &ctx->launches,
+                                  t->conv_thresh, t->d_seeds + s0, t->d_obs + s0, t->d_seed_scratch, t->S, s0, s_seeds, &ctx->launches,
                                   (marks && t->profiling) ? &t->ev[8] : nullptr))
     return fail(ctx, SVOB200_ERR_CUDA, "tracker_step: seeds_update failed");
   if (s_seeds != s) { CU(cudaEventRecord(t->fork_ev[3], s_seeds)); CU(cudaStreamWaitEvent(s, t->fork_ev[3], 0)); }
@@ -957,71 +939,53 @@ int svob200_tracker_step(svob200_tracker* t, const uint8_t* cur_imgs, int stride
     }
     // level 0 of the current frames aliases the caller's device buffer: no copy at all
     if (int e = svob200_frame_bind_only(ctx, t->fid_cur, cur_imgs, stride)) return e;
-    const bool use_graph = !t->profiling && B <= t->graph_max_batch && t->graph_max_batch > 0;
+    const bool use_graph = !t->profiling && B <= svob200_tracker::GRAPH_MAX_BATCH;
     // everything the kernels of a step receive BY VALUE: the buffers of this call and the two frame views
     FrameRec* last = find_frame(ctx, t->fid_last);
     const std::vector<uintptr_t> key = {1, (uintptr_t)cur_imgs, (uintptr_t)stride, (uintptr_t)T_last_w, (uintptr_t)last_px, (uintptr_t)stats,
                                         (uintptr_t)px_refined, (uintptr_t)match_ok, (uintptr_t)t->fid_cur, (uintptr_t)t->fid_last,
                                         (uintptr_t)last->f.lvl[0], (uintptr_t)last->f.pitch[0]};
-    if (use_graph && t->graph_fork && !t->fork_stream) {
+    if (use_graph && !t->fork_stream) {
       CU(cudaStreamCreateWithFlags(&t->fork_stream, cudaStreamNonBlocking));
       for (auto& e : t->fork_ev) CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
     }
-    // direct launches of a big batch: sub-ranges alternate between two streams (chain mode keeps one range: its reprojector
-    // scratch is shared), and the depth filter of the whole batch follows on its own stream
-    int n_ranges = 1;
-    if (!use_graph && !t->profiling && t->chain_cell <= 0) n_ranges = std::max(1, std::min(std::min(t->ranges, 4), B / std::max(1, t->min_range)));   // (<= 4 <= SEED_RANGES)
-    if (n_ranges > 1 && !t->range_stream) {
-      CU(cudaStreamCreateWithFlags(&t->range_stream, cudaStreamNonBlocking));
-      for (auto& e : t->range_ev) CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    }
-    const bool async_df = t->async_df && !use_graph && !t->profiling && t->chain_cell <= 0 && t->S > 0;
-    if (async_df && !t->df_stream) {
+    // direct launches of a big batch: the depth filter follows on its own stream (graphs, profiling and chain mode run it in place)
+    const bool df_on_stream = !use_graph && !t->profiling && t->chain_cell <= 0 && t->S > 0;
+    if (df_on_stream && !t->df_stream) {
       CU(cudaStreamCreateWithFlags(&t->df_stream, cudaStreamNonBlocking));
       if (int e = ctx_add_aux(ctx, t->df_stream)) return e;
       for (auto& e : t->df_done) CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-      for (auto& e : t->ev_pose) CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-      for (auto& e : t->ev_track) CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+      CU(cudaEventCreateWithFlags(&t->ev_pose, cudaEventDisableTiming));
+      CU(cudaEventCreateWithFlags(&t->ev_track, cudaEventDisableTiming));
     }
     const int par = (int)(t->step_no & 1);
-    if (!async_df && (t->df_pending[0] || t->df_pending[1])) {     // a step that runs the depth filter in place after asynchronous ones
+    if (!df_on_stream && (t->df_pending[0] || t->df_pending[1])) {     // a step that runs the depth filter in place after asynchronous ones
       if (int e = ctx_join_aux(ctx)) return e;
       t->df_pending[0] = t->df_pending[1] = false;
     }
     const int rc = graph_or_direct(t, use_graph, key, [&]() -> int {
-      if (async_df) {
+      if (df_on_stream) {
         t->df_defer = 1;
         t->cur_pose_table = par ? t->d_seed_poses2 : t->d_seed_poses;
         t->cur_stats = par ? t->d_stats2 : t->d_stats;
       }
-      int e0 = 0;
-      if (n_ranges > 1) {
-        CU(cudaEventRecord(t->range_ev[0], s));
-        CU(cudaStreamWaitEvent(t->range_stream, t->range_ev[0], 0));
-        for (int r = 0; r < n_ranges && !e0; ++r) {
-          const int c0 = (int)((long long)B * r / n_ranges), c1 = (int)((long long)B * (r + 1) / n_ranges);
-          e0 = run_range(t, c0, c1, T_last_w, last_px, false, px_refined, match_ok, (r & 1) ? t->range_stream : s, r);
-        }
-        if (!e0) { CU(cudaEventRecord(t->range_ev[1], t->range_stream)); CU(cudaStreamWaitEvent(s, t->range_ev[1], 0)); }
-      } else {
-        t->forking = use_graph && t->graph_fork;     // only a capture runs this body when use_graph is set
-        e0 = run_range(t, 0, B, T_last_w, last_px, true, px_refined, match_ok);
-        t->forking = false;
-      }
+      t->forking = use_graph;     // only a capture runs this body when use_graph is set
+      const int e0 = run_range(t, 0, B, T_last_w, last_px, true, px_refined, match_ok);
+      t->forking = false;
       svob200_step_stats* d_stats = t->cur_stats ? t->cur_stats : t->d_stats;
       SeedPoseRec* table = t->cur_pose_table;
       t->df_defer = 0; t->cur_pose_table = nullptr; t->cur_stats = nullptr;
       if (e0) return e0;
-      if (async_df) {
-        // the depth filter of the whole batch on its own stream: it starts as soon as every range has its pose rows, and its
+      if (df_on_stream) {
+        // the depth filter of the whole batch on its own stream: it starts as soon as the pose rows are written, and its
         // half of the step records (and their copy to the caller) follows the tracking half
         cudaStream_t df = t->df_stream;
-        for (int r = 0; r < n_ranges; ++r) CU(cudaStreamWaitEvent(df, t->ev_pose[r], 0));
+        CU(cudaStreamWaitEvent(df, t->ev_pose, 0));
         FrameRec* cur = find_frame(ctx, t->fid_cur);
         if (launch_seeds_update_compact(ctx->d_table, cur->slot, to_cam(&t->cam), t->S, t->d_seed_refs, t->d_kf_slot, t->batch, table, t->batch_counter, t->max_n_kfs, t->mopts,
-                                        t->conv_thresh, t->d_seeds, t->d_obs, t->d_seed_scratch, t->S, 0, 0, df, &ctx->launches, nullptr))
+                                        t->conv_thresh, t->d_seeds, t->d_obs, t->d_seed_scratch, t->S, 0, df, &ctx->launches, nullptr))
           return fail(ctx, SVOB200_ERR_CUDA, "tracker_step: seeds_update failed");
-        for (int r = 0; r < n_ranges; ++r) CU(cudaStreamWaitEvent(df, t->ev_track[r], 0));
+        CU(cudaStreamWaitEvent(df, t->ev_track, 0));
         step_stats_kernel<<<B, 128, 0, df>>>(t->d_ftr_off, t->d_seed_off, t->d_align, t->d_T_cur, t->d_match_ok, t->d_obs, t->d_seeds, t->seed_init,
                                              t->reseed, d_stats, 2, t->d_seed_refs);
         ++ctx->launches;
@@ -1072,7 +1036,7 @@ int svob200_tracker_step(svob200_tracker* t, const uint8_t* cur_imgs, int stride
         CU(cudaMemcpyAsync(t->d_step_in, t->h_pinned, in_bytes, cudaMemcpyHostToDevice, s));
       }
     }
-    const int chunk = (t->profiling || B <= t->chunk) ? B : t->chunk;
+    const int chunk = (t->profiling || B <= svob200_tracker::CHUNK) ? B : svob200_tracker::CHUNK;
     const int n_chunks = (B + chunk - 1) / chunk;
     if (!t->copy_stream) CU(cudaStreamCreateWithFlags(&t->copy_stream, cudaStreamNonBlocking));
     while ((int)t->chunk_ev.size() < n_chunks + 1) { cudaEvent_t e; CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming)); t->chunk_ev.push_back(e); }
@@ -1096,22 +1060,15 @@ int svob200_tracker_step(svob200_tracker* t, const uint8_t* cur_imgs, int stride
     // replayed as the same forked graph as in device mode; the kernels only see the tracker's own buffers here, so two
     // graphs (the frame pair swaps every step) serve every call.  (A graph WITHOUT the parallel branches gained nothing in
     // host mode: 0.202 -> 0.199 ms for C2.)
-    const bool use_graph = !t->profiling && n_chunks == 1 && B <= t->graph_max_batch && t->graph_max_batch > 0 && t->graph_fork;
+    const bool use_graph = !t->profiling && n_chunks == 1 && B <= svob200_tracker::GRAPH_MAX_BATCH;
     if (use_graph && !t->fork_stream) {
       CU(cudaStreamCreateWithFlags(&t->fork_stream, cudaStreamNonBlocking));
       for (auto& e : t->fork_ev) CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
     }
-    // chunks alternate between the two compute streams (see `ranges`), each waiting for its own frame copy
-    const bool two_streams = n_chunks > 1 && t->ranges > 1 && t->chain_cell <= 0 && n_chunks <= (int)SEED_RANGES;   // one job region per chunk in flight
-    if (two_streams && !t->range_stream) {
-      CU(cudaStreamCreateWithFlags(&t->range_stream, cudaStreamNonBlocking));
-      for (auto& e : t->range_ev) CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    }
-    if (two_streams) { CU(cudaEventRecord(t->range_ev[0], s)); CU(cudaStreamWaitEvent(t->range_stream, t->range_ev[0], 0)); }
+    // each chunk's kernels wait for its own frame copy
     for (int c = 0; c < n_chunks; ++c) {
       const int c0 = c * chunk, c1 = std::min(B, c0 + chunk);
-      cudaStream_t sc = (two_streams && (c & 1)) ? t->range_stream : s;
-      CU(cudaStreamWaitEvent(sc, t->chunk_ev[c], 0));
+      CU(cudaStreamWaitEvent(s, t->chunk_ev[c], 0));
       if (use_graph) {
         FrameRec* last = find_frame(ctx, t->fid_last);
         const std::vector<uintptr_t> key = {2, (uintptr_t)t->fid_cur, (uintptr_t)t->fid_last, (uintptr_t)r->f.lvl[0], (uintptr_t)r->f.pitch[0],
@@ -1123,9 +1080,8 @@ int svob200_tracker_step(svob200_tracker* t, const uint8_t* cur_imgs, int stride
           return e0;
         });
         if (rc) return rc;
-      } else if (int e = run_range(t, c0, c1, d_T_last, d_last_px, n_chunks == 1, nullptr, nullptr, sc, two_streams ? c : 0)) return e;
+      } else if (int e = run_range(t, c0, c1, d_T_last, d_last_px, n_chunks == 1)) return e;
     }
-    if (two_streams) { CU(cudaEventRecord(t->range_ev[1], t->range_stream)); CU(cudaStreamWaitEvent(s, t->range_ev[1], 0)); }
     uint8_t* ho = t->h_pinned + ((in_bytes + 255) & ~(size_t)255);
     uint8_t* h_stats = ho; uint8_t* h_px = h_stats + sizeof(svob200_step_stats) * B; uint8_t* h_ok = h_px + sizeof(double) * 2 * (size_t)N;
     if (stats) CU(cudaMemcpyAsync(h_stats, t->d_stats, sizeof(svob200_step_stats) * B, cudaMemcpyDeviceToHost, s));

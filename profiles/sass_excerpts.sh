@@ -19,7 +19,6 @@ dump() {  # object, function-name regex, output name
   echo "$name: $(grep -cE '^\s+/\*[0-9a-f]{4,6}\*/' /tmp/sass_$name.txt) instructions"
 }
 dump pyramid 'pyramid_fused_kernelILb0ELi4' pyramid_fused_kernel
-dump pyramid 'pyramid_tma_kernelILi4' pyramid_tma_kernel
 dump fast 'fast_kernel' fast_kernel
 dump sparse_align 'sparse_align_kernelILi128ELi1' sparse_align_kernel_128_1
 dump matcher 'match_prepare_kernel' match_prepare_kernel

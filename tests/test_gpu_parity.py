@@ -60,15 +60,31 @@ def test_pyramid_bit_exact(ctx, oracle, shape, n_levels, mode):
         ctx.frame_release(fid)
 
 
-def test_pyramid_tma_kernel_bit_exact():
-    """The opt-in TMA-load pyramid kernel (SVOB200_PYRAMID_TMA=R, batches of 64+ frames; pyramid.cu) against the oracle, in a
-    process of its own because the library reads the knob once: frame sizes with partial tiles, 2 to 7 levels, both roundings."""
-    import os, subprocess, sys
-    here = os.path.dirname(os.path.abspath(__file__))
-    env = dict(os.environ, SVOB200_PYRAMID_TMA="6")
-    out = subprocess.run([sys.executable, os.path.join(here, "tma_pyramid_check.py")], env=env, capture_output=True, text=True, timeout=600)
-    assert out.returncode == 0, out.stdout + out.stderr
-    assert "TMA pyramid OK" in out.stdout
+@pytest.mark.parametrize("shape,n_levels,batch,modes", [((480, 640), 4, 96, None), ((480, 752), 5, 80, None), ((1080, 1920), 5, 64, None),
+                                                         ((480, 640), 4, 70, [0, 0, 0]), ((480, 640), 3, 65, [1, 0]), ((66, 144), 4, 64, None),
+                                                         ((64, 64), 7, 64, None), ((480, 640), 2, 64, None)])
+def test_pyramid_bound_batch_bit_exact(ctx, oracle, shape, n_levels, batch, modes):
+    """The fused pyramid kernel on batches of 64+ frames bound from a device buffer (the tracker's device-memory path), against
+    the oracle's vk::halfSample (vision.cpp:20-110), every level of a sample of the images, bit for bit: frame sizes with
+    partial tiles, 2 to 7 levels, both roundings."""
+    h, w = shape
+    base = [scenes.noise_image(h, w, s, blur=(s % 2 == 0)) for s in range(4)]
+    imgs = np.stack([base[i % 4] if i % 5 else np.roll(base[i % 4], i, axis=1) for i in range(batch)])
+    d = ctx.dev_alloc(imgs.nbytes)
+    ctx.dev_upload(d, imgs)
+    fid = new_id()
+    ctx.frame_create(fid, batch, w, h, n_levels)
+    try:
+        ctx.frame_bind(fid, d, w, round_modes=modes)
+        ctx.sync()
+        for im in (0, 1, 5, batch // 2, batch - 1):
+            po = oracle.pyramid(imgs[im], n_levels, modes)
+            for l in range(1, n_levels):
+                got = ctx.frame_download(fid, im, l)
+                assert np.array_equal(got, po[l]), "%dx%d batch %d image %d level %d: %d px differ" % (w, h, batch, im, l, (got != po[l]).sum())
+    finally:
+        ctx.frame_release(fid)
+        ctx.dev_free(d)
 
 
 def test_pyramid_odd_width_scalar_walk(ctx, oracle):

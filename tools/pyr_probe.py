@@ -1,12 +1,11 @@
 """The fused pyramid kernel alone: B VGA frames (4 levels) per launch from device memory (svob200_frame_bind), two alternating
-input batches; and a digest of every level of a few images at three frame sizes, to compare kernel variants bit for bit.
-   [SVOB200_PYRAMID_TMA=R] python tools/pyr_probe.py [batch] [digest.npz]"""
+input batches; and a digest of every level of a few images at three frame sizes, to compare library builds (SVOB200_LIB) bit for bit.
+   python tools/pyr_probe.py [batch] [digest.npz]"""
 import sys, os, ctypes as C, hashlib
 import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from android_svo_b200 import capi
 B = int(sys.argv[1]) if len(sys.argv) > 1 else 4096
-tag = "tma=%s" % os.environ.get("SVOB200_PYRAMID_TMA", "0")
 ctx = capi.Context(0)
 V = C.c_void_p
 rng = np.random.default_rng(1)
@@ -25,7 +24,7 @@ if len(sys.argv) > 2:
         ctx.frame_release(7)
         ctx.dev_free(d)
     np.savez(sys.argv[2], **dig)
-    print(tag, "digest of %d level images written" % len(dig))
+    print("digest of %d level images written" % len(dig))
 w, h, nl = 640, 480, 4
 img = rng.integers(0, 256, (h, w), dtype=np.uint8)
 d = [ctx.dev_alloc(B * w * h) for _ in range(2)]
@@ -47,4 +46,4 @@ for rep in range(5):
     best.append(ctx.timer_stop_ms() / 20)
 alg = B * (w * h + sum((w >> l) * (h >> l) for l in range(1, nl)))
 ms = float(np.median(best))
-print("%s %s: pyramid alone %.4f ms per %d frames (min %.4f), %.0f GB/s algorithmic" % (os.environ.get("SVOB200_LIB", "base").split("/")[-1], tag, ms, B, min(best), alg / ms / 1e6))
+print("%s: pyramid alone %.4f ms per %d frames (min %.4f), %.0f GB/s algorithmic" % (os.environ.get("SVOB200_LIB", "base").split("/")[-1], ms, B, min(best), alg / ms / 1e6))
