@@ -558,7 +558,7 @@ class Tracker:
 
     def step_device(self, cur_imgs, T_last_w, last_px, want_px=False):
         """The same step with EVERY argument resident in device memory (SVOB200_MEM_DEVICE): level 0 of the current
-        frame aliases the caller's device buffer (svob200_frame_bind_only), nothing is staged, the whole batch runs on the
+        frame aliases the caller's device buffer, nothing is staged, the whole batch runs on the
         context's stream (a CUDA graph with forked branches for small batches, the depth filter on its own stream for larger
         ones).  This is the path bench.py's `value` times.  The images go through a ring of three device buffers (the aliased
         frame must stay valid through the next two steps)."""

@@ -83,6 +83,25 @@ int resolve_slots(svob200_ctx* ctx, svob200_feature_ref* staged, int n)
 
 }  // namespace
 
+int frame_bind_level0(svob200_ctx* ctx, FrameRec* r, const uint8_t* dev_gray, int stride)
+{
+  if (stride < r->f.w[0] || (stride & 15) || (reinterpret_cast<uintptr_t>(dev_gray) & 15))
+    return fail(ctx, SVOB200_ERR_ARG, "frame_bind: buffer and stride must be 16-byte aligned and stride >= width");
+  r->f.lvl[0] = const_cast<uint8_t*>(dev_gray); r->f.pitch[0] = stride; r->f.img_stride[0] = (unsigned long long)stride * r->f.h[0];
+  CU(cudaMemcpyAsync(ctx->d_table + r->slot, &r->f, sizeof(DevFrame), cudaMemcpyHostToDevice, ctx->stream));
+  return 0;
+}
+
+int frame_own_level0(svob200_ctx* ctx, FrameRec* r, bool copy_pixels)
+{
+  if (r->f.lvl[0] == r->own_l0) return 0;
+  if (copy_pixels)
+    CU(cudaMemcpy2DAsync(r->own_l0, r->own_pitch0, r->f.lvl[0], r->f.pitch[0], r->f.w[0], (size_t)r->f.h[0] * r->f.batch, cudaMemcpyDeviceToDevice, ctx->stream));
+  r->f.lvl[0] = r->own_l0; r->f.pitch[0] = r->own_pitch0; r->f.img_stride[0] = (unsigned long long)r->own_pitch0 * r->f.h[0];
+  CU(cudaMemcpyAsync(ctx->d_table + r->slot, &r->f, sizeof(DevFrame), cudaMemcpyHostToDevice, ctx->stream));
+  return 0;
+}
+
 extern "C" {
 
 int svob200_ctx_create(int device, svob200_ctx** out)
@@ -212,7 +231,7 @@ int svob200_frame_create(svob200_ctx* ctx, int64_t frame_id, int batch, int w, i
 static int build_levels(svob200_ctx* ctx, FrameRec* r, const int* round_modes)
 {
   int modes[SVOB200_MAX_LEVELS];
-  for (int l = 0; l + 1 < r->f.n_levels; ++l) modes[l] = round_modes ? round_modes[l] : svob200_round_mode_x86(r->f.w[l]);
+  pyramid_round_modes(r->f, round_modes, modes);
   if (launch_pyramid(r->f, modes, ctx->stream, &ctx->launches)) return fail(ctx, SVOB200_ERR_CUDA, "pyramid launch failed: %s", cudaGetErrorString(cudaGetLastError()));
   return 0;
 }
@@ -223,10 +242,7 @@ int svob200_frame_upload(svob200_ctx* ctx, int64_t frame_id, const uint8_t* gray
   FrameRec* r = find_frame(ctx, frame_id);
   if (!r) return fail(ctx, SVOB200_ERR_NOFRAME, "frame %lld not found", (long long)frame_id);
   if (stride < r->f.w[0]) return fail(ctx, SVOB200_ERR_ARG, "frame_upload: stride < width");
-  if (r->f.lvl[0] != r->own_l0) {                       // undo a previous bind
-    r->f.lvl[0] = r->own_l0; r->f.pitch[0] = r->own_pitch0; r->f.img_stride[0] = (unsigned long long)r->own_pitch0 * r->f.h[0];
-    CU(cudaMemcpyAsync(ctx->d_table + r->slot, &r->f, sizeof(DevFrame), cudaMemcpyHostToDevice, ctx->stream));
-  }
+  if (int e = frame_own_level0(ctx, r, false)) return e;
   CU(cudaMemcpy2DAsync(r->f.lvl[0], r->f.pitch[0], gray, stride, r->f.w[0], (size_t)r->f.h[0] * r->f.batch,
                        mem == SVOB200_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, ctx->stream));
   if (int e = build_levels(ctx, r, round_modes)) return e;
@@ -241,23 +257,8 @@ int svob200_frame_bind(svob200_ctx* ctx, int64_t frame_id, const uint8_t* dev_gr
   if (!ctx || !dev_gray) return fail(ctx, SVOB200_ERR_ARG, "frame_bind: null argument");
   FrameRec* r = find_frame(ctx, frame_id);
   if (!r) return fail(ctx, SVOB200_ERR_NOFRAME, "frame %lld not found", (long long)frame_id);
-  if (stride < r->f.w[0] || (stride & 15) || (reinterpret_cast<uintptr_t>(dev_gray) & 15))
-    return fail(ctx, SVOB200_ERR_ARG, "frame_bind: buffer and stride must be 16-byte aligned and stride >= width");
-  r->f.lvl[0] = const_cast<uint8_t*>(dev_gray); r->f.pitch[0] = stride; r->f.img_stride[0] = (unsigned long long)stride * r->f.h[0];
-  CU(cudaMemcpyAsync(ctx->d_table + r->slot, &r->f, sizeof(DevFrame), cudaMemcpyHostToDevice, ctx->stream));
+  if (int e = frame_bind_level0(ctx, r, dev_gray, stride)) return e;
   return build_levels(ctx, r, round_modes);
-}
-
-// bind level 0 without building the pyramid (tracker: the pyramid launch is part of the step)
-int svob200_frame_bind_only(svob200_ctx* ctx, int64_t frame_id, const uint8_t* dev_gray, int stride)
-{
-  FrameRec* r = ctx ? find_frame(ctx, frame_id) : nullptr;
-  if (!r) return fail(ctx, SVOB200_ERR_NOFRAME, "frame %lld not found", (long long)frame_id);
-  if (stride < r->f.w[0] || (stride & 15) || (reinterpret_cast<uintptr_t>(dev_gray) & 15))
-    return fail(ctx, SVOB200_ERR_ARG, "frame_bind: buffer and stride must be 16-byte aligned and stride >= width");
-  r->f.lvl[0] = const_cast<uint8_t*>(dev_gray); r->f.pitch[0] = stride; r->f.img_stride[0] = (unsigned long long)stride * r->f.h[0];
-  CU(cudaMemcpyAsync(ctx->d_table + r->slot, &r->f, sizeof(DevFrame), cudaMemcpyHostToDevice, ctx->stream));
-  return SVOB200_OK;
 }
 
 int svob200_frame_download(svob200_ctx* ctx, int64_t frame_id, int image, int level, uint8_t* out, int out_stride)
@@ -648,10 +649,7 @@ int svob200_frame_upload_level(svob200_ctx* ctx, int64_t frame_id, int image, in
   FrameRec* r = find_frame(ctx, frame_id);
   if (!r) return fail(ctx, SVOB200_ERR_NOFRAME, "frame %lld not found", (long long)frame_id);
   if (level < 0 || level >= r->f.n_levels || image < 0 || image >= r->f.batch || stride < r->f.w[level]) return fail(ctx, SVOB200_ERR_ARG, "frame_upload_level: bad level/image/stride");
-  if (level == 0 && r->f.lvl[0] != r->own_l0) {          // undo a previous bind
-    r->f.lvl[0] = r->own_l0; r->f.pitch[0] = r->own_pitch0; r->f.img_stride[0] = (unsigned long long)r->own_pitch0 * r->f.h[0];
-    CU(cudaMemcpyAsync(ctx->d_table + r->slot, &r->f, sizeof(DevFrame), cudaMemcpyHostToDevice, ctx->stream));
-  }
+  if (level == 0) if (int e = frame_own_level0(ctx, r, false)) return e;
   CU(cudaMemcpy2DAsync(r->f.lvl[level] + (size_t)image * r->f.img_stride[level], r->f.pitch[level], data, stride, r->f.w[level], r->f.h[level],
                        cudaMemcpyHostToDevice, ctx->stream));
   CU(cudaStreamSynchronize(ctx->stream));
@@ -753,10 +751,7 @@ int svob200_frame_upload_yuv420(svob200_ctx* ctx, int64_t frame_id, const uint8_
   const int cw = (w + 1) / 2, ch = (h + 1) / 2;
   const int uv_row_bytes = (cw - 1) * uv_pixel_stride + 1;
   if (uv_stride < uv_row_bytes) return fail(ctx, SVOB200_ERR_ARG, "frame_upload_yuv420: uv_stride too small");
-  if (r->f.lvl[0] != r->own_l0) {                       // level 0 is produced here: undo a previous bind
-    r->f.lvl[0] = r->own_l0; r->f.pitch[0] = r->own_pitch0; r->f.img_stride[0] = (unsigned long long)r->own_pitch0 * r->f.h[0];
-    CU(cudaMemcpyAsync(ctx->d_table + r->slot, &r->f, sizeof(DevFrame), cudaMemcpyHostToDevice, ctx->stream));
-  }
+  if (int e = frame_own_level0(ctx, r, false)) return e;      // level 0 is produced here
   YuvPlanes P;
   if (mem == SVOB200_MEM_DEVICE) {
     P.y = y; P.u = u; P.v = v; P.y_stride = y_stride; P.uv_stride = uv_stride; P.uv_pixel_stride = uv_pixel_stride;
@@ -789,7 +784,7 @@ int svob200_frame_upload_yuv420(svob200_ctx* ctx, int64_t frame_id, const uint8_
     else { P.u = dc0; P.v = dc1; }
   }
   int modes[SVOB200_MAX_LEVELS];
-  for (int l = 0; l + 1 < r->f.n_levels; ++l) modes[l] = round_modes ? round_modes[l] : svob200_round_mode_x86(r->f.w[l]);
+  pyramid_round_modes(r->f, round_modes, modes);
   if (launch_pyramid_yuv(r->f, P, modes, ctx->stream, &ctx->launches))
     return fail(ctx, SVOB200_ERR_CUDA, "yuv pyramid launch failed: %s", cudaGetErrorString(cudaGetLastError()));
   if (mem == SVOB200_MEM_HOST) CU(cudaStreamSynchronize(ctx->stream));

@@ -17,7 +17,7 @@ struct FrameRec {
   DevFrame f;
   uint8_t* base = nullptr;       // owned allocation (all levels)
   size_t bytes = 0;              // its size
-  uint8_t* own_l0 = nullptr;     // owned level-0 storage (f.lvl[0] may alias caller memory after bind)
+  uint8_t* own_l0 = nullptr;     // owned level-0 storage (f.lvl[0] may alias caller memory: frame_bind_level0)
   int own_pitch0 = 0;
   int slot = -1;
 };
@@ -109,5 +109,14 @@ inline int ensure_host_stage(svob200_ctx* ctx, size_t n)
   return 0;
 }
 
+// Level 0 of a frame is its own storage or aliases a caller's device buffer; only these two switch it, and they rewrite the
+// frame's row of the device table on ctx->stream.  Bind rejects (SVOB200_ERR_ARG, nothing changes) a buffer or stride that
+// is not 16-byte aligned and a stride below the width; copy_pixels copies the aliased images into the frame's own storage.
+int frame_bind_level0(svob200_ctx* ctx, FrameRec* r, const uint8_t* dev_gray, int stride);
+int frame_own_level0(svob200_ctx* ctx, FrameRec* r, bool copy_pixels);
 
-extern "C" int svob200_frame_bind_only(svob200_ctx* ctx, int64_t frame_id, const uint8_t* dev_gray, int stride);
+// rounding of every pyramid step l -> l+1: the caller's round_modes, or the reference's x86 dispatch on the level's width
+inline void pyramid_round_modes(const DevFrame& f, const int* round_modes, int* modes)
+{
+  for (int l = 0; l + 1 < f.n_levels; ++l) modes[l] = round_modes ? round_modes[l] : svob200_round_mode_x86(f.w[l]);
+}

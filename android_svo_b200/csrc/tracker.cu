@@ -5,8 +5,11 @@
 // It chains the operators exactly the way FrameHandlerMono::processFrame + DepthFilter do
 // (frame_handler_mono.cpp:171-262, depth_filter.cpp:237-341), minus the host-only stages that are
 // out of scope (pose_optimizer, map management): everything between the operators that the
-// reference does in host code is done by the glue kernels, so a step is 14 launches (15 when the depth
-// filter runs on its own stream and the step records are written in two halves) with no host round trip; in SVOB200_MEM_HOST mode it is bracketed by one H2D of the frame(s), one
+// reference does in host code is done by the glue kernels, so a step is 14 launches with no host round trip.  It runs in one
+// of three shapes (RangeShape): graph + fork (up to GRAPH_MAX_BATCH sequences, no profiling: a CUDA graph replay whose
+// independent stages run on forked branches); asynchronous depth filter (device memory, more sequences, not chain mode: the
+// depth filter on df_stream, the step records in two halves, 15 launches); in place (everything else: host-memory chunks of
+// CHUNK sequences, profiling, chain mode).  In SVOB200_MEM_HOST mode the step is bracketed by one H2D of the frame(s), one
 // H2D of the small per-step inputs and one D2H of the per-sequence results.
 #include <atomic>
 #include "ctx_internal.h"
@@ -277,13 +280,6 @@ __global__ void __launch_bounds__(256) kf_append_seeds_kernel(DevCam cam, const 
   if (tid == 0) { appended[b] = n_fill; dropped[b] = s_new_total - n_fill; }
 }
 
-template <class T> int dalloc(svob200_ctx* ctx, T** p, size_t n)
-{
-  *p = nullptr;
-  if (cudaMalloc((void**)p, sizeof(T) * (n ? n : 1)) != cudaSuccess) { cudaGetLastError(); return fail(ctx, SVOB200_ERR_NOMEM, "tracker: device alloc of %zu bytes failed", sizeof(T) * n); }
-  return 0;
-}
-
 }  // namespace
 
 // CUDA-event stage marks of one step (svob200_tracker_stage_ms / _stage_name): one entry per kernel of the
@@ -302,6 +298,7 @@ struct svob200_tracker {
   double conv_thresh = 100.0;
   svob200_seed seed_init{};
   int reseed = 1;
+  int64_t uid = 0;                     // frame ids of this tracker: -(uid << 8 | n), n = 1, 2, ... (new_frame)
   int64_t fid_last = 0, fid_cur = 0;
   // keyframes: up to max_kfs frames of the pool are keyframes (index k = position in the tables d_kf_slot / d_T_kf); the frame
   // of a keyframe may at the same time be the `last` frame of the tracking chain
@@ -342,9 +339,9 @@ struct svob200_tracker {
   svob200_align_result* d_align = nullptr;
   svob200_seed_obs* d_obs = nullptr;
   svob200_step_stats* d_stats = nullptr;
-  void* d_align_scratch = nullptr;
-  void* d_seed_scratch = nullptr;
-  void* d_match_scratch = nullptr;
+  uint8_t* d_align_scratch = nullptr;
+  uint8_t* d_seed_scratch = nullptr;
+  uint8_t* d_match_scratch = nullptr;
   uint8_t* h_pinned = nullptr; size_t h_cap = 0;
   std::vector<void*> owned;
   std::vector<int> h_ftr_off, h_seed_off;
@@ -354,17 +351,13 @@ struct svob200_tracker {
   // the tracking chain (pyramid -> alignment -> matching) of frame k+1 is already in flight: the latency-bound alignment wave
   // overlaps the issue-bound epipolar search.  Everything a chain reads that the next steps overwrite is double-buffered by
   // step parity (pose table, step records) or guarded by an event (the frame slot it searches in is reused two steps later).
-  // Every synchronising entry point joins the stream (ctx_join_aux).
+  // Every synchronising entry point joins the stream (ctx_join_aux; df_join where frame roles change).
   cudaStream_t df_stream = nullptr;
   cudaEvent_t df_done[2] = {}, ev_pose = nullptr, ev_track = nullptr;
   bool df_pending[2] = {false, false};
   long long step_no = 0;
   SeedPoseRec* d_seed_poses2 = nullptr;      // second pose table (odd steps)
   svob200_step_stats* d_stats2 = nullptr;    // second step-record array (odd steps)
-  // what the current run_range call does with the depth filter: 0 = runs it in place, 1 = leaves it to the df stream
-  int df_defer = 0;
-  SeedPoseRec* cur_pose_table = nullptr;
-  svob200_step_stats* cur_stats = nullptr;
   cudaStream_t copy_stream = nullptr;
   std::vector<cudaEvent_t> chunk_ev;
   // chain mode (svob200_tracker_set_chain): reprojector grid rules + pose optimiser instead of refining every map point
@@ -377,7 +370,7 @@ struct svob200_tracker {
   int *d_winner = nullptr, *d_m_level = nullptr, *d_m_point = nullptr, *d_m_count = nullptr, *d_seg_begin = nullptr, *d_seg_end = nullptr;
   double *d_m_f = nullptr, *d_m_pos = nullptr, *d_pose_work = nullptr;
   uint8_t* d_outlier = nullptr;
-  void* d_reproj_scratch = nullptr;
+  uint8_t* d_reproj_scratch = nullptr;
   // single-stream latency: in device mode with small batches the 14 launches of a step are replayed as ONE CUDA graph
   // (captured once per distinct set of buffer addresses: a camera ring buffer has only a few), which removes the
   // per-launch driver cost and most of the inter-kernel gaps
@@ -388,12 +381,53 @@ struct svob200_tracker {
   // branches and its critical path is 7 kernels instead of 13
   cudaStream_t fork_stream = nullptr;
   cudaEvent_t fork_ev[4] = {};
-  bool forking = false;
   // optional per-stage CUDA-event timing (bench.py's stage breakdown / roofline)
   bool profiling = false;
   cudaEvent_t ev[kNumStages + 1] = {};
 };
 
+// a device buffer of n elements that the tracker owns (freed by svob200_tracker_destroy)
+template <class T> static int alloc_owned(svob200_tracker* t, T*& p, size_t n)
+{
+  p = nullptr;
+  if (cudaMalloc((void**)&p, sizeof(T) * (n ? n : 1)) != cudaSuccess) { cudaGetLastError(); return fail(t->ctx, SVOB200_ERR_NOMEM, "tracker: device alloc of %zu bytes failed", sizeof(T) * n); }
+  t->owned.push_back(p);
+  return 0;
+}
+
+// a new frame of the tracker's pool
+static int new_frame(svob200_tracker* t, int64_t* out_id)
+{
+  const int64_t id = -((t->uid << 8) | t->next_fid++);
+  if (int e = svob200_frame_create(t->ctx, id, t->batch, t->cam.width, t->cam.height, t->n_levels)) return e;
+  t->frame_pool.push_back(id); *out_id = id;
+  return 0;
+}
+
+// the context's stream waits for every depth-filter chain in flight, so none is pending any more (before frame roles change)
+static int df_join(svob200_tracker* t)
+{
+  if (int e = ctx_join_aux(t->ctx)) return e;
+  t->df_pending[0] = t->df_pending[1] = false;
+  return 0;
+}
+
+// captured steps hold the addresses and values they were captured with: drop them when those change
+static void drop_graphs(svob200_tracker* t)
+{
+  for (auto& g : t->graphs) cudaGraphExecDestroy(g.exec);
+  t->graphs.clear();
+}
+
+// the second stream of captured steps and its events, created with the first graph
+static int ensure_fork_stream(svob200_tracker* t)
+{
+  svob200_ctx* ctx = t->ctx;
+  if (t->fork_stream) return 0;
+  CU(cudaStreamCreateWithFlags(&t->fork_stream, cudaStreamNonBlocking));
+  for (auto& e : t->fork_ev) CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+  return 0;
+}
 
 // Enqueue `body` on the context's stream, either directly or — single-stream latency — as a replay of a CUDA graph captured
 // from it the first time this `key` (every address the kernels receive by value) is seen.
@@ -420,7 +454,7 @@ static int graph_or_direct(svob200_tracker* t, bool use_graph, const std::vector
   const cudaError_t ie = cudaGraphInstantiate(&exec, graph, 0);
   cudaGraphDestroy(graph);
   if (ie != cudaSuccess) return fail(ctx, SVOB200_ERR_CUDA, "tracker_step: graph instantiate failed: %s", cudaGetErrorString(ie));
-  if (t->graphs.size() >= 64) { for (auto& g : t->graphs) cudaGraphExecDestroy(g.exec); t->graphs.clear(); }
+  if (t->graphs.size() >= 64) drop_graphs(t);
   t->graphs.push_back({key, exec, ctx->launches - launches0});
   CU(cudaGraphLaunch(exec, s));
   return 0;
@@ -443,23 +477,17 @@ int svob200_tracker_create(svob200_ctx* ctx, const svob200_camera* cam, int batc
   if (mopts->max_epi_search_steps < 0) return fail(ctx, SVOB200_ERR_ARG, "tracker_create: negative max_epi_search_steps %d", mopts->max_epi_search_steps);
   if (cam->width <= 0 || cam->height <= 0) return fail(ctx, SVOB200_ERR_ARG, "tracker_create: bad camera size");
   static std::atomic<int64_t> uid_counter{0};
-  const int64_t uid = ++uid_counter;
   svob200_tracker* t = new svob200_tracker();
+  t->uid = ++uid_counter;
   t->ctx = ctx; t->cam = *cam; t->batch = batch; t->n_levels = n_levels; t->aopts = *aopts; t->mopts = *mopts;
   t->conv_thresh = conv_thresh; t->reseed = reseed;
   // Seed ctor depth_filter.cpp:36-45
   t->seed_init.a = 10; t->seed_init.b = 10; t->seed_init.mu = (float)(1.0 / depth_mean); t->seed_init.z_range = (float)(1.0 / depth_min);
   t->seed_init.sigma2 = t->seed_init.z_range * t->seed_init.z_range / 36;
-  // frame ids of this tracker: -(uid << 8 | n); three to start with (keyframe 0, last, cur), more as keyframes are inserted
+  // three frames to start with (keyframe 0, last, cur), more as keyframes are inserted
   t->next_fid = 1;
-  auto new_frame = [&](int64_t* out_id) -> int {
-    const int64_t id = -((uid << 8) | t->next_fid++);
-    if (int e = svob200_frame_create(ctx, id, batch, cam->width, cam->height, n_levels)) return e;
-    t->frame_pool.push_back(id); *out_id = id;
-    return 0;
-  };
   for (int64_t* pid : {&t->fid_kfs[0], &t->fid_last, &t->fid_cur})
-    if (int e = new_frame(pid)) { for (int64_t id : t->frame_pool) svob200_frame_release(ctx, id); delete t; return e; }
+    if (int e = new_frame(t, pid)) { for (int64_t id : t->frame_pool) svob200_frame_release(ctx, id); delete t; return e; }
   *out = t;
   return SVOB200_OK;
 }
@@ -474,7 +502,7 @@ void svob200_tracker_destroy(svob200_tracker* t)
   for (void* p : t->owned) cudaFree(p);
   if (t->h_pinned) cudaFreeHost(t->h_pinned);
   for (auto e : t->chunk_ev) cudaEventDestroy(e);
-  for (auto& g : t->graphs) cudaGraphExecDestroy(g.exec);
+  drop_graphs(t);
   if (t->copy_stream) cudaStreamDestroy(t->copy_stream);
   if (t->df_stream) { cudaStreamSynchronize(t->df_stream); ctx_remove_aux(ctx, t->df_stream); cudaStreamDestroy(t->df_stream); }
   for (auto e : t->df_done) if (e) cudaEventDestroy(e);
@@ -541,33 +569,23 @@ int svob200_tracker_set_keyframe(svob200_tracker* t, const uint8_t* imgs, int st
       if (i < seed_offsets[b + 1]) { r.px[0] = seed_px[2 * i]; r.px[1] = seed_px[2 * i + 1]; r.level = (uint8_t)seed_level[i]; r.kf = 0; r.batch_id = 0; r.state = 0; }
     }
   }
-  // an allocation that fails midway leaves the tracker as it was before the call (it can be retried or destroyed)
-  auto rollback = [&]() {
+  int err = 0;
+  auto own = [&](auto*& p, size_t n) { if (!err) err = alloc_owned(t, p, n); };
+  own(t->d_ftr_off, B + 1); own(t->d_seed_off, B + 1); own(t->d_ftr_image, N); own(t->d_match_ok, N); own(t->d_has_point, N);
+  own(t->d_ftrs, N); own(t->d_seed_refs, S); own(t->d_pt_world, 3 * (size_t)N); own(t->d_T_kf_ftr, 7 * (size_t)N);
+  own(t->d_pobs, (size_t)N * t->max_kfs); own(t->d_T_pobs, 7 * (size_t)N * t->max_kfs); own(t->d_active, N); own(t->d_match_level, N); own(t->d_match_A, 4 * (size_t)N); own(t->d_sel, N);
+  own(t->d_points, N);
+  own(t->d_T_kf, 7 * (size_t)B * t->max_kfs); own(t->d_kf_slot, t->max_kfs); own(t->d_seed_poses, (size_t)B * t->max_kfs); own(t->d_seed_poses2, (size_t)B * t->max_kfs);
+  own(t->d_seeds, S); own(t->d_step_in, 7 * (size_t)B + 2 * (size_t)N); own(t->d_xyz, 3 * (size_t)N); own(t->d_T_init, 7 * (size_t)B);
+  own(t->d_T_cur, 7 * (size_t)B); own(t->d_depth_ref, N); own(t->d_px_in, 2 * (size_t)N); own(t->d_px_out, 2 * (size_t)N);
+  own(t->d_align, B); own(t->d_obs, S); own(t->d_stats, B); own(t->d_stats2, B);
+  own(t->d_align_scratch, sparse_align_scratch_bytes(N)); own(t->d_seed_scratch, seeds_scratch_bytes(S)); own(t->d_match_scratch, match_scratch_bytes(N));
+  if (err) {                 // an allocation that failed leaves the tracker as it was before the call (it can be retried or destroyed)
     for (void* q : t->owned) cudaFree(q);
     t->owned.clear();
     t->N = t->S = 0; t->max_per = 0; t->d_stats = nullptr; t->d_reproj = nullptr; t->det_cells_alloc = 0; t->d_det_counts = nullptr;
-  };
-#define DA(ptr, n) do { if (int e_ = dalloc(ctx, &ptr, (size_t)(n))) { rollback(); return e_; } t->owned.push_back(ptr); } while (0)
-  DA(t->d_ftr_off, B + 1); DA(t->d_seed_off, B + 1); DA(t->d_ftr_image, N); DA(t->d_match_ok, N); DA(t->d_has_point, N);
-  DA(t->d_ftrs, N); DA(t->d_seed_refs, S); DA(t->d_pt_world, 3 * (size_t)N); DA(t->d_T_kf_ftr, 7 * (size_t)N);
-  DA(t->d_pobs, (size_t)N * t->max_kfs); DA(t->d_T_pobs, 7 * (size_t)N * t->max_kfs); DA(t->d_active, N); DA(t->d_match_level, N); DA(t->d_match_A, 4 * (size_t)N); DA(t->d_sel, N);
-  DA(t->d_points, N);
-  DA(t->d_T_kf, 7 * (size_t)B * t->max_kfs); DA(t->d_kf_slot, t->max_kfs); DA(t->d_seed_poses, (size_t)B * t->max_kfs); DA(t->d_seed_poses2, (size_t)B * t->max_kfs);
-  DA(t->d_seeds, S); DA(t->d_step_in, 7 * (size_t)B + 2 * (size_t)N); DA(t->d_xyz, 3 * (size_t)N); DA(t->d_T_init, 7 * (size_t)B);
-  DA(t->d_T_cur, 7 * (size_t)B); DA(t->d_depth_ref, N); DA(t->d_px_in, 2 * (size_t)N); DA(t->d_px_out, 2 * (size_t)N);
-  DA(t->d_align, B); DA(t->d_obs, S); DA(t->d_stats, B); DA(t->d_stats2, B);
-  {
-    uint8_t* p = nullptr;
-    if (int e = dalloc(ctx, &p, sparse_align_scratch_bytes(N))) { rollback(); return e; }
-    t->owned.push_back(p); t->d_align_scratch = p;
-    uint8_t* q = nullptr;
-    if (int e = dalloc(ctx, &q, seeds_scratch_bytes(S))) { rollback(); return e; }
-    t->owned.push_back(q); t->d_seed_scratch = q;
-    uint8_t* m = nullptr;
-    if (int e = dalloc(ctx, &m, match_scratch_bytes(N))) { rollback(); return e; }
-    t->owned.push_back(m); t->d_match_scratch = m;
+    return err;
   }
-#undef DA
   cudaStream_t s = ctx->stream;
   CU(cudaMemcpyAsync(t->d_ftr_off, ftr_offsets, sizeof(int) * (B + 1), cudaMemcpyHostToDevice, s));
   CU(cudaMemcpyAsync(t->d_seed_off, pool_off.data(), sizeof(int) * (B + 1), cudaMemcpyHostToDevice, s));
@@ -618,11 +636,9 @@ int svob200_tracker_set_seed_pool(svob200_tracker* t, int capacity_per_sequence,
     return fail(ctx, SVOB200_ERR_ARG, "tracker_set_seed_pool: bad arguments");
   t->seed_capacity = capacity_per_sequence; t->max_kfs = max_keyframes; t->max_n_kfs = max_n_kfs; t->reseed = reseed;
   // the whole frame pool now (keyframe ring + last + cur), so that no keyframe insertion allocates
-  while ((int)t->frame_pool.size() < t->max_kfs + 2) {
-    const int64_t id = -(((-t->frame_pool[0]) & ~(int64_t)0xff) | t->next_fid++);
-    if (int e = svob200_frame_create(ctx, id, t->batch, t->cam.width, t->cam.height, t->n_levels)) return e;
-    t->frame_pool.push_back(id);
-  }
+  int64_t id;
+  while ((int)t->frame_pool.size() < t->max_kfs + 2)
+    if (int e = new_frame(t, &id)) return e;
   return SVOB200_OK;
 }
 
@@ -646,10 +662,8 @@ int svob200_tracker_add_keyframe(svob200_tracker* t, const float* depth_mean, co
   if (t->chain_cell > 0) return fail(ctx, SVOB200_ERR_UNSUPPORTED, "tracker_add_keyframe: not available in chain mode");
   const int B = t->batch, N = t->N, S = t->S;
   cudaStream_t s = ctx->stream;
-  if (int e = ctx_join_aux(ctx)) return e;                 // the depth filter of the last step may still be running
-  t->df_pending[0] = t->df_pending[1] = false;
-  for (auto& g : t->graphs) cudaGraphExecDestroy(g.exec);  // captured steps hold the old keyframe tables' values / frame roles
-  t->graphs.clear();
+  if (int e = df_join(t)) return e;                        // the depth filter of the last step may still be running
+  drop_graphs(t);                                          // captured steps hold the old keyframe tables' values / frame roles
   // 1. the keyframe's index in the ring: a free one, else the oldest keyframe leaves (its seeds with it: removeKeyframe)
   int k = -1;
   for (int i = 0; i < t->max_kfs; ++i) if (t->fid_kfs[i] == 0) { k = i; break; }
@@ -666,11 +680,7 @@ int svob200_tracker_add_keyframe(svob200_tracker* t, const float* depth_mean, co
   // 2. the frame: the last step's current frame (now `last`).  Its level 0 may alias the caller's buffer: the keyframe owns a copy.
   FrameRec* r = find_frame(ctx, t->fid_last);
   if (!r) return fail(ctx, SVOB200_ERR_NOFRAME, "tracker_add_keyframe: last frame missing");
-  if (r->f.lvl[0] != r->own_l0) {
-    CU(cudaMemcpy2DAsync(r->own_l0, r->own_pitch0, r->f.lvl[0], r->f.pitch[0], r->f.w[0], (size_t)r->f.h[0] * B, cudaMemcpyDeviceToDevice, s));
-    r->f.lvl[0] = r->own_l0; r->f.pitch[0] = r->own_pitch0; r->f.img_stride[0] = (unsigned long long)r->own_pitch0 * r->f.h[0];
-    CU(cudaMemcpyAsync(ctx->d_table + r->slot, &r->f, sizeof(DevFrame), cudaMemcpyHostToDevice, s));
-  }
+  if (int e = frame_own_level0(ctx, r, true)) return e;
   t->fid_kfs[k] = t->fid_last;
   t->kf_batch[k] = ++t->batch_counter;                      // ++Seed::batch_counter (depth_filter.cpp:139)
   if (t->batch_counter >= 65535) return fail(ctx, SVOB200_ERR_UNSUPPORTED, "tracker_add_keyframe: batch counter exhausted");
@@ -683,11 +693,12 @@ int svob200_tracker_add_keyframe(svob200_tracker* t, const float* depth_mean, co
   const int n_cells = gc * gr;
   if (n_cells > 8192) return fail(ctx, SVOB200_ERR_UNSUPPORTED, "tracker_add_keyframe: grid of %d cells exceeds the kernel's table (8192)", n_cells);
   if (t->det_cells_alloc < n_cells) {
-#define DA(ptr, n) do { if (int e_ = dalloc(ctx, &ptr, (size_t)(n))) return e_; t->owned.push_back(ptr); } while (0)
     const size_t M = (size_t)B * n_cells;
-    DA(t->d_occ, M); DA(t->d_det_keys, M); DA(t->d_det_cells, M);
-    if (!t->d_det_counts) { DA(t->d_det_counts, B); DA(t->d_kf_appended, B); DA(t->d_kf_dropped, B); DA(t->d_depth_mean, B); DA(t->d_depth_min, B); }
-#undef DA
+    int err = 0;
+    auto own = [&](auto*& p, size_t n) { if (!err) err = alloc_owned(t, p, n); };
+    own(t->d_occ, M); own(t->d_det_keys, M); own(t->d_det_cells, M);
+    if (!t->d_det_counts) { own(t->d_det_counts, B); own(t->d_kf_appended, B); own(t->d_kf_dropped, B); own(t->d_depth_mean, B); own(t->d_depth_min, B); }
+    if (err) return err;
     t->det_cells_alloc = n_cells;
   }
   CU(cudaMemcpyAsync(t->d_depth_mean, depth_mean, sizeof(float) * B, cudaMemcpyHostToDevice, s));
@@ -743,19 +754,19 @@ int svob200_tracker_set_chain(svob200_tracker* t, int cell_size, int max_fts, in
   if (!t->d_stats) return fail(ctx, SVOB200_ERR_ARG, "tracker_set_chain: set_keyframe first");
   if (int e = ctx_join_aux(ctx)) return e;
   CU(cudaStreamSynchronize(ctx->stream));
-  for (auto& g : t->graphs) cudaGraphExecDestroy(g.exec);          // captured steps belong to the other mode
-  t->graphs.clear();
+  drop_graphs(t);                                                  // captured steps belong to the other mode
   if (cell_size <= 0) { t->chain_cell = 0; return SVOB200_OK; }
   const int B = t->batch, N = t->N;
   const int n_cells = ((t->cam.width + cell_size - 1) / cell_size) * ((t->cam.height + cell_size - 1) / cell_size);
   if (n_cells > 8192) return fail(ctx, SVOB200_ERR_UNSUPPORTED, "tracker_set_chain: grid of %d cells exceeds the kernel's table (8192)", n_cells);
   if (!t->d_reproj || n_cells != t->chain_cells) {
-#define DA(ptr, n) do { if (int e_ = dalloc(ctx, &ptr, (size_t)(n))) return e_; t->owned.push_back(ptr); } while (0)
     const size_t M = (size_t)B * n_cells;
-    if (!t->d_reproj) { DA(t->d_reproj, N); DA(t->d_rstats, B); DA(t->d_pose, B); DA(t->d_m_count, B); DA(t->d_seg_begin, B); DA(t->d_seg_end, B);
-      uint8_t* q = nullptr; if (int e = dalloc(ctx, &q, reproject_scratch_bytes(N))) return e; t->owned.push_back(q); t->d_reproj_scratch = q; }
-    DA(t->d_winner, M); DA(t->d_m_level, M); DA(t->d_m_point, M); DA(t->d_m_f, 3 * M); DA(t->d_m_pos, 3 * M); DA(t->d_pose_work, M); DA(t->d_outlier, M);
-#undef DA
+    int err = 0;
+    auto own = [&](auto*& p, size_t n) { if (!err) err = alloc_owned(t, p, n); };
+    if (!t->d_reproj) { own(t->d_reproj, N); own(t->d_rstats, B); own(t->d_pose, B); own(t->d_m_count, B); own(t->d_seg_begin, B); own(t->d_seg_end, B);
+                        own(t->d_reproj_scratch, reproject_scratch_bytes(N)); }
+    own(t->d_winner, M); own(t->d_m_level, M); own(t->d_m_point, M); own(t->d_m_f, 3 * M); own(t->d_m_pos, 3 * M); own(t->d_pose_work, M); own(t->d_outlier, M);
+    if (err) return err;
   }
   // the map points as reprojector candidates: insertion order = the keyframe's fts_ order, every point TYPE_UNKNOWN (d_points /
   // d_obs / d_T_obs already hold them with their observation lists)
@@ -768,8 +779,7 @@ int svob200_tracker_set_chain(svob200_tracker* t, int cell_size, int max_fts, in
 int svob200_tracker_set_last(svob200_tracker* t, const uint8_t* imgs, int stride, int mem)
 {
   if (!t || !imgs) return SVOB200_ERR_ARG;
-  if (int e = ctx_join_aux(t->ctx)) return e;          // a depth-filter chain may still be reading the frame slots
-  t->df_pending[0] = t->df_pending[1] = false;
+  if (int e = df_join(t)) return e;                    // a depth-filter chain may still be reading the frame slots
   return svob200_frame_upload(t->ctx, t->fid_last, imgs, stride, nullptr, mem);
 }
 
@@ -782,10 +792,45 @@ static DevFrame frame_view(const DevFrame& f, int c0, int cnt)
   return v;
 }
 
-// all stages of one step for the sequences [c0, c1) on the compute stream (level 0 of cur is in place)
+// the shape of one run_range call (see the head of the file)
+struct RangeShape {
+  cudaStream_t side;               // the fork branch of a captured step, else the context's stream
+  bool defer_df;                   // the range stops after the tracking half of the step records: the depth filter goes to df_stream
+  SeedPoseRec* pose_table;         // the pose table and the step records of this step (of its parity when deferred)
+  svob200_step_stats* stats;
+};
+
+// DepthFilter::updateSeeds(cur) for the seeds of the sequences [c0, c1), on stream st
+static int enqueue_seeds_update(svob200_tracker* t, int c0, int c1, const SeedPoseRec* table, cudaStream_t st, cudaEvent_t* marks)
+{
+  svob200_ctx* ctx = t->ctx;
+  const int s0 = t->h_seed_off[c0], ns = t->h_seed_off[c1] - s0;
+  if (launch_seeds_update_compact(ctx->d_table, find_frame(ctx, t->fid_cur)->slot, to_cam(&t->cam), ns, t->d_seed_refs + s0, t->d_kf_slot, t->batch, table,
+                                  t->batch_counter, t->max_n_kfs, t->mopts, t->conv_thresh, t->d_seeds + s0, t->d_obs + s0, t->d_seed_scratch, t->S, s0,
+                                  st, &ctx->launches, marks))
+    return fail(ctx, SVOB200_ERR_CUDA, "tracker_step: seeds_update failed");
+  return 0;
+}
+
+// the step records of the sequences [c0, c1), on stream st: `parts` of step_stats_kernel, then the chain-mode fields
+static int enqueue_step_stats(svob200_tracker* t, int c0, int c1, int parts, svob200_step_stats* d_stats, cudaStream_t st)
+{
+  svob200_ctx* ctx = t->ctx;
+  const int cnt = c1 - c0;
+  step_stats_kernel<<<cnt, 128, 0, st>>>(t->d_ftr_off + c0, t->d_seed_off + c0, t->d_align + c0, t->d_T_cur + 7 * (size_t)c0, t->d_match_ok, t->d_obs,
+                                         t->d_seeds, t->seed_init, t->reseed, d_stats + c0, parts, t->d_seed_refs);
+  ++ctx->launches;
+  if (t->chain_cell > 0) {
+    chain_stats_kernel<<<(cnt + 127) / 128, 128, 0, st>>>(cnt, t->d_rstats + c0, t->d_pose + c0, t->chain_pose_opt, d_stats + c0); ++ctx->launches;
+  }
+  if (cudaGetLastError() != cudaSuccess) return fail(ctx, SVOB200_ERR_CUDA, "tracker_step: launch error");
+  return 0;
+}
+
+// all stages of one step for the sequences [c0, c1) on the context's stream, in the shape sh (level 0 of cur is in place)
 // out_px / out_ok: optional device destinations of the refined pixels / match flags (device-mode callers): copied as soon as
 // the matching stage is done, beside the depth filter in a forked step
-static int run_range(svob200_tracker* t, int c0, int c1, const double* d_T_last, const double* d_last_px, bool marks,
+static int run_range(svob200_tracker* t, int c0, int c1, const double* d_T_last, const double* d_last_px, bool marks, const RangeShape& sh,
                      double* out_px = nullptr, int* out_ok = nullptr)
 {
   svob200_ctx* ctx = t->ctx;
@@ -795,19 +840,18 @@ static int run_range(svob200_tracker* t, int c0, int c1, const double* d_T_last,
   FrameRec* cur = find_frame(ctx, t->fid_cur);
   const int cnt = c1 - c0;
   const int f0 = t->h_ftr_off[c0], nf = t->h_ftr_off[c1] - f0;
-  const int s0 = t->h_seed_off[c0], ns = t->h_seed_off[c1] - s0;
   const DevFrame vlast = frame_view(last->f, c0, cnt), vcur = frame_view(cur->f, c0, cnt);
 #define MARK(k) do { if (marks && t->profiling) cudaEventRecord(t->ev[k], s); } while (0)
   // Captured steps (single-stream latency) fork: the per-feature preparation does not read the new pyramid, and the depth
   // filter and the map-point matching both depend on the aligned pose only (default mode), so each pair runs as parallel
   // branches of the graph; s2 == s everywhere else.
-  const bool fork = t->forking;
-  cudaStream_t s2 = fork ? t->fork_stream : s;
+  cudaStream_t s2 = sh.side;
+  const bool fork = s2 != s;
   if (fork) { CU(cudaEventRecord(t->fork_ev[0], s)); CU(cudaStreamWaitEvent(s2, t->fork_ev[0], 0)); }
   // 1. fused pyramid of the current frames
   {
     int modes[SVOB200_MAX_LEVELS];
-    for (int l = 0; l + 1 < vcur.n_levels; ++l) modes[l] = svob200_round_mode_x86(vcur.w[l]);
+    pyramid_round_modes(vcur, nullptr, modes);
     if (launch_pyramid(vcur, modes, s, &ctx->launches)) return fail(ctx, SVOB200_ERR_CUDA, "tracker_step: pyramid launch failed");
   }
   MARK(1);
@@ -838,7 +882,6 @@ static int run_range(svob200_tracker* t, int c0, int c1, const double* d_T_last,
     // 4b-5. chain mode: Reprojector::reprojectMap (grid, every in-frame candidate matched in parallel, per-cell first success,
     // maxFts) over the keyframe's map points, then pose_optimizer::optimizeGaussNewton on the frame's new features (in place
     // on T_cur, so the depth filter sees the optimised pose).
-    MARK(4);
     const size_t cb = (size_t)c0 * t->chain_cells;
     const int rc = launch_reproject_map(ctx->d_table, cur->slot, cam, cnt, t->d_T_cur + 7 * (size_t)c0, t->d_ftr_off + c0, t->N, t->d_points, t->d_pobs,
                                         t->d_T_pobs, t->chain_cell, t->chain_max_fts, t->mopts, t->d_reproj, t->d_winner + cb, t->d_rstats + c0,
@@ -866,38 +909,22 @@ static int run_range(svob200_tracker* t, int c0, int c1, const double* d_T_last,
   }
   if (out_px) CU(cudaMemcpyAsync(out_px + 2 * (size_t)f0, t->d_px_out + 2 * (size_t)f0, sizeof(double) * 2 * (size_t)nf, cudaMemcpyDeviceToDevice, s));
   if (out_ok) CU(cudaMemcpyAsync(out_ok + f0, t->d_match_ok + f0, sizeof(int) * (size_t)nf, cudaMemcpyDeviceToDevice, s));
-  SeedPoseRec* table = t->cur_pose_table ? t->cur_pose_table : t->d_seed_poses;
-  svob200_step_stats* d_stats = t->cur_stats ? t->cur_stats : t->d_stats;
-  if (t->df_defer) {
-    // asynchronous depth filter: this range only prepares what the df stream needs of it — its rows of the pose table (from
-    // the step's final T_cur) — and writes the tracking half of the step records; the events tell the df stream when
-    if (launch_seed_pose_table(cam, t->batch, t->n_kfs, c0, cnt, t->d_T_kf, t->d_T_cur, table, s, &ctx->launches))
-      return fail(ctx, SVOB200_ERR_CUDA, "tracker_step: seed pose table failed");
+  // 6. DepthFilter::updateSeeds(cur): this range's rows of the pose table (from the step's final T_cur), then the seeds
+  if (launch_seed_pose_table(cam, t->batch, t->n_kfs, c0, cnt, t->d_T_kf, t->d_T_cur, sh.pose_table, s_seeds, &ctx->launches))
+    return fail(ctx, SVOB200_ERR_CUDA, "tracker_step: seed pose table failed");
+  if (sh.defer_df) {
+    // asynchronous depth filter (never forked: s_seeds == s): the df stream starts from the pose rows and writes its half of
+    // the step records after the tracking half; the events tell it when
     CU(cudaEventRecord(t->ev_pose, s));
-    step_stats_kernel<<<cnt, 128, 0, s>>>(t->d_ftr_off + c0, t->d_seed_off + c0, t->d_align + c0, t->d_T_cur + 7 * (size_t)c0, t->d_match_ok, t->d_obs,
-                                          t->d_seeds, t->seed_init, t->reseed, d_stats + c0, 1, t->d_seed_refs);
-    ++ctx->launches;
+    if (int e = enqueue_step_stats(t, c0, c1, 1, sh.stats, s)) return e;
     CU(cudaEventRecord(t->ev_track, s));
-    if (cudaGetLastError() != cudaSuccess) return fail(ctx, SVOB200_ERR_CUDA, "tracker_step: launch error");
     return 0;
   }
-  // 6. DepthFilter::updateSeeds(cur)
-  if (launch_seed_pose_table(cam, t->batch, t->n_kfs, c0, cnt, t->d_T_kf, t->d_T_cur, table, s_seeds, &ctx->launches))
-    return fail(ctx, SVOB200_ERR_CUDA, "tracker_step: seed pose table failed");
-  if (launch_seeds_update_compact(ctx->d_table, cur->slot, cam, ns, t->d_seed_refs + s0, t->d_kf_slot, t->batch, table, t->batch_counter, t->max_n_kfs, t->mopts,
-                                  t->conv_thresh, t->d_seeds + s0, t->d_obs + s0, t->d_seed_scratch, t->S, s0, s_seeds, &ctx->launches,
-                                  (marks && t->profiling) ? &t->ev[8] : nullptr))
-    return fail(ctx, SVOB200_ERR_CUDA, "tracker_step: seeds_update failed");
+  if (int e = enqueue_seeds_update(t, c0, c1, sh.pose_table, s_seeds, (marks && t->profiling) ? &t->ev[8] : nullptr)) return e;
   if (s_seeds != s) { CU(cudaEventRecord(t->fork_ev[3], s_seeds)); CU(cudaStreamWaitEvent(s, t->fork_ev[3], 0)); }
   MARK(11);
   // 7. per-sequence statistics (+ steady-state re-seeding)
-  step_stats_kernel<<<cnt, 128, 0, s>>>(t->d_ftr_off + c0, t->d_seed_off + c0, t->d_align + c0, t->d_T_cur + 7 * (size_t)c0, t->d_match_ok, t->d_obs,
-                                        t->d_seeds, t->seed_init, t->reseed, d_stats + c0, 3, t->d_seed_refs);
-  ++ctx->launches;
-  if (t->chain_cell > 0) {
-    chain_stats_kernel<<<(cnt + 127) / 128, 128, 0, s>>>(cnt, t->d_rstats + c0, t->d_pose + c0, t->chain_pose_opt, d_stats + c0); ++ctx->launches;
-  }
-  if (cudaGetLastError() != cudaSuccess) return fail(ctx, SVOB200_ERR_CUDA, "tracker_step: launch error");
+  if (int e = enqueue_step_stats(t, c0, c1, 3, sh.stats, s)) return e;
   MARK(12);
 #undef MARK
   return 0;
@@ -917,15 +944,10 @@ int svob200_tracker_step(svob200_tracker* t, const uint8_t* cur_imgs, int stride
   {
     auto is_kf = [&](int64_t id) { for (int i = 0; i < svob200_tracker::MAX_KFS; ++i) if (t->fid_kfs[i] == id) return true; return false; };
     if (is_kf(t->fid_cur)) {
-      if (int e = ctx_join_aux(ctx)) return e;            // frame roles change: no depth-filter chain may be in flight
-      t->df_pending[0] = t->df_pending[1] = false;
+      if (int e = df_join(t)) return e;                   // frame roles change: no depth-filter chain may be in flight
       int64_t pick = 0;
       for (int64_t id : t->frame_pool) if (id != t->fid_last && !is_kf(id)) { pick = id; break; }
-      if (!pick) {
-        pick = -(((-t->frame_pool[0]) & ~(int64_t)0xff) | t->next_fid++);
-        if (int e = svob200_frame_create(ctx, pick, B, t->cam.width, t->cam.height, t->n_levels)) return e;
-        t->frame_pool.push_back(pick);
-      }
+      if (!pick) if (int e = new_frame(t, &pick)) return e;
       t->fid_cur = pick;
     }
   }
@@ -933,22 +955,17 @@ int svob200_tracker_step(svob200_tracker* t, const uint8_t* cur_imgs, int stride
   if (mem == SVOB200_MEM_DEVICE) {
     // the frame slot that becomes `cur` now, the pose table and the step records of this parity were last used by the depth
     // filter chain of two steps ago: wait for it (the chain of the previous step keeps running beside this step's tracking)
-    {
-      const int par = (int)(t->step_no & 1);
-      if (t->df_pending[par]) { CU(cudaStreamWaitEvent(s, t->df_done[par], 0)); t->df_pending[par] = false; }
-    }
+    const int par = (int)(t->step_no & 1);
+    if (t->df_pending[par]) { CU(cudaStreamWaitEvent(s, t->df_done[par], 0)); t->df_pending[par] = false; }
     // level 0 of the current frames aliases the caller's device buffer: no copy at all
-    if (int e = svob200_frame_bind_only(ctx, t->fid_cur, cur_imgs, stride)) return e;
+    if (int e = frame_bind_level0(ctx, find_frame(ctx, t->fid_cur), cur_imgs, stride)) return e;
     const bool use_graph = !t->profiling && B <= svob200_tracker::GRAPH_MAX_BATCH;
     // everything the kernels of a step receive BY VALUE: the buffers of this call and the two frame views
     FrameRec* last = find_frame(ctx, t->fid_last);
     const std::vector<uintptr_t> key = {1, (uintptr_t)cur_imgs, (uintptr_t)stride, (uintptr_t)T_last_w, (uintptr_t)last_px, (uintptr_t)stats,
                                         (uintptr_t)px_refined, (uintptr_t)match_ok, (uintptr_t)t->fid_cur, (uintptr_t)t->fid_last,
                                         (uintptr_t)last->f.lvl[0], (uintptr_t)last->f.pitch[0]};
-    if (use_graph && !t->fork_stream) {
-      CU(cudaStreamCreateWithFlags(&t->fork_stream, cudaStreamNonBlocking));
-      for (auto& e : t->fork_ev) CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    }
+    if (use_graph) if (int e = ensure_fork_stream(t)) return e;
     // direct launches of a big batch: the depth filter follows on its own stream (graphs, profiling and chain mode run it in place)
     const bool df_on_stream = !use_graph && !t->profiling && t->chain_cell <= 0 && t->S > 0;
     if (df_on_stream && !t->df_stream) {
@@ -958,56 +975,37 @@ int svob200_tracker_step(svob200_tracker* t, const uint8_t* cur_imgs, int stride
       CU(cudaEventCreateWithFlags(&t->ev_pose, cudaEventDisableTiming));
       CU(cudaEventCreateWithFlags(&t->ev_track, cudaEventDisableTiming));
     }
-    const int par = (int)(t->step_no & 1);
-    if (!df_on_stream && (t->df_pending[0] || t->df_pending[1])) {     // a step that runs the depth filter in place after asynchronous ones
-      if (int e = ctx_join_aux(ctx)) return e;
-      t->df_pending[0] = t->df_pending[1] = false;
-    }
+    if (!df_on_stream && (t->df_pending[0] || t->df_pending[1]))       // a step that runs the depth filter in place after asynchronous ones
+      if (int e = df_join(t)) return e;
+    // graph + fork (only a capture runs the body then), asynchronous depth filter on this parity's pose table and step
+    // records, or in place
+    const RangeShape shape = {use_graph ? t->fork_stream : s, df_on_stream, (df_on_stream && par) ? t->d_seed_poses2 : t->d_seed_poses,
+                              (df_on_stream && par) ? t->d_stats2 : t->d_stats};
     const int rc = graph_or_direct(t, use_graph, key, [&]() -> int {
-      if (df_on_stream) {
-        t->df_defer = 1;
-        t->cur_pose_table = par ? t->d_seed_poses2 : t->d_seed_poses;
-        t->cur_stats = par ? t->d_stats2 : t->d_stats;
-      }
-      t->forking = use_graph;     // only a capture runs this body when use_graph is set
-      const int e0 = run_range(t, 0, B, T_last_w, last_px, true, px_refined, match_ok);
-      t->forking = false;
-      svob200_step_stats* d_stats = t->cur_stats ? t->cur_stats : t->d_stats;
-      SeedPoseRec* table = t->cur_pose_table;
-      t->df_defer = 0; t->cur_pose_table = nullptr; t->cur_stats = nullptr;
-      if (e0) return e0;
-      if (df_on_stream) {
-        // the depth filter of the whole batch on its own stream: it starts as soon as the pose rows are written, and its
-        // half of the step records (and their copy to the caller) follows the tracking half
-        cudaStream_t df = t->df_stream;
-        CU(cudaStreamWaitEvent(df, t->ev_pose, 0));
-        FrameRec* cur = find_frame(ctx, t->fid_cur);
-        if (launch_seeds_update_compact(ctx->d_table, cur->slot, to_cam(&t->cam), t->S, t->d_seed_refs, t->d_kf_slot, t->batch, table, t->batch_counter, t->max_n_kfs, t->mopts,
-                                        t->conv_thresh, t->d_seeds, t->d_obs, t->d_seed_scratch, t->S, 0, df, &ctx->launches, nullptr))
-          return fail(ctx, SVOB200_ERR_CUDA, "tracker_step: seeds_update failed");
-        CU(cudaStreamWaitEvent(df, t->ev_track, 0));
-        step_stats_kernel<<<B, 128, 0, df>>>(t->d_ftr_off, t->d_seed_off, t->d_align, t->d_T_cur, t->d_match_ok, t->d_obs, t->d_seeds, t->seed_init,
-                                             t->reseed, d_stats, 2, t->d_seed_refs);
-        ++ctx->launches;
-        if (stats) CU(cudaMemcpyAsync(stats, d_stats, sizeof(svob200_step_stats) * B, cudaMemcpyDeviceToDevice, df));
-        CU(cudaEventRecord(t->df_done[par], df));
-        t->df_pending[par] = true;
+      if (int e = run_range(t, 0, B, T_last_w, last_px, true, shape, px_refined, match_ok)) return e;
+      if (!df_on_stream) {
+        if (stats) CU(cudaMemcpyAsync(stats, shape.stats, sizeof(svob200_step_stats) * B, cudaMemcpyDeviceToDevice, s));
         return 0;
       }
-      if (stats) CU(cudaMemcpyAsync(stats, d_stats, sizeof(svob200_step_stats) * B, cudaMemcpyDeviceToDevice, s));
+      // the depth filter of the whole batch on its own stream: it starts as soon as the pose rows are written, and its
+      // half of the step records (and their copy to the caller) follows the tracking half
+      cudaStream_t df = t->df_stream;
+      CU(cudaStreamWaitEvent(df, t->ev_pose, 0));
+      if (int e = enqueue_seeds_update(t, 0, B, shape.pose_table, df, nullptr)) return e;
+      CU(cudaStreamWaitEvent(df, t->ev_track, 0));
+      if (int e = enqueue_step_stats(t, 0, B, 2, shape.stats, df)) return e;
+      if (stats) CU(cudaMemcpyAsync(stats, shape.stats, sizeof(svob200_step_stats) * B, cudaMemcpyDeviceToDevice, df));
+      CU(cudaEventRecord(t->df_done[par], df));
+      t->df_pending[par] = true;
       return 0;
     });
     if (rc) return rc;
   } else {
     // host buffers: the frame copy is split into chunks on a copy stream so that chunk c+1 crosses
     // PCIe while chunk c is being processed; one small H2D for the per-step inputs, one D2H for results
-    if (int e = ctx_join_aux(ctx)) return e;           // a depth-filter chain of earlier device-memory steps
-    t->df_pending[0] = t->df_pending[1] = false;
+    if (int e = df_join(t)) return e;                  // a depth-filter chain of earlier device-memory steps
     FrameRec* r = find_frame(ctx, t->fid_cur);
-    if (r->f.lvl[0] != r->own_l0) {   // drop an earlier device binding
-      r->f.lvl[0] = r->own_l0; r->f.pitch[0] = r->own_pitch0; r->f.img_stride[0] = (unsigned long long)r->own_pitch0 * r->f.h[0];
-      CU(cudaMemcpyAsync(ctx->d_table + r->slot, &r->f, sizeof(DevFrame), cudaMemcpyHostToDevice, s));
-    }
+    if (int e = frame_own_level0(ctx, r, false)) return e;    // drop an earlier device binding
     const size_t out_bytes = sizeof(svob200_step_stats) * B + sizeof(double) * 2 * (size_t)N + sizeof(int) * (size_t)N;
     if (t->h_cap < in_bytes + out_bytes + 512) {
       if (t->h_pinned) cudaFreeHost(t->h_pinned);
@@ -1061,10 +1059,8 @@ int svob200_tracker_step(svob200_tracker* t, const uint8_t* cur_imgs, int stride
     // graphs (the frame pair swaps every step) serve every call.  (A graph WITHOUT the parallel branches gained nothing in
     // host mode: 0.202 -> 0.199 ms for C2.)
     const bool use_graph = !t->profiling && n_chunks == 1 && B <= svob200_tracker::GRAPH_MAX_BATCH;
-    if (use_graph && !t->fork_stream) {
-      CU(cudaStreamCreateWithFlags(&t->fork_stream, cudaStreamNonBlocking));
-      for (auto& e : t->fork_ev) CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    }
+    if (use_graph) if (int e = ensure_fork_stream(t)) return e;
+    const RangeShape shape = {use_graph ? t->fork_stream : s, false, t->d_seed_poses, t->d_stats};
     // each chunk's kernels wait for its own frame copy
     for (int c = 0; c < n_chunks; ++c) {
       const int c0 = c * chunk, c1 = std::min(B, c0 + chunk);
@@ -1073,14 +1069,8 @@ int svob200_tracker_step(svob200_tracker* t, const uint8_t* cur_imgs, int stride
         FrameRec* last = find_frame(ctx, t->fid_last);
         const std::vector<uintptr_t> key = {2, (uintptr_t)t->fid_cur, (uintptr_t)t->fid_last, (uintptr_t)r->f.lvl[0], (uintptr_t)r->f.pitch[0],
                                             (uintptr_t)last->f.lvl[0], (uintptr_t)last->f.pitch[0], (uintptr_t)d_T_last};
-        const int rc = graph_or_direct(t, true, key, [&]() -> int {
-          t->forking = true;
-          const int e0 = run_range(t, 0, B, d_T_last, d_last_px, true);
-          t->forking = false;
-          return e0;
-        });
-        if (rc) return rc;
-      } else if (int e = run_range(t, c0, c1, d_T_last, d_last_px, n_chunks == 1)) return e;
+        if (int e = graph_or_direct(t, true, key, [&]() { return run_range(t, 0, B, d_T_last, d_last_px, true, shape); })) return e;
+      } else if (int e = run_range(t, c0, c1, d_T_last, d_last_px, n_chunks == 1, shape)) return e;
     }
     uint8_t* ho = t->h_pinned + ((in_bytes + 255) & ~(size_t)255);
     uint8_t* h_stats = ho; uint8_t* h_px = h_stats + sizeof(svob200_step_stats) * B; uint8_t* h_ok = h_px + sizeof(double) * 2 * (size_t)N;

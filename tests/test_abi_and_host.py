@@ -28,6 +28,16 @@ def test_library_exports_every_declared_symbol():
         assert n in names, "%s is bound in capi.py but not declared in include/svob200.h" % n
 
 
+def test_every_exported_symbol_is_declared():
+    """The library's C ABI is what include/svob200.h declares: no svob200_* function is exported by accident."""
+    import subprocess
+    out = subprocess.run(["nm", "-D", "--defined-only", capi.LIB_PATH], capture_output=True, text=True, check=True).stdout
+    exported = sorted({line.split()[-1] for line in out.splitlines() if line.split() and line.split()[-1].startswith("svob200_")})
+    assert len(exported) >= 40
+    undeclared = sorted(set(exported) - set(declared_symbols()))
+    assert not undeclared, "exported by libsvob200.so but not declared in include/svob200.h: %s" % undeclared
+
+
 def test_abi_struct_layout():
     c_sizes, py_sizes = capi.abi_sizes()
     assert c_sizes == py_sizes

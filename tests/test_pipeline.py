@@ -217,10 +217,11 @@ def test_tracker_step_matches_oracle(ctx, oracle, name, batch, n_frames, mode, r
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("chain", [0, 1])
-@pytest.mark.parametrize("batch", [1, 3, 70])
+@pytest.mark.parametrize("batch", [1, 3, 70, 300])
 def test_tracker_device_mode_bit_identical_to_host_mode(ctx, oracle, batch, chain):
     """SVOB200_MEM_DEVICE (frame_bind aliasing, forked CUDA graph for batch <= 64, plain launches above) must return the
-    bit-identical step record, refined pixels, seed state and seed observations as SVOB200_MEM_HOST on the same inputs."""
+    bit-identical step record, refined pixels, seed state and seed observations as SVOB200_MEM_HOST on the same inputs.
+    A host-memory batch of 300 runs in two chunks, 256 + 44."""
     from android_svo_b200 import capi
     n_frames, n_distinct = 6, min(batch, 3)
     seqs = [make_sequence(oracle, "C2", 0x00C0FFEE + 40 + i, n_frames + 1) for i in range(n_distinct)]
@@ -296,7 +297,7 @@ def test_tracker_c5_size_replicas(ctx, oracle):
     the batch holds 32 distinct sequences, each replicated 128 times at scattered batch positions; every replica must
     return the bit-identical step record, refined pixels, seed state and seed observations (no cross-talk, no dependence
     on the position in the batch or on which SM / group processed it), and replica 0 of each sequence must match the oracle.
-    Runs the EXACT path bench.py's `value` times — SVOB200_MEM_DEVICE: svob200_frame_bind_only aliasing + ONE 4,096-wide
+    Runs the EXACT path bench.py's `value` times — SVOB200_MEM_DEVICE: level-0 aliasing + ONE 4,096-wide
     range (491 k candidates, 3.1 M seeds per launch) — and the SVOB200_MEM_HOST path (16 chunks of 256 on a copy stream):
     the two must agree bit for bit.  Four steps, so that the frame slot the asynchronous depth filter searches is reused while
     that filter runs; in both seed regimes of bench.py."""
