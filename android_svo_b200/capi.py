@@ -127,6 +127,9 @@ def load_library():
     L.svob200_tracker_add_keyframe.argtypes = [V, V, V, V, V]
     L.svob200_tracker_get_seed_refs.argtypes = [V, V, V, V, V, V]
     L.svob200_tracker_num_seed_slots.argtypes = [V]
+    L.svob200_tracker_set_point_pool.argtypes = [V, C.c_int]
+    L.svob200_tracker_num_point_slots.argtypes = [V]
+    L.svob200_tracker_get_points.argtypes = [V, V, V, V, V, V]
     L.svob200_tracker_step.argtypes = [V, V, C.c_int, V, V, V, V, V, C.c_int]
     L.svob200_tracker_get_seeds.argtypes = [V, V]
     L.svob200_tracker_enable_profiling.argtypes = [V, C.c_int]
@@ -177,7 +180,7 @@ EXPORTED_SYMBOLS = [
     "svob200_frame_upload_yuv420", "svob200_reproject_map", "svob200_pose_opt_opts_default", "svob200_pose_optimize",
     "svob200_points_optimize", "svob200_seeds_initialize", "svob200_tracker_debug_align", "svob200_tracker_set_chain",
     "svob200_tracker_set_seed_pool", "svob200_tracker_set_detector", "svob200_tracker_add_keyframe", "svob200_tracker_get_seed_refs",
-    "svob200_tracker_num_seed_slots",
+    "svob200_tracker_num_seed_slots", "svob200_tracker_set_point_pool", "svob200_tracker_num_point_slots", "svob200_tracker_get_points",
 ]
 
 
@@ -510,10 +513,28 @@ class Tracker:
                 a(seed_px, np.float64), a(seed_level, np.int32)]
         self.ctx._ck(self.L.svob200_tracker_set_keyframe(self.h, _ptr(imgs), imgs.shape[-1], *[_ptr(x) for x in args]))
         self.S = int(self.L.svob200_tracker_num_seed_slots(self.h))          # pool slots (>= the seeds given)
+        self.N = int(self.L.svob200_tracker_num_point_slots(self.h))         # point slots (>= the map points given)
+
+    @property
+    def P(self):
+        """point slots: the length of every per-map-feature array of a step"""
+        return self.N
 
     # ---- keyframe insertion inside the tracker
     def set_seed_pool(self, capacity_per_sequence, max_keyframes=4, max_n_kfs=3, reseed=3):
         self.ctx._ck(self.L.svob200_tracker_set_seed_pool(self.h, int(capacity_per_sequence), int(max_keyframes), int(max_n_kfs), int(reseed)))
+
+    def set_point_pool(self, capacity_per_sequence):
+        """converged seeds become map points (svob200_tracker_set_point_pool): call before set_keyframe"""
+        self.ctx._ck(self.L.svob200_tracker_set_point_pool(self.h, int(capacity_per_sequence)))
+
+    def points(self):
+        """(pos[P,3], type[P], n_obs[P], created[batch], dropped[batch]) of the point slots; type SVOB200_POINT_*"""
+        P = self.N
+        pos = np.zeros((max(P, 1), 3)); ty = np.zeros(max(P, 1), np.int32); no = np.zeros(max(P, 1), np.int32)
+        cr = np.zeros(self.batch, np.int32); dr = np.zeros(self.batch, np.int32)
+        self.ctx._ck(self.L.svob200_tracker_get_points(self.h, _ptr(pos), _ptr(ty), _ptr(no), _ptr(cr), _ptr(dr)))
+        return pos[:P], ty[:P], no[:P], cr, dr
 
     def set_detector(self, cell, levels, thr):
         self.ctx._ck(self.L.svob200_tracker_set_detector(self.h, int(cell), int(levels), float(thr)))

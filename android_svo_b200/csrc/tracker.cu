@@ -10,7 +10,9 @@
 // independent stages run on forked branches); asynchronous depth filter (device memory, more sequences, not chain mode: the
 // depth filter on df_stream, the step records in two halves, 15 launches); in place (everything else: host-memory chunks of
 // CHUNK sequences, profiling, chain mode).  In SVOB200_MEM_HOST mode the step is bracketed by one H2D of the frame(s), one
-// H2D of the small per-step inputs and one D2H of the per-sequence results.
+// H2D of the small per-step inputs and one D2H of the per-sequence results.  With a point pool (svob200_tracker_set_point_pool)
+// the step-record kernel also turns converged seeds into candidate points, and one more launch at the head of the step inserts
+// the candidates of two steps ago (cand_insert_kernel): the same in every shape.
 #include <atomic>
 #include "ctx_internal.h"
 
@@ -27,15 +29,90 @@ __global__ void init_pose_kernel(int batch, const double* T_last, double* T_init
   for (int k = 0; k < 7; ++k) T_init[7 * (size_t)b + k] = out[k];
 }
 
+// ---- point pool (svob200_tracker_set_point_pool): a converged seed becomes a candidate point (DepthFilter::updateSeeds ->
+// seed_converged_cb_ -> MapPointCandidates::newCandidatePoint), which enters an empty point slot two steps later
+struct CandRec { double pos[3], px[2], f[3]; int level, kf, batch_id, pad; };   // one candidate, with its one observation
+struct CandStage {                       // where step_stats_kernel records the candidates of the step (rec == nullptr: no pool)
+  CandRec* rec; int* count; int* created;  // rec: the sequence's point-slot block of this parity's staging; count / created: per sequence
+  const int* pt_off; const double* T_kf; int batch, b0;   // point-slot offsets, keyframe poses [kf][batch][7], first sequence of the range
+};
+struct KfBatches { int v[16]; };         // Seed::batch_id of every keyframe index of the ring (svob200_tracker::kf_batch)
+
+// exclusive prefix sum over a 128-thread block (every thread calls it); *total = the block's sum
+__device__ int block_scan128(int v, int* total)
+{
+  __shared__ int s_w[4];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  int x = v;
+  for (int o = 1; o < 32; o <<= 1) { const int y = __shfl_up_sync(0xffffffffu, x, o); if (lane >= o) x += y; }
+  if (lane == 31) s_w[w] = x;
+  __syncthreads();
+  int before = 0;
+  for (int k = 0; k < w; ++k) before += s_w[k];
+  *total = s_w[0] + s_w[1] + s_w[2] + s_w[3];
+  __syncthreads();
+  return before + x - v;
+}
+
+// The candidates of sequence b in the reference's list order (seeds_ is ordered by ascending Seed::batch_id, and inside one
+// batch by slot, since kf_append_seeds_kernel fills slots in cell order): one pass per batch id, each a block scan over
+// contiguous slot chunks, so placement never depends on scheduling.  xyz_world = kf.T_f_w.inverse() * (f * (1.0 / mu))
+// (depth_filter.cpp:318-325 -> MapPointCandidates::newCandidatePoint); runs before the seed is re-initialised.
+__device__ void create_candidates(const CandStage& cs, int b, int p0, int np, const svob200_seed_obs* obs, const svob200_seed* seeds,
+                                  const SeedRef* refs)
+{
+  __shared__ int s_min;
+  const int tid = threadIdx.x, ab = cs.b0 + b;
+  const int chunk = (np + 127) / 128, q0 = min(tid * chunk, np), q1 = min(q0 + chunk, np);
+  const int cap = cs.pt_off[ab + 1] - cs.pt_off[ab];
+  CandRec* out = cs.rec + cs.pt_off[ab];
+  int n_out = 0, prev = -1;
+  for (;;) {
+    if (tid == 0) s_min = 0x7fffffff;
+    __syncthreads();
+    int m = 0x7fffffff;
+    for (int q = q0; q < q1; ++q)
+      if (obs[p0 + q].status == SVOB200_SEED_CONVERGED && (int)refs[p0 + q].batch_id > prev) m = min(m, (int)refs[p0 + q].batch_id);
+    if (m != 0x7fffffff) atomicMin(&s_min, m);
+    __syncthreads();
+    const int bid = s_min;
+    if (bid == 0x7fffffff) break;
+    int local = 0;
+    for (int q = q0; q < q1; ++q) local += obs[p0 + q].status == SVOB200_SEED_CONVERGED && refs[p0 + q].batch_id == bid;
+    int total;
+    int r = n_out + block_scan128(local, &total);
+    for (int q = q0; q < q1; ++q) {
+      if (obs[p0 + q].status != SVOB200_SEED_CONVERGED || refs[p0 + q].batch_id != bid) continue;
+      if (r < cap) {
+        const SeedRef sr = refs[p0 + q];
+        double inv[7];
+        se3_inverse(cs.T_kf + 7 * ((size_t)sr.kf * cs.batch + ab), inv);
+        const double s = 1.0 / (double)seeds[p0 + q].mu;
+        const v3d p = se3_transform(inv, {sr.f[0] * s, sr.f[1] * s, sr.f[2] * s});
+        CandRec c;
+        c.pos[0] = p.x; c.pos[1] = p.y; c.pos[2] = p.z; c.px[0] = sr.px[0]; c.px[1] = sr.px[1];
+        c.f[0] = sr.f[0]; c.f[1] = sr.f[1]; c.f[2] = sr.f[2]; c.level = sr.level; c.kf = sr.kf; c.batch_id = sr.batch_id; c.pad = 0;
+        out[r] = c;
+      }
+      ++r;
+    }
+    n_out += total; prev = bid;
+  }
+  if (tid == 0) { cs.count[ab] = n_out; cs.created[ab] += n_out; }
+}
+
 // one CTA per sequence: per-sequence statistics + steady-state re-seeding of finished seeds
 // parts: 1 = the tracking fields (pose, alignment, matches), 2 = the depth-filter fields (+ re-seeding); 3 = both.  The
-// asynchronous depth filter runs part 2 on its own stream, after the tracking chain of the same step ran part 1.
+// asynchronous depth filter runs part 2 on its own stream, after the tracking chain of the same step ran part 1.  kPool: the
+// tracker has a point pool, and part 2 first records the step's candidates (the instance without it keeps the lean kernel).
+template <bool kPool>
 __global__ void __launch_bounds__(128) step_stats_kernel(const int* ftr_off, const int* seed_off, const svob200_align_result* align,
                                                          const double* T_cur_w, const int* match_ok, const svob200_seed_obs* obs,
                                                          svob200_seed* seeds, svob200_seed init, int reseed, svob200_step_stats* stats, int parts,
-                                                         SeedRef* refs)
+                                                         SeedRef* refs, CandStage cand)
 {
   const int b = blockIdx.x, tid = threadIdx.x;
+  if (kPool && (parts & 2)) create_candidates(cand, b, seed_off[b], seed_off[b + 1] - seed_off[b], obs, seeds, refs);
   int matched = 0, upd = 0, conv = 0, fail = 0, skipped = 0;
   if (parts & 1) for (int i = ftr_off[b] + tid; i < ftr_off[b + 1]; i += 128) matched += match_ok[i] ? 1 : 0;
   if (parts & 2) for (int i = seed_off[b] + tid; i < seed_off[b + 1]; i += 128) {
@@ -123,8 +200,9 @@ __device__ __forceinline__ v3d kf_frame_pos(const double* T)
   return {inv[0], inv[1], inv[2]};
 }
 
-__global__ void points_init_kernel(int n, int K, const svob200_feature_ref* ftrs, const double* T_kf, const double* pt_world, svob200_map_point* pts,
-                                   svob200_feature_ref* obs, double* T_obs)
+// (an empty slot of a point pool, has_point 0: TYPE_DELETED with no observation)
+__global__ void points_init_kernel(int n, int K, const svob200_feature_ref* ftrs, const double* T_kf, const double* pt_world, const uint8_t* has_point,
+                                   svob200_map_point* pts, svob200_feature_ref* obs, double* T_obs)
 {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
@@ -134,7 +212,64 @@ __global__ void points_init_kernel(int n, int K, const svob200_feature_ref* ftrs
   svob200_map_point p;
   for (int k = 0; k < 3; ++k) p.pos[k] = pt_world[3 * (size_t)i + k];
   p.type = SVOB200_POINT_UNKNOWN; p.obs_begin = slot; p.obs_end = (i + 1) * K; p.reserved = 0;
+  if (!has_point[i]) { p.type = SVOB200_POINT_DELETED; p.obs_begin = p.obs_end; }
   pts[i] = p;
+}
+
+// The candidates of step k enter at the head of step k + 2 (the reference's depth filter runs one frame behind tracking):
+// into the sequence's empty slots in slot order, in their list order.  A candidate whose keyframe left the ring since (its
+// batch id is no longer that keyframe index's) or that finds no empty slot is dropped.  One CTA per sequence; ranks come from
+// block scans, so placement never depends on scheduling.
+__global__ void __launch_bounds__(128) cand_insert_kernel(int K, int batch, const int* pt_off, const CandRec* cand, const int* cand_n, KfBatches kfb,
+                                                          const int* kf_slot, const double* T_kf, svob200_map_point* pts, double* pt_world,
+                                                          svob200_feature_ref* obs, double* T_obs, int* sel, uint8_t* has_point,
+                                                          int* slot_of_rank, int* dropped)
+{
+  const int b = blockIdx.x, tid = threadIdx.x;
+  const int P0 = pt_off[b], P = pt_off[b + 1] - P0, n = cand_n[b], stored = min(n, P);
+  const CandRec* C = cand + P0;
+  const int cc = (stored + 127) / 128, c0 = min(tid * cc, stored), c1 = min(c0 + cc, stored);
+  int nv = 0;
+  for (int c = c0; c < c1; ++c) nv += C[c].batch_id == kfb.v[C[c].kf];
+  int v_total;
+  const int v_rank = block_scan128(nv, &v_total);
+  const int pc = (P + 127) / 128, q0 = min(tid * pc, P), q1 = min(q0 + pc, P);
+  int nf = 0;
+  for (int q = q0; q < q1; ++q) nf += pts[P0 + q].type == SVOB200_POINT_DELETED;
+  int f_total;
+  const int f_rank = block_scan128(nf, &f_total);
+  const int n_fill = min(v_total, f_total);
+  { int r = f_rank; for (int q = q0; q < q1 && r < n_fill; ++q) if (pts[P0 + q].type == SVOB200_POINT_DELETED) slot_of_rank[P0 + r++] = P0 + q; }
+  __syncthreads();
+  int r = v_rank;
+  for (int c = c0; c < c1 && r < n_fill; ++c) {
+    const CandRec cr = C[c];
+    if (cr.batch_id != kfb.v[cr.kf]) continue;
+    const int j = slot_of_rank[P0 + r++], o = j * K + K - 1;
+    svob200_feature_ref f;
+    f.ref_frame_id = kf_slot[cr.kf]; f.ref_image = b; f.cur_image = b; f.level = cr.level; f.type = 0;
+    f.px[0] = cr.px[0]; f.px[1] = cr.px[1]; f.f[0] = cr.f[0]; f.f[1] = cr.f[1]; f.f[2] = cr.f[2]; f.grad[0] = 1.0; f.grad[1] = 0.0;
+    for (int k = 0; k < 7; ++k) { f.T_cur_ref[k] = 0.0; T_obs[7 * (size_t)o + k] = T_kf[7 * ((size_t)cr.kf * batch + b) + k]; }
+    obs[o] = f;
+    svob200_map_point p;
+    for (int k = 0; k < 3; ++k) { p.pos[k] = cr.pos[k]; pt_world[3 * (size_t)j + k] = cr.pos[k]; }
+    p.type = SVOB200_POINT_CANDIDATE; p.obs_begin = o; p.obs_end = (j + 1) * K; p.reserved = 0;
+    pts[j] = p;
+    sel[j] = -1; has_point[j] = 1;
+  }
+  if (tid == 0) dropped[b] += n - n_fill;
+}
+
+// MapPointCandidates::removeFrameCandidates: the candidates of the keyframe that leaves the ring are deleted, except those
+// matched in the new keyframe (the reference promotes them first: addCandidatePointToFrame runs before the ring drops a keyframe)
+__global__ void kf_drop_candidates_kernel(int n, svob200_map_point* pts, const svob200_feature_ref* obs, const int* match_ok, uint8_t* has_point, int kf_slot)
+{
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const svob200_map_point p = pts[i];
+  if (p.type != SVOB200_POINT_CANDIDATE || match_ok[i] || (int)obs[p.obs_begin].ref_frame_id != kf_slot) return;
+  pts[i].type = SVOB200_POINT_DELETED; pts[i].obs_begin = p.obs_end;
+  has_point[i] = 0;
 }
 
 // The head of Matcher::findMatchDirect for every map point (matcher.cpp:156-173): Point::getCloseViewObs (point.cpp:101-125: arg-max of
@@ -201,6 +336,7 @@ __global__ void kf_add_obs_kernel(DevCam cam, int n, int K, svob200_map_point* p
   for (int k = 0; k < 7; ++k) { f.T_cur_ref[k] = 0.0; T_obs[7 * (size_t)slot + k] = T_cur_w[7 * (size_t)image[i] + k]; }
   obs[slot] = f;
   pts[i].obs_begin = slot;
+  if (p.type == SVOB200_POINT_CANDIDATE) pts[i].type = SVOB200_POINT_UNKNOWN;   // MapPointCandidates::addCandidatePointToFrame
 }
 
 // Map::safeDeleteFrame -> Point::deleteFrameRef for every point seen in the keyframe that leaves the ring
@@ -326,6 +462,12 @@ struct svob200_tracker {
   svob200_feature_ref* d_pobs = nullptr; double* d_T_pobs = nullptr; uint8_t* d_active = nullptr;
   int* d_match_level = nullptr; double* d_match_A = nullptr;
   int* d_sel = nullptr;                    // observation slot currently copied into d_ftrs[i] (-1: none)
+  // point pool (svob200_tracker_set_point_pool): every sequence owns max(its set_keyframe points, pt_capacity) point slots;
+  // the candidates of the steps of each parity wait in d_cand[parity] (one entry per point slot) until two steps later
+  int pt_capacity = -1;                    // -1: no pool
+  CandRec* d_cand[2] = {};
+  int* d_cand_n[2] = {};                   // candidates of the sequence in that step (the entries beyond its slots are dropped)
+  int *d_pt_created = nullptr, *d_pt_dropped = nullptr, *d_pt_rank = nullptr;
   // depth-filter seeds: 32-byte compact records + keyframe tables (pose per (keyframe, image), frame slot per keyframe)
   SeedRef* d_seed_refs = nullptr;
   double* d_T_kf = nullptr;            // [max_kfs][batch][7]
@@ -524,42 +666,52 @@ int svob200_tracker_set_keyframe(svob200_tracker* t, const uint8_t* imgs, int st
   svob200_ctx* ctx = t->ctx;
   if (t->d_stats) return fail(ctx, SVOB200_ERR_UNSUPPORTED, "tracker_set_keyframe: keyframe already set (svob200_tracker_add_keyframe inserts further ones)");
   const int B = t->batch;
-  const int N = ftr_offsets[B];
+  const int N_in = ftr_offsets[B];
   int S = seed_offsets[B];
   // validate everything BEFORE the first launch / allocation
-  if (N < 0 || S < 0 || ftr_offsets[0] != 0 || seed_offsets[0] != 0) return fail(ctx, SVOB200_ERR_ARG, "tracker_set_keyframe: bad offsets");
+  if (N_in < 0 || S < 0 || ftr_offsets[0] != 0 || seed_offsets[0] != 0) return fail(ctx, SVOB200_ERR_ARG, "tracker_set_keyframe: bad offsets");
   for (int b = 0; b < B; ++b)
     if (ftr_offsets[b + 1] < ftr_offsets[b] || seed_offsets[b + 1] < seed_offsets[b]) return fail(ctx, SVOB200_ERR_ARG, "tracker_set_keyframe: offsets must be non-decreasing");
-  if (N > 0 && (!kf_px || !kf_level || !pt_world)) return fail(ctx, SVOB200_ERR_ARG, "tracker_set_keyframe: null feature arrays with %d features", N);
+  if (N_in > 0 && (!kf_px || !kf_level || !pt_world)) return fail(ctx, SVOB200_ERR_ARG, "tracker_set_keyframe: null feature arrays with %d features", N_in);
   if (S > 0 && (!seed_px || !seed_level)) return fail(ctx, SVOB200_ERR_ARG, "tracker_set_keyframe: null seed arrays with %d seeds", S);
-  for (int i = 0; i < N; ++i) if (kf_level[i] < 0 || kf_level[i] >= t->n_levels) return fail(ctx, SVOB200_ERR_ARG, "tracker_set_keyframe: kf_level[%d] = %d outside the pyramid", i, kf_level[i]);
+  for (int i = 0; i < N_in; ++i) if (kf_level[i] < 0 || kf_level[i] >= t->n_levels) return fail(ctx, SVOB200_ERR_ARG, "tracker_set_keyframe: kf_level[%d] = %d outside the pyramid", i, kf_level[i]);
   for (int i = 0; i < S; ++i) if (seed_level[i] < 0 || seed_level[i] >= t->n_levels) return fail(ctx, SVOB200_ERR_ARG, "tracker_set_keyframe: seed_level[%d] = %d outside the pyramid", i, seed_level[i]);
   if (int e = svob200_frame_upload(ctx, t->fid_kfs[0], imgs, stride, nullptr, SVOB200_MEM_HOST)) return e;
   // seed pool: sequence b owns slots [pool_off[b], pool_off[b+1]) = its seeds followed by empty slots up to the capacity
   std::vector<int> pool_off(B + 1, 0);
   for (int b = 0; b < B; ++b) pool_off[b + 1] = pool_off[b] + std::max(seed_offsets[b + 1] - seed_offsets[b], t->seed_capacity);
   const int S_pool = pool_off[B];
+  // point slots: sequence b owns [pt_off[b], pt_off[b+1]) = its map points followed, with a point pool, by empty slots
+  std::vector<int> pt_off(B + 1, 0);
+  for (int b = 0; b < B; ++b) pt_off[b + 1] = pt_off[b] + std::max(ftr_offsets[b + 1] - ftr_offsets[b], t->pt_capacity);
+  const int N = pt_off[B];
   t->N = N; t->S = S_pool;
   S = S_pool;                                                            // from here on S counts pool slots
-  t->h_ftr_off.assign(ftr_offsets, ftr_offsets + B + 1);
-  t->h_pt_world.assign(pt_world, pt_world + 3 * (size_t)N);
+  t->h_ftr_off = pt_off;
+  t->h_pt_world.assign(3 * (size_t)N, 0.0);
   t->h_seed_off = pool_off;
-  for (int b = 0; b < B; ++b) t->max_per = std::max(t->max_per, ftr_offsets[b + 1] - ftr_offsets[b]);
+  for (int b = 0; b < B; ++b) t->max_per = std::max(t->max_per, pt_off[b + 1] - pt_off[b]);
   const int slot = svob200_frame_slot(ctx, t->fid_kfs[0]);
   t->kf_batch[0] = 0; t->n_kfs = 1;
   std::vector<svob200_feature_ref> ftrs(N);
   std::vector<SeedRef> srefs(S_pool);
   std::vector<int> image(N);
-  std::vector<double> Tf((size_t)7 * N);
+  std::vector<uint8_t> has_point(N, 0);
+  std::vector<double> Tf((size_t)7 * N, 0.0);
   std::vector<svob200_seed> seeds(S_pool, t->seed_init);
   for (int b = 0; b < B; ++b) {
-    for (int i = ftr_offsets[b]; i < ftr_offsets[b + 1]; ++i) {
-      svob200_feature_ref& f = ftrs[i];
+    for (int j = pt_off[b]; j < pt_off[b + 1]; ++j) {
+      svob200_feature_ref& f = ftrs[j];
       memset(&f, 0, sizeof(f));
-      f.ref_frame_id = slot; f.ref_image = b; f.cur_image = b; f.level = kf_level[i]; f.type = 0;
+      f.ref_image = b; f.cur_image = b;
+      image[j] = b;
+      const int i = ftr_offsets[b] + (j - pt_off[b]);
+      if (i >= ftr_offsets[b + 1]) continue;                             // empty slot of the point pool
+      f.ref_frame_id = slot; f.level = kf_level[i]; f.type = 0;
       f.px[0] = kf_px[2 * i]; f.px[1] = kf_px[2 * i + 1]; f.grad[0] = 1.0; f.grad[1] = 0.0;
-      image[i] = b;
-      memcpy(&Tf[(size_t)7 * i], T_kf_w + 7 * b, 7 * sizeof(double));
+      memcpy(&Tf[(size_t)7 * j], T_kf_w + 7 * b, 7 * sizeof(double));
+      memcpy(&t->h_pt_world[3 * (size_t)j], pt_world + 3 * (size_t)i, 3 * sizeof(double));
+      has_point[j] = 1;
     }
     for (int q = pool_off[b]; q < pool_off[b + 1]; ++q) {
       SeedRef& r = srefs[q];
@@ -580,6 +732,10 @@ int svob200_tracker_set_keyframe(svob200_tracker* t, const uint8_t* imgs, int st
   own(t->d_T_cur, 7 * (size_t)B); own(t->d_depth_ref, N); own(t->d_px_in, 2 * (size_t)N); own(t->d_px_out, 2 * (size_t)N);
   own(t->d_align, B); own(t->d_obs, S); own(t->d_stats, B); own(t->d_stats2, B);
   own(t->d_align_scratch, sparse_align_scratch_bytes(N)); own(t->d_seed_scratch, seeds_scratch_bytes(S)); own(t->d_match_scratch, match_scratch_bytes(N));
+  if (t->pt_capacity >= 0) {
+    for (int p = 0; p < 2; ++p) { own(t->d_cand[p], N); own(t->d_cand_n[p], B); }
+    own(t->d_pt_created, B); own(t->d_pt_dropped, B); own(t->d_pt_rank, N);
+  }
   if (err) {                 // an allocation that failed leaves the tracker as it was before the call (it can be retried or destroyed)
     for (void* q : t->owned) cudaFree(q);
     t->owned.clear();
@@ -587,15 +743,20 @@ int svob200_tracker_set_keyframe(svob200_tracker* t, const uint8_t* imgs, int st
     return err;
   }
   cudaStream_t s = ctx->stream;
-  CU(cudaMemcpyAsync(t->d_ftr_off, ftr_offsets, sizeof(int) * (B + 1), cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(t->d_ftr_off, pt_off.data(), sizeof(int) * (B + 1), cudaMemcpyHostToDevice, s));
   CU(cudaMemcpyAsync(t->d_seed_off, pool_off.data(), sizeof(int) * (B + 1), cudaMemcpyHostToDevice, s));
   CU(cudaMemcpyAsync(t->d_ftr_image, image.data(), sizeof(int) * N, cudaMemcpyHostToDevice, s));
-  CU(cudaMemsetAsync(t->d_has_point, 1, N ? N : 1, s));
+  CU(cudaMemcpyAsync(t->d_has_point, has_point.data(), N, cudaMemcpyHostToDevice, s));
+  if (t->pt_capacity >= 0) {
+    for (int p = 0; p < 2; ++p) CU(cudaMemsetAsync(t->d_cand_n[p], 0, sizeof(int) * B, s));
+    CU(cudaMemsetAsync(t->d_pt_created, 0, sizeof(int) * B, s));
+    CU(cudaMemsetAsync(t->d_pt_dropped, 0, sizeof(int) * B, s));
+  }
   CU(cudaMemcpyAsync(t->d_ftrs, ftrs.data(), sizeof(svob200_feature_ref) * N, cudaMemcpyHostToDevice, s));
   CU(cudaMemcpyAsync(t->d_seed_refs, srefs.data(), sizeof(SeedRef) * S, cudaMemcpyHostToDevice, s));
   CU(cudaMemcpyAsync(t->d_T_kf, T_kf_w, sizeof(double) * 7 * B, cudaMemcpyHostToDevice, s));
   CU(cudaMemcpyAsync(t->d_kf_slot, &slot, sizeof(int), cudaMemcpyHostToDevice, s));
-  CU(cudaMemcpyAsync(t->d_pt_world, pt_world, sizeof(double) * 3 * N, cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(t->d_pt_world, t->h_pt_world.data(), sizeof(double) * 3 * N, cudaMemcpyHostToDevice, s));
   CU(cudaMemcpyAsync(t->d_T_kf_ftr, Tf.data(), sizeof(double) * 7 * N, cudaMemcpyHostToDevice, s));
   CU(cudaMemcpyAsync(t->d_seeds, seeds.data(), sizeof(svob200_seed) * S, cudaMemcpyHostToDevice, s));
   CU(cudaStreamSynchronize(s));
@@ -615,7 +776,8 @@ int svob200_tracker_set_keyframe(svob200_tracker* t, const uint8_t* imgs, int st
         CU(cudaMemcpyAsync(t->d_ftrs, ftrs.data(), sizeof(svob200_feature_ref) * n, cudaMemcpyHostToDevice, s));
         // every map point starts with ONE observation, in keyframe 0: the last slot of its block of K
         CU(cudaMemsetAsync(t->d_sel, 0xff, sizeof(int) * (size_t)n, s));
-        points_init_kernel<<<(n + 255) / 256, 256, 0, s>>>(n, t->max_kfs, t->d_ftrs, t->d_T_kf_ftr, t->d_pt_world, t->d_points, t->d_pobs, t->d_T_pobs);
+        points_init_kernel<<<(n + 255) / 256, 256, 0, s>>>(n, t->max_kfs, t->d_ftrs, t->d_T_kf_ftr, t->d_pt_world, t->d_has_point, t->d_points, t->d_pobs,
+                                                           t->d_T_pobs);
         ++ctx->launches;
       } else {
         for (int i = 0; i < n; ++i) { srefs[i].f[0] = f[3 * i]; srefs[i].f[1] = f[3 * i + 1]; srefs[i].f[2] = f[3 * i + 2]; }
@@ -639,6 +801,16 @@ int svob200_tracker_set_seed_pool(svob200_tracker* t, int capacity_per_sequence,
   int64_t id;
   while ((int)t->frame_pool.size() < t->max_kfs + 2)
     if (int e = new_frame(t, &id)) return e;
+  return SVOB200_OK;
+}
+
+int svob200_tracker_set_point_pool(svob200_tracker* t, int capacity_per_sequence)
+{
+  if (!t) return SVOB200_ERR_ARG;
+  svob200_ctx* ctx = t->ctx;
+  if (t->d_stats) return fail(ctx, SVOB200_ERR_ARG, "tracker_set_point_pool: call before set_keyframe");
+  if (capacity_per_sequence < 0) return fail(ctx, SVOB200_ERR_ARG, "tracker_set_point_pool: negative capacity %d", capacity_per_sequence);
+  t->pt_capacity = capacity_per_sequence;
   return SVOB200_OK;
 }
 
@@ -673,6 +845,9 @@ int svob200_tracker_add_keyframe(svob200_tracker* t, const float* depth_mean, co
     if (S) { kf_erase_seeds_kernel<<<(S + 255) / 256, 256, 0, s>>>(S, t->d_seed_refs, k); ++ctx->launches; }
     if (N) {                                                 // Map::safeDeleteFrame: the points forget the keyframe
       FrameRec* old = find_frame(ctx, t->fid_kfs[k]);
+      if (t->pt_capacity >= 0) {
+        kf_drop_candidates_kernel<<<(N + 255) / 256, 256, 0, s>>>(N, t->d_points, t->d_pobs, t->d_match_ok, t->d_has_point, old->slot); ++ctx->launches;
+      }
       kf_drop_obs_kernel<<<(N + 255) / 256, 256, 0, s>>>(N, t->max_kfs, t->d_points, t->d_pobs, t->d_T_pobs, old->slot, t->d_sel); ++ctx->launches;
     }
     t->fid_kfs[k] = 0;
@@ -747,11 +922,39 @@ int svob200_tracker_get_seed_refs(svob200_tracker* t, double* px, int* level, in
 }
 int svob200_tracker_num_seed_slots(svob200_tracker* t) { return t ? t->S : 0; }
 
+// the point slots as they stand (host arrays of N slots: 3 doubles pos, SVOB200_POINT_* type, observation count) and the
+// candidates created / dropped so far (one int per sequence); any pointer may be NULL
+int svob200_tracker_get_points(svob200_tracker* t, double* pos, int* type, int* n_obs, int* created, int* dropped)
+{
+  if (!t) return SVOB200_ERR_ARG;
+  svob200_ctx* ctx = t->ctx;
+  if (int e = ctx_join_aux(ctx)) return e;
+  const int B = t->batch;
+  std::vector<svob200_map_point> pts((size_t)std::max(t->N, 1));
+  std::vector<int> cr(B, 0), dr(B, 0);
+  if (t->N) CU(cudaMemcpyAsync(pts.data(), t->d_points, sizeof(svob200_map_point) * (size_t)t->N, cudaMemcpyDeviceToHost, ctx->stream));
+  if (t->d_pt_created) {
+    CU(cudaMemcpyAsync(cr.data(), t->d_pt_created, sizeof(int) * B, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaMemcpyAsync(dr.data(), t->d_pt_dropped, sizeof(int) * B, cudaMemcpyDeviceToHost, ctx->stream));
+  }
+  CU(cudaStreamSynchronize(ctx->stream));
+  for (int i = 0; i < t->N; ++i) {
+    if (pos) for (int k = 0; k < 3; ++k) pos[3 * (size_t)i + k] = pts[i].pos[k];
+    if (type) type[i] = pts[i].type;
+    if (n_obs) n_obs[i] = pts[i].obs_end - pts[i].obs_begin;
+  }
+  if (created) memcpy(created, cr.data(), sizeof(int) * B);
+  if (dropped) memcpy(dropped, dr.data(), sizeof(int) * B);
+  return SVOB200_OK;
+}
+int svob200_tracker_num_point_slots(svob200_tracker* t) { return t ? t->N : 0; }
+
 int svob200_tracker_set_chain(svob200_tracker* t, int cell_size, int max_fts, int pose_opt)
 {
   if (!t) return SVOB200_ERR_ARG;
   svob200_ctx* ctx = t->ctx;
   if (!t->d_stats) return fail(ctx, SVOB200_ERR_ARG, "tracker_set_chain: set_keyframe first");
+  if (t->pt_capacity >= 0) return fail(ctx, SVOB200_ERR_UNSUPPORTED, "tracker_set_chain: not available with a point pool");
   if (int e = ctx_join_aux(ctx)) return e;
   CU(cudaStreamSynchronize(ctx->stream));
   drop_graphs(t);                                                  // captured steps belong to the other mode
@@ -816,14 +1019,33 @@ static int enqueue_seeds_update(svob200_tracker* t, int c0, int c1, const SeedPo
 static int enqueue_step_stats(svob200_tracker* t, int c0, int c1, int parts, svob200_step_stats* d_stats, cudaStream_t st)
 {
   svob200_ctx* ctx = t->ctx;
-  const int cnt = c1 - c0;
-  step_stats_kernel<<<cnt, 128, 0, st>>>(t->d_ftr_off + c0, t->d_seed_off + c0, t->d_align + c0, t->d_T_cur + 7 * (size_t)c0, t->d_match_ok, t->d_obs,
-                                         t->d_seeds, t->seed_init, t->reseed, d_stats + c0, parts, t->d_seed_refs);
+  const int cnt = c1 - c0, par = (int)(t->step_no & 1);
+  const CandStage cand = {t->d_cand[par], t->d_cand_n[par], t->d_pt_created, t->d_ftr_off, t->d_T_kf, t->batch, c0};
+  auto kernel = cand.rec ? step_stats_kernel<true> : step_stats_kernel<false>;
+  kernel<<<cnt, 128, 0, st>>>(t->d_ftr_off + c0, t->d_seed_off + c0, t->d_align + c0, t->d_T_cur + 7 * (size_t)c0, t->d_match_ok, t->d_obs,
+                              t->d_seeds, t->seed_init, t->reseed, d_stats + c0, parts, t->d_seed_refs, cand);
   ++ctx->launches;
   if (t->chain_cell > 0) {
     chain_stats_kernel<<<(cnt + 127) / 128, 128, 0, st>>>(cnt, t->d_rstats + c0, t->d_pose + c0, t->chain_pose_opt, d_stats + c0); ++ctx->launches;
   }
   if (cudaGetLastError() != cudaSuccess) return fail(ctx, SVOB200_ERR_CUDA, "tracker_step: launch error");
+  return 0;
+}
+
+// point pool: the candidates of two steps ago take their slots, at the head of the step on the context's stream (outside any
+// captured graph).  Every shape waits for that step's depth filter first, so every shape inserts the same candidates.
+static int enqueue_insert_candidates(svob200_tracker* t)
+{
+  if (t->pt_capacity < 0) return 0;
+  svob200_ctx* ctx = t->ctx;
+  const int par = (int)(t->step_no & 1);
+  KfBatches kfb;
+  for (int k = 0; k < svob200_tracker::MAX_KFS; ++k) kfb.v[k] = t->kf_batch[k];
+  cand_insert_kernel<<<t->batch, 128, 0, ctx->stream>>>(t->max_kfs, t->batch, t->d_ftr_off, t->d_cand[par], t->d_cand_n[par], kfb, t->d_kf_slot, t->d_T_kf,
+                                                        t->d_points, t->d_pt_world, t->d_pobs, t->d_T_pobs, t->d_sel, t->d_has_point, t->d_pt_rank,
+                                                        t->d_pt_dropped);
+  ++ctx->launches;
+  if (cudaGetLastError() != cudaSuccess) return fail(ctx, SVOB200_ERR_CUDA, "tracker_step: candidate insertion launch error");
   return 0;
 }
 
@@ -964,7 +1186,7 @@ int svob200_tracker_step(svob200_tracker* t, const uint8_t* cur_imgs, int stride
     FrameRec* last = find_frame(ctx, t->fid_last);
     const std::vector<uintptr_t> key = {1, (uintptr_t)cur_imgs, (uintptr_t)stride, (uintptr_t)T_last_w, (uintptr_t)last_px, (uintptr_t)stats,
                                         (uintptr_t)px_refined, (uintptr_t)match_ok, (uintptr_t)t->fid_cur, (uintptr_t)t->fid_last,
-                                        (uintptr_t)last->f.lvl[0], (uintptr_t)last->f.pitch[0]};
+                                        (uintptr_t)last->f.lvl[0], (uintptr_t)last->f.pitch[0], (uintptr_t)(t->pt_capacity >= 0 ? par : 0)};
     if (use_graph) if (int e = ensure_fork_stream(t)) return e;
     // direct launches of a big batch: the depth filter follows on its own stream (graphs, profiling and chain mode run it in place)
     const bool df_on_stream = !use_graph && !t->profiling && t->chain_cell <= 0 && t->S > 0;
@@ -977,8 +1199,9 @@ int svob200_tracker_step(svob200_tracker* t, const uint8_t* cur_imgs, int stride
     }
     if (!df_on_stream && (t->df_pending[0] || t->df_pending[1]))       // a step that runs the depth filter in place after asynchronous ones
       if (int e = df_join(t)) return e;
+    if (int e = enqueue_insert_candidates(t)) return e;
     // graph + fork (only a capture runs the body then), asynchronous depth filter on this parity's pose table and step
-    // records, or in place
+    // records, or in place; with a point pool the captured step records its candidates into this parity's staging
     const RangeShape shape = {use_graph ? t->fork_stream : s, df_on_stream, (df_on_stream && par) ? t->d_seed_poses2 : t->d_seed_poses,
                               (df_on_stream && par) ? t->d_stats2 : t->d_stats};
     const int rc = graph_or_direct(t, use_graph, key, [&]() -> int {
@@ -1034,6 +1257,7 @@ int svob200_tracker_step(svob200_tracker* t, const uint8_t* cur_imgs, int stride
         CU(cudaMemcpyAsync(t->d_step_in, t->h_pinned, in_bytes, cudaMemcpyHostToDevice, s));
       }
     }
+    if (int e = enqueue_insert_candidates(t)) return e;
     const int chunk = (t->profiling || B <= svob200_tracker::CHUNK) ? B : svob200_tracker::CHUNK;
     const int n_chunks = (B + chunk - 1) / chunk;
     if (!t->copy_stream) CU(cudaStreamCreateWithFlags(&t->copy_stream, cudaStreamNonBlocking));
@@ -1068,7 +1292,8 @@ int svob200_tracker_step(svob200_tracker* t, const uint8_t* cur_imgs, int stride
       if (use_graph) {
         FrameRec* last = find_frame(ctx, t->fid_last);
         const std::vector<uintptr_t> key = {2, (uintptr_t)t->fid_cur, (uintptr_t)t->fid_last, (uintptr_t)r->f.lvl[0], (uintptr_t)r->f.pitch[0],
-                                            (uintptr_t)last->f.lvl[0], (uintptr_t)last->f.pitch[0], (uintptr_t)d_T_last};
+                                            (uintptr_t)last->f.lvl[0], (uintptr_t)last->f.pitch[0], (uintptr_t)d_T_last,
+                                            (uintptr_t)(t->pt_capacity >= 0 ? (t->step_no & 1) : 0)};
         if (int e = graph_or_direct(t, true, key, [&]() { return run_range(t, 0, B, d_T_last, d_last_px, true, shape); })) return e;
       } else if (int e = run_range(t, c0, c1, d_T_last, d_last_px, n_chunks == 1, shape)) return e;
     }

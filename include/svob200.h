@@ -311,6 +311,30 @@ int  svob200_tracker_set_detector(svob200_tracker* t, int cell_size, int n_detec
 int  svob200_tracker_add_keyframe(svob200_tracker* t, const float* depth_mean, const float* depth_min, int* n_new_seeds, int* n_dropped);
 int  svob200_tracker_get_seed_refs(svob200_tracker* t, double* px, int* level, int* kf, int* batch_id, int* state);
 int  svob200_tracker_num_seed_slots(svob200_tracker* t);
+/* ---- point pool: converged seeds become map points on the device (DepthFilter::updateSeeds -> seed_converged_cb_ ->
+ * MapPointCandidates::newCandidatePoint, addCandidatePointToFrame, removeFrameCandidates).  Opt-in: without the call nothing changes.
+ * svob200_tracker_set_point_pool (before set_keyframe; SVOB200_ERR_ARG after it or for a negative capacity): sequence b owns
+ *   max(its set_keyframe points, capacity_per_sequence) point slots, its set_keyframe points first, then empty slots.  From then
+ *   on every per-map-feature array of svob200_tracker_step (last_px, px_refined, match_ok) has one entry per SLOT
+ *   (svob200_tracker_num_point_slots).  svob200_tracker_set_chain returns SVOB200_ERR_UNSUPPORTED on such a tracker.
+ * Creation: a seed whose status in step k is SVOB200_SEED_CONVERGED becomes a candidate, whatever reseed then does to the seed:
+ *   position kf.T_f_w.inverse() * (f * (1.0 / mu)), one observation (the seed's feature in its keyframe), type
+ *   SVOB200_POINT_CANDIDATE.  A step records at most as many candidates per sequence as the sequence has point slots.
+ * Insertion at the head of step k + 2: the reference's depth filter runs one frame behind tracking (its own thread), and so does
+ *   the tracker's asynchronous depth filter, whose step k has finished only when step k + 2 starts; every shape (graph, in
+ *   place, asynchronous, host or device memory) inserts then, so all give the same results.  Candidates take the sequence's
+ *   empty slots in slot order, in the reference's list order (ascending Seed::batch_id, then seed slot).  A candidate that
+ *   finds no empty slot, or whose keyframe left the ring in between, is dropped.  From its insertion a candidate is selected,
+ *   matched and used in sparse alignment (with the caller's last_px) like every map point; empty slots report match_ok 0.
+ * Promotion (svob200_tracker_add_keyframe): a candidate matched in the new keyframe gains the observation and becomes
+ *   SVOB200_POINT_UNKNOWN; it marks the detector's occupancy grid like every matched point.  Removal: when a keyframe leaves
+ *   the ring, its candidates that were not matched in the new keyframe are deleted and their slots become empty.
+ * svob200_tracker_get_points (host arrays, any may be NULL; joins the asynchronous depth filter): per slot 3 doubles pos, the
+ *   SVOB200_POINT_* type (DELETED: empty slot) and the observation count; per sequence the candidates created and dropped so far.
+ * svob200_tracker_num_point_slots: the slot count (without a pool: the set_keyframe point count). */
+int  svob200_tracker_set_point_pool(svob200_tracker* t, int capacity_per_sequence);
+int  svob200_tracker_num_point_slots(svob200_tracker* t);
+int  svob200_tracker_get_points(svob200_tracker* t, double* pos, int* type, int* n_obs, int* created, int* dropped);
 /* Chain mode (call after set_keyframe): between sparse alignment and the depth filter the step runs
  * Reprojector::reprojectMap over the keyframe's map points (grid of cell_size, first success per cell, max_fts) and, with
  * pose_opt != 0, pose_optimizer::optimizeGaussNewton on the matched features — FrameHandlerMono::processFrame's Step 2 and
