@@ -29,6 +29,17 @@ struct DevCam { int width, height; double fx, fy, cx, cy; };
 
 __host__ __device__ inline int align_up_i(int v, int a) { return (v + a - 1) / a * a; }
 
+// (int) of a double the way x86 cvttsd2si does it (NaN / out of range -> INT_MIN); Eigen's cast<int>() on the host
+__device__ __forceinline__ int x86_d2i(double v) { return (v > -2147483649.0 && v < 2147483648.0) ? (int)v : (int)0x80000000; }
+
+// Seed ctor depth_filter.cpp:36-45
+__host__ __device__ inline svob200_seed seed_prior(float depth_mean, float depth_min)
+{
+  svob200_seed s;
+  s.a = 10; s.b = 10; s.mu = (float)(1.0 / depth_mean); s.z_range = (float)(1.0 / depth_min); s.sigma2 = s.z_range * s.z_range / 36;
+  return s;
+}
+
 // ---------------------------------------------------------------- SE3 / SO3 (SE3.h, SO3.h)
 struct v3d { double x, y, z; };
 __device__ __forceinline__ v3d v3_add(v3d a, v3d b) { return {a.x + b.x, a.y + b.y, a.z + b.z}; }
@@ -173,4 +184,22 @@ __device__ __forceinline__ int warp_sum_i(int v)
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
   return v;
+}
+
+// exclusive prefix sum over an NT-thread block (every thread calls it); *total = the block's sum.  It ends with a barrier, so
+// one call may follow another (they share the partials).
+template <int NT>
+__device__ int block_exclusive_scan(int v, int* total)
+{
+  __shared__ int s_w[NT / 32];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  int x = v;
+  for (int o = 1; o < 32; o <<= 1) { const int y = __shfl_up_sync(0xffffffffu, x, o); if (lane >= o) x += y; }
+  if (lane == 31) s_w[w] = x;
+  __syncthreads();
+  int before = 0, sum = 0;
+  for (int k = 0; k < NT / 32; ++k) { if (k < w) before += s_w[k]; sum += s_w[k]; }
+  *total = sum;
+  __syncthreads();
+  return before + x - v;
 }

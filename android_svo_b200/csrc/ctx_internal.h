@@ -109,6 +109,66 @@ inline int ensure_host_stage(svob200_ctx* ctx, size_t n)
   return 0;
 }
 
+// Three-region staging plan: IN | INOUT | OUT.  Device copies cover [0, end(INOUT)) on the way in
+// and [begin(INOUT), end) on the way out — one cudaMemcpyAsync each way per call.
+struct Stage {
+  svob200_ctx* ctx; int mem;
+  struct Item { const void* src; void* dst; size_t bytes, off; int kind; };   // kind 0 in, 1 inout, 2 out
+  std::vector<Item> items;
+  size_t total = 0, in_end = 0, io_begin = 0;
+  bool pushed = false, drained = false;
+  Stage(svob200_ctx* c, int m) : ctx(c), mem(m) {}
+  // a call that fails between push() and download() must not leave its host->device copy in flight: the next call's upload()
+  // writes the same pinned staging buffer
+  ~Stage() { if (pushed && !drained) cudaStreamSynchronize(ctx->stream); }
+  // returns an index; resolve() gives the device pointer
+  int add(const void* src, void* dst, size_t bytes, int kind) { items.push_back({src, dst, bytes, 0, kind}); return (int)items.size() - 1; }
+  int layout()
+  {
+    if (mem == SVOB200_MEM_DEVICE) return 0;
+    size_t off = 0;
+    for (int kind = 0; kind < 3; ++kind) {
+      if (kind == 1) io_begin = off;
+      for (auto& it : items) if (it.kind == kind) { it.off = off; off += (it.bytes + 255) & ~(size_t)255; }
+      if (kind == 1) in_end = off;
+    }
+    total = off;
+    if (int r = ensure_host_stage(ctx, total)) return r;
+    if (ctx->d_stage.ensure(total) != cudaSuccess) return fail(ctx, SVOB200_ERR_NOMEM, "device staging alloc of %zu bytes failed", total);
+    return 0;
+  }
+  template <class T> T* dev(int idx)
+  {
+    Item& it = items[idx];
+    if (mem == SVOB200_MEM_DEVICE) return (T*)(it.kind == 2 ? it.dst : (it.kind == 1 ? it.dst : const_cast<void*>(it.src)));
+    return reinterpret_cast<T*>(static_cast<uint8_t*>(ctx->d_stage.p) + it.off);
+  }
+  template <class T> T* host(int idx) { return reinterpret_cast<T*>(ctx->h_stage + items[idx].off); }   // staged host copy (HOST mode)
+  int upload()
+  {
+    if (mem == SVOB200_MEM_DEVICE) return 0;
+    for (auto& it : items) if (it.kind <= 1 && it.src && it.bytes) memcpy(ctx->h_stage + it.off, it.src, it.bytes);
+    return 0;
+  }
+  int push()
+  {
+    if (mem == SVOB200_MEM_DEVICE || in_end == 0) return 0;
+    pushed = true;
+    CU(cudaMemcpyAsync(ctx->d_stage.p, ctx->h_stage, in_end, cudaMemcpyHostToDevice, ctx->stream));
+    return 0;
+  }
+  int download()
+  {
+    if (mem == SVOB200_MEM_DEVICE) return 0;
+    if (total > io_begin)
+      CU(cudaMemcpyAsync(ctx->h_stage + io_begin, static_cast<uint8_t*>(ctx->d_stage.p) + io_begin, total - io_begin, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    drained = true;
+    for (auto& it : items) if (it.kind >= 1 && it.dst && it.bytes) memcpy(it.dst, ctx->h_stage + it.off, it.bytes);
+    return 0;
+  }
+};
+
 // Level 0 of a frame is its own storage or aliases a caller's device buffer; only these two switch it, and they rewrite the
 // frame's row of the device table on ctx->stream.  Bind rejects (SVOB200_ERR_ARG, nothing changes) a buffer or stride that
 // is not 16-byte aligned and a stride below the width; copy_pixels copies the aliased images into the frame's own storage.

@@ -18,9 +18,6 @@
 
 namespace {
 
-// (int) of a double the way x86 cvttsd2si does it (NaN / out of range -> INT_MIN); Eigen's cast<int>() on the host
-__device__ __forceinline__ int x86_d2i(double v) { return (v > -2147483649.0 && v < 2147483648.0) ? (int)v : (int)0x80000000; }
-
 __device__ __forceinline__ v3d frame_pos(const double* T)           // Frame::pos() frame.h:105
 {
   double inv[7];
@@ -97,7 +94,6 @@ __global__ void __launch_bounds__(REPROJ_T) reproj_cells_kernel(DevCam cam, cons
                                                                 double* m_f, int* m_level, double* m_pos, int* m_point, int* m_count)
 {
   __shared__ uint32_t s_best[REPROJ_MAX_CELLS];
-  __shared__ int s_scan[REPROJ_T];
   __shared__ int s_cnt[4];
   const int b = blockIdx.x, tid = threadIdx.x;
   const int p0 = pt_off[b], p1 = pt_off[b + 1];
@@ -115,15 +111,8 @@ __global__ void __launch_bounds__(REPROJ_T) reproj_cells_kernel(DevCam cam, cons
   const int c0 = min(tid * chunk, n_cells), c1 = min(c0 + chunk, n_cells);
   int local = 0;
   for (int c = c0; c < c1; ++c) local += s_best[c] != 0xffffffffu;
-  s_scan[tid] = local;
-  __syncthreads();
-  for (int off = 1; off < REPROJ_T; off <<= 1) {
-    const int v = tid >= off ? s_scan[tid - off] : 0;
-    __syncthreads();
-    s_scan[tid] += v;
-    __syncthreads();
-  }
-  int run = s_scan[tid] - local;                       // matched cells before c0
+  int total;
+  int run = block_exclusive_scan<REPROJ_T>(local, &total);   // matched cells before c0
   int my_matches = 0;
   for (int c = c0; c < c1; ++c) {
     const bool has = s_best[c] != 0xffffffffu;
@@ -428,31 +417,22 @@ __global__ void __launch_bounds__(256) seeds_compact_kernel(const svob200_corner
                                                             const float* depth_min, svob200_corner* corners_out, svob200_seed* seeds_out,
                                                             int* counts)
 {
-  __shared__ int s_scan[256];
   const int b = blockIdx.x, tid = threadIdx.x;
   const svob200_corner* C = cells + (size_t)b * n_cells;
   const int chunk = (n_cells + 255) / 256;
   const int c0 = min(tid * chunk, n_cells), c1 = min(c0 + chunk, n_cells);
   int local = 0;
   for (int c = c0; c < c1; ++c) local += (double)C[c].score > thr;
-  s_scan[tid] = local;
-  __syncthreads();
-  for (int off = 1; off < 256; off <<= 1) {
-    const int v = tid >= off ? s_scan[tid - off] : 0;
-    __syncthreads();
-    s_scan[tid] += v;
-    __syncthreads();
-  }
-  int run = s_scan[tid] - local;
-  svob200_seed sd;
-  sd.a = 10; sd.b = 10; sd.mu = (float)(1.0 / depth_mean[b]); sd.z_range = (float)(1.0 / depth_min[b]); sd.sigma2 = sd.z_range * sd.z_range / 36;
+  int total;
+  int run = block_exclusive_scan<256>(local, &total);
+  const svob200_seed sd = seed_prior(depth_mean[b], depth_min[b]);
   for (int c = c0; c < c1; ++c) {
     if (!((double)C[c].score > thr)) continue;
     corners_out[(size_t)b * n_cells + run] = C[c];
     seeds_out[(size_t)b * n_cells + run] = sd;
     ++run;
   }
-  if (tid == 255) counts[b] = s_scan[255];
+  if (tid == 0) counts[b] = total;
 }
 
 inline size_t up256(size_t b) { return (b + 255) & ~(size_t)255; }

@@ -281,7 +281,8 @@ def test_tracker_points_shapes_identical(ctx, oracle, seqs):
 @pytest.mark.gpu
 def test_tracker_point_pool_validation(ctx, seqs):
     """set_point_pool after set_keyframe or with a negative capacity is rejected; chain mode refuses a pool; without a pool the
-    slot count is the set_keyframe point count and no candidate is counted."""
+    slot count is the set_keyframe point count and no candidate is counted.  With unequal counts per sequence, the point and
+    seed slots right after set_keyframe equal the caller's arrays laid out in numpy."""
     from android_svo_b200 import capi
     cfg = seqs[0][0]
     which = np.arange(2)
@@ -309,3 +310,29 @@ def test_tracker_point_pool_validation(ctx, seqs):
         assert rc == -4                                            # SVOB200_ERR_UNSUPPORTED
     finally:
         t2.close()
+    # unequal counts per sequence (one without map points, one without seeds), pool capacities above and below them: right after
+    # set_keyframe each sequence's slots hold its map points / seeds in order, then empty slots
+    n_pt, n_sd, cap_pt, cap_sd = [cfg["n_features"], 0, 37, 90], [S0, 50, 0, 7], 100, 60
+    src = [seqs[b % 2] for b in range(4)]
+    take = lambda key, n: np.concatenate([src[b][3][key][:n[b]] for b in range(4)])
+    t3 = capi.Tracker(ctx, scenes.cam_of(cfg, capi.Camera), 4, cfg["n_levels"], cfg["max_level"], cfg["min_level"], cfg["n_pyr"])
+    try:
+        t3.set_seed_pool(cap_sd, *POOL)
+        t3.set_point_pool(cap_pt)
+        t3.set_keyframe(np.stack([s[2][0] for s in src]), np.stack([s[1][0] for s in src]), np.cumsum([0] + n_pt), take("kf_px", n_pt),
+                        take("kf_level", n_pt), take("pt_world", n_pt), np.cumsum([0] + n_sd), take("seed_px", n_sd), take("seed_level", n_sd))
+
+        def slots(key, n, cap, width):
+            return np.concatenate([np.concatenate([np.asarray(src[b][3][key], np.float64)[:n[b]].reshape(-1, width), np.zeros((max(n[b], cap) - n[b], width))])
+                                   for b in range(4)])
+        real_pt = np.concatenate([np.arange(max(n, cap_pt)) < n for n in n_pt])
+        real_sd = np.concatenate([np.arange(max(n, cap_sd)) < n for n in n_sd])
+        assert t3.P == len(real_pt) == 120 + 3 * 100 and t3.S == len(real_sd) == S0 + 3 * 60
+        pos, ty, no, cr, dr = t3.points()
+        assert np.array_equal(bits(pos), bits(slots("pt_world", n_pt, cap_pt, 3)))
+        assert np.array_equal(ty, np.where(real_pt, UNKNOWN, DELETED)) and np.array_equal(no, real_pt) and not cr.any() and not dr.any()
+        px, lv, kf, bt, st = t3.seed_refs()
+        assert np.array_equal(bits(px), bits(slots("seed_px", n_sd, cap_sd, 2))) and np.array_equal(lv, slots("seed_level", n_sd, cap_sd, 1)[:, 0])
+        assert not kf.any() and not bt.any() and np.array_equal(st, ~real_sd)
+    finally:
+        t3.close()
