@@ -125,6 +125,8 @@ def load_library():
     L.svob200_tracker_set_seed_pool.argtypes = [V, C.c_int, C.c_int, C.c_int, C.c_int]
     L.svob200_tracker_set_detector.argtypes = [V, C.c_int, C.c_int, C.c_double]
     L.svob200_tracker_add_keyframe.argtypes = [V, V, V, V, V]
+    L.svob200_tracker_add_keyframes.argtypes = [V, V, V, V, V, V, C.c_int]
+    L.svob200_tracker_scene_depth.argtypes = [V, V, V, V, C.c_int]
     L.svob200_tracker_get_seed_refs.argtypes = [V, V, V, V, V, V]
     L.svob200_tracker_num_seed_slots.argtypes = [V]
     L.svob200_tracker_set_point_pool.argtypes = [V, C.c_int]
@@ -181,6 +183,7 @@ EXPORTED_SYMBOLS = [
     "svob200_points_optimize", "svob200_seeds_initialize", "svob200_tracker_debug_align", "svob200_tracker_set_chain",
     "svob200_tracker_set_seed_pool", "svob200_tracker_set_detector", "svob200_tracker_add_keyframe", "svob200_tracker_get_seed_refs",
     "svob200_tracker_num_seed_slots", "svob200_tracker_set_point_pool", "svob200_tracker_num_point_slots", "svob200_tracker_get_points",
+    "svob200_tracker_add_keyframes", "svob200_tracker_scene_depth",
 ]
 
 
@@ -546,6 +549,37 @@ class Tracker:
         n_new = np.zeros(self.batch, np.int32); n_drop = np.zeros(self.batch, np.int32)
         self.ctx._ck(self.L.svob200_tracker_add_keyframe(self.h, _ptr(dm), _ptr(dn), _ptr(n_new), _ptr(n_drop)))
         return n_new, n_drop
+
+    def add_keyframes(self, which, depth_mean, depth_min):
+        """the frame of the most recent step becomes a keyframe of the sequences with which[b] != 0 (None: every sequence), each
+        in its own ring: returns (new seeds, dropped corners) per sequence, 0 for the sequences not selected and -1 for a
+        selected sequence that has used up its 65,534 keyframes"""
+        w = None if which is None else np.ascontiguousarray(np.broadcast_to(np.asarray(which) != 0, (self.batch,)), dtype=np.uint8)
+        dm = np.ascontiguousarray(np.broadcast_to(np.asarray(depth_mean, np.float32), (self.batch,)))
+        dn = np.ascontiguousarray(np.broadcast_to(np.asarray(depth_min, np.float32), (self.batch,)))
+        n_new = np.zeros(self.batch, np.int32); n_drop = np.zeros(self.batch, np.int32)
+        self.ctx._ck(self.L.svob200_tracker_add_keyframes(self.h, _ptr(w), _ptr(dm), _ptr(dn), _ptr(n_new), _ptr(n_drop), MEM_HOST))
+        return n_new, n_drop
+
+    def add_keyframes_raw(self, which_ptr, depth_mean_ptr, depth_min_ptr, n_new_ptr=0, n_dropped_ptr=0, mem=MEM_DEVICE):
+        """Pointer-level add_keyframes (device addresses by default: ordered on the context's stream, no synchronisation);
+        0 for which_ptr = every sequence, 0 for an output = not wanted."""
+        V = lambda p: C.c_void_p(p) if p else None
+        self.ctx._ck(self.L.svob200_tracker_add_keyframes(self.h, V(which_ptr), V(depth_mean_ptr), V(depth_min_ptr), V(n_new_ptr), V(n_dropped_ptr), int(mem)))
+
+    def scene_depth(self, depth_mean=None, depth_min=None):
+        """frame_utils::getSceneDepth of the most recent step's frame per sequence: (depth_mean, depth_min, n_points); a sequence
+        without a matched point keeps the value of the arrays passed in (default NaN)"""
+        dm = np.array(np.broadcast_to(np.nan if depth_mean is None else np.asarray(depth_mean, np.float32), (self.batch,)), np.float32)
+        dn = np.array(np.broadcast_to(np.nan if depth_min is None else np.asarray(depth_min, np.float32), (self.batch,)), np.float32)
+        n = np.zeros(self.batch, np.int32)
+        self.ctx._ck(self.L.svob200_tracker_scene_depth(self.h, _ptr(dm), _ptr(dn), _ptr(n), MEM_HOST))
+        return dm, dn, n
+
+    def scene_depth_raw(self, depth_mean_ptr, depth_min_ptr, n_points_ptr=0, mem=MEM_DEVICE):
+        """Pointer-level scene_depth (device addresses by default: ordered on the context's stream, no synchronisation)"""
+        self.ctx._ck(self.L.svob200_tracker_scene_depth(self.h, C.c_void_p(depth_mean_ptr), C.c_void_p(depth_min_ptr),
+                                                         C.c_void_p(n_points_ptr) if n_points_ptr else None, int(mem)))
 
     def seed_refs(self):
         """(px[S,2], level, kf, batch_id, state) of every pool slot; state 0 = alive"""

@@ -32,11 +32,9 @@ int frame_bind_level0(svob200_ctx* ctx, FrameRec* r, const uint8_t* dev_gray, in
   return 0;
 }
 
-int frame_own_level0(svob200_ctx* ctx, FrameRec* r, bool copy_pixels)
+int frame_own_level0(svob200_ctx* ctx, FrameRec* r)
 {
   if (r->f.lvl[0] == r->own_l0) return 0;
-  if (copy_pixels)
-    CU(cudaMemcpy2DAsync(r->own_l0, r->own_pitch0, r->f.lvl[0], r->f.pitch[0], r->f.w[0], (size_t)r->f.h[0] * r->f.batch, cudaMemcpyDeviceToDevice, ctx->stream));
   r->f.lvl[0] = r->own_l0; r->f.pitch[0] = r->own_pitch0; r->f.img_stride[0] = (unsigned long long)r->own_pitch0 * r->f.h[0];
   CU(cudaMemcpyAsync(ctx->d_table + r->slot, &r->f, sizeof(DevFrame), cudaMemcpyHostToDevice, ctx->stream));
   return 0;
@@ -182,7 +180,7 @@ int svob200_frame_upload(svob200_ctx* ctx, int64_t frame_id, const uint8_t* gray
   FrameRec* r = find_frame(ctx, frame_id);
   if (!r) return fail(ctx, SVOB200_ERR_NOFRAME, "frame %lld not found", (long long)frame_id);
   if (stride < r->f.w[0]) return fail(ctx, SVOB200_ERR_ARG, "frame_upload: stride < width");
-  if (int e = frame_own_level0(ctx, r, false)) return e;
+  if (int e = frame_own_level0(ctx, r)) return e;
   CU(cudaMemcpy2DAsync(r->f.lvl[0], r->f.pitch[0], gray, stride, r->f.w[0], (size_t)r->f.h[0] * r->f.batch,
                        mem == SVOB200_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, ctx->stream));
   if (int e = build_levels(ctx, r, round_modes)) return e;
@@ -589,7 +587,7 @@ int svob200_frame_upload_level(svob200_ctx* ctx, int64_t frame_id, int image, in
   FrameRec* r = find_frame(ctx, frame_id);
   if (!r) return fail(ctx, SVOB200_ERR_NOFRAME, "frame %lld not found", (long long)frame_id);
   if (level < 0 || level >= r->f.n_levels || image < 0 || image >= r->f.batch || stride < r->f.w[level]) return fail(ctx, SVOB200_ERR_ARG, "frame_upload_level: bad level/image/stride");
-  if (level == 0) if (int e = frame_own_level0(ctx, r, false)) return e;
+  if (level == 0) if (int e = frame_own_level0(ctx, r)) return e;
   CU(cudaMemcpy2DAsync(r->f.lvl[level] + (size_t)image * r->f.img_stride[level], r->f.pitch[level], data, stride, r->f.w[level], r->f.h[level],
                        cudaMemcpyHostToDevice, ctx->stream));
   CU(cudaStreamSynchronize(ctx->stream));
@@ -691,7 +689,7 @@ int svob200_frame_upload_yuv420(svob200_ctx* ctx, int64_t frame_id, const uint8_
   const int cw = (w + 1) / 2, ch = (h + 1) / 2;
   const int uv_row_bytes = (cw - 1) * uv_pixel_stride + 1;
   if (uv_stride < uv_row_bytes) return fail(ctx, SVOB200_ERR_ARG, "frame_upload_yuv420: uv_stride too small");
-  if (int e = frame_own_level0(ctx, r, false)) return e;      // level 0 is produced here
+  if (int e = frame_own_level0(ctx, r)) return e;      // level 0 is produced here
   YuvPlanes P;
   if (mem == SVOB200_MEM_DEVICE) {
     P.y = y; P.u = u; P.v = v; P.y_stride = y_stride; P.uv_stride = uv_stride; P.uv_pixel_stride = uv_pixel_stride;

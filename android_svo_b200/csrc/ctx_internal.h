@@ -171,9 +171,9 @@ struct Stage {
 
 // Level 0 of a frame is its own storage or aliases a caller's device buffer; only these two switch it, and they rewrite the
 // frame's row of the device table on ctx->stream.  Bind rejects (SVOB200_ERR_ARG, nothing changes) a buffer or stride that
-// is not 16-byte aligned and a stride below the width; copy_pixels copies the aliased images into the frame's own storage.
+// is not 16-byte aligned and a stride below the width; own switches back to the frame's own storage (without its pixels).
 int frame_bind_level0(svob200_ctx* ctx, FrameRec* r, const uint8_t* dev_gray, int stride);
-int frame_own_level0(svob200_ctx* ctx, FrameRec* r, bool copy_pixels);
+int frame_own_level0(svob200_ctx* ctx, FrameRec* r);
 
 // rounding of every pyramid step l -> l+1: the caller's round_modes, or the reference's x86 dispatch on the level's width
 inline void pyramid_round_modes(const DevFrame& f, const int* round_modes, int* modes)

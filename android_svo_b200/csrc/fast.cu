@@ -170,6 +170,7 @@ struct FastArgs {
   int cell, grid_cols, n_cells;
   float thr_f;
   const uint8_t* occupancy;
+  const int* image_sel;    // optional: images with a negative entry are skipped
   unsigned long long* keys;
   // raw mode (svob200_fast_corners): single image / level, write score map instead of cells
   uint8_t* raw_scores; int raw_image, raw_level, raw_threshold, raw_nonmax;
@@ -200,6 +201,7 @@ __global__ void __launch_bounds__(NT, 3) fast_kernel(FastArgs A)
   if (raw) level = A.raw_level;
   else { while (level + 1 < A.n_levels && (int)blockIdx.x >= A.tile_begin[level + 1]) ++level; }
   const int b = raw ? A.raw_image : (int)blockIdx.y;
+  if (A.image_sel && A.image_sel[b] < 0) return;           // (uniform over the CTA)
   const int w = A.f.w[level], h = A.f.h[level], pitch = A.f.pitch[level];
   const int tile = (int)blockIdx.x - (raw ? 0 : A.tile_begin[level]);
   const int tiles_x = (w + TW - 1) / TW;
@@ -332,9 +334,10 @@ __global__ void fast_init_keys_kernel(unsigned long long* keys, int n, float thr
 
 // decode cell records; one CTA per image counts its features
 __global__ void fast_finalize_kernel(const unsigned long long* keys, int n_cells, float thr_f, double thr,
-                                     svob200_corner* cells, int* counts)
+                                     svob200_corner* cells, int* counts, const int* image_sel)
 {
   const int b = blockIdx.x;
+  if (image_sel && image_sel[b] < 0) { if (threadIdx.x == 0 && counts) counts[b] = 0; return; }
   int local = 0;
   for (int k = threadIdx.x; k < n_cells; k += blockDim.x) {
     const unsigned long long key = keys[(size_t)b * n_cells + k];
@@ -388,7 +391,7 @@ __global__ void shi_tomasi_points_kernel(const uint8_t* img, int pitch, int cols
 
 int launch_fast_detect(const DevFrame& f, int n_detect_levels, int cell, int grid_cols, int grid_rows, double thr,
                        const uint8_t* d_occupancy, unsigned long long* d_keys, svob200_corner* d_cells, int* d_counts,
-                       cudaStream_t s, long long* launches)
+                       cudaStream_t s, long long* launches, const int* d_image_sel)
 {
   const int n_cells = grid_cols * grid_rows;
   const int total = n_cells * f.batch;
@@ -396,7 +399,7 @@ int launch_fast_detect(const DevFrame& f, int n_detect_levels, int cell, int gri
   fast_init_keys_kernel<<<(total + 255) / 256, 256, 0, s>>>(d_keys, total, thr_f);
   FastArgs A{};
   A.f = f; A.n_levels = n_detect_levels; A.cell = cell; A.grid_cols = grid_cols; A.n_cells = n_cells; A.thr_f = thr_f;
-  A.occupancy = d_occupancy; A.keys = d_keys; A.raw_scores = nullptr;
+  A.occupancy = d_occupancy; A.image_sel = d_image_sel; A.keys = d_keys; A.raw_scores = nullptr;
   A.tile_begin[0] = 0;
   for (int l = 0; l < n_detect_levels; ++l) {
     A.tiles_x[l] = (f.w[l] + TW - 1) / TW;
@@ -404,7 +407,7 @@ int launch_fast_detect(const DevFrame& f, int n_detect_levels, int cell, int gri
   }
   dim3 grid(A.tile_begin[n_detect_levels], f.batch);
   fast_kernel<<<grid, NT, 0, s>>>(A);
-  fast_finalize_kernel<<<f.batch, 256, 0, s>>>(d_keys, n_cells, thr_f, thr, d_cells, d_counts);
+  fast_finalize_kernel<<<f.batch, 256, 0, s>>>(d_keys, n_cells, thr_f, thr, d_cells, d_counts, d_image_sel);
   *launches += 3;
   return cudaGetLastError() == cudaSuccess ? 0 : -1;
 }

@@ -18,10 +18,11 @@ int launch_half_sample_single(const uint8_t* in, int in_pitch, int w, int h, uin
 
 // fast.cu
 // keys: batch*n_cells 64-bit cell records (device scratch); raw_scores: optional w*h score map of
-// (raw_image, raw_level) for svob200_fast_corners.
+// (raw_image, raw_level) for svob200_fast_corners.  d_image_sel (optional, one int per image): images with a negative entry
+// are not scored (their cells are not written, their count is 0).
 int launch_fast_detect(const DevFrame& f, int n_detect_levels, int cell, int grid_cols, int grid_rows, double thr,
                        const uint8_t* d_occupancy, unsigned long long* d_keys, svob200_corner* d_cells, int* d_counts,
-                       cudaStream_t s, long long* launches);
+                       cudaStream_t s, long long* launches, const int* d_image_sel = nullptr);
 int launch_fast_raw(const DevFrame& f, int image, int level, int threshold, int nonmax, uint8_t* d_scores,
                     cudaStream_t s, long long* launches);
 
@@ -79,9 +80,10 @@ static_assert(sizeof(SeedPoseRec) == 176, "SeedPoseRec layout");
 // rows (keyframe k, image b), b in [image0, image0 + n_images), of the pose table: run after the step's final T_cur_w is known
 int launch_seed_pose_table(const DevCam& cam, int batch, int n_kfs, int image0, int n_images, const double* d_T_kf_w, const double* d_T_cur_w,
                            SeedPoseRec* d_pose_table, cudaStream_t s, long long* launches);
-// batch_counter / max_n_kfs: Seed::batch_counter and DepthFilter::Options::max_n_kfs (seeds older than that are erased, :258-261)
+// d_batch_counter / max_n_kfs: Seed::batch_counter of every sequence (indexed by SeedRef::image) and DepthFilter::Options::max_n_kfs
+// (seeds older than that are erased, :258-261)
 int launch_seeds_update_compact(const DevFrame* d_frames, int cur_slot, const DevCam& cam, int n, SeedRef* d_refs,
-                                const int* d_kf_slot, int batch, const SeedPoseRec* d_pose_table, int batch_counter, int max_n_kfs,
+                                const int* d_kf_slot, int batch, const SeedPoseRec* d_pose_table, const int* d_batch_counter, int max_n_kfs,
                                 svob200_matcher_opts opts, double conv_thresh,
                                 svob200_seed* d_seeds, svob200_seed_obs* d_obs, void* d_scratch, int scratch_total, int first,
                                 cudaStream_t s, long long* launches, cudaEvent_t* marks = nullptr);

@@ -947,7 +947,8 @@ struct SeedSrcApi {
 // frame are row (k * batch + b) of the table seed_pose_table_kernel refreshed
 struct SeedSrcCompact {
   SeedRef* refs; const SeedPoseRec* table; const int* kf_slot; int batch;
-  int batch_counter, max_n_kfs;          // Seed::batch_counter and DepthFilter::Options::max_n_kfs for the ageing rule
+  const int* batch_counter;              // Seed::batch_counter of every sequence (one DepthFilter each), for the ageing rule
+  int max_n_kfs;                         // DepthFilter::Options::max_n_kfs
   __device__ __forceinline__ RefFtr get(int i) const
   {
     const uint4* q = reinterpret_cast<const uint4*>(&refs[i]);
@@ -967,7 +968,7 @@ struct SeedSrcCompact {
   __device__ __forceinline__ int early_status(const RefFtr& f) const
   {
     if (f.state != 0) return -1;
-    return (batch_counter - f.batch_id) > max_n_kfs ? SVOB200_SEED_TOO_OLD : 0;
+    return (__ldg(&batch_counter[f.ref_image]) - f.batch_id) > max_n_kfs ? SVOB200_SEED_TOO_OLD : 0;
   }
   __device__ __forceinline__ void erase(int i) const { reinterpret_cast<uint8_t*>(&refs[i])[48] = 1; }
   __device__ __forceinline__ void poses(const DevCam&, int, const RefFtr& f, SeedPoses& P) const
@@ -1522,12 +1523,12 @@ int launch_seed_pose_table(const DevCam& cam, int batch, int n_kfs, int image0, 
 }
 
 int launch_seeds_update_compact(const DevFrame* d_frames, int cur_slot, const DevCam& cam, int n, SeedRef* d_refs,
-                                const int* d_kf_slot, int batch, const SeedPoseRec* d_pose_table, int batch_counter, int max_n_kfs,
+                                const int* d_kf_slot, int batch, const SeedPoseRec* d_pose_table, const int* d_batch_counter, int max_n_kfs,
                                 svob200_matcher_opts opts, double conv_thresh,
                                 svob200_seed* d_seeds, svob200_seed_obs* d_obs, void* d_scratch, int scratch_total, int first,
                                 cudaStream_t s, long long* launches, cudaEvent_t* marks)
 {
-  SeedSrcCompact src{d_refs, d_pose_table, d_kf_slot, batch, batch_counter, max_n_kfs};
+  SeedSrcCompact src{d_refs, d_pose_table, d_kf_slot, batch, d_batch_counter, max_n_kfs};
   return seeds_update_impl(d_frames, cur_slot, cam, n, src, opts, conv_thresh, d_seeds, d_obs, d_scratch, scratch_total, first, s, launches, marks);
 }
 

@@ -36,7 +36,6 @@ struct CandStage {                       // where step_stats_kernel records the 
   CandRec* rec; int* count; int* created;  // rec: the sequence's point-slot block of this parity's staging; count / created: per sequence
   const int* pt_off; const double* T_kf; int batch, b0;   // point-slot offsets, keyframe poses [kf][batch][7], first sequence of the range
 };
-struct KfBatches { int v[16]; };         // Seed::batch_id of every keyframe index of the ring (svob200_tracker::kf_batch)
 
 // Order-preserving fill of one sequence's empty slots by one CTA of NT threads: the r-th selected item (is_item, in index
 // order) goes to the r-th free slot (is_free, in slot order), put(item, slot) for r < min(#items, #free).  Every thread owns
@@ -184,13 +183,15 @@ __global__ void chain_stats_kernel(int batch, const svob200_reproj_stats* rs, co
   stats[b].n_pose_obs = pose_opt ? pr[b].num_obs : rs[b].n_matches;
 }
 
-// ---- keyframe insertion (svob200_tracker_add_keyframe)
+// ---- keyframe insertion (svob200_tracker_add_keyframes): a kernel of a sequence that is not selected (kf_new < 0) or loses no
+// keyframe (kf_old < 0) leaves it untouched
 // occupancy of the frame's existing features = the map points matched in it (AbstractDetector::setExistingFeatures,
 // feature_detection.cpp:40-58: cell of (px.y / cell, px.x / cell) with the x86 double -> int conversion)
-__global__ void kf_occupancy_kernel(int n, const int* ftr_image, const double* px, const int* match_ok, int cell, int grid_cols, int n_cells, uint8_t* occ)
+__global__ void kf_occupancy_kernel(int n, const int* ftr_image, const double* px, const int* match_ok, const int* kf_new, int cell, int grid_cols,
+                                    int n_cells, uint8_t* occ)
 {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n || !match_ok[i]) return;
+  if (i >= n || !match_ok[i] || kf_new[ftr_image[i]] < 0) return;
   const long long k = (long long)x86_d2i(px[2 * (size_t)i + 1] / cell) * grid_cols + x86_d2i(px[2 * (size_t)i] / cell);
   if (k >= 0 && k < n_cells) occ[(size_t)ftr_image[i] * n_cells + k] = 1;
 }
@@ -250,7 +251,7 @@ __global__ void __launch_bounds__(128) kf_init_slots_kernel(DevCam cam, int K, i
 // The candidates of step k enter at the head of step k + 2 (the reference's depth filter runs one frame behind tracking):
 // into the sequence's empty slots in slot order, in their list order.  A candidate whose keyframe left the ring since (its
 // batch id is no longer that keyframe index's) or that finds no empty slot is dropped.  One CTA per sequence.
-__global__ void __launch_bounds__(128) cand_insert_kernel(int K, int batch, const int* pt_off, const CandRec* cand, const int* cand_n, KfBatches kfb,
+__global__ void __launch_bounds__(128) cand_insert_kernel(int K, int batch, const int* pt_off, const CandRec* cand, const int* cand_n, const int* kf_batch,
                                                           const int* kf_slot, const double* T_kf, svob200_map_point* pts, double* pt_world,
                                                           svob200_feature_ref* obs, double* T_obs, int* sel, uint8_t* has_point,
                                                           int* slot_of_rank, int* dropped)
@@ -258,7 +259,7 @@ __global__ void __launch_bounds__(128) cand_insert_kernel(int K, int batch, cons
   const int b = blockIdx.x, tid = threadIdx.x;
   const int P0 = pt_off[b], P = pt_off[b + 1] - P0, n = cand_n[b];
   const CandRec* C = cand + P0;
-  auto valid = [&](int c) { return C[c].batch_id == kfb.v[C[c].kf]; };
+  auto valid = [&](int c) { return C[c].batch_id == kf_batch[C[c].kf * batch + b]; };
   auto empty = [&](int q) { return pts[P0 + q].type == SVOB200_POINT_DELETED; };
   auto put = [&](int c, int q) {
     const CandRec cr = C[c];
@@ -281,12 +282,15 @@ __global__ void __launch_bounds__(128) cand_insert_kernel(int K, int batch, cons
 
 // MapPointCandidates::removeFrameCandidates: the candidates of the keyframe that leaves the ring are deleted, except those
 // matched in the new keyframe (the reference promotes them first: addCandidatePointToFrame runs before the ring drops a keyframe)
-__global__ void kf_drop_candidates_kernel(int n, svob200_map_point* pts, const svob200_feature_ref* obs, const int* match_ok, uint8_t* has_point, int kf_slot)
+__global__ void kf_drop_candidates_kernel(int n, svob200_map_point* pts, const svob200_feature_ref* obs, const int* match_ok, uint8_t* has_point,
+                                          const int* image, const int* kf_old, const int* kf_slot)
 {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
+  const int k = kf_old[image[i]];
+  if (k < 0) return;
   const svob200_map_point p = pts[i];
-  if (p.type != SVOB200_POINT_CANDIDATE || match_ok[i] || (int)obs[p.obs_begin].ref_frame_id != kf_slot) return;
+  if (p.type != SVOB200_POINT_CANDIDATE || match_ok[i] || (int)obs[p.obs_begin].ref_frame_id != kf_slot[k]) return;
   pts[i].type = SVOB200_POINT_DELETED; pts[i].obs_begin = p.obs_end;
   has_point[i] = 0;
 }
@@ -340,10 +344,11 @@ __global__ void __launch_bounds__(128) points_select_kernel(DevCam cam, int n, c
 // frame_handler_mono.cpp:277-279: every feature of the new keyframe with a point adds a frame reference to it (push_front).
 // The keyframe's features are the map points matched in it: Feature(frame, px_refined, search_level) (reprojector.cpp:219-231).
 __global__ void kf_add_obs_kernel(DevCam cam, int n, int K, svob200_map_point* pts, svob200_feature_ref* obs, double* T_obs, const int* image,
-                                  const int* match_ok, const double* px, const int* level, int kf_slot, const double* T_cur_w)
+                                  const int* match_ok, const double* px, const int* level, const int* kf_new, const int* kf_slot_of, const double* T_cur_w)
 {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n || !match_ok[i]) return;
+  if (i >= n || !match_ok[i] || kf_new[image[i]] < 0) return;
+  const int kf_slot = kf_slot_of[kf_new[image[i]]];
   svob200_map_point p = pts[i];
   if (p.obs_end - p.obs_begin >= K) return;                      // (cannot happen: at most one observation per resident keyframe)
   const int slot = p.obs_begin - 1;
@@ -359,10 +364,12 @@ __global__ void kf_add_obs_kernel(DevCam cam, int n, int K, svob200_map_point* p
 }
 
 // Map::safeDeleteFrame -> Point::deleteFrameRef for every point seen in the keyframe that leaves the ring
-__global__ void kf_drop_obs_kernel(int n, int K, svob200_map_point* pts, svob200_feature_ref* obs, double* T_obs, int kf_slot, int* sel)
+__global__ void kf_drop_obs_kernel(int n, int K, svob200_map_point* pts, svob200_feature_ref* obs, double* T_obs, const int* image, const int* kf_old,
+                                   const int* kf_slot_of, int* sel)
 {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
+  if (i >= n || kf_old[image[i]] < 0) return;
+  const int kf_slot = kf_slot_of[kf_old[image[i]]];
   sel[i] = -1;                                                   // slots move: the next step copies its choice afresh
   const svob200_map_point p = pts[i];
   int w = p.obs_end;                                             // compact towards the top end, keeping the list order
@@ -375,20 +382,22 @@ __global__ void kf_drop_obs_kernel(int n, int K, svob200_map_point* pts, svob200
 }
 
 // seeds of a dropped keyframe leave the pool (DepthFilter::removeKeyframe, depth_filter.cpp:153-170)
-__global__ void kf_erase_seeds_kernel(int n, SeedRef* refs, int kf)
+__global__ void kf_erase_seeds_kernel(int n, SeedRef* refs, const int* kf_old)
 {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n && refs[i].state == 0 && refs[i].kf == kf) refs[i].state = 1;
+  if (i < n && refs[i].state == 0 && refs[i].kf == kf_old[refs[i].image]) refs[i].state = 1;
 }
 
 // DepthFilter::initializeSeeds (depth_filter.cpp:129-151): one Seed (ctor :36-45) per new corner, in cell order, into the empty
 // slots of the sequence's pool in slot order.  One CTA per sequence; corners that find no slot are counted as dropped.
 __global__ void __launch_bounds__(256) kf_append_seeds_kernel(DevCam cam, const svob200_corner* cells, int n_cells, double thr, const float* depth_mean,
-                                                              const float* depth_min, const int* seed_off, SeedRef* refs, svob200_seed* seeds, int kf,
-                                                              int batch_id, int* appended, int* dropped)
+                                                              const float* depth_min, const int* seed_off, SeedRef* refs, svob200_seed* seeds,
+                                                              const int* kf_new, const int* batch_counter, int* appended, int* dropped)
 {
   __shared__ int s_slot_of_rank[8192];                // grids up to 8,192 cells (svob200_tracker_set_detector / _add_keyframe)
   const int b = blockIdx.x, tid = threadIdx.x;
+  const int kf = kf_new[b], batch_id = batch_counter[b];
+  if (kf < 0) { if (tid == 0) appended[b] = dropped[b] = kf == -2 ? -1 : 0; return; }   // refused (batch counter exhausted) / not selected
   const svob200_corner* C = cells + (size_t)b * n_cells;
   const int p0 = seed_off[b], np = seed_off[b + 1] - p0;
   const svob200_seed sd = seed_prior(depth_mean[b], depth_min[b]);
@@ -407,7 +416,93 @@ __global__ void __launch_bounds__(256) kf_append_seeds_kernel(DevCam cam, const 
   };
   int n_new;
   const int n_fill = fill_free_slots<256>(n_cells, is_new, np, empty, s_slot_of_rank, &n_new, put);
-  if (tid == 0) { appended[b] = n_fill; dropped[b] = n_new - n_fill; }
+  // without a seed pool (no slot anywhere) the counts are the corners found, every one of them dropped
+  if (tid == 0) { appended[b] = seed_off[gridDim.x] ? n_fill : n_new; dropped[b] = n_new - n_fill; }
+}
+
+// ---- per-sequence keyframe rings (svob200_tracker_add_keyframes): ring index k of sequence b is image b of store frame k;
+// kf_batch[k * batch + b] is the Seed::batch_id of that keyframe (-1: free), batch_counter[b] the sequence's Seed::batch_counter.
+// One thread per sequence: a selected sequence takes its first free index, else its oldest keyframe leaves (kf_old = that index);
+// the new keyframe is the frame of the most recent step, with its pose.  kf_new / kf_old = -1: not selected / nothing leaves.
+// Seed::batch_id is 16 bits wide (SeedRef): a sequence whose counter reached kMaxBatchId takes no further keyframe (kf_new = -2).
+constexpr int kMaxBatchId = 65534;
+__global__ void kf_select_kernel(int batch, int max_kfs, const uint8_t* which, int* kf_batch, int* batch_counter, int* kf_new, int* kf_old,
+                                 const double* T_cur_w, double* T_kf)
+{
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= batch) return;
+  kf_old[b] = -1;
+  if (which && !which[b]) { kf_new[b] = -1; return; }
+  if (batch_counter[b] >= kMaxBatchId) { kf_new[b] = -2; return; }
+  int k = -1, old = -1;
+  for (int i = 0; i < max_kfs; ++i) if (kf_batch[i * batch + b] < 0) { k = i; break; }
+  if (k < 0) {
+    old = 0;
+    for (int i = 1; i < max_kfs; ++i) if (kf_batch[i * batch + b] < kf_batch[old * batch + b]) old = i;
+    k = old;
+  }
+  const int id = ++batch_counter[b];                        // ++Seed::batch_counter (depth_filter.cpp:139)
+  kf_batch[k * batch + b] = id;
+  kf_new[b] = k; kf_old[b] = old;
+  for (int j = 0; j < 7; ++j) T_kf[7 * ((size_t)k * batch + b) + j] = T_cur_w[7 * (size_t)b + j];
+}
+
+// The images of the selected sequences, every pyramid level, into their keyframe's store frame (frames[kf_slot[kf_new[b]]]).
+// Rows are copied in 16-byte words up to the width rounded up to 16: both pitches are multiples of 16 and at least that.
+__global__ void __launch_bounds__(256) kf_store_copy_kernel(DevFrame src, const DevFrame* frames, const int* kf_slot, const int* kf_new)
+{
+  const int b = blockIdx.y;
+  const int k = kf_new[b];
+  if (k < 0) return;
+  const DevFrame& dst = frames[kf_slot[k]];
+  for (int l = 0; l < src.n_levels; ++l) {
+    const int words = (src.w[l] + 15) / 16, n = words * src.h[l];
+    const uint8_t* in = src.lvl[l] + (size_t)b * src.img_stride[l];
+    uint8_t* out = dst.lvl[l] + (size_t)b * dst.img_stride[l];
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+      const int y = i / words, x = 16 * (i - y * words);
+      *reinterpret_cast<uint4*>(out + (size_t)y * dst.pitch[l] + x) = __ldg(reinterpret_cast<const uint4*>(in + (size_t)y * src.pitch[l] + x));
+    }
+  }
+}
+
+// frame_utils::getSceneDepth of the most recent step's frame, one CTA per sequence: the depths z = (T_cur_w * pos).z of the
+// point slots matched in it, compacted in slot order into z_buf; depth_mean = (float) the element of rank n/2 of the ascending
+// depths (vk::getMedian: nth_element), depth_min = (float)(0.5 * min).  n == 0 leaves depth_mean / depth_min as they are.
+__global__ void __launch_bounds__(128) scene_depth_kernel(const int* pt_off, const svob200_map_point* pts, const int* match_ok, const double* T_cur_w,
+                                                          double* z_buf, float* depth_mean, float* depth_min, int* n_points)
+{
+  const int b = blockIdx.x, tid = threadIdx.x;
+  const int p0 = pt_off[b], np = pt_off[b + 1] - p0;
+  const int chunk = (np + 127) / 128, q0 = min(tid * chunk, np), q1 = min(q0 + chunk, np);
+  const double* T = T_cur_w + 7 * (size_t)b;
+  int local = 0;
+  for (int q = q0; q < q1; ++q) local += match_ok[p0 + q] != 0;
+  int n;
+  int r = block_exclusive_scan<128>(local, &n);
+  double zmin = INFINITY;
+  for (int q = q0; q < q1; ++q) {
+    if (!match_ok[p0 + q]) continue;
+    const svob200_map_point p = pts[p0 + q];
+    const double z = se3_transform(T, {p.pos[0], p.pos[1], p.pos[2]}).z;
+    z_buf[p0 + r++] = z;
+    zmin = fmin(zmin, z);
+  }
+  __shared__ double s_min[4];
+  for (int o = 16; o > 0; o >>= 1) zmin = fmin(zmin, __shfl_xor_sync(0xffffffffu, zmin, o));
+  if ((tid & 31) == 0) s_min[tid >> 5] = zmin;
+  __syncthreads();                                         // (also publishes z_buf to the CTA)
+  if (tid == 0 && n_points) n_points[b] = n;
+  if (n == 0) return;
+  if (tid == 0) depth_min[b] = (float)(0.5 * fmin(fmin(s_min[0], s_min[1]), fmin(s_min[2], s_min[3])));
+  const double* Z = z_buf + p0;
+  const int want = n / 2;
+  for (int i = tid; i < n; i += 128) {                     // the element whose rank (ties by position) is n/2
+    const double zi = Z[i];
+    int rank = 0;
+    for (int j = 0; j < n; ++j) rank += (Z[j] < zi) || (Z[j] == zi && j < i);
+    if (rank == want) depth_mean[b] = (float)zi;
+  }
 }
 
 }  // namespace
@@ -430,14 +525,18 @@ struct svob200_tracker {
   int reseed = 1;
   int64_t uid = 0;                     // frame ids of this tracker: -(uid << 8 | n), n = 1, 2, ... (new_frame)
   int64_t fid_last = 0, fid_cur = 0;
-  // keyframes: up to max_kfs frames of the pool are keyframes (index k = position in the tables d_kf_slot / d_T_kf); the frame
-  // of a keyframe may at the same time be the `last` frame of the tracking chain
+  // keyframes: every sequence has its own ring of max_kfs keyframes.  Ring index k of sequence b is image b of the keyframe
+  // store's frame fid_kfs[k] (frame slot d_kf_slot[k], pose d_T_kf[k][b]); the ring state lives on the device, per sequence:
+  // d_kf_batch[k][b] = Seed::batch_id of that keyframe (-1: free), d_batch_counter[b] = Seed::batch_counter (depth_filter.cpp:139)
   static constexpr int MAX_KFS = 16;
   int64_t fid_kfs[MAX_KFS] = {};
-  int kf_batch[MAX_KFS] = {};          // Seed::batch_id of the seeds initialised in keyframe k (0 = unused slot of the ring)
   std::vector<int64_t> frame_pool;     // every frame this tracker created
   int64_t next_fid = 0;
-  int batch_counter = 0;               // Seed::batch_counter (depth_filter.cpp:139)
+  int *d_kf_batch = nullptr, *d_batch_counter = nullptr;
+  int *d_kf_new = nullptr, *d_kf_old = nullptr;     // of the latest insertion: the ring index taken / left, per sequence (-1: none)
+  uint8_t* d_kf_which = nullptr;                    // host-memory insertion masks, staged
+  double* d_sd_z = nullptr;            // svob200_tracker_scene_depth: the depths of the matched point slots
+  int* d_sd_n = nullptr;
   int max_n_kfs = 3;                   // DepthFilter::Options::max_n_kfs (depth_filter.h:75)
   int seed_capacity = 0;               // slots per sequence of the seed pool (0: exactly the seeds of set_keyframe)
   int det_cell = 30, det_levels = 3;   // Config::gridSize / nPyrLevels, Config::triangMinCornerScore
@@ -467,7 +566,7 @@ struct svob200_tracker {
   double* d_T_kf = nullptr;            // [max_kfs][batch][7]
   int* d_kf_slot = nullptr;            // [max_kfs]
   SeedPoseRec* d_seed_poses = nullptr; // [max_kfs][batch], refreshed every step
-  int n_kfs = 1;                       // rows of the tables in use (highest keyframe index + 1)
+  int n_kfs = 1;                       // rows of the tables in use (no sequence has more keyframes: min(max_kfs, 1 + insertions))
   int max_kfs = 4;                     // keyframe ring (svob200_tracker_set_keyframe_ring)
   svob200_seed* d_seeds = nullptr;
   double *d_step_in = nullptr;      // [T_last_w 7B | last_px 2N]
@@ -595,6 +694,16 @@ static int graph_or_direct(svob200_tracker* t, bool use_graph, const std::vector
   return 0;
 }
 
+// the frame slot of every store frame that exists (d_kf_slot, constant once the store is complete)
+static int upload_kf_slots(svob200_tracker* t)
+{
+  svob200_ctx* ctx = t->ctx;
+  int slots[svob200_tracker::MAX_KFS] = {};
+  for (int k = 0; k < t->max_kfs; ++k) if (t->fid_kfs[k]) slots[k] = svob200_frame_slot(ctx, t->fid_kfs[k]);
+  CU(cudaMemcpyAsync(t->d_kf_slot, slots, sizeof(int) * t->max_kfs, cudaMemcpyHostToDevice, ctx->stream));
+  return 0;
+}
+
 extern "C" {
 
 int svob200_tracker_create(svob200_ctx* ctx, const svob200_camera* cam, int batch, int n_levels, const svob200_align_opts* aopts,
@@ -616,7 +725,7 @@ int svob200_tracker_create(svob200_ctx* ctx, const svob200_camera* cam, int batc
   t->uid = ++uid_counter;
   t->ctx = ctx; t->cam = *cam; t->batch = batch; t->n_levels = n_levels; t->aopts = *aopts; t->mopts = *mopts;
   t->conv_thresh = conv_thresh; t->reseed = reseed; t->seed_init = seed_prior(depth_mean, depth_min);
-  // three frames to start with (keyframe 0, last, cur), more as keyframes are inserted
+  // three frames to start with (store frame 0, last, cur); the other store frames come with set_seed_pool or the first insertion
   t->next_fid = 1;
   for (int64_t* pid : {&t->fid_kfs[0], &t->fid_last, &t->fid_cur})
     if (int e = new_frame(t, pid)) { for (int64_t id : t->frame_pool) svob200_frame_release(ctx, id); delete t; return e; }
@@ -681,7 +790,7 @@ int svob200_tracker_set_keyframe(svob200_tracker* t, const uint8_t* imgs, int st
   t->h_seed_off = pool_off;
   for (int b = 0; b < B; ++b) t->max_per = std::max(t->max_per, pt_off[b + 1] - pt_off[b]);
   const int slot = svob200_frame_slot(ctx, t->fid_kfs[0]);
-  t->kf_batch[0] = 0; t->n_kfs = 1;
+  t->n_kfs = 1;
   int err = 0;
   auto own = [&](auto*& p, size_t n) { if (!err) err = alloc_owned(t, p, n); };
   own(t->d_ftr_off, B + 1); own(t->d_seed_off, B + 1); own(t->d_ftr_image, N); own(t->d_match_ok, N); own(t->d_has_point, N);
@@ -692,6 +801,8 @@ int svob200_tracker_set_keyframe(svob200_tracker* t, const uint8_t* imgs, int st
   own(t->d_seeds, S); own(t->d_step_in, 7 * (size_t)B + 2 * (size_t)N); own(t->d_xyz, 3 * (size_t)N); own(t->d_T_init, 7 * (size_t)B);
   own(t->d_T_cur, 7 * (size_t)B); own(t->d_depth_ref, N); own(t->d_px_in, 2 * (size_t)N); own(t->d_px_out, 2 * (size_t)N);
   own(t->d_align, B); own(t->d_obs, S); own(t->d_stats, B); own(t->d_stats2, B);
+  own(t->d_kf_batch, (size_t)B * t->max_kfs); own(t->d_batch_counter, B); own(t->d_kf_new, B); own(t->d_kf_old, B); own(t->d_kf_which, B);
+  own(t->d_depth_mean, B); own(t->d_depth_min, B); own(t->d_sd_n, B); own(t->d_sd_z, N);
   own(t->d_align_scratch, sparse_align_scratch_bytes(N)); own(t->d_seed_scratch, seeds_scratch_bytes(S)); own(t->d_match_scratch, match_scratch_bytes(N));
   if (t->pt_capacity >= 0) {
     for (int p = 0; p < 2; ++p) { own(t->d_cand[p], N); own(t->d_cand_n[p], B); }
@@ -700,7 +811,7 @@ int svob200_tracker_set_keyframe(svob200_tracker* t, const uint8_t* imgs, int st
   if (err) {                 // an allocation that failed leaves the tracker as it was before the call (it can be retried or destroyed)
     for (void* q : t->owned) cudaFree(q);
     t->owned.clear();
-    t->N = t->S = 0; t->max_per = 0; t->d_stats = nullptr; t->d_reproj = nullptr; t->det_cells_alloc = 0; t->d_det_counts = nullptr;
+    t->N = t->S = 0; t->max_per = 0; t->d_stats = nullptr; t->d_reproj = nullptr; t->det_cells_alloc = 0; t->d_det_counts = nullptr; t->d_kf_batch = nullptr;
     return err;
   }
   cudaStream_t s = ctx->stream;
@@ -711,8 +822,15 @@ int svob200_tracker_set_keyframe(svob200_tracker* t, const uint8_t* imgs, int st
     CU(cudaMemsetAsync(t->d_pt_created, 0, sizeof(int) * B, s));
     CU(cudaMemsetAsync(t->d_pt_dropped, 0, sizeof(int) * B, s));
   }
-  CU(cudaMemcpyAsync(t->d_T_kf, T_kf_w, sizeof(double) * 7 * B, cudaMemcpyHostToDevice, s));
-  CU(cudaMemcpyAsync(t->d_kf_slot, &slot, sizeof(int), cudaMemcpyHostToDevice, s));
+  // every ring index starts with keyframe 0's pose: the pose table of a step covers rows whose index a sequence has not used yet
+  for (int k = 0; k < t->max_kfs; ++k) CU(cudaMemcpyAsync(t->d_T_kf + 7 * (size_t)B * k, T_kf_w, sizeof(double) * 7 * B, cudaMemcpyHostToDevice, s));
+  {                                                      // every sequence's ring holds keyframe 0 (batch id 0), nothing else
+    std::vector<int> kb((size_t)B * t->max_kfs, -1);
+    std::fill(kb.begin(), kb.begin() + B, 0);
+    CU(cudaMemcpyAsync(t->d_kf_batch, kb.data(), sizeof(int) * kb.size(), cudaMemcpyHostToDevice, s));
+    CU(cudaMemsetAsync(t->d_batch_counter, 0, sizeof(int) * B, s));
+  }
+  if (int e = upload_kf_slots(t)) return e;
   // the caller's arrays in one copy; every point slot and seed slot is written on the device
   Stage st(ctx, SVOB200_MEM_HOST);
   const int i_fo = st.add(ftr_offsets, nullptr, sizeof(int) * (B + 1), 0), i_px = st.add(kf_px, nullptr, sizeof(double) * 2 * N_in, 0);
@@ -741,10 +859,9 @@ int svob200_tracker_set_seed_pool(svob200_tracker* t, int capacity_per_sequence,
   if (capacity_per_sequence < 0 || max_keyframes < 1 || max_keyframes > svob200_tracker::MAX_KFS || max_n_kfs < 0 || reseed < 0 || reseed > 3)
     return fail(ctx, SVOB200_ERR_ARG, "tracker_set_seed_pool: bad arguments");
   t->seed_capacity = capacity_per_sequence; t->max_kfs = max_keyframes; t->max_n_kfs = max_n_kfs; t->reseed = reseed;
-  // the whole frame pool now (keyframe ring + last + cur), so that no keyframe insertion allocates
-  int64_t id;
-  while ((int)t->frame_pool.size() < t->max_kfs + 2)
-    if (int e = new_frame(t, &id)) return e;
+  // the whole frame pool now (keyframe store + last + cur), so that no keyframe insertion allocates
+  for (int k = 1; k < t->max_kfs; ++k)
+    if (!t->fid_kfs[k]) if (int e = new_frame(t, &t->fid_kfs[k])) return e;
   return SVOB200_OK;
 }
 
@@ -769,80 +886,129 @@ int svob200_tracker_set_detector(svob200_tracker* t, int cell_size, int n_detect
   return SVOB200_OK;
 }
 
-// The frame of the most recent step becomes a keyframe of every sequence.
-int svob200_tracker_add_keyframe(svob200_tracker* t, const float* depth_mean, const float* depth_min, int* n_new_seeds, int* n_dropped)
+// The frame of the most recent step becomes a keyframe of the sequences `which` selects (NULL: every sequence), each in its
+// own ring: what svob200_tracker_add_keyframe did for a tracker of that sequence alone.  Every per-sequence choice is made on
+// the device, so in SVOB200_MEM_DEVICE mode nothing here waits for the device.
+int svob200_tracker_add_keyframes(svob200_tracker* t, const uint8_t* which, const float* depth_mean, const float* depth_min, int* n_new_seeds,
+                                  int* n_dropped, int mem)
 {
   if (!t || !depth_mean || !depth_min) return SVOB200_ERR_ARG;
   svob200_ctx* ctx = t->ctx;
-  if (!t->d_stats || t->steps_done == 0) return fail(ctx, SVOB200_ERR_ARG, "tracker_add_keyframe: needs a keyframe and at least one step");
-  if (t->chain_cell > 0) return fail(ctx, SVOB200_ERR_UNSUPPORTED, "tracker_add_keyframe: not available in chain mode");
+  if (mem != SVOB200_MEM_HOST && mem != SVOB200_MEM_DEVICE) return fail(ctx, SVOB200_ERR_ARG, "tracker_add_keyframes: bad mem %d", mem);
+  if (!t->d_stats || t->steps_done == 0) return fail(ctx, SVOB200_ERR_ARG, "tracker_add_keyframes: needs a keyframe and at least one step");
+  if (t->chain_cell > 0) return fail(ctx, SVOB200_ERR_UNSUPPORTED, "tracker_add_keyframes: not available in chain mode");
   const int B = t->batch, N = t->N, S = t->S;
-  cudaStream_t s = ctx->stream;
-  if (int e = df_join(t)) return e;                        // the depth filter of the last step may still be running
-  drop_graphs(t);                                          // captured steps hold the old keyframe tables' values / frame roles
-  // 1. the keyframe's index in the ring: a free one, else the oldest keyframe leaves (its seeds with it: removeKeyframe)
-  int k = -1;
-  for (int i = 0; i < t->max_kfs; ++i) if (t->fid_kfs[i] == 0) { k = i; break; }
-  if (k < 0) {
-    k = 0;
-    for (int i = 1; i < t->max_kfs; ++i) if (t->kf_batch[i] < t->kf_batch[k]) k = i;
-    if (S) { kf_erase_seeds_kernel<<<(S + 255) / 256, 256, 0, s>>>(S, t->d_seed_refs, k); ++ctx->launches; }
-    if (N) {                                                 // Map::safeDeleteFrame: the points forget the keyframe
-      FrameRec* old = find_frame(ctx, t->fid_kfs[k]);
-      if (t->pt_capacity >= 0) {
-        kf_drop_candidates_kernel<<<(N + 255) / 256, 256, 0, s>>>(N, t->d_points, t->d_pobs, t->d_match_ok, t->d_has_point, old->slot); ++ctx->launches;
-      }
-      kf_drop_obs_kernel<<<(N + 255) / 256, 256, 0, s>>>(N, t->max_kfs, t->d_points, t->d_pobs, t->d_T_pobs, old->slot, t->d_sel); ++ctx->launches;
-    }
-    t->fid_kfs[k] = 0;
-  }
-  // 2. the frame: the last step's current frame (now `last`).  Its level 0 may alias the caller's buffer: the keyframe owns a copy.
-  FrameRec* r = find_frame(ctx, t->fid_last);
-  if (!r) return fail(ctx, SVOB200_ERR_NOFRAME, "tracker_add_keyframe: last frame missing");
-  if (int e = frame_own_level0(ctx, r, true)) return e;
-  t->fid_kfs[k] = t->fid_last;
-  t->kf_batch[k] = ++t->batch_counter;                      // ++Seed::batch_counter (depth_filter.cpp:139)
-  if (t->batch_counter >= 65535) return fail(ctx, SVOB200_ERR_UNSUPPORTED, "tracker_add_keyframe: batch counter exhausted");
-  t->n_kfs = std::max(t->n_kfs, k + 1);
-  const int slot = r->slot;
-  CU(cudaMemcpyAsync(t->d_kf_slot + k, &slot, sizeof(int), cudaMemcpyHostToDevice, s));
-  CU(cudaMemcpyAsync(t->d_T_kf + 7 * (size_t)B * k, t->d_T_cur, sizeof(double) * 7 * B, cudaMemcpyDeviceToDevice, s));   // the frame's pose
-  // 3. detector scratch
   const int gc = (t->cam.width + t->det_cell - 1) / t->det_cell, gr = (t->cam.height + t->det_cell - 1) / t->det_cell;
   const int n_cells = gc * gr;
-  if (n_cells > 8192) return fail(ctx, SVOB200_ERR_UNSUPPORTED, "tracker_add_keyframe: grid of %d cells exceeds the kernel's table (8192)", n_cells);
+  if (n_cells > 8192) return fail(ctx, SVOB200_ERR_UNSUPPORTED, "tracker_add_keyframes: grid of %d cells exceeds the kernel's table (8192)", n_cells);
+  cudaStream_t s = ctx->stream;
+  // the keyframe store (allocated here when set_seed_pool did not) and the detector scratch
+  bool new_store = false;
+  for (int k = 1; k < t->max_kfs; ++k)
+    if (!t->fid_kfs[k]) { if (int e = new_frame(t, &t->fid_kfs[k])) return e; new_store = true; }
+  if (new_store) if (int e = upload_kf_slots(t)) return e;
   if (t->det_cells_alloc < n_cells) {
     const size_t M = (size_t)B * n_cells;
     int err = 0;
     auto own = [&](auto*& p, size_t n) { if (!err) err = alloc_owned(t, p, n); };
     own(t->d_occ, M); own(t->d_det_keys, M); own(t->d_det_cells, M);
-    if (!t->d_det_counts) { own(t->d_det_counts, B); own(t->d_kf_appended, B); own(t->d_kf_dropped, B); own(t->d_depth_mean, B); own(t->d_depth_min, B); }
+    if (!t->d_det_counts) { own(t->d_det_counts, B); own(t->d_kf_appended, B); own(t->d_kf_dropped, B); }
     if (err) return err;
     t->det_cells_alloc = n_cells;
   }
-  CU(cudaMemcpyAsync(t->d_depth_mean, depth_mean, sizeof(float) * B, cudaMemcpyHostToDevice, s));
-  CU(cudaMemcpyAsync(t->d_depth_min, depth_min, sizeof(float) * B, cudaMemcpyHostToDevice, s));
-  // 4. occupancy from the frame's features (the map points matched in it), FAST + Shi-Tomasi + grid, one seed per new corner
+  if (int e = df_join(t)) return e;                        // the depth filter of the last step may still be running
+  const float *d_dm = depth_mean, *d_dn = depth_min;
+  const uint8_t* d_which = which;
+  if (mem == SVOB200_MEM_HOST) {
+    CU(cudaMemcpyAsync(t->d_depth_mean, depth_mean, sizeof(float) * B, cudaMemcpyHostToDevice, s));
+    CU(cudaMemcpyAsync(t->d_depth_min, depth_min, sizeof(float) * B, cudaMemcpyHostToDevice, s));
+    if (which) CU(cudaMemcpyAsync(t->d_kf_which, which, (size_t)B, cudaMemcpyHostToDevice, s));
+    d_dm = t->d_depth_mean; d_dn = t->d_depth_min; d_which = which ? t->d_kf_which : nullptr;
+  }
+  // 1. every selected sequence's ring index: a free one, else its oldest keyframe leaves (its seeds with it: removeKeyframe)
+  const bool may_evict = t->n_kfs == t->max_kfs;           // (no sequence holds more keyframes than n_kfs)
+  kf_select_kernel<<<(B + 127) / 128, 128, 0, s>>>(B, t->max_kfs, d_which, t->d_kf_batch, t->d_batch_counter, t->d_kf_new, t->d_kf_old, t->d_T_cur, t->d_T_kf);
+  ++ctx->launches;
+  if (!may_evict) { t->n_kfs = std::min(t->max_kfs, t->n_kfs + 1); drop_graphs(t); }   // captured steps hold n_kfs
+  if (may_evict) {
+    if (S) { kf_erase_seeds_kernel<<<(S + 255) / 256, 256, 0, s>>>(S, t->d_seed_refs, t->d_kf_old); ++ctx->launches; }
+    if (N) {                                                 // Map::safeDeleteFrame: the points forget the keyframe
+      if (t->pt_capacity >= 0) {
+        kf_drop_candidates_kernel<<<(N + 255) / 256, 256, 0, s>>>(N, t->d_points, t->d_pobs, t->d_match_ok, t->d_has_point, t->d_ftr_image, t->d_kf_old,
+                                                                  t->d_kf_slot);
+        ++ctx->launches;
+      }
+      kf_drop_obs_kernel<<<(N + 255) / 256, 256, 0, s>>>(N, t->max_kfs, t->d_points, t->d_pobs, t->d_T_pobs, t->d_ftr_image, t->d_kf_old, t->d_kf_slot,
+                                                         t->d_sel);
+      ++ctx->launches;
+    }
+  }
+  // 2. the frame: the last step's current frame (now `last`), every level, into the store
+  FrameRec* r = find_frame(ctx, t->fid_last);
+  if (!r) return fail(ctx, SVOB200_ERR_NOFRAME, "tracker_add_keyframes: last frame missing");
+  kf_store_copy_kernel<<<dim3(16, B), 256, 0, s>>>(r->f, ctx->d_table, t->d_kf_slot, t->d_kf_new);
+  ++ctx->launches;
+  // 3. occupancy from the frame's features (the map points matched in it), FAST + Shi-Tomasi + grid on the selected images,
+  // one seed per new corner
   CU(cudaMemsetAsync(t->d_occ, 0, (size_t)B * n_cells, s));
-  if (N) { kf_occupancy_kernel<<<(N + 255) / 256, 256, 0, s>>>(N, t->d_ftr_image, t->d_px_out, t->d_match_ok, t->det_cell, gc, n_cells, t->d_occ); ++ctx->launches; }
-  if (launch_fast_detect(r->f, t->det_levels, t->det_cell, gc, gr, t->det_thr, t->d_occ, t->d_det_keys, t->d_det_cells, t->d_det_counts, s, &ctx->launches))
-    return fail(ctx, SVOB200_ERR_CUDA, "tracker_add_keyframe: detector launch failed");
-  if (S) {
-    kf_append_seeds_kernel<<<B, 256, 0, s>>>(to_cam(&t->cam), t->d_det_cells, n_cells, t->det_thr, t->d_depth_mean, t->d_depth_min, t->d_seed_off, t->d_seed_refs,
-                                             t->d_seeds, k, t->batch_counter, t->d_kf_appended, t->d_kf_dropped);
+  if (N) {
+    kf_occupancy_kernel<<<(N + 255) / 256, 256, 0, s>>>(N, t->d_ftr_image, t->d_px_out, t->d_match_ok, t->d_kf_new, t->det_cell, gc, n_cells, t->d_occ);
     ++ctx->launches;
   }
-  // 5. the matched map points gain an observation in the new keyframe (frame_handler_mono.cpp:277-279)
+  if (launch_fast_detect(r->f, t->det_levels, t->det_cell, gc, gr, t->det_thr, t->d_occ, t->d_det_keys, t->d_det_cells, t->d_det_counts, s, &ctx->launches,
+                         t->d_kf_new))
+    return fail(ctx, SVOB200_ERR_CUDA, "tracker_add_keyframes: detector launch failed");
+  kf_append_seeds_kernel<<<B, 256, 0, s>>>(to_cam(&t->cam), t->d_det_cells, n_cells, t->det_thr, d_dm, d_dn, t->d_seed_off, t->d_seed_refs,
+                                           t->d_seeds, t->d_kf_new, t->d_batch_counter, t->d_kf_appended, t->d_kf_dropped);
+  ++ctx->launches;
+  // 4. the matched map points gain an observation in the new keyframe (frame_handler_mono.cpp:277-279)
   if (N) {
     kf_add_obs_kernel<<<(N + 255) / 256, 256, 0, s>>>(to_cam(&t->cam), N, t->max_kfs, t->d_points, t->d_pobs, t->d_T_pobs, t->d_ftr_image, t->d_match_ok, t->d_px_out,
-                                                      t->d_match_level, slot, t->d_T_cur);
+                                                      t->d_match_level, t->d_kf_new, t->d_kf_slot, t->d_T_cur);
     ++ctx->launches;
   }
-  if (cudaGetLastError() != cudaSuccess) return fail(ctx, SVOB200_ERR_CUDA, "tracker_add_keyframe: launch error");
-  if (n_new_seeds) CU(cudaMemcpyAsync(n_new_seeds, S ? t->d_kf_appended : t->d_det_counts, sizeof(int) * B, cudaMemcpyDeviceToHost, s));
-  if (n_dropped && S) CU(cudaMemcpyAsync(n_dropped, t->d_kf_dropped, sizeof(int) * B, cudaMemcpyDeviceToHost, s));
-  CU(cudaStreamSynchronize(s));                             // depth_mean / depth_min are the caller's; the counts go back
-  if (n_dropped && !S) for (int b = 0; b < B; ++b) n_dropped[b] = n_new_seeds ? n_new_seeds[b] : 0;
+  if (cudaGetLastError() != cudaSuccess) return fail(ctx, SVOB200_ERR_CUDA, "tracker_add_keyframes: launch error");
+  // the counts (unselected sequences: 0, refused ones: -1).  Without a seed pool n_dropped repeats n_new_seeds, and is 0 when
+  // n_new_seeds is not asked for (as svob200_tracker_add_keyframe always reported it)
+  const cudaMemcpyKind kind = mem == SVOB200_MEM_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
+  if (n_new_seeds) CU(cudaMemcpyAsync(n_new_seeds, t->d_kf_appended, sizeof(int) * B, kind, s));
+  const bool zero_dropped = n_dropped && !S && !n_new_seeds;
+  if (n_dropped && !zero_dropped) CU(cudaMemcpyAsync(n_dropped, t->d_kf_dropped, sizeof(int) * B, kind, s));
+  if (zero_dropped && mem == SVOB200_MEM_DEVICE) CU(cudaMemsetAsync(n_dropped, 0, sizeof(int) * B, s));
+  if (mem == SVOB200_MEM_HOST) CU(cudaStreamSynchronize(s));   // depth_mean / depth_min / which are the caller's; the counts go back
+  if (zero_dropped && mem == SVOB200_MEM_HOST) memset(n_dropped, 0, sizeof(int) * B);
+  return SVOB200_OK;
+}
+
+int svob200_tracker_add_keyframe(svob200_tracker* t, const float* depth_mean, const float* depth_min, int* n_new_seeds, int* n_dropped)
+{
+  return svob200_tracker_add_keyframes(t, nullptr, depth_mean, depth_min, n_new_seeds, n_dropped, SVOB200_MEM_HOST);
+}
+
+int svob200_tracker_scene_depth(svob200_tracker* t, float* depth_mean, float* depth_min, int* n_points, int mem)
+{
+  if (!t || !depth_mean || !depth_min) return SVOB200_ERR_ARG;
+  svob200_ctx* ctx = t->ctx;
+  if (mem != SVOB200_MEM_HOST && mem != SVOB200_MEM_DEVICE) return fail(ctx, SVOB200_ERR_ARG, "tracker_scene_depth: bad mem %d", mem);
+  if (!t->d_stats || t->steps_done == 0) return fail(ctx, SVOB200_ERR_ARG, "tracker_scene_depth: needs a keyframe and at least one step");
+  const int B = t->batch;
+  cudaStream_t s = ctx->stream;
+  const bool dev = mem == SVOB200_MEM_DEVICE;
+  scene_depth_kernel<<<B, 128, 0, s>>>(t->d_ftr_off, t->d_points, t->d_match_ok, t->d_T_cur, t->d_sd_z, dev ? depth_mean : t->d_depth_mean,
+                                       dev ? depth_min : t->d_depth_min, dev ? n_points : t->d_sd_n);
+  ++ctx->launches;
+  if (cudaGetLastError() != cudaSuccess) return fail(ctx, SVOB200_ERR_CUDA, "tracker_scene_depth: launch error");
+  if (dev) return SVOB200_OK;
+  std::vector<float> dm(B), dn(B);
+  std::vector<int> n(B);
+  CU(cudaMemcpyAsync(dm.data(), t->d_depth_mean, sizeof(float) * B, cudaMemcpyDeviceToHost, s));
+  CU(cudaMemcpyAsync(dn.data(), t->d_depth_min, sizeof(float) * B, cudaMemcpyDeviceToHost, s));
+  CU(cudaMemcpyAsync(n.data(), t->d_sd_n, sizeof(int) * B, cudaMemcpyDeviceToHost, s));
+  CU(cudaStreamSynchronize(s));
+  for (int b = 0; b < B; ++b) {
+    if (n[b] > 0) { depth_mean[b] = dm[b]; depth_min[b] = dn[b]; }
+    if (n_points) n_points[b] = n[b];
+  }
   return SVOB200_OK;
 }
 
@@ -953,7 +1119,7 @@ static int enqueue_seeds_update(svob200_tracker* t, int c0, int c1, const SeedPo
   svob200_ctx* ctx = t->ctx;
   const int s0 = t->h_seed_off[c0], ns = t->h_seed_off[c1] - s0;
   if (launch_seeds_update_compact(ctx->d_table, find_frame(ctx, t->fid_cur)->slot, to_cam(&t->cam), ns, t->d_seed_refs + s0, t->d_kf_slot, t->batch, table,
-                                  t->batch_counter, t->max_n_kfs, t->mopts, t->conv_thresh, t->d_seeds + s0, t->d_obs + s0, t->d_seed_scratch, t->S, s0,
+                                  t->d_batch_counter, t->max_n_kfs, t->mopts, t->conv_thresh, t->d_seeds + s0, t->d_obs + s0, t->d_seed_scratch, t->S, s0,
                                   st, &ctx->launches, marks))
     return fail(ctx, SVOB200_ERR_CUDA, "tracker_step: seeds_update failed");
   return 0;
@@ -983,9 +1149,7 @@ static int enqueue_insert_candidates(svob200_tracker* t)
   if (t->pt_capacity < 0) return 0;
   svob200_ctx* ctx = t->ctx;
   const int par = (int)(t->step_no & 1);
-  KfBatches kfb;
-  for (int k = 0; k < svob200_tracker::MAX_KFS; ++k) kfb.v[k] = t->kf_batch[k];
-  cand_insert_kernel<<<t->batch, 128, 0, ctx->stream>>>(t->max_kfs, t->batch, t->d_ftr_off, t->d_cand[par], t->d_cand_n[par], kfb, t->d_kf_slot, t->d_T_kf,
+  cand_insert_kernel<<<t->batch, 128, 0, ctx->stream>>>(t->max_kfs, t->batch, t->d_ftr_off, t->d_cand[par], t->d_cand_n[par], t->d_kf_batch, t->d_kf_slot, t->d_T_kf,
                                                         t->d_points, t->d_pt_world, t->d_pobs, t->d_T_pobs, t->d_sel, t->d_has_point, t->d_pt_rank,
                                                         t->d_pt_dropped);
   ++ctx->launches;
@@ -1105,18 +1269,6 @@ int svob200_tracker_step(svob200_tracker* t, const uint8_t* cur_imgs, int stride
   const int B = t->batch, N = t->N;
   cudaStream_t s = ctx->stream;
   const size_t in_bytes = sizeof(double) * (7 * (size_t)B + 2 * (size_t)N);
-  // the frame that receives the new images must not be a keyframe's (the frame of the step before a keyframe insertion is one):
-  // take a free frame of the pool, or create one (the pool holds at most max_kfs + 2 frames)
-  {
-    auto is_kf = [&](int64_t id) { for (int i = 0; i < svob200_tracker::MAX_KFS; ++i) if (t->fid_kfs[i] == id) return true; return false; };
-    if (is_kf(t->fid_cur)) {
-      if (int e = df_join(t)) return e;                   // frame roles change: no depth-filter chain may be in flight
-      int64_t pick = 0;
-      for (int64_t id : t->frame_pool) if (id != t->fid_last && !is_kf(id)) { pick = id; break; }
-      if (!pick) if (int e = new_frame(t, &pick)) return e;
-      t->fid_cur = pick;
-    }
-  }
   if (t->profiling) cudaEventRecord(t->ev[0], s);
   if (mem == SVOB200_MEM_DEVICE) {
     // the frame slot that becomes `cur` now, the pose table and the step records of this parity were last used by the depth
@@ -1172,7 +1324,7 @@ int svob200_tracker_step(svob200_tracker* t, const uint8_t* cur_imgs, int stride
     // PCIe while chunk c is being processed; one small H2D for the per-step inputs, one D2H for results
     if (int e = df_join(t)) return e;                  // a depth-filter chain of earlier device-memory steps
     FrameRec* r = find_frame(ctx, t->fid_cur);
-    if (int e = frame_own_level0(ctx, r, false)) return e;    // drop an earlier device binding
+    if (int e = frame_own_level0(ctx, r)) return e;           // drop an earlier device binding
     const size_t out_bytes = sizeof(svob200_step_stats) * B + sizeof(double) * 2 * (size_t)N + sizeof(int) * (size_t)N;
     if (t->h_cap < in_bytes + out_bytes + 512) {
       if (t->h_pinned) cudaFreeHost(t->h_pinned);

@@ -295,20 +295,43 @@ int  svob200_tracker_set_last(svob200_tracker* t, const uint8_t* imgs, int strid
  *   svob200_tracker_create, plus 3 = finished seeds (converged / NaN) leave the pool like they leave the reference's list.
  * svob200_tracker_set_detector: FastDetector(cell size = Config::gridSize, levels = Config::nPyrLevels) and the threshold
  *   DepthFilter::initializeSeeds passes (Config::triangMinCornerScore).
- * svob200_tracker_add_keyframe: the frame of the most recent step becomes a keyframe of every sequence, with the pose the step
- *   gave it: occupancy grid from the frame's features (= the map points matched in it, AbstractDetector::setExistingFeatures),
- *   FAST + Shi-Tomasi + grid selection on its pyramid, one Seed(ftr, depth_mean, depth_min) per new corner in cell order
- *   (batch_id = ++Seed::batch_counter) into the empty slots of the sequence's pool; every map point matched in the frame gains
- *   an observation in it (Feature(frame, px_refined, search_level) + Point::addFrameRef, reprojector.cpp:219-231,
- *   frame_handler_mono.cpp:277-279), and from then on each step matches a point against its closest-view observation
- *   (Point::getCloseViewObs, point.cpp:101-125); when the oldest keyframe leaves the ring its seeds are erased
- *   (DepthFilter::removeKeyframe) and the points forget it (Map::safeDeleteFrame).  depth_mean / depth_min: one per sequence,
- *   host memory (FrameHandlerMono passes frame_utils::getSceneDepth's mean and 0.5 * min).  n_new_seeds / n_dropped (host,
- *   one int per sequence, may be NULL): seeds created / corners that found no empty slot.
- * svob200_tracker_get_seed_refs: the pool slot by slot (host arrays of svob200_tracker_num_seed_slots entries, any may be NULL). */
+ * Every sequence has its own keyframe ring, as if it were its own FrameHandlerMono + DepthFilter: its own ring indices
+ *   (a free one, else its oldest keyframe leaves), its own Seed::batch_counter and its own evictions.  The keyframe images live
+ *   in a store of max_keyframes frame batches (ring index k of sequence b = image b of store frame k); an insertion copies the
+ *   selected sequences' images, every pyramid level, into it.
+ * svob200_tracker_add_keyframes: the frame of the most recent step becomes a keyframe of the sequences with which[b] != 0
+ *   (which: one byte per sequence, NULL = every sequence), with the pose the step gave it: occupancy grid from the frame's
+ *   features (= the map points matched in it, AbstractDetector::setExistingFeatures), FAST + Shi-Tomasi + grid selection on
+ *   its pyramid, one Seed(ftr, depth_mean, depth_min) per new corner in cell order (batch_id = ++Seed::batch_counter of the
+ *   sequence) into the empty slots of the sequence's pool; every map point matched in the frame gains an observation in it
+ *   (Feature(frame, px_refined, search_level) + Point::addFrameRef, reprojector.cpp:219-231, frame_handler_mono.cpp:277-279),
+ *   and from then on each step matches a point against its closest-view observation (Point::getCloseViewObs,
+ *   point.cpp:101-125); when the sequence's oldest keyframe leaves its ring, its seeds are erased (DepthFilter::removeKeyframe)
+ *   and its points forget it (Map::safeDeleteFrame).  For a selected sequence the result is what a tracker holding only that
+ *   sequence computes; an unselected sequence is left untouched, its counter included.
+ *   depth_mean / depth_min: one float per sequence (what FrameHandlerMono passes to DepthFilter::addKeyframe: the mean and
+ *   0.5 * min of frame_utils::getSceneDepth, see svob200_tracker_scene_depth).  n_new_seeds / n_dropped (one int per
+ *   sequence, may be NULL): seeds created / corners that found no empty slot (0 for an unselected sequence; without a seed
+ *   pool, the corners found for both, and n_dropped 0 when n_new_seeds is NULL).  Seed::batch_id is 16 bits wide: a sequence
+ *   takes at most 65,534 keyframes; a selected sequence past that is left untouched and reports -1 in both counts (the limit
+ *   counts the sequence's own keyframes, not calls).  mem: where ALL
+ *   the arrays live.  In SVOB200_MEM_DEVICE mode the call is ordered on the context's stream and does not synchronise with
+ *   the host (the first insertion allocates the keyframe store when svob200_tracker_set_seed_pool did not).  Not available in
+ *   chain mode (SVOB200_ERR_UNSUPPORTED); SVOB200_ERR_ARG before set_keyframe, before the first step, or for a bad mem.
+ * svob200_tracker_add_keyframe(t, dm, dn, nn, nd) = svob200_tracker_add_keyframes(t, NULL, dm, dn, nn, nd, SVOB200_MEM_HOST).
+ * svob200_tracker_scene_depth: frame_utils::getSceneDepth of the most recent step's frame, per sequence, over the point slots
+ *   matched in it (candidates included, like the occupancy grid), z = (T_cur_w * pos).z: depth_mean = (float) the element of
+ *   rank n/2 of the ascending depths (vk::getMedian's nth_element), depth_min = (float)(0.5 * min) (the value processFrame
+ *   passes), n_points = n (may be NULL).  n == 0 leaves that sequence's depth_mean / depth_min untouched.  mem as above; in
+ *   SVOB200_MEM_DEVICE mode the call does not synchronise with the host.
+ * svob200_tracker_get_seed_refs: the pool slot by slot (host arrays of svob200_tracker_num_seed_slots entries, any may be NULL);
+ *   kf is the ring index of the seed's keyframe in its own sequence's ring, batch_id its sequence's Seed::batch_id. */
 int  svob200_tracker_set_seed_pool(svob200_tracker* t, int capacity_per_sequence, int max_keyframes, int max_n_kfs, int reseed);
 int  svob200_tracker_set_detector(svob200_tracker* t, int cell_size, int n_detect_levels, double detection_threshold);
+int  svob200_tracker_add_keyframes(svob200_tracker* t, const uint8_t* which, const float* depth_mean, const float* depth_min,
+                                   int* n_new_seeds, int* n_dropped, int mem);
 int  svob200_tracker_add_keyframe(svob200_tracker* t, const float* depth_mean, const float* depth_min, int* n_new_seeds, int* n_dropped);
+int  svob200_tracker_scene_depth(svob200_tracker* t, float* depth_mean, float* depth_min, int* n_points, int mem);
 int  svob200_tracker_get_seed_refs(svob200_tracker* t, double* px, int* level, int* kf, int* batch_id, int* state);
 int  svob200_tracker_num_seed_slots(svob200_tracker* t);
 /* ---- point pool: converged seeds become map points on the device (DepthFilter::updateSeeds -> seed_converged_cb_ ->
