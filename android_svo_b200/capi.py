@@ -437,14 +437,15 @@ class Context:
         return seeds
 
     def debug_chi2_chain(self, res, visible, contrib, block=256):
-        """The device replays of the reference's sequential float chi2 chain: [(sum, count)] for serial, parallel (latency mode), parallel (batch mode)."""
+        """The device replays of the reference's sequential float chi2 chain: [(sum, count)] for serial, parallel (latency mode),
+        parallel (128-thread batch kernel, one staging buffer), parallel (256/512-thread batch kernels, double-buffered)."""
         res = np.ascontiguousarray(res, dtype=np.float32).reshape(-1, 16)
         vis = np.ascontiguousarray(visible, dtype=np.uint8)
         con = np.ascontiguousarray(contrib, dtype=np.uint8)
-        sums = np.zeros(3, np.float32)
-        cnts = np.zeros(3, np.int32)
+        sums = np.zeros(4, np.float32)
+        cnts = np.zeros(4, np.int32)
         self._ck(self.L.svob200_debug_chi2_chain(self.h, int(block), len(res), _ptr(res), _ptr(vis), _ptr(con), _ptr(sums), _ptr(cnts)))
-        return [(sums[i], int(cnts[i])) for i in range(3)]
+        return [(sums[i], int(cnts[i])) for i in range(4)]
 
     def compute_tau(self, T_ref_cur, f, z, ang):
         T = np.ascontiguousarray(T_ref_cur, dtype=np.float64)

@@ -492,8 +492,8 @@ int svob200_debug_chi2_chain(svob200_ctx* ctx, int block, int n_features, const 
   const int i_r = st.add(res, nullptr, sizeof(float) * 16 * (size_t)n_features, 0);
   const int i_v = st.add(visible, nullptr, (size_t)n_features, 0);
   const int i_c = st.add(contrib, nullptr, (size_t)n_features, 0);
-  const int i_s = st.add(nullptr, sums, sizeof(float) * 3, 2);
-  const int i_n = st.add(nullptr, counts, sizeof(int) * 3, 2);
+  const int i_s = st.add(nullptr, sums, sizeof(float) * 4, 2);
+  const int i_n = st.add(nullptr, counts, sizeof(int) * 4, 2);
   if (int e = st.layout()) return e;
   st.upload();
   if (int e = st.push()) return e;

@@ -739,7 +739,8 @@ __global__ void __launch_bounds__(BLOCK, CLUSTER > 1 ? 1 : (BLOCK == 128 ? ALIGN
 }
 
 // diagnostics (svob200_debug_chi2_chain): the replays of the float chi2 chain over caller-supplied residuals, one CTA:
-// [0] one thread adding, [1] the parallel replay as the latency-mode kernels run it, [2] as the batch kernels run it
+// [0] one thread adding, [1] the parallel replay as the latency-mode kernels run it, [2] as the 128-thread batch kernel runs
+// it (one staging buffer), [3] as the 256- and 512-thread batch kernels run it (sequential head, double-buffered)
 template <int BLOCK>
 __global__ void __launch_bounds__(BLOCK) chi2_chain_test_kernel(const float* res, const uint8_t* visible, const uint8_t* contrib, int N, float* sums, int* cnts)
 {
@@ -750,6 +751,8 @@ __global__ void __launch_bounds__(BLOCK) chi2_chain_test_kernel(const float* res
   exact_chi2_chain_parallel<BLOCK, CHAIN_HEAD_LATENCY, 2>(res, visible, contrib, N, &s_chainmem, sums + 1, cnts + 1, tid);
   __syncthreads();
   exact_chi2_chain_parallel<BLOCK, CHAIN_TERMS, 1>(res, visible, contrib, N, reinterpret_cast<ChainSmem<1>*>(&s_chainmem), sums + 2, cnts + 2, tid);
+  __syncthreads();
+  exact_chi2_chain_parallel<BLOCK, CHAIN_TERMS, 2>(res, visible, contrib, N, &s_chainmem, sums + 3, cnts + 3, tid);
 }
 
 }  // namespace

@@ -230,8 +230,9 @@ int svob200_update_seed(svob200_ctx* ctx, int n, const float* x, const float* ta
  * sequentially accumulated `float chi2` (sparse_img_align.cpp:259-263) when the double sums are too close to call.  This entry
  * runs the device replays of that chain over caller-supplied residuals (16 per feature, host memory) with a CTA of `block`
  * threads (128, 256 or 512): sums[0]/counts[0] = one thread adding in order, [1] = the parallel exact replay as the
- * latency-mode (cluster) alignment kernels run it, [2] = as the batch kernels run it.  sums and counts hold 3 entries; all
- * three must be bit-identical for any input. */
+ * latency-mode (cluster) alignment kernels run it, [2] = as the 128-thread batch kernel runs it (one staging buffer),
+ * [3] = as the 256- and 512-thread batch kernels run it (double-buffered).  sums and counts hold 4 entries; all four must
+ * be bit-identical for any input. */
 int svob200_debug_chi2_chain(svob200_ctx* ctx, int block, int n_features, const float* res, const uint8_t* visible,
                              const uint8_t* contrib, float* sums, int* counts);
 int svob200_compute_tau(svob200_ctx* ctx, int n, const double* T_ref_cur, const double* f, const double* z,

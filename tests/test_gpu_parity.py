@@ -633,9 +633,15 @@ def _chain_reference(res, visible, contrib):
 
 @pytest.mark.parametrize("block", [128, 256, 512])
 def test_exact_chi2_chain_parallel_property(ctx, block):
+    """Every replay instance the alignment kernels run, against the sequential float32 chain: the cluster kernels'
+    (short sequential head), the 128-thread batch kernel's (one staging buffer) and the 256- / 512-thread batch kernels'
+    (a whole chunk as the sequential head, double-buffered)."""
+    names = ("serial", "parallel/latency", "parallel/batch128", "parallel/batch256-512")
     for name, res, vis, con in _chain_cases():
         want, want_n = _chain_reference(res, vis, con)
         bits = lambda v: int(np.float32(v).view(np.uint32))
-        for which, (got, got_n) in zip(("serial", "parallel/latency", "parallel/batch"), ctx.debug_chi2_chain(res, vis, con, block=block)):
+        got_all = ctx.debug_chi2_chain(res, vis, con, block=block)
+        assert len(got_all) == len(names)
+        for which, (got, got_n) in zip(names, got_all):
             assert got_n == want_n, (name, which, got_n, want_n)
             assert bits(got) == bits(want), "%s: %s device chain %r (%08x) != reference %r (%08x)" % (name, which, got, bits(got), want, bits(want))
