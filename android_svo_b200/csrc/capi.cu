@@ -21,6 +21,21 @@ int resolve_slots(svob200_ctx* ctx, svob200_feature_ref* staged, int n)
   return 0;
 }
 
+// total = off[n] and the largest count off[i + 1] - off[i] of an offsets array in caller memory; of device-resident offsets
+// one small read-back of off[n] (scratch sizes depend on it), and the total stands in for the largest count
+int offsets_extent(svob200_ctx* ctx, const int* off, int n, int mem, int* total, int* max_count = nullptr)
+{
+  if (mem == SVOB200_MEM_HOST) {
+    *total = off[n];
+    if (max_count) { *max_count = 0; for (int i = 0; i < n; ++i) *max_count = std::max(*max_count, off[i + 1] - off[i]); }
+    return 0;
+  }
+  CU(cudaMemcpyAsync(total, off + n, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+  CU(cudaStreamSynchronize(ctx->stream));
+  if (max_count) *max_count = *total;
+  return 0;
+}
+
 }  // namespace
 
 int frame_bind_level0(svob200_ctx* ctx, FrameRec* r, const uint8_t* dev_gray, int stride)
@@ -166,24 +181,23 @@ int svob200_frame_create(svob200_ctx* ctx, int64_t frame_id, int batch, int w, i
   return SVOB200_OK;
 }
 
-static int build_levels(svob200_ctx* ctx, FrameRec* r, const int* round_modes)
+static int build_levels(svob200_ctx* ctx, FrameRec* r, const int* round_modes, const char* who)
 {
   int modes[SVOB200_MAX_LEVELS];
   pyramid_round_modes(r->f, round_modes, modes);
-  if (launch_pyramid(r->f, modes, ctx->stream, &ctx->launches)) return fail(ctx, SVOB200_ERR_CUDA, "pyramid launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+  CU_AT(who, launch_pyramid(r->f, modes, ctx->stream, &ctx->launches));
   return 0;
 }
 
 int svob200_frame_upload(svob200_ctx* ctx, int64_t frame_id, const uint8_t* gray, int stride, const int* round_modes, int mem)
 {
   if (!ctx || !gray) return fail(ctx, SVOB200_ERR_ARG, "frame_upload: null argument");
-  FrameRec* r = find_frame(ctx, frame_id);
-  if (!r) return fail(ctx, SVOB200_ERR_NOFRAME, "frame %lld not found", (long long)frame_id);
+  FrameRec* r = resident_frame(ctx, frame_id, "frame_upload"); if (!r) return SVOB200_ERR_NOFRAME;
   if (stride < r->f.w[0]) return fail(ctx, SVOB200_ERR_ARG, "frame_upload: stride < width");
   if (int e = frame_own_level0(ctx, r)) return e;
   CU(cudaMemcpy2DAsync(r->f.lvl[0], r->f.pitch[0], gray, stride, r->f.w[0], (size_t)r->f.h[0] * r->f.batch,
                        mem == SVOB200_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, ctx->stream));
-  if (int e = build_levels(ctx, r, round_modes)) return e;
+  if (int e = build_levels(ctx, r, round_modes, "frame_upload: launch_pyramid")) return e;
   if (mem == SVOB200_MEM_HOST) CU(cudaStreamSynchronize(ctx->stream));
   return SVOB200_OK;
 }
@@ -193,17 +207,15 @@ int svob200_frame_upload(svob200_ctx* ctx, int64_t frame_id, const uint8_t* gray
 int svob200_frame_bind(svob200_ctx* ctx, int64_t frame_id, const uint8_t* dev_gray, int stride, const int* round_modes)
 {
   if (!ctx || !dev_gray) return fail(ctx, SVOB200_ERR_ARG, "frame_bind: null argument");
-  FrameRec* r = find_frame(ctx, frame_id);
-  if (!r) return fail(ctx, SVOB200_ERR_NOFRAME, "frame %lld not found", (long long)frame_id);
+  FrameRec* r = resident_frame(ctx, frame_id, "frame_bind"); if (!r) return SVOB200_ERR_NOFRAME;
   if (int e = frame_bind_level0(ctx, r, dev_gray, stride)) return e;
-  return build_levels(ctx, r, round_modes);
+  return build_levels(ctx, r, round_modes, "frame_bind: launch_pyramid");
 }
 
 int svob200_frame_download(svob200_ctx* ctx, int64_t frame_id, int image, int level, uint8_t* out, int out_stride)
 {
   if (!ctx || !out) return fail(ctx, SVOB200_ERR_ARG, "frame_download: null argument");
-  FrameRec* r = find_frame(ctx, frame_id);
-  if (!r) return fail(ctx, SVOB200_ERR_NOFRAME, "frame %lld not found", (long long)frame_id);
+  FrameRec* r = resident_frame(ctx, frame_id, "frame_download"); if (!r) return SVOB200_ERR_NOFRAME;
   if (level < 0 || level >= r->f.n_levels || image < 0 || image >= r->f.batch || out_stride < r->f.w[level]) return fail(ctx, SVOB200_ERR_ARG, "frame_download: bad level/image/stride");
   CU(cudaMemcpy2DAsync(out, out_stride, r->f.lvl[level] + (size_t)image * r->f.img_stride[level], r->f.pitch[level], r->f.w[level], r->f.h[level],
                        cudaMemcpyDeviceToHost, ctx->stream));
@@ -215,23 +227,21 @@ int svob200_frame_release(svob200_ctx* ctx, int64_t frame_id)
 {
   if (!ctx) return SVOB200_ERR_ARG;
   std::lock_guard<std::mutex> lk(ctx->mu);
-  auto it = ctx->frames.find(frame_id);
-  if (it == ctx->frames.end()) return fail(ctx, SVOB200_ERR_NOFRAME, "frame %lld not found", (long long)frame_id);
+  FrameRec* r = resident_frame(ctx, frame_id, "frame_release"); if (!r) return SVOB200_ERR_NOFRAME;
   if (int e = ctx_join_aux(ctx)) return e;
   CU(cudaStreamSynchronize(ctx->stream));
   // frames of up to 8 MB (single camera images with their pyramid) go to the spare list, at most kSpareFrames of them
   constexpr size_t kSpareFrames = 8, kSpareBytes = 8u << 20;
-  if (it->second.bytes <= kSpareBytes && ctx->spare_frames.size() < kSpareFrames) ctx->spare_frames.push_back({it->second.bytes, it->second.base});
-  else cudaFree(it->second.base);
-  ctx->free_slots.push_back(it->second.slot);
-  ctx->frames.erase(it);
+  if (r->bytes <= kSpareBytes && ctx->spare_frames.size() < kSpareFrames) ctx->spare_frames.push_back({r->bytes, r->base});
+  else cudaFree(r->base);
+  ctx->free_slots.push_back(r->slot);
+  ctx->frames.erase(frame_id);
   return SVOB200_OK;
 }
 
 int svob200_frame_info(svob200_ctx* ctx, int64_t frame_id, int* batch, int* w, int* h, int* n_levels)
 {
-  FrameRec* r = ctx ? find_frame(ctx, frame_id) : nullptr;
-  if (!r) return fail(ctx, SVOB200_ERR_NOFRAME, "frame %lld not found", (long long)frame_id);
+  FrameRec* r = resident_frame(ctx, frame_id, "frame_info"); if (!r) return SVOB200_ERR_NOFRAME;
   if (batch) *batch = r->f.batch;
   if (w) *w = r->f.w[0];
   if (h) *h = r->f.h[0];
@@ -241,8 +251,8 @@ int svob200_frame_info(svob200_ctx* ctx, int64_t frame_id, int* batch, int* w, i
 
 int svob200_frame_slot(svob200_ctx* ctx, int64_t frame_id)
 {
-  FrameRec* r = ctx ? find_frame(ctx, frame_id) : nullptr;
-  return r ? r->slot : fail(ctx, SVOB200_ERR_NOFRAME, "frame %lld not found", (long long)frame_id);
+  FrameRec* r = resident_frame(ctx, frame_id, "frame_slot");
+  return r ? r->slot : SVOB200_ERR_NOFRAME;
 }
 
 int svob200_half_sample(svob200_ctx* ctx, const uint8_t* in, int w, int h, int in_stride, uint8_t* out, int out_stride, int round_mode)
@@ -254,7 +264,7 @@ int svob200_half_sample(svob200_ctx* ctx, const uint8_t* in, int w, int h, int i
   uint8_t* d_in = static_cast<uint8_t*>(ctx->d_scratch.p);
   uint8_t* d_out = d_in + ((in_b + 255) & ~(size_t)255);
   CU(cudaMemcpy2DAsync(d_in, ip, in, in_stride, w, h, cudaMemcpyHostToDevice, ctx->stream));
-  if (launch_half_sample_single(d_in, ip, w, h, d_out, op, round_mode, ctx->stream, &ctx->launches)) return fail(ctx, SVOB200_ERR_CUDA, "half_sample launch failed");
+  CU_AT("half_sample: launch_half_sample_single", launch_half_sample_single(d_in, ip, w, h, d_out, op, round_mode, ctx->stream, &ctx->launches));
   CU(cudaMemcpy2DAsync(out, out_stride, d_out, op, w / 2, h / 2, cudaMemcpyDeviceToHost, ctx->stream));
   CU(cudaStreamSynchronize(ctx->stream));
   return SVOB200_OK;
@@ -265,8 +275,7 @@ int svob200_fast_detect(svob200_ctx* ctx, int64_t frame_id, int n_detect_levels,
                         const uint8_t* occupancy, svob200_corner* cells_out, int* n_features_out, int mem)
 {
   if (!ctx || !cells_out || cell_size <= 0) return fail(ctx, SVOB200_ERR_ARG, "fast_detect: bad arguments");
-  FrameRec* r = find_frame(ctx, frame_id);
-  if (!r) return fail(ctx, SVOB200_ERR_NOFRAME, "frame %lld not found", (long long)frame_id);
+  FrameRec* r = resident_frame(ctx, frame_id, "fast_detect"); if (!r) return SVOB200_ERR_NOFRAME;
   if (n_detect_levels < 1 || n_detect_levels > r->f.n_levels) return fail(ctx, SVOB200_ERR_ARG, "fast_detect: n_detect_levels out of range");
   if (r->f.w[0] >= 16384 || r->f.h[0] >= 16384) return fail(ctx, SVOB200_ERR_UNSUPPORTED, "fast_detect: image larger than 16383");
   const int gc = (r->f.w[0] + cell_size - 1) / cell_size, gr = (r->f.h[0] + cell_size - 1) / cell_size;
@@ -276,14 +285,13 @@ int svob200_fast_detect(svob200_ctx* ctx, int64_t frame_id, int n_detect_levels,
   const int i_cells = st.add(nullptr, cells_out, total * sizeof(svob200_corner), 2);
   const int i_cnt = st.add(nullptr, n_features_out, sizeof(int) * r->f.batch, 2);
   if (int e = st.layout()) return e;
-  st.upload();
   if (int e = st.push()) return e;
   if (ctx->d_scratch.ensure(total * 8 + sizeof(int) * r->f.batch + 256) != cudaSuccess) return fail(ctx, SVOB200_ERR_NOMEM, "fast_detect: scratch alloc failed");
   unsigned long long* d_keys = static_cast<unsigned long long*>(ctx->d_scratch.p);
   int* d_cnt = (mem == SVOB200_MEM_DEVICE && !n_features_out) ? reinterpret_cast<int*>(d_keys + total) : st.dev<int>(i_cnt);
-  if (launch_fast_detect(r->f, n_detect_levels, cell_size, gc, gr, thr, occupancy ? st.dev<uint8_t>(i_occ) : nullptr, d_keys,
-                         st.dev<svob200_corner>(i_cells), d_cnt, ctx->stream, &ctx->launches))
-    return fail(ctx, SVOB200_ERR_CUDA, "fast_detect launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+  CU_AT("fast_detect: launch_fast_detect",
+        launch_fast_detect(r->f, n_detect_levels, cell_size, gc, gr, thr, occupancy ? st.dev<uint8_t>(i_occ) : nullptr, d_keys,
+                           st.dev<svob200_corner>(i_cells), d_cnt, ctx->stream, &ctx->launches));
   return st.download();
 }
 
@@ -291,15 +299,14 @@ int svob200_fast_corners(svob200_ctx* ctx, int64_t frame_id, int image, int leve
                          int* xs, int* ys, int* scores)
 {
   if (!ctx) return SVOB200_ERR_ARG;
-  FrameRec* r = find_frame(ctx, frame_id);
-  if (!r) return fail(ctx, SVOB200_ERR_NOFRAME, "frame %lld not found", (long long)frame_id);
+  FrameRec* r = resident_frame(ctx, frame_id, "fast_corners"); if (!r) return SVOB200_ERR_NOFRAME;
   if (level < 0 || level >= r->f.n_levels || image < 0 || image >= r->f.batch) return fail(ctx, SVOB200_ERR_ARG, "fast_corners: bad level/image");
   const int w = r->f.w[level], h = r->f.h[level];
   const size_t n = (size_t)w * h;
   if (ctx->d_scratch.ensure(n + 256) != cudaSuccess) return fail(ctx, SVOB200_ERR_NOMEM, "fast_corners: scratch alloc failed");
   uint8_t* d_sc = static_cast<uint8_t*>(ctx->d_scratch.p);
   threshold = std::min(std::max(threshold, 0), 255);
-  if (launch_fast_raw(r->f, image, level, threshold, nonmax, d_sc, ctx->stream, &ctx->launches)) return fail(ctx, SVOB200_ERR_CUDA, "fast_corners launch failed");
+  CU_AT("fast_corners: launch_fast_raw", launch_fast_raw(r->f, image, level, threshold, nonmax, d_sc, ctx->stream, &ctx->launches));
   std::vector<uint8_t> sc(n);
   CU(cudaMemcpyAsync(sc.data(), d_sc, n, cudaMemcpyDeviceToHost, ctx->stream));
   CU(cudaStreamSynchronize(ctx->stream));
@@ -320,22 +327,13 @@ int svob200_sparse_align(svob200_ctx* ctx, int64_t ref_frame_id, int64_t cur_fra
                          const double* T_cur_ref, const svob200_align_opts* opts, svob200_align_result* results, int mem)
 {
   if (!ctx || !cam || !ftr_offsets || !opts || !results || batch <= 0) return fail(ctx, SVOB200_ERR_ARG, "sparse_align: bad arguments");
-  FrameRec* ref = find_frame(ctx, ref_frame_id);
-  FrameRec* cur = find_frame(ctx, cur_frame_id);
-  if (!ref || !cur) return fail(ctx, SVOB200_ERR_NOFRAME, "sparse_align: frame not resident");
+  FrameRec* ref = resident_frame(ctx, ref_frame_id, "sparse_align"); if (!ref) return SVOB200_ERR_NOFRAME;
+  FrameRec* cur = resident_frame(ctx, cur_frame_id, "sparse_align"); if (!cur) return SVOB200_ERR_NOFRAME;
   if (batch > ref->f.batch || batch > cur->f.batch) return fail(ctx, SVOB200_ERR_ARG, "sparse_align: batch exceeds the frames' batch");
   if (opts->max_level >= ref->f.n_levels || opts->max_level >= cur->f.n_levels || opts->min_level < 0 || opts->min_level > opts->max_level)
     return fail(ctx, SVOB200_ERR_ARG, "sparse_align: level range [%d,%d] outside the pyramid", opts->min_level, opts->max_level);
   int total = 0, max_per = 0;
-  if (mem == SVOB200_MEM_HOST) {
-    total = ftr_offsets[batch];
-    for (int b = 0; b < batch; ++b) max_per = std::max(max_per, ftr_offsets[b + 1] - ftr_offsets[b]);
-  } else {
-    // device-resident offsets: one small read-back of the final offset (the scratch size depends on it)
-    CU(cudaMemcpyAsync(&total, ftr_offsets + batch, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
-    max_per = total;
-  }
+  if (int e = offsets_extent(ctx, ftr_offsets, batch, mem, &total, &max_per)) return e;
   Stage st(ctx, mem);
   const int i_off = st.add(ftr_offsets, nullptr, sizeof(int) * (batch + 1), 0);
   const int i_px = st.add(px, nullptr, sizeof(double) * 2 * total, 0);
@@ -344,13 +342,12 @@ int svob200_sparse_align(svob200_ctx* ctx, int64_t ref_frame_id, int64_t cur_fra
   const int i_T = st.add(T_cur_ref, nullptr, sizeof(double) * 7 * batch, 0);
   const int i_res = st.add(nullptr, results, sizeof(svob200_align_result) * batch, 2);
   if (int e = st.layout()) return e;
-  st.upload();
   if (int e = st.push()) return e;
   if (ctx->d_scratch.ensure(sparse_align_scratch_bytes(total)) != cudaSuccess) return fail(ctx, SVOB200_ERR_NOMEM, "sparse_align: scratch alloc failed");
-  if (launch_sparse_align(ref->f, cur->f, to_cam(cam), batch, total, max_per, st.dev<int>(i_off), st.dev<double>(i_px), st.dev<double>(i_xyz),
-                          st.dev<uint8_t>(i_hp), st.dev<double>(i_T), *opts, st.dev<svob200_align_result>(i_res), ctx->d_scratch.p,
-                          ctx->stream, &ctx->launches))
-    return fail(ctx, SVOB200_ERR_CUDA, "sparse_align launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+  CU_AT("sparse_align: launch_sparse_align",
+        launch_sparse_align(ref->f, cur->f, to_cam(cam), batch, total, max_per, st.dev<int>(i_off), st.dev<double>(i_px), st.dev<double>(i_xyz),
+                            st.dev<uint8_t>(i_hp), st.dev<double>(i_T), *opts, st.dev<svob200_align_result>(i_res), ctx->d_scratch.p,
+                            ctx->stream, &ctx->launches));
   return st.download();
 }
 
@@ -359,8 +356,7 @@ int svob200_align_patches(svob200_ctx* ctx, int64_t frame_id, int level, int n, 
                           const uint8_t* patch, const float* dir, int n_iter, double* px, int* converged, double* h_inv, int mem)
 {
   if (!ctx || n < 0 || !image || !pwb || !patch || !px || !converged) return fail(ctx, SVOB200_ERR_ARG, "align_patches: bad arguments");
-  FrameRec* r = find_frame(ctx, frame_id);
-  if (!r) return fail(ctx, SVOB200_ERR_NOFRAME, "frame %lld not found", (long long)frame_id);
+  FrameRec* r = resident_frame(ctx, frame_id, "align_patches"); if (!r) return SVOB200_ERR_NOFRAME;
   if (level < 0 || level >= r->f.n_levels) return fail(ctx, SVOB200_ERR_ARG, "align_patches: bad level");
   if (n == 0) return SVOB200_OK;
   Stage st(ctx, mem);
@@ -372,12 +368,11 @@ int svob200_align_patches(svob200_ctx* ctx, int64_t frame_id, int level, int n, 
   const int i_cv = st.add(nullptr, converged, sizeof(int) * n, 2);
   const int i_hi = h_inv ? st.add(nullptr, h_inv, sizeof(double) * n, 2) : -1;
   if (int e = st.layout()) return e;
-  st.upload();
   if (int e = st.push()) return e;
   if (ctx->d_scratch.ensure(lk_jobs_bytes(n)) != cudaSuccess) return fail(ctx, SVOB200_ERR_NOMEM, "align_patches: scratch alloc failed");
-  if (launch_align_patches(ctx->d_table, r->slot, level, n, st.dev<int>(i_img), st.dev<uint8_t>(i_pwb), st.dev<uint8_t>(i_pat), dir ? st.dev<float>(i_dir) : nullptr,
-                           n_iter, st.dev<double>(i_px), st.dev<int>(i_cv), h_inv ? st.dev<double>(i_hi) : nullptr, ctx->d_scratch.p, ctx->stream, &ctx->launches))
-    return fail(ctx, SVOB200_ERR_CUDA, "align_patches launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+  CU_AT("align_patches: launch_align_patches",
+        launch_align_patches(ctx->d_table, r->slot, level, n, st.dev<int>(i_img), st.dev<uint8_t>(i_pwb), st.dev<uint8_t>(i_pat), dir ? st.dev<float>(i_dir) : nullptr,
+                             n_iter, st.dev<double>(i_px), st.dev<int>(i_cv), h_inv ? st.dev<double>(i_hi) : nullptr, ctx->d_scratch.p, ctx->stream, &ctx->launches));
   return st.download();
 }
 
@@ -393,8 +388,7 @@ int svob200_match_direct(svob200_ctx* ctx, int64_t cur_frame_id, const svob200_c
                          svob200_match_result* results, int mem)
 {
   if (!ctx || !cam || n < 0 || !ftrs || !depth_ref || !px_cur_in || !opts || !results) return fail(ctx, SVOB200_ERR_ARG, "match_direct: bad arguments");
-  FrameRec* cur = find_frame(ctx, cur_frame_id);
-  if (!cur) return fail(ctx, SVOB200_ERR_NOFRAME, "match_direct: current frame not resident");
+  FrameRec* cur = resident_frame(ctx, cur_frame_id, "match_direct"); if (!cur) return SVOB200_ERR_NOFRAME;
   if (opts->max_search_level >= cur->f.n_levels) return fail(ctx, SVOB200_ERR_ARG, "match_direct: max_search_level outside the pyramid");
   if (opts->max_epi_search_steps < 0) return fail(ctx, SVOB200_ERR_ARG, "match_direct: negative max_epi_search_steps");
   if (n == 0) return SVOB200_OK;
@@ -404,13 +398,12 @@ int svob200_match_direct(svob200_ctx* ctx, int64_t cur_frame_id, const svob200_c
   const int i_p = st.add(px_cur_in, nullptr, sizeof(double) * 2 * n, 0);
   const int i_r = st.add(nullptr, results, sizeof(svob200_match_result) * n, 2);
   if (int e = st.layout()) return e;
-  st.upload();
   if (mem == SVOB200_MEM_HOST) if (int e = resolve_slots(ctx, st.host<svob200_feature_ref>(i_f), n)) return e;
   if (int e = st.push()) return e;
   if (ctx->d_scratch.ensure(match_scratch_bytes(n)) != cudaSuccess) return fail(ctx, SVOB200_ERR_NOMEM, "match_direct: scratch alloc failed");
-  if (launch_match_direct(ctx->d_table, cur->slot, to_cam(cam), n, st.dev<svob200_feature_ref>(i_f), st.dev<double>(i_d),
-                          st.dev<double>(i_p), *opts, st.dev<svob200_match_result>(i_r), nullptr, nullptr, ctx->d_scratch.p, n, 0, ctx->stream, &ctx->launches))
-    return fail(ctx, SVOB200_ERR_CUDA, "match_direct launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+  CU_AT("match_direct: launch_match_direct",
+        launch_match_direct(ctx->d_table, cur->slot, to_cam(cam), n, st.dev<svob200_feature_ref>(i_f), st.dev<double>(i_d),
+                            st.dev<double>(i_p), *opts, st.dev<svob200_match_result>(i_r), nullptr, nullptr, ctx->d_scratch.p, n, 0, ctx->stream, &ctx->launches));
   return st.download();
 }
 
@@ -418,8 +411,7 @@ int svob200_epipolar_match(svob200_ctx* ctx, int64_t cur_frame_id, const svob200
                            const double* d, const svob200_matcher_opts* opts, svob200_epi_result* results, int mem)
 {
   if (!ctx || !cam || n < 0 || !ftrs || !d || !opts || !results) return fail(ctx, SVOB200_ERR_ARG, "epipolar_match: bad arguments");
-  FrameRec* cur = find_frame(ctx, cur_frame_id);
-  if (!cur) return fail(ctx, SVOB200_ERR_NOFRAME, "epipolar_match: current frame not resident");
+  FrameRec* cur = resident_frame(ctx, cur_frame_id, "epipolar_match"); if (!cur) return SVOB200_ERR_NOFRAME;
   if (opts->max_search_level >= cur->f.n_levels) return fail(ctx, SVOB200_ERR_ARG, "epipolar_match: max_search_level outside the pyramid");
   if (opts->max_epi_search_steps < 0) return fail(ctx, SVOB200_ERR_ARG, "epipolar_match: negative max_epi_search_steps");
   if (n == 0) return SVOB200_OK;
@@ -428,13 +420,12 @@ int svob200_epipolar_match(svob200_ctx* ctx, int64_t cur_frame_id, const svob200
   const int i_d = st.add(d, nullptr, sizeof(double) * 3 * n, 0);
   const int i_r = st.add(nullptr, results, sizeof(svob200_epi_result) * n, 2);
   if (int e = st.layout()) return e;
-  st.upload();
   if (mem == SVOB200_MEM_HOST) if (int e = resolve_slots(ctx, st.host<svob200_feature_ref>(i_f), n)) return e;
   if (int e = st.push()) return e;
   if (ctx->d_scratch.ensure(epipolar_scratch_bytes(n)) != cudaSuccess) return fail(ctx, SVOB200_ERR_NOMEM, "epipolar_match: scratch alloc failed");
-  if (launch_epipolar(ctx->d_table, cur->slot, to_cam(cam), n, st.dev<svob200_feature_ref>(i_f), st.dev<double>(i_d), *opts,
-                      st.dev<svob200_epi_result>(i_r), ctx->d_scratch.p, ctx->stream, &ctx->launches))
-    return fail(ctx, SVOB200_ERR_CUDA, "epipolar launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+  CU_AT("epipolar_match: launch_epipolar",
+        launch_epipolar(ctx->d_table, cur->slot, to_cam(cam), n, st.dev<svob200_feature_ref>(i_f), st.dev<double>(i_d), *opts,
+                        st.dev<svob200_epi_result>(i_r), ctx->d_scratch.p, ctx->stream, &ctx->launches));
   return st.download();
 }
 
@@ -444,8 +435,7 @@ int svob200_seeds_update(svob200_ctx* ctx, int64_t cur_frame_id, const svob200_c
                          svob200_seed* seeds, svob200_seed_obs* obs, int mem)
 {
   if (!ctx || !cam || n < 0 || !ftrs || !T_ref_w || !T_cur_w || !opts || !seeds || !obs) return fail(ctx, SVOB200_ERR_ARG, "seeds_update: bad arguments");
-  FrameRec* cur = find_frame(ctx, cur_frame_id);
-  if (!cur) return fail(ctx, SVOB200_ERR_NOFRAME, "seeds_update: current frame not resident");
+  FrameRec* cur = resident_frame(ctx, cur_frame_id, "seeds_update"); if (!cur) return SVOB200_ERR_NOFRAME;
   if (opts->max_search_level >= cur->f.n_levels) return fail(ctx, SVOB200_ERR_ARG, "seeds_update: max_search_level outside the pyramid");
   if (opts->max_epi_search_steps < 0) return fail(ctx, SVOB200_ERR_ARG, "seeds_update: negative max_epi_search_steps");
   if (n == 0) return SVOB200_OK;
@@ -456,14 +446,13 @@ int svob200_seeds_update(svob200_ctx* ctx, int64_t cur_frame_id, const svob200_c
   const int i_s = st.add(seeds, seeds, sizeof(svob200_seed) * n, 1);
   const int i_o = st.add(nullptr, obs, sizeof(svob200_seed_obs) * n, 2);
   if (int e = st.layout()) return e;
-  st.upload();
   if (mem == SVOB200_MEM_HOST) if (int e = resolve_slots(ctx, st.host<svob200_feature_ref>(i_f), n)) return e;
   if (int e = st.push()) return e;
   if (ctx->d_scratch.ensure(seeds_scratch_bytes(n)) != cudaSuccess) return fail(ctx, SVOB200_ERR_NOMEM, "seeds_update: scratch alloc failed");
-  if (launch_seeds_update(ctx->d_table, cur->slot, to_cam(cam), n, st.dev<svob200_feature_ref>(i_f), st.dev<double>(i_tr),
-                          st.dev<double>(i_tc), *opts, conv_thresh, st.dev<svob200_seed>(i_s), st.dev<svob200_seed_obs>(i_o),
-                          ctx->d_scratch.p, n, 0, ctx->stream, &ctx->launches))
-    return fail(ctx, SVOB200_ERR_CUDA, "seeds_update launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+  CU_AT("seeds_update: launch_seeds_update",
+        launch_seeds_update(ctx->d_table, cur->slot, to_cam(cam), n, st.dev<svob200_feature_ref>(i_f), st.dev<double>(i_tr),
+                            st.dev<double>(i_tc), *opts, conv_thresh, st.dev<svob200_seed>(i_s), st.dev<svob200_seed_obs>(i_o),
+                            ctx->d_scratch.p, n, 0, ctx->stream, &ctx->launches));
   return st.download();
 }
 
@@ -476,10 +465,9 @@ int svob200_update_seed(svob200_ctx* ctx, int n, const float* x, const float* ta
   const int i_t = st.add(tau2, nullptr, sizeof(float) * n, 0);
   const int i_s = st.add(seeds, seeds, sizeof(svob200_seed) * n, 1);
   if (int e = st.layout()) return e;
-  st.upload();
   if (int e = st.push()) return e;
-  if (launch_update_seed(n, st.dev<float>(i_x), st.dev<float>(i_t), st.dev<svob200_seed>(i_s), ctx->stream, &ctx->launches))
-    return fail(ctx, SVOB200_ERR_CUDA, "update_seed launch failed");
+  CU_AT("update_seed: launch_update_seed",
+        launch_update_seed(n, st.dev<float>(i_x), st.dev<float>(i_t), st.dev<svob200_seed>(i_s), ctx->stream, &ctx->launches));
   return st.download();
 }
 
@@ -495,11 +483,10 @@ int svob200_debug_chi2_chain(svob200_ctx* ctx, int block, int n_features, const 
   const int i_s = st.add(nullptr, sums, sizeof(float) * 4, 2);
   const int i_n = st.add(nullptr, counts, sizeof(int) * 4, 2);
   if (int e = st.layout()) return e;
-  st.upload();
   if (int e = st.push()) return e;
-  if (launch_chi2_chain_test(block, st.dev<float>(i_r), st.dev<uint8_t>(i_v), st.dev<uint8_t>(i_c), n_features, st.dev<float>(i_s), st.dev<int>(i_n),
-                             ctx->stream, &ctx->launches))
-    return fail(ctx, SVOB200_ERR_CUDA, "debug_chi2_chain launch failed");
+  CU_AT("debug_chi2_chain: launch_chi2_chain_test",
+        launch_chi2_chain_test(block, st.dev<float>(i_r), st.dev<uint8_t>(i_v), st.dev<uint8_t>(i_c), n_features, st.dev<float>(i_s), st.dev<int>(i_n),
+                               ctx->stream, &ctx->launches));
   return st.download();
 }
 
@@ -513,10 +500,9 @@ int svob200_compute_tau(svob200_ctx* ctx, int n, const double* T_ref_cur, const 
   const int i_z = st.add(z, nullptr, sizeof(double) * n, 0);
   const int i_o = st.add(nullptr, tau_out, sizeof(double) * n, 2);
   if (int e = st.layout()) return e;
-  st.upload();
   if (int e = st.push()) return e;
-  if (launch_compute_tau(n, st.dev<double>(i_T), st.dev<double>(i_f), st.dev<double>(i_z), px_error_angle, st.dev<double>(i_o), ctx->stream, &ctx->launches))
-    return fail(ctx, SVOB200_ERR_CUDA, "compute_tau launch failed");
+  CU_AT("compute_tau: launch_compute_tau",
+        launch_compute_tau(n, st.dev<double>(i_T), st.dev<double>(i_f), st.dev<double>(i_z), px_error_angle, st.dev<double>(i_o), ctx->stream, &ctx->launches));
   return st.download();
 }
 
@@ -534,11 +520,10 @@ int svob200_features_prepare(svob200_ctx* ctx, const svob200_camera* cam, int n,
   const int i_f = f_out ? st.add(nullptr, f_out, sizeof(double) * 3 * n, 2) : -1;
   const int i_x = st.add(nullptr, xyz_ref_out, sizeof(double) * 3 * n, 2);
   if (int e = st.layout()) return e;
-  st.upload();
   if (int e = st.push()) return e;
-  if (launch_features_prepare(to_cam(cam), n, st.dev<double>(i_px), st.dev<double>(i_pt), st.dev<int>(i_im), st.dev<double>(i_T),
-                              f_out ? st.dev<double>(i_f) : nullptr, st.dev<double>(i_x), ctx->stream, &ctx->launches))
-    return fail(ctx, SVOB200_ERR_CUDA, "features_prepare launch failed");
+  CU_AT("features_prepare: launch_features_prepare",
+        launch_features_prepare(to_cam(cam), n, st.dev<double>(i_px), st.dev<double>(i_pt), st.dev<int>(i_im), st.dev<double>(i_T),
+                                f_out ? st.dev<double>(i_f) : nullptr, st.dev<double>(i_x), ctx->stream, &ctx->launches));
   return st.download();
 }
 
@@ -550,10 +535,9 @@ int svob200_compose_poses(svob200_ctx* ctx, int batch, const svob200_align_resul
   const int i_T = st.add(T_ref_w, nullptr, sizeof(double) * 7 * batch, 0);
   const int i_o = st.add(nullptr, T_cur_w, sizeof(double) * 7 * batch, 2);
   if (int e = st.layout()) return e;
-  st.upload();
   if (int e = st.push()) return e;
-  if (launch_compose_poses(batch, st.dev<svob200_align_result>(i_r), st.dev<double>(i_T), st.dev<double>(i_o), ctx->stream, &ctx->launches))
-    return fail(ctx, SVOB200_ERR_CUDA, "compose_poses launch failed");
+  CU_AT("compose_poses: launch_compose_poses",
+        launch_compose_poses(batch, st.dev<svob200_align_result>(i_r), st.dev<double>(i_T), st.dev<double>(i_o), ctx->stream, &ctx->launches));
   return st.download();
 }
 
@@ -571,11 +555,10 @@ int svob200_reproject_prepare(svob200_ctx* ctx, const svob200_camera* cam, int n
   const int i_d = st.add(nullptr, depth_ref_out, sizeof(double) * n, 2);
   const int i_p = st.add(nullptr, px_cur_out, sizeof(double) * 2 * n, 2);
   if (int e = st.layout()) return e;
-  st.upload();
   if (int e = st.push()) return e;
-  if (launch_reproject_prepare(to_cam(cam), n, st.dev<svob200_feature_ref>(i_f), st.dev<double>(i_pt), st.dev<double>(i_Tk), st.dev<double>(i_Tc),
-                               st.dev<double>(i_d), st.dev<double>(i_p), ctx->stream, &ctx->launches))
-    return fail(ctx, SVOB200_ERR_CUDA, "reproject_prepare launch failed");
+  CU_AT("reproject_prepare: launch_reproject_prepare",
+        launch_reproject_prepare(to_cam(cam), n, st.dev<svob200_feature_ref>(i_f), st.dev<double>(i_pt), st.dev<double>(i_Tk), st.dev<double>(i_Tc),
+                                 st.dev<double>(i_d), st.dev<double>(i_p), ctx->stream, &ctx->launches));
   return st.download();
 }
 
@@ -584,8 +567,7 @@ int svob200_reproject_prepare(svob200_ctx* ctx, const svob200_camera* cam, int n
 int svob200_frame_upload_level(svob200_ctx* ctx, int64_t frame_id, int image, int level, const uint8_t* data, int stride)
 {
   if (!ctx || !data) return fail(ctx, SVOB200_ERR_ARG, "frame_upload_level: null argument");
-  FrameRec* r = find_frame(ctx, frame_id);
-  if (!r) return fail(ctx, SVOB200_ERR_NOFRAME, "frame %lld not found", (long long)frame_id);
+  FrameRec* r = resident_frame(ctx, frame_id, "frame_upload_level"); if (!r) return SVOB200_ERR_NOFRAME;
   if (level < 0 || level >= r->f.n_levels || image < 0 || image >= r->f.batch || stride < r->f.w[level]) return fail(ctx, SVOB200_ERR_ARG, "frame_upload_level: bad level/image/stride");
   if (level == 0) if (int e = frame_own_level0(ctx, r)) return e;
   CU(cudaMemcpy2DAsync(r->f.lvl[level] + (size_t)image * r->f.img_stride[level], r->f.pitch[level], data, stride, r->f.w[level], r->f.h[level],
@@ -607,7 +589,7 @@ int svob200_shi_tomasi(svob200_ctx* ctx, const uint8_t* img, int w, int h, int s
   float* d_out = reinterpret_cast<float*>(d_img + img_b + uv_b);
   CU(cudaMemcpy2DAsync(d_img, pitch, img, stride, w, h, cudaMemcpyHostToDevice, ctx->stream));
   CU(cudaMemcpyAsync(d_uv, uv, (size_t)n * 8, cudaMemcpyHostToDevice, ctx->stream));
-  if (launch_shi_tomasi_points(d_img, pitch, w, h, n, d_uv, d_out, ctx->stream, &ctx->launches)) return fail(ctx, SVOB200_ERR_CUDA, "shi_tomasi launch failed");
+  CU_AT("shi_tomasi: launch_shi_tomasi_points", launch_shi_tomasi_points(d_img, pitch, w, h, n, d_uv, d_out, ctx->stream, &ctx->launches));
   CU(cudaMemcpyAsync(scores, d_out, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
   CU(cudaStreamSynchronize(ctx->stream));
   return SVOB200_OK;
@@ -627,11 +609,10 @@ int svob200_warp_matrix_affine(svob200_ctx* ctx, const svob200_camera* cam, int 
   const int i_l = st.add(level_ref, nullptr, sizeof(int) * n, 0);
   const int i_A = st.add(nullptr, A_out, sizeof(double) * 4 * n, 2);
   if (int e = st.layout()) return e;
-  st.upload();
   if (int e = st.push()) return e;
-  if (launch_warp_matrix(to_cam(cam), n, st.dev<double>(i_px), st.dev<double>(i_f), st.dev<double>(i_d), st.dev<double>(i_T), st.dev<int>(i_l),
-                         st.dev<double>(i_A), ctx->stream, &ctx->launches))
-    return fail(ctx, SVOB200_ERR_CUDA, "warp_matrix_affine launch failed");
+  CU_AT("warp_matrix_affine: launch_warp_matrix",
+        launch_warp_matrix(to_cam(cam), n, st.dev<double>(i_px), st.dev<double>(i_f), st.dev<double>(i_d), st.dev<double>(i_T), st.dev<int>(i_l),
+                           st.dev<double>(i_A), ctx->stream, &ctx->launches));
   return st.download();
 }
 
@@ -650,8 +631,8 @@ int svob200_warp_affine(svob200_ctx* ctx, const uint8_t* img, int w, int h, int 
   uint8_t* d_patch = d_img + img_b;
   CU(cudaMemcpy2DAsync(d_img, pitch, img, stride, w, h, cudaMemcpyHostToDevice, ctx->stream));
   CU(cudaMemcpyAsync(d_patch, patch, np, cudaMemcpyHostToDevice, ctx->stream));
-  if (launch_warp_affine(d_img, pitch, w, h, A_cur_ref, px_ref, level_ref, search_level, halfpatch_size, d_patch, ctx->stream, &ctx->launches))
-    return fail(ctx, SVOB200_ERR_CUDA, "warp_affine launch failed");
+  CU_AT("warp_affine: launch_warp_affine",
+        launch_warp_affine(d_img, pitch, w, h, A_cur_ref, px_ref, level_ref, search_level, halfpatch_size, d_patch, ctx->stream, &ctx->launches));
   CU(cudaMemcpyAsync(patch, d_patch, np, cudaMemcpyDeviceToHost, ctx->stream));
   CU(cudaStreamSynchronize(ctx->stream));
   return SVOB200_OK;
@@ -670,10 +651,9 @@ int svob200_depth_from_triangulation(svob200_ctx* ctx, int n, const double* T_se
   const int i_d = st.add(depth, depth, sizeof(double) * n, 1);
   const int i_o = st.add(nullptr, ok, sizeof(int) * n, 2);
   if (int e = st.layout()) return e;
-  st.upload();
   if (int e = st.push()) return e;
-  if (launch_triangulate(n, st.dev<double>(i_T), st.dev<double>(i_a), st.dev<double>(i_b), st.dev<double>(i_d), st.dev<int>(i_o), ctx->stream, &ctx->launches))
-    return fail(ctx, SVOB200_ERR_CUDA, "depth_from_triangulation launch failed");
+  CU_AT("depth_from_triangulation: launch_triangulate",
+        launch_triangulate(n, st.dev<double>(i_T), st.dev<double>(i_a), st.dev<double>(i_b), st.dev<double>(i_d), st.dev<int>(i_o), ctx->stream, &ctx->launches));
   return st.download();
 }
 
@@ -682,8 +662,7 @@ int svob200_frame_upload_yuv420(svob200_ctx* ctx, int64_t frame_id, const uint8_
                                 int uv_stride, int uv_pixel_stride, size_t y_image_stride, size_t uv_image_stride, const int* round_modes, int mem)
 {
   if (!ctx || !y || !u || !v) return fail(ctx, SVOB200_ERR_ARG, "frame_upload_yuv420: null argument");
-  FrameRec* r = find_frame(ctx, frame_id);
-  if (!r) return fail(ctx, SVOB200_ERR_NOFRAME, "frame %lld not found", (long long)frame_id);
+  FrameRec* r = resident_frame(ctx, frame_id, "frame_upload_yuv420"); if (!r) return SVOB200_ERR_NOFRAME;
   const int w = r->f.w[0], h = r->f.h[0], B = r->f.batch;
   if (y_stride < w || uv_pixel_stride < 1 || uv_pixel_stride > 2) return fail(ctx, SVOB200_ERR_ARG, "frame_upload_yuv420: bad strides");
   const int cw = (w + 1) / 2, ch = (h + 1) / 2;
@@ -723,8 +702,7 @@ int svob200_frame_upload_yuv420(svob200_ctx* ctx, int64_t frame_id, const uint8_
   }
   int modes[SVOB200_MAX_LEVELS];
   pyramid_round_modes(r->f, round_modes, modes);
-  if (launch_pyramid_yuv(r->f, P, modes, ctx->stream, &ctx->launches))
-    return fail(ctx, SVOB200_ERR_CUDA, "yuv pyramid launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+  CU_AT("frame_upload_yuv420: launch_pyramid_yuv", launch_pyramid_yuv(r->f, P, modes, ctx->stream, &ctx->launches));
   if (mem == SVOB200_MEM_HOST) CU(cudaStreamSynchronize(ctx->stream));
   return SVOB200_OK;
 }
@@ -738,13 +716,12 @@ int svob200_reproject_map(svob200_ctx* ctx, int64_t cur_frame_id, const svob200_
   if (!ctx || !cam || batch <= 0 || !T_cur_w || !point_offsets || n_points < 0 || n_obs < 0 || !opts || !results || !cell_winner || !stats || cell_size <= 0)
     return fail(ctx, SVOB200_ERR_ARG, "reproject_map: bad arguments");
   if (n_points > 0 && (!points || !obs || !T_obs_w)) return fail(ctx, SVOB200_ERR_ARG, "reproject_map: null point / observation arrays");
-  FrameRec* cur = find_frame(ctx, cur_frame_id);
-  if (!cur) return fail(ctx, SVOB200_ERR_NOFRAME, "reproject_map: current frame not resident");
+  FrameRec* cur = resident_frame(ctx, cur_frame_id, "reproject_map"); if (!cur) return SVOB200_ERR_NOFRAME;
   if (batch != cur->f.batch) return fail(ctx, SVOB200_ERR_ARG, "reproject_map: batch differs from the frame's");
   if (opts->max_search_level >= cur->f.n_levels) return fail(ctx, SVOB200_ERR_ARG, "reproject_map: max_search_level outside the pyramid");
   if (opts->max_epi_search_steps < 0) return fail(ctx, SVOB200_ERR_ARG, "reproject_map: negative max_epi_search_steps");
-  const int gc = (cam->width + cell_size - 1) / cell_size, gr = (cam->height + cell_size - 1) / cell_size;
-  const size_t n_cells = (size_t)gc * gr;
+  const long long n_cells = grid_cells(cam->width, cam->height, cell_size);
+  if (n_cells > kMaxGridCells) return fail(ctx, SVOB200_ERR_UNSUPPORTED, "reproject_map: grid of %lld cells exceeds the limit of %d", n_cells, kMaxGridCells);
   Stage st(ctx, mem);
   const int i_T = st.add(T_cur_w, nullptr, sizeof(double) * 7 * batch, 0);
   const int i_off = st.add(point_offsets, nullptr, sizeof(int) * (batch + 1), 0);
@@ -752,20 +729,18 @@ int svob200_reproject_map(svob200_ctx* ctx, int64_t cur_frame_id, const svob200_
   const int i_o = st.add(obs, nullptr, sizeof(svob200_feature_ref) * n_obs, 0);
   const int i_To = st.add(T_obs_w, nullptr, sizeof(double) * 7 * n_obs, 0);
   const int i_r = st.add(nullptr, results, sizeof(svob200_reproj_result) * n_points, 2);
-  const int i_w = st.add(nullptr, cell_winner, sizeof(int) * n_cells * batch, 2);
+  const int i_w = st.add(nullptr, cell_winner, sizeof(int) * (size_t)n_cells * batch, 2);
   const int i_s = st.add(nullptr, stats, sizeof(svob200_reproj_stats) * batch, 2);
   if (int e = st.layout()) return e;
-  st.upload();
   if (mem == SVOB200_MEM_HOST && n_obs > 0) if (int e = resolve_slots(ctx, st.host<svob200_feature_ref>(i_o), n_obs)) return e;
   if (int e = st.push()) return e;
   if (ctx->d_scratch.ensure(match_scratch_bytes(n_points)) != cudaSuccess || ctx->d_scratch2.ensure(reproject_scratch_bytes(n_points)) != cudaSuccess)
     return fail(ctx, SVOB200_ERR_NOMEM, "reproject_map: scratch alloc failed");
-  const int rc = launch_reproject_map(ctx->d_table, cur->slot, to_cam(cam), batch, st.dev<double>(i_T), st.dev<int>(i_off), n_points,
-                                      st.dev<svob200_map_point>(i_p), st.dev<svob200_feature_ref>(i_o), st.dev<double>(i_To), cell_size, max_fts,
-                                      *opts, st.dev<svob200_reproj_result>(i_r), st.dev<int>(i_w), st.dev<svob200_reproj_stats>(i_s),
-                                      ctx->d_scratch2.p, ctx->d_scratch.p, nullptr, nullptr, nullptr, nullptr, nullptr, ctx->stream, &ctx->launches);
-  if (rc == -2) return fail(ctx, SVOB200_ERR_UNSUPPORTED, "reproject_map: grid of %zu cells exceeds the kernel's table (8192)", n_cells);
-  if (rc) return fail(ctx, SVOB200_ERR_CUDA, "reproject_map launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+  CU_AT("reproject_map: launch_reproject_map",
+        launch_reproject_map(ctx->d_table, cur->slot, to_cam(cam), batch, st.dev<double>(i_T), st.dev<int>(i_off), n_points,
+                             st.dev<svob200_map_point>(i_p), st.dev<svob200_feature_ref>(i_o), st.dev<double>(i_To), cell_size, max_fts,
+                             *opts, st.dev<svob200_reproj_result>(i_r), st.dev<int>(i_w), st.dev<svob200_reproj_stats>(i_s),
+                             ctx->d_scratch2.p, ctx->d_scratch.p, nullptr, nullptr, nullptr, nullptr, nullptr, ctx->stream, &ctx->launches));
   return st.download();
 }
 
@@ -784,8 +759,7 @@ int svob200_pose_optimize(svob200_ctx* ctx, const svob200_camera* cam, int batch
 {
   if (!ctx || !cam || batch <= 0 || !ftr_offsets || !opts || !T_f_w || !results) return fail(ctx, SVOB200_ERR_ARG, "pose_optimize: bad arguments");
   int n = 0;
-  if (mem == SVOB200_MEM_HOST) n = ftr_offsets[batch];
-  else { CU(cudaMemcpyAsync(&n, ftr_offsets + batch, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream)); CU(cudaStreamSynchronize(ctx->stream)); }
+  if (int e = offsets_extent(ctx, ftr_offsets, batch, mem, &n)) return e;
   if (n < 0 || (n > 0 && (!f || !level || !pos || !outlier))) return fail(ctx, SVOB200_ERR_ARG, "pose_optimize: null feature arrays");
   Stage st(ctx, mem);
   const int i_off = st.add(ftr_offsets, nullptr, sizeof(int) * (batch + 1), 0);
@@ -796,14 +770,13 @@ int svob200_pose_optimize(svob200_ctx* ctx, const svob200_camera* cam, int batch
   const int i_r = st.add(nullptr, results, sizeof(svob200_pose_opt_result) * batch, 2);
   const int i_o = st.add(nullptr, outlier, (size_t)n, 2);
   if (int e = st.layout()) return e;
-  st.upload();
   if (int e = st.push()) return e;
   if (ctx->d_scratch.ensure(sizeof(double) * (size_t)(n > 0 ? n : 1)) != cudaSuccess) return fail(ctx, SVOB200_ERR_NOMEM, "pose_optimize: scratch alloc failed");
   const int* d_off = st.dev<int>(i_off);
-  if (launch_pose_optimize(to_cam(cam), batch, d_off, d_off + 1, st.dev<double>(i_f), st.dev<int>(i_l), st.dev<double>(i_p), opts->reproj_thresh,
-                           opts->n_iter, opts->eps, opts->tukey_b, st.dev<double>(i_T), st.dev<svob200_pose_opt_result>(i_r), st.dev<uint8_t>(i_o),
-                           static_cast<double*>(ctx->d_scratch.p), ctx->stream, &ctx->launches))
-    return fail(ctx, SVOB200_ERR_CUDA, "pose_optimize launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+  CU_AT("pose_optimize: launch_pose_optimize",
+        launch_pose_optimize(to_cam(cam), batch, d_off, d_off + 1, st.dev<double>(i_f), st.dev<int>(i_l), st.dev<double>(i_p), opts->reproj_thresh,
+                             opts->n_iter, opts->eps, opts->tukey_b, st.dev<double>(i_T), st.dev<svob200_pose_opt_result>(i_r), st.dev<uint8_t>(i_o),
+                             static_cast<double*>(ctx->d_scratch.p), ctx->stream, &ctx->launches));
   return st.download();
 }
 
@@ -813,8 +786,7 @@ int svob200_points_optimize(svob200_ctx* ctx, int n, const int* obs_offsets, con
   if (!ctx || n < 0 || !obs_offsets || !pos) return fail(ctx, SVOB200_ERR_ARG, "points_optimize: bad arguments");
   if (n == 0) return SVOB200_OK;
   int m = 0;
-  if (mem == SVOB200_MEM_HOST) m = obs_offsets[n];
-  else { CU(cudaMemcpyAsync(&m, obs_offsets + n, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream)); CU(cudaStreamSynchronize(ctx->stream)); }
+  if (int e = offsets_extent(ctx, obs_offsets, n, mem, &m)) return e;
   if (m < 0 || (m > 0 && (!T_f_w || !f))) return fail(ctx, SVOB200_ERR_ARG, "points_optimize: null observation arrays");
   Stage st(ctx, mem);
   const int i_off = st.add(obs_offsets, nullptr, sizeof(int) * (n + 1), 0);
@@ -823,11 +795,10 @@ int svob200_points_optimize(svob200_ctx* ctx, int n, const int* obs_offsets, con
   const int i_p = st.add(pos, pos, sizeof(double) * 3 * n, 1);
   const int i_it = iters_out ? st.add(nullptr, iters_out, sizeof(int) * n, 2) : -1;
   if (int e = st.layout()) return e;
-  st.upload();
   if (int e = st.push()) return e;
-  if (launch_points_optimize(n, st.dev<int>(i_off), st.dev<double>(i_T), st.dev<double>(i_f), n_iter, eps, st.dev<double>(i_p),
-                             iters_out ? st.dev<int>(i_it) : nullptr, ctx->stream, &ctx->launches))
-    return fail(ctx, SVOB200_ERR_CUDA, "points_optimize launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+  CU_AT("points_optimize: launch_points_optimize",
+        launch_points_optimize(n, st.dev<int>(i_off), st.dev<double>(i_T), st.dev<double>(i_f), n_iter, eps, st.dev<double>(i_p),
+                               iters_out ? st.dev<int>(i_it) : nullptr, ctx->stream, &ctx->launches));
   return st.download();
 }
 
@@ -838,16 +809,14 @@ int svob200_seeds_initialize(svob200_ctx* ctx, int64_t frame_id, int n_detect_le
 {
   if (!ctx || cell_size <= 0 || !existing_offsets || !depth_mean || !depth_min || !corners_out || !seeds_out || !counts)
     return fail(ctx, SVOB200_ERR_ARG, "seeds_initialize: bad arguments");
-  FrameRec* r = find_frame(ctx, frame_id);
-  if (!r) return fail(ctx, SVOB200_ERR_NOFRAME, "frame %lld not found", (long long)frame_id);
+  FrameRec* r = resident_frame(ctx, frame_id, "seeds_initialize"); if (!r) return SVOB200_ERR_NOFRAME;
   if (n_detect_levels < 1 || n_detect_levels > r->f.n_levels) return fail(ctx, SVOB200_ERR_ARG, "seeds_initialize: n_detect_levels out of range");
   if (r->f.w[0] >= 16384 || r->f.h[0] >= 16384) return fail(ctx, SVOB200_ERR_UNSUPPORTED, "seeds_initialize: image larger than 16383");
   const int B = r->f.batch;
   const int gc = (r->f.w[0] + cell_size - 1) / cell_size, gr = (r->f.h[0] + cell_size - 1) / cell_size;
   const size_t n_cells = (size_t)gc * gr, total = n_cells * B;
   int n = 0, max_per = 0;
-  if (mem == SVOB200_MEM_HOST) { n = existing_offsets[B]; for (int b = 0; b < B; ++b) max_per = std::max(max_per, existing_offsets[b + 1] - existing_offsets[b]); }
-  else { CU(cudaMemcpyAsync(&n, existing_offsets + B, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream)); CU(cudaStreamSynchronize(ctx->stream)); max_per = n; }
+  if (int e = offsets_extent(ctx, existing_offsets, B, mem, &n, &max_per)) return e;
   if (n < 0 || (n > 0 && !existing_px)) return fail(ctx, SVOB200_ERR_ARG, "seeds_initialize: null existing_px");
   Stage st(ctx, mem);
   const int i_off = st.add(existing_offsets, nullptr, sizeof(int) * (B + 1), 0);
@@ -858,7 +827,6 @@ int svob200_seeds_initialize(svob200_ctx* ctx, int64_t frame_id, int n_detect_le
   const int i_s = st.add(nullptr, seeds_out, sizeof(svob200_seed) * total, 2);
   const int i_n = st.add(nullptr, counts, sizeof(int) * B, 2);
   if (int e = st.layout()) return e;
-  st.upload();
   if (int e = st.push()) return e;
   // scratch: cell keys (8 B) | cell records | occupancy | detector counts
   const size_t need = total * 8 + total * sizeof(svob200_corner) + ((total + 255) & ~(size_t)255) + sizeof(int) * B + 1024;
@@ -868,11 +836,13 @@ int svob200_seeds_initialize(svob200_ctx* ctx, int64_t frame_id, int n_detect_le
   uint8_t* d_occ = reinterpret_cast<uint8_t*>(d_cells + total);
   int* d_cnt = reinterpret_cast<int*>(d_occ + ((total + 255) & ~(size_t)255));
   CU(cudaMemsetAsync(d_occ, 0, total, ctx->stream));
-  if (launch_occupancy(B, max_per, st.dev<int>(i_off), st.dev<double>(i_px), cell_size, gc, (int)n_cells, d_occ, ctx->stream, &ctx->launches) ||
-      launch_fast_detect(r->f, n_detect_levels, cell_size, gc, gr, thr, d_occ, d_keys, d_cells, d_cnt, ctx->stream, &ctx->launches) ||
-      launch_seeds_compact(B, d_cells, (int)n_cells, thr, st.dev<float>(i_dm), st.dev<float>(i_dn), st.dev<svob200_corner>(i_c),
-                           st.dev<svob200_seed>(i_s), st.dev<int>(i_n), ctx->stream, &ctx->launches))
-    return fail(ctx, SVOB200_ERR_CUDA, "seeds_initialize launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+  CU_AT("seeds_initialize: launch_occupancy",
+        launch_occupancy(B, max_per, st.dev<int>(i_off), st.dev<double>(i_px), cell_size, gc, (int)n_cells, d_occ, ctx->stream, &ctx->launches));
+  CU_AT("seeds_initialize: launch_fast_detect",
+        launch_fast_detect(r->f, n_detect_levels, cell_size, gc, gr, thr, d_occ, d_keys, d_cells, d_cnt, ctx->stream, &ctx->launches));
+  CU_AT("seeds_initialize: launch_seeds_compact",
+        launch_seeds_compact(B, d_cells, (int)n_cells, thr, st.dev<float>(i_dm), st.dev<float>(i_dn), st.dev<svob200_corner>(i_c),
+                             st.dev<svob200_seed>(i_s), st.dev<int>(i_n), ctx->stream, &ctx->launches));
   return st.download();
 }
 
@@ -921,9 +891,9 @@ int svob200_synth_render(svob200_ctx* ctx, const uint8_t* dev_texture, int tex_s
   if (ctx->d_scratch2.ensure(rc.size() * sizeof(double)) != cudaSuccess) return fail(ctx, SVOB200_ERR_NOMEM, "synth_render: scratch alloc failed");
   CU(cudaMemcpyAsync(ctx->d_scratch2.p, rc.data(), rc.size() * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
   CU(cudaStreamSynchronize(ctx->stream));
-  if (launch_synth_render(dev_texture, tex_size, ppm, plane_z, to_cam(cam), batch, static_cast<const double*>(ctx->d_scratch2.p), dev_out,
-                          ctx->stream, &ctx->launches))
-    return fail(ctx, SVOB200_ERR_CUDA, "synth_render launch failed");
+  CU_AT("synth_render: launch_synth_render",
+        launch_synth_render(dev_texture, tex_size, ppm, plane_z, to_cam(cam), batch, static_cast<const double*>(ctx->d_scratch2.p), dev_out,
+                            ctx->stream, &ctx->launches));
   return SVOB200_OK;
 }
 

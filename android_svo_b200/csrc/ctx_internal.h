@@ -65,7 +65,9 @@ inline int fail(svob200_ctx* c, int code, const char* fmt, ...)
   if (c) c->err = buf;
   return code;
 }
-#define CU(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return fail(ctx, SVOB200_ERR_CUDA, "%s: %s", #call, cudaGetErrorString(e_)); } while (0)
+// a CUDA call, a launcher or cudaGetLastError() right after a raw launch: its error is reported as "<what>: <error string>"
+#define CU_AT(what, call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return fail(ctx, SVOB200_ERR_CUDA, "%s: %s", what, cudaGetErrorString(e_)); } while (0)
+#define CU(call) CU_AT(#call, call)
 
 // make ctx->stream wait for everything enqueued so far on the auxiliary streams
 inline int ctx_join_aux(svob200_ctx* ctx)
@@ -96,6 +98,13 @@ inline FrameRec* find_frame(svob200_ctx* ctx, int64_t id)
   auto it = ctx->frames.find(id);
   return it == ctx->frames.end() ? nullptr : &it->second;
 }
+// the frame an entry point (`who`) was given, or nullptr with SVOB200_ERR_NOFRAME reported
+inline FrameRec* resident_frame(svob200_ctx* ctx, int64_t id, const char* who)
+{
+  FrameRec* r = ctx ? find_frame(ctx, id) : nullptr;
+  if (!r) fail(ctx, SVOB200_ERR_NOFRAME, "%s: frame %lld is not resident", who, (long long)id);
+  return r;
+}
 
 inline int ensure_host_stage(svob200_ctx* ctx, size_t n)
 {
@@ -118,11 +127,12 @@ struct Stage {
   size_t total = 0, in_end = 0, io_begin = 0;
   bool pushed = false, drained = false;
   Stage(svob200_ctx* c, int m) : ctx(c), mem(m) {}
-  // a call that fails between push() and download() must not leave its host->device copy in flight: the next call's upload()
+  // a call that fails between push() and download() must not leave its host->device copy in flight: the next call's layout()
   // writes the same pinned staging buffer
   ~Stage() { if (pushed && !drained) cudaStreamSynchronize(ctx->stream); }
-  // returns an index; resolve() gives the device pointer
+  // returns an index; dev() gives the device pointer
   int add(const void* src, void* dst, size_t bytes, int kind) { items.push_back({src, dst, bytes, 0, kind}); return (int)items.size() - 1; }
+  // places the items and copies the host inputs into the pinned staging buffer (HOST mode); push() sends them
   int layout()
   {
     if (mem == SVOB200_MEM_DEVICE) return 0;
@@ -135,6 +145,7 @@ struct Stage {
     total = off;
     if (int r = ensure_host_stage(ctx, total)) return r;
     if (ctx->d_stage.ensure(total) != cudaSuccess) return fail(ctx, SVOB200_ERR_NOMEM, "device staging alloc of %zu bytes failed", total);
+    for (auto& it : items) if (it.kind <= 1 && it.src && it.bytes) memcpy(ctx->h_stage + it.off, it.src, it.bytes);
     return 0;
   }
   template <class T> T* dev(int idx)
@@ -144,12 +155,6 @@ struct Stage {
     return reinterpret_cast<T*>(static_cast<uint8_t*>(ctx->d_stage.p) + it.off);
   }
   template <class T> T* host(int idx) { return reinterpret_cast<T*>(ctx->h_stage + items[idx].off); }   // staged host copy (HOST mode)
-  int upload()
-  {
-    if (mem == SVOB200_MEM_DEVICE) return 0;
-    for (auto& it : items) if (it.kind <= 1 && it.src && it.bytes) memcpy(ctx->h_stage + it.off, it.src, it.bytes);
-    return 0;
-  }
   int push()
   {
     if (mem == SVOB200_MEM_DEVICE || in_end == 0) return 0;

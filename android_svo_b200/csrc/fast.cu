@@ -389,9 +389,9 @@ __global__ void shi_tomasi_points_kernel(const uint8_t* img, int pitch, int cols
 
 }  // namespace
 
-int launch_fast_detect(const DevFrame& f, int n_detect_levels, int cell, int grid_cols, int grid_rows, double thr,
-                       const uint8_t* d_occupancy, unsigned long long* d_keys, svob200_corner* d_cells, int* d_counts,
-                       cudaStream_t s, long long* launches, const int* d_image_sel)
+cudaError_t launch_fast_detect(const DevFrame& f, int n_detect_levels, int cell, int grid_cols, int grid_rows, double thr,
+                               const uint8_t* d_occupancy, unsigned long long* d_keys, svob200_corner* d_cells, int* d_counts,
+                               cudaStream_t s, long long* launches, const int* d_image_sel)
 {
   const int n_cells = grid_cols * grid_rows;
   const int total = n_cells * f.batch;
@@ -409,11 +409,11 @@ int launch_fast_detect(const DevFrame& f, int n_detect_levels, int cell, int gri
   fast_kernel<<<grid, NT, 0, s>>>(A);
   fast_finalize_kernel<<<f.batch, 256, 0, s>>>(d_keys, n_cells, thr_f, thr, d_cells, d_counts, d_image_sel);
   *launches += 3;
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+  return cudaGetLastError();
 }
 
-int launch_fast_raw(const DevFrame& f, int image, int level, int threshold, int nonmax, uint8_t* d_scores,
-                    cudaStream_t s, long long* launches)
+cudaError_t launch_fast_raw(const DevFrame& f, int image, int level, int threshold, int nonmax, uint8_t* d_scores,
+                            cudaStream_t s, long long* launches)
 {
   FastArgs A{};
   A.f = f; A.n_levels = 1; A.raw_scores = d_scores; A.raw_image = image; A.raw_level = level;
@@ -421,14 +421,14 @@ int launch_fast_raw(const DevFrame& f, int image, int level, int threshold, int 
   const int tiles = ((f.w[level] + TW - 1) / TW) * ((f.h[level] + TH - 1) / TH);
   fast_kernel<<<dim3(tiles, 1), NT, 0, s>>>(A);
   ++*launches;
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+  return cudaGetLastError();
 }
 
-int launch_shi_tomasi_points(const uint8_t* d_img, int pitch, int cols, int rows, int n, const int* d_uv, float* d_out,
-                             cudaStream_t s, long long* launches)
+cudaError_t launch_shi_tomasi_points(const uint8_t* d_img, int pitch, int cols, int rows, int n, const int* d_uv, float* d_out,
+                                     cudaStream_t s, long long* launches)
 {
-  if (n <= 0) return 0;
+  if (n <= 0) return cudaSuccess;
   shi_tomasi_points_kernel<<<(n + 127) / 128, 128, 0, s>>>(d_img, pitch, cols, rows, n, d_uv, d_out);
   ++*launches;
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+  return cudaGetLastError();
 }

@@ -65,29 +65,29 @@ __global__ void reproject_prepare_kernel(DevCam cam, int n, svob200_feature_ref*
 
 }  // namespace
 
-int launch_features_prepare(const DevCam& cam, int n, const double* d_px, const double* d_pt, const int* d_image,
-                            const double* d_T_ref_w, double* d_f, double* d_xyz, cudaStream_t s, long long* launches)
+cudaError_t launch_features_prepare(const DevCam& cam, int n, const double* d_px, const double* d_pt, const int* d_image,
+                                    const double* d_T_ref_w, double* d_f, double* d_xyz, cudaStream_t s, long long* launches)
 {
-  if (n <= 0) return 0;
+  if (n <= 0) return cudaSuccess;
   features_prepare_kernel<<<(n + 127) / 128, 128, 0, s>>>(cam, n, d_px, d_pt, d_image, d_T_ref_w, d_f, d_xyz);
   ++*launches;
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+  return cudaGetLastError();
 }
 
-int launch_compose_poses(int batch, const svob200_align_result* d_res, const double* d_T_ref_w, double* d_T_cur_w,
-                         cudaStream_t s, long long* launches)
+cudaError_t launch_compose_poses(int batch, const svob200_align_result* d_res, const double* d_T_ref_w, double* d_T_cur_w,
+                                 cudaStream_t s, long long* launches)
 {
-  if (batch <= 0) return 0;
+  if (batch <= 0) return cudaSuccess;
   compose_poses_kernel<<<(batch + 127) / 128, 128, 0, s>>>(batch, d_res, d_T_ref_w, d_T_cur_w);
   ++*launches;
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+  return cudaGetLastError();
 }
 
-int launch_reproject_prepare(const DevCam& cam, int n, svob200_feature_ref* d_ftrs, const double* d_pt, const double* d_T_kf_w,
-                             const double* d_T_cur_w, double* d_depth_ref, double* d_px_cur, cudaStream_t s, long long* launches)
+cudaError_t launch_reproject_prepare(const DevCam& cam, int n, svob200_feature_ref* d_ftrs, const double* d_pt, const double* d_T_kf_w,
+                                     const double* d_T_cur_w, double* d_depth_ref, double* d_px_cur, cudaStream_t s, long long* launches)
 {
-  if (n <= 0) return 0;
+  if (n <= 0) return cudaSuccess;
   reproject_prepare_kernel<<<(n + 127) / 128, 128, 0, s>>>(cam, n, d_ftrs, d_pt, d_T_kf_w, d_T_cur_w, d_depth_ref, d_px_cur);
   ++*launches;
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+  return cudaGetLastError();
 }

@@ -84,7 +84,6 @@ __global__ void __launch_bounds__(128) reproj_select_kernel(DevCam cam, const do
 
 // ---------------------------------------------------------------- reprojector, phase 2: per image, the sequential rules
 constexpr int REPROJ_T = 256;
-constexpr int REPROJ_MAX_CELLS = 8192;       // 32 KB of keys in shared memory (1080p at cell 20 has 5,184)
 
 __global__ void __launch_bounds__(REPROJ_T) reproj_cells_kernel(DevCam cam, const int* pt_off, const svob200_map_point* pts, const uint8_t* active,
                                                                 const int* ok, const double* px_refined, const int* level, const double* A,
@@ -93,7 +92,7 @@ __global__ void __launch_bounds__(REPROJ_T) reproj_cells_kernel(DevCam cam, cons
                                                                 // optional compacted matches of image b at [b * n_cells, ...) in cell order
                                                                 double* m_f, int* m_level, double* m_pos, int* m_point, int* m_count)
 {
-  __shared__ uint32_t s_best[REPROJ_MAX_CELLS];
+  __shared__ uint32_t s_best[kMaxGridCells];        // 32 KB of keys (1080p at cell 20 has 5,184 cells)
   __shared__ int s_cnt[4];
   const int b = blockIdx.x, tid = threadIdx.x;
   const int p0 = pt_off[b], p1 = pt_off[b + 1];
@@ -439,25 +438,25 @@ inline size_t up256(size_t b) { return (b + 255) & ~(size_t)255; }
 
 }  // namespace
 
-int launch_occupancy(int batch, int max_per_image, const int* d_off, const double* d_px, int cell_size, int grid_cols, int n_cells, uint8_t* d_occ,
-                     cudaStream_t s, long long* launches)
+cudaError_t launch_occupancy(int batch, int max_per_image, const int* d_off, const double* d_px, int cell_size, int grid_cols, int n_cells, uint8_t* d_occ,
+                             cudaStream_t s, long long* launches)
 {
-  if (batch <= 0) return 0;
+  if (batch <= 0) return cudaSuccess;
   int bx = (max_per_image + 127) / 128;
   if (bx < 1) bx = 1;
   if (bx > 64) bx = 64;
   occupancy_kernel<<<dim3(bx, batch), 128, 0, s>>>(batch, d_off, d_px, cell_size, grid_cols, n_cells, d_occ);
   ++*launches;
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+  return cudaGetLastError();
 }
 
-int launch_seeds_compact(int batch, const svob200_corner* d_cells, int n_cells, double thr, const float* d_depth_mean, const float* d_depth_min,
-                         svob200_corner* d_corners_out, svob200_seed* d_seeds_out, int* d_counts, cudaStream_t s, long long* launches)
+cudaError_t launch_seeds_compact(int batch, const svob200_corner* d_cells, int n_cells, double thr, const float* d_depth_mean, const float* d_depth_min,
+                                 svob200_corner* d_corners_out, svob200_seed* d_seeds_out, int* d_counts, cudaStream_t s, long long* launches)
 {
-  if (batch <= 0) return 0;
+  if (batch <= 0) return cudaSuccess;
   seeds_compact_kernel<<<batch, 256, 0, s>>>(d_cells, n_cells, thr, d_depth_mean, d_depth_min, d_corners_out, d_seeds_out, d_counts);
   ++*launches;
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+  return cudaGetLastError();
 }
 
 // ---------------------------------------------------------------- launchers
@@ -468,20 +467,18 @@ size_t reproject_scratch_bytes(int n_points)
          + up256(m * 4 * sizeof(double)) + 256;
 }
 
-int launch_reproject_map(const DevFrame* d_frames, int cur_slot, const DevCam& cam, int batch, const double* d_T_cur_w, const int* d_pt_off,
-                         int n_points, const svob200_map_point* d_points, const svob200_feature_ref* d_obs, const double* d_T_obs_w,
-                         int cell_size, int max_fts, svob200_matcher_opts opts, svob200_reproj_result* d_results, int* d_cell_winner,
-                         svob200_reproj_stats* d_stats, void* d_scratch, void* d_match_scratch,
-                         double* d_m_f, int* d_m_level, double* d_m_pos, int* d_m_point, int* d_m_count,
-                         cudaStream_t s, long long* launches, int image_base, int point_base, int n_range)
+cudaError_t launch_reproject_map(const DevFrame* d_frames, int cur_slot, const DevCam& cam, int batch, const double* d_T_cur_w, const int* d_pt_off,
+                                 int n_points, const svob200_map_point* d_points, const svob200_feature_ref* d_obs, const double* d_T_obs_w,
+                                 int cell_size, int max_fts, svob200_matcher_opts opts, svob200_reproj_result* d_results, int* d_cell_winner,
+                                 svob200_reproj_stats* d_stats, void* d_scratch, void* d_match_scratch,
+                                 double* d_m_f, int* d_m_level, double* d_m_pos, int* d_m_point, int* d_m_count,
+                                 cudaStream_t s, long long* launches, int image_base, int point_base, int n_range)
 {
   // d_T_cur_w, d_pt_off, d_cell_winner, d_stats, d_m_* already point at image `image_base` (offsets in d_pt_off stay
   // ABSOLUTE indices into d_points / d_results); this call covers the points [point_base, point_base + n_range)
   if (n_range < 0) n_range = n_points - point_base;
-  if (batch <= 0) return 0;
-  const int cols = (cam.width + cell_size - 1) / cell_size, rows = (cam.height + cell_size - 1) / cell_size;
-  const int n_cells = cols * rows;
-  if (n_cells > REPROJ_MAX_CELLS) return -2;
+  if (batch <= 0) return cudaSuccess;
+  const int cols = (cam.width + cell_size - 1) / cell_size, n_cells = (int)grid_cells(cam.width, cam.height, cell_size);
   const size_t m = (size_t)(n_points > 0 ? n_points : 1);
   char* p = static_cast<char*>(d_scratch);
   svob200_feature_ref* ftr = reinterpret_cast<svob200_feature_ref*>(p); p += up256(m * sizeof(svob200_feature_ref));
@@ -494,34 +491,35 @@ int launch_reproject_map(const DevFrame* d_frames, int cur_slot, const DevCam& c
   double* A = reinterpret_cast<double*>(p);
   reproj_select_kernel<<<batch, 128, 0, s>>>(cam, d_T_cur_w, d_pt_off, d_points, d_obs, d_T_obs_w, cell_size, cols, image_base, ftr, depth, px_in, active, d_results);
   ++*launches;
+  if (cudaError_t e = cudaGetLastError()) return e;
   if (n_range > 0) {
     const size_t o = (size_t)point_base;
-    if (launch_match_direct(d_frames, cur_slot, cam, n_range, ftr + o, depth + o, px_in + 2 * o, opts, nullptr, px_out + 2 * o, ok + o, d_match_scratch,
-                            n_points, point_base, s, launches, nullptr, active + o, level + o, A + 4 * o))
-      return -1;
+    if (cudaError_t e = launch_match_direct(d_frames, cur_slot, cam, n_range, ftr + o, depth + o, px_in + 2 * o, opts, nullptr, px_out + 2 * o, ok + o,
+                                            d_match_scratch, n_points, point_base, s, launches, nullptr, active + o, level + o, A + 4 * o))
+      return e;
   }
   reproj_cells_kernel<<<batch, REPROJ_T, 0, s>>>(cam, d_pt_off, d_points, active, ok, px_out, level, A, n_cells, max_fts, d_results, d_cell_winner, d_stats,
                                                  d_m_f, d_m_level, d_m_pos, d_m_point, d_m_count);
   ++*launches;
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+  return cudaGetLastError();
 }
 
-int launch_pose_optimize(const DevCam& cam, int batch, const int* d_seg_begin, const int* d_seg_end, const double* d_f, const int* d_level,
-                         const double* d_pos, double reproj_thresh, int n_iter, double eps, float tukey_b, double* d_T_io,
-                         svob200_pose_opt_result* d_results, uint8_t* d_outlier, double* d_work, cudaStream_t s, long long* launches)
+cudaError_t launch_pose_optimize(const DevCam& cam, int batch, const int* d_seg_begin, const int* d_seg_end, const double* d_f, const int* d_level,
+                                 const double* d_pos, double reproj_thresh, int n_iter, double eps, float tukey_b, double* d_T_io,
+                                 svob200_pose_opt_result* d_results, uint8_t* d_outlier, double* d_work, cudaStream_t s, long long* launches)
 {
-  if (batch <= 0) return 0;
+  if (batch <= 0) return cudaSuccess;
   pose_optimize_kernel<<<batch, POSE_T, 0, s>>>(cam, d_seg_begin, d_seg_end, d_f, d_level, d_pos, reproj_thresh, n_iter, eps, tukey_b, d_T_io,
                                                d_results, d_outlier, d_work);
   ++*launches;
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+  return cudaGetLastError();
 }
 
-int launch_points_optimize(int n, const int* d_obs_off, const double* d_T_f_w, const double* d_f, int n_iter, double eps, double* d_pos_io,
-                           int* d_iters, cudaStream_t s, long long* launches)
+cudaError_t launch_points_optimize(int n, const int* d_obs_off, const double* d_T_f_w, const double* d_f, int n_iter, double eps, double* d_pos_io,
+                                   int* d_iters, cudaStream_t s, long long* launches)
 {
-  if (n <= 0) return 0;
+  if (n <= 0) return cudaSuccess;
   points_optimize_kernel<<<(n + 127) / 128, 128, 0, s>>>(n, d_obs_off, d_T_f_w, d_f, n_iter, eps, d_pos_io, d_iters);
   ++*launches;
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+  return cudaGetLastError();
 }

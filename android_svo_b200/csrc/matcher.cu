@@ -893,13 +893,13 @@ __global__ void __launch_bounds__(LK_T, LK_CTAS) lk_refine_kernel(const DevFrame
   }
 }
 
-int launch_lk_refine(const DevFrame* d_frames, int cur_slot, const LkJob* d_jobs, const int* d_count, int n_max, int n_iter, const LkSink& sink,
-                     cudaStream_t s, long long* launches)
+cudaError_t launch_lk_refine(const DevFrame* d_frames, int cur_slot, const LkJob* d_jobs, const int* d_count, int n_max, int n_iter, const LkSink& sink,
+                             cudaStream_t s, long long* launches)
 {
-  if (n_max <= 0) return 0;
+  if (n_max <= 0) return cudaSuccess;
   lk_refine_kernel<<<(n_max + LK_T - 1) / LK_T, LK_T, 0, s>>>(d_frames, cur_slot, d_jobs, d_count, n_max, n_iter, sink);
   ++*launches;
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+  return cudaGetLastError();
 }
 
 // ---------------------------------------------------------------- depth filter: DepthFilter::updateSeeds loop body
@@ -1368,18 +1368,18 @@ static inline size_t up256(size_t b) { return (b + 255) & ~(size_t)255; }
 
 size_t lk_jobs_bytes(int n) { return up256((size_t)(n > 0 ? n : 1) * sizeof(LkJob)) + 256; }
 
-int launch_align_patches(const DevFrame* d_frames, int slot, int level, int n, const int* d_image, const uint8_t* d_pwb, const uint8_t* d_patch,
-                         const float* d_dir, int n_iter, double* d_px, int* d_converged, double* d_h_inv, void* d_scratch,
-                         cudaStream_t s, long long* launches)
+cudaError_t launch_align_patches(const DevFrame* d_frames, int slot, int level, int n, const int* d_image, const uint8_t* d_pwb, const uint8_t* d_patch,
+                                 const float* d_dir, int n_iter, double* d_px, int* d_converged, double* d_h_inv, void* d_scratch,
+                                 cudaStream_t s, long long* launches)
 {
-  if (n <= 0) return 0;
+  if (n <= 0) return cudaSuccess;
   LkJob* jobs = static_cast<LkJob*>(d_scratch);
   align_jobs_kernel<<<(n + 127) / 128, 128, 0, s>>>(level, n, d_image, d_pwb, d_dir, d_px, jobs);
   ++*launches;
+  if (cudaError_t e = cudaGetLastError()) return e;
   LkSink sink{};
   sink.kind = LK_SINK_ARRAYS; sink.px_out = d_px; sink.ok_out = d_converged; sink.h_inv_out = d_h_inv; sink.patches = d_patch;
-  if (launch_lk_refine(d_frames, slot, jobs, nullptr, n, n_iter, sink, s, launches)) return -1;
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+  return launch_lk_refine(d_frames, slot, jobs, nullptr, n, n_iter, sink, s, launches);
 }
 
 size_t match_scratch_bytes(int n)
@@ -1392,12 +1392,12 @@ size_t match_scratch_bytes(int n)
 // results: full records (API) or nullptr; px_out / ok_out: compact outputs (tracker) or nullptr.
 // The scratch was sized for scratch_total candidates; this call covers [first, first + n) of it (all other
 // pointers already point at candidate `first`).  marks: optional 2 events recorded between the three kernels.
-int launch_match_direct(const DevFrame* d_frames, int cur_slot, const DevCam& cam, int n, const svob200_feature_ref* d_ftrs,
-                        const double* d_depth_ref, const double* d_px_in, svob200_matcher_opts opts, svob200_match_result* d_results,
-                        double* d_px_out, int* d_ok_out, void* d_scratch, int scratch_total, int first, cudaStream_t s, long long* launches,
-                        cudaEvent_t* marks, const uint8_t* d_active, int* d_level_out, double* d_A_out)
+cudaError_t launch_match_direct(const DevFrame* d_frames, int cur_slot, const DevCam& cam, int n, const svob200_feature_ref* d_ftrs,
+                                const double* d_depth_ref, const double* d_px_in, svob200_matcher_opts opts, svob200_match_result* d_results,
+                                double* d_px_out, int* d_ok_out, void* d_scratch, int scratch_total, int first, cudaStream_t s, long long* launches,
+                                cudaEvent_t* marks, const uint8_t* d_active, int* d_level_out, double* d_A_out)
 {
-  if (n <= 0) return 0;
+  if (n <= 0) return cudaSuccess;
   const size_t m = (size_t)(scratch_total > 0 ? scratch_total : 1);
   char* p = static_cast<char*>(d_scratch);
   LkJob* jobs = reinterpret_cast<LkJob*>(p) + first; p += up256(m * sizeof(LkJob));
@@ -1407,12 +1407,12 @@ int launch_match_direct(const DevFrame* d_frames, int cur_slot, const DevCam& ca
   if (marks) cudaEventRecord(marks[0], s);
   match_prepare_kernel<<<(n + 4 * GPW - 1) / (4 * GPW), 128, 0, s>>>(d_frames, n, d_ftrs, d_px_in, geom, jobs, d_results);
   *launches += 2;
+  if (cudaError_t e = cudaGetLastError()) return e;
   if (marks) cudaEventRecord(marks[1], s);
   LkSink sink{};
   if (d_results) { sink.kind = LK_SINK_MATCH_RESULT; sink.mres = d_results; }
   else { sink.kind = LK_SINK_MATCH_COMPACT; sink.px_out = d_px_out; sink.ok_out = d_ok_out; }
-  if (launch_lk_refine(d_frames, cur_slot, jobs, nullptr, n, opts.align_max_iter, sink, s, launches)) return -1;
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+  return launch_lk_refine(d_frames, cur_slot, jobs, nullptr, n, opts.align_max_iter, sink, s, launches);
 }
 
 // persistent grid of the search kernel: SEARCH_CTAS CTAs of 4 warps (16 groups) per SM
@@ -1441,10 +1441,10 @@ size_t epipolar_scratch_bytes(int n)
   return up256(m * sizeof(EpiCold)) + up256(m * sizeof(SearchTask)) + up256(m * sizeof(EpiSearch)) + up256(job_capacity(m) * sizeof(LkJob)) + 512;
 }
 
-int launch_epipolar(const DevFrame* d_frames, int cur_slot, const DevCam& cam, int n, const svob200_feature_ref* d_ftrs, const double* d_d,
-                    svob200_matcher_opts opts, svob200_epi_result* d_results, void* d_scratch, cudaStream_t s, long long* launches)
+cudaError_t launch_epipolar(const DevFrame* d_frames, int cur_slot, const DevCam& cam, int n, const svob200_feature_ref* d_ftrs, const double* d_d,
+                            svob200_matcher_opts opts, svob200_epi_result* d_results, void* d_scratch, cudaStream_t s, long long* launches)
 {
-  if (n <= 0) return 0;
+  if (n <= 0) return cudaSuccess;
   const size_t m = (size_t)n;
   char* p = static_cast<char*>(d_scratch);
   EpiCold* cold = reinterpret_cast<EpiCold*>(p); p += up256(m * sizeof(EpiCold));
@@ -1455,12 +1455,13 @@ int launch_epipolar(const DevFrame* d_frames, int cur_slot, const DevCam& cam, i
   epi_geom_kernel<<<(n + 127) / 128, 128, 0, s>>>(cam, n, d_ftrs, d_d, opts, cold, tasks, count);
   epi_search_kernel<<<search_grid(n), 128, 0, s>>>(d_frames, cur_slot, cam, n, opts, tasks, search, nullptr, jobs, count, d_results);
   *launches += 2;
+  if (cudaError_t e = cudaGetLastError()) return e;
   LkSink sink{};
   sink.kind = LK_SINK_EPI; sink.search = search;
-  if (launch_lk_refine(d_frames, cur_slot, jobs, count, (int)job_capacity(m), opts.align_max_iter, sink, s, launches)) return -1;
+  if (cudaError_t e = launch_lk_refine(d_frames, cur_slot, jobs, count, (int)job_capacity(m), opts.align_max_iter, sink, s, launches)) return e;
   epi_result_kernel<<<(n + 127) / 128, 128, 0, s>>>(cam, n, d_ftrs, cold, search, d_results);
   ++*launches;
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+  return cudaGetLastError();
 }
 
 size_t seeds_scratch_bytes(int n)
@@ -1473,11 +1474,11 @@ size_t seeds_scratch_bytes(int n)
 // The scratch was sized for scratch_total seeds and is indexed by absolute seed number; `src`, d_seeds and d_obs already point at
 // seed `first`.  marks: optional 3 events recorded between the four kernels.
 template <class SRC>
-static int seeds_update_impl(const DevFrame* d_frames, int cur_slot, const DevCam& cam, int n, const SRC& src,
-                             svob200_matcher_opts opts, double conv_thresh, svob200_seed* d_seeds, svob200_seed_obs* d_obs, void* d_scratch,
-                             int scratch_total, int first, cudaStream_t s, long long* launches, cudaEvent_t* marks)
+static cudaError_t seeds_update_impl(const DevFrame* d_frames, int cur_slot, const DevCam& cam, int n, const SRC& src,
+                                     svob200_matcher_opts opts, double conv_thresh, svob200_seed* d_seeds, svob200_seed_obs* d_obs, void* d_scratch,
+                                     int scratch_total, int first, cudaStream_t s, long long* launches, cudaEvent_t* marks)
 {
-  if (n <= 0) return 0;
+  if (n <= 0) return cudaSuccess;
   const size_t m = (size_t)(scratch_total > 0 ? scratch_total : 1);
   char* p = static_cast<char*>(d_scratch);
   SearchTask* tasks = reinterpret_cast<SearchTask*>(p) + first; p += up256(m * sizeof(SearchTask));
@@ -1493,87 +1494,88 @@ static int seeds_update_impl(const DevFrame* d_frames, int cur_slot, const DevCa
   epi_search_kernel<<<search_grid(n, waves), 128, 0, s>>>(d_frames, cur_slot, cam, n, opts, tasks, nullptr, match, jobs, count, nullptr);
   if (marks) cudaEventRecord(marks[1], s);
   *launches += 2;
+  if (cudaError_t e = cudaGetLastError()) return e;
   LkSink sink{};
   sink.kind = LK_SINK_SEED; sink.seed_match = match;
-  if (launch_lk_refine(d_frames, cur_slot, jobs, count, (int)job_capacity((size_t)n), opts.align_max_iter, sink, s, launches)) return -1;
+  if (cudaError_t e = launch_lk_refine(d_frames, cur_slot, jobs, count, (int)job_capacity((size_t)n), opts.align_max_iter, sink, s, launches)) return e;
   if (marks) cudaEventRecord(marks[2], s);
   seeds_finish_kernel<SRC><<<(n + 127) / 128, 128, 0, s>>>(cam, n, src, conv_thresh, tasks, match, d_seeds, d_obs);
   ++*launches;
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+  return cudaGetLastError();
 }
 
-int launch_seeds_update(const DevFrame* d_frames, int cur_slot, const DevCam& cam, int n, const svob200_feature_ref* d_ftrs,
-                        const double* d_T_ref_w, const double* d_T_cur_w, svob200_matcher_opts opts, double conv_thresh,
-                        svob200_seed* d_seeds, svob200_seed_obs* d_obs, void* d_scratch, int scratch_total, int first,
-                        cudaStream_t s, long long* launches, cudaEvent_t* marks)
+cudaError_t launch_seeds_update(const DevFrame* d_frames, int cur_slot, const DevCam& cam, int n, const svob200_feature_ref* d_ftrs,
+                                const double* d_T_ref_w, const double* d_T_cur_w, svob200_matcher_opts opts, double conv_thresh,
+                                svob200_seed* d_seeds, svob200_seed_obs* d_obs, void* d_scratch, int scratch_total, int first,
+                                cudaStream_t s, long long* launches, cudaEvent_t* marks)
 {
   SeedSrcApi src{d_ftrs, d_T_ref_w, d_T_cur_w};
   return seeds_update_impl(d_frames, cur_slot, cam, n, src, opts, conv_thresh, d_seeds, d_obs, d_scratch, scratch_total, first, s, launches, marks);
 }
 
 // rows (keyframe k, image b), b in [image0, image0 + n_images), of the pose table the compact seed kernels read
-int launch_seed_pose_table(const DevCam& cam, int batch, int n_kfs, int image0, int n_images, const double* d_T_kf_w, const double* d_T_cur_w,
-                           SeedPoseRec* d_pose_table, cudaStream_t s, long long* launches)
+cudaError_t launch_seed_pose_table(const DevCam& cam, int batch, int n_kfs, int image0, int n_images, const double* d_T_kf_w, const double* d_T_cur_w,
+                                   SeedPoseRec* d_pose_table, cudaStream_t s, long long* launches)
 {
   const int rows = n_kfs * n_images;
-  if (rows <= 0) return 0;
+  if (rows <= 0) return cudaSuccess;
   seed_pose_table_kernel<<<(rows + 127) / 128, 128, 0, s>>>(cam, batch, n_kfs, image0, n_images, d_T_kf_w, d_T_cur_w, d_pose_table);
   ++*launches;
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+  return cudaGetLastError();
 }
 
-int launch_seeds_update_compact(const DevFrame* d_frames, int cur_slot, const DevCam& cam, int n, SeedRef* d_refs,
-                                const int* d_kf_slot, int batch, const SeedPoseRec* d_pose_table, const int* d_batch_counter, int max_n_kfs,
-                                svob200_matcher_opts opts, double conv_thresh,
-                                svob200_seed* d_seeds, svob200_seed_obs* d_obs, void* d_scratch, int scratch_total, int first,
-                                cudaStream_t s, long long* launches, cudaEvent_t* marks)
+cudaError_t launch_seeds_update_compact(const DevFrame* d_frames, int cur_slot, const DevCam& cam, int n, SeedRef* d_refs,
+                                        const int* d_kf_slot, int batch, const SeedPoseRec* d_pose_table, const int* d_batch_counter, int max_n_kfs,
+                                        svob200_matcher_opts opts, double conv_thresh,
+                                        svob200_seed* d_seeds, svob200_seed_obs* d_obs, void* d_scratch, int scratch_total, int first,
+                                        cudaStream_t s, long long* launches, cudaEvent_t* marks)
 {
   SeedSrcCompact src{d_refs, d_pose_table, d_kf_slot, batch, d_batch_counter, max_n_kfs};
   return seeds_update_impl(d_frames, cur_slot, cam, n, src, opts, conv_thresh, d_seeds, d_obs, d_scratch, scratch_total, first, s, launches, marks);
 }
 
-int launch_update_seed(int n, const float* d_x, const float* d_tau2, svob200_seed* d_seeds, cudaStream_t s, long long* launches)
+cudaError_t launch_update_seed(int n, const float* d_x, const float* d_tau2, svob200_seed* d_seeds, cudaStream_t s, long long* launches)
 {
-  if (n <= 0) return 0;
+  if (n <= 0) return cudaSuccess;
   update_seed_kernel<<<(n + 127) / 128, 128, 0, s>>>(n, d_x, d_tau2, d_seeds);
   ++*launches;
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+  return cudaGetLastError();
 }
 
-int launch_compute_tau(int n, const double* d_T, const double* d_f, const double* d_z, double angle, double* d_out,
-                       cudaStream_t s, long long* launches)
+cudaError_t launch_compute_tau(int n, const double* d_T, const double* d_f, const double* d_z, double angle, double* d_out,
+                               cudaStream_t s, long long* launches)
 {
-  if (n <= 0) return 0;
+  if (n <= 0) return cudaSuccess;
   compute_tau_kernel<<<(n + 127) / 128, 128, 0, s>>>(n, d_T, d_f, d_z, angle, d_out);
   ++*launches;
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+  return cudaGetLastError();
 }
 
-int launch_warp_matrix(const DevCam& cam, int n, const double* d_px_ref, const double* d_f_ref, const double* d_depth_ref,
-                       const double* d_T_cur_ref, const int* d_level_ref, double* d_A_out, cudaStream_t s, long long* launches)
+cudaError_t launch_warp_matrix(const DevCam& cam, int n, const double* d_px_ref, const double* d_f_ref, const double* d_depth_ref,
+                               const double* d_T_cur_ref, const int* d_level_ref, double* d_A_out, cudaStream_t s, long long* launches)
 {
-  if (n <= 0) return 0;
+  if (n <= 0) return cudaSuccess;
   warp_matrix_kernel<<<(n + 127) / 128, 128, 0, s>>>(cam, n, d_px_ref, d_f_ref, d_depth_ref, d_T_cur_ref, d_level_ref, d_A_out);
   ++*launches;
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+  return cudaGetLastError();
 }
 
-int launch_warp_affine(const uint8_t* d_img, int pitch, int cols, int rows, const double* A, const double* px_ref, int level_ref,
-                       int search_level, int halfpatch, uint8_t* d_patch, cudaStream_t s, long long* launches)
+cudaError_t launch_warp_affine(const uint8_t* d_img, int pitch, int cols, int rows, const double* A, const double* px_ref, int level_ref,
+                               int search_level, int halfpatch, uint8_t* d_patch, cudaStream_t s, long long* launches)
 {
   const int n = 4 * halfpatch * halfpatch;
-  if (n <= 0) return 0;
+  if (n <= 0) return cudaSuccess;
   warp_affine_kernel<<<(n + 127) / 128, 128, 0, s>>>(d_img, pitch, cols, rows, A[0], A[1], A[2], A[3], px_ref[0], px_ref[1], level_ref,
                                                      search_level, halfpatch, d_patch);
   ++*launches;
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+  return cudaGetLastError();
 }
 
-int launch_triangulate(int n, const double* d_T, const double* d_f_ref, const double* d_f_cur, double* d_depth, int* d_ok,
-                       cudaStream_t s, long long* launches)
+cudaError_t launch_triangulate(int n, const double* d_T, const double* d_f_ref, const double* d_f_cur, double* d_depth, int* d_ok,
+                               cudaStream_t s, long long* launches)
 {
-  if (n <= 0) return 0;
+  if (n <= 0) return cudaSuccess;
   triangulate_kernel<<<(n + 127) / 128, 128, 0, s>>>(n, d_T, d_f_ref, d_f_cur, d_depth, d_ok);
   ++*launches;
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+  return cudaGetLastError();
 }

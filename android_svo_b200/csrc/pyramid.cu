@@ -282,8 +282,10 @@ __global__ void __launch_bounds__(128) yuv_gray_kernel(DevFrame f, YuvPlanes yuv
 }  // namespace
 
 template <bool YUV>
-static void launch_fused(const DevFrame& f, int mask, const YuvPlanes& yuv, cudaStream_t s)
+static cudaError_t launch_fused(const DevFrame& f, const int* modes, const YuvPlanes& yuv, cudaStream_t s)
 {
+  int mask = 0;
+  for (int l = 0; l + 1 < f.n_levels; ++l) if (modes[l] == SVOB200_ROUND_SSE2) mask |= 1 << l;
   dim3 grid((f.w[0] + PTW - 1) / PTW, (f.h[0] + PTH - 1) / PTH, f.batch);
   switch (f.n_levels) {
     case 2: pyramid_fused_kernel<YUV, 2><<<grid, PNT, 0, s>>>(f, mask, yuv); break;
@@ -293,6 +295,7 @@ static void launch_fused(const DevFrame& f, int mask, const YuvPlanes& yuv, cuda
     case 6: pyramid_fused_kernel<YUV, 6><<<grid, PNT, 0, s>>>(f, mask, yuv); break;
     default: pyramid_fused_kernel<YUV, 7><<<grid, PNT, 0, s>>>(f, mask, yuv); break;
   }
+  return cudaGetLastError();
 }
 
 static bool fused_ok(const DevFrame& f)
@@ -303,48 +306,40 @@ static bool fused_ok(const DevFrame& f)
 }
 
 // level 0 from YUV planes (+ all coarser levels); level 0 must be owned storage with a 16-byte pitch
-int launch_pyramid_yuv(const DevFrame& f, const YuvPlanes& yuv, const int* modes, cudaStream_t s, long long* launches)
+cudaError_t launch_pyramid_yuv(const DevFrame& f, const YuvPlanes& yuv, const int* modes, cudaStream_t s, long long* launches)
 {
-  if (fused_ok(f)) {
-    int mask = 0;
-    for (int l = 0; l + 1 < f.n_levels; ++l) if (modes[l] == SVOB200_ROUND_SSE2) mask |= 1 << l;
-    launch_fused<true>(f, mask, yuv, s);
-    ++*launches;
-    return cudaGetLastError() == cudaSuccess ? 0 : -1;
-  }
+  ++*launches;
+  if (fused_ok(f)) return launch_fused<true>(f, modes, yuv, s);
   dim3 grid((f.w[0] + 511) / 512, (f.h[0] + 7) / 8, f.batch);
   yuv_gray_kernel<<<grid, 128, 0, s>>>(f, yuv);
-  ++*launches;
-  if (cudaGetLastError() != cudaSuccess) return -1;
+  if (cudaError_t e = cudaGetLastError()) return e;
   return launch_pyramid(f, modes, s, launches);
 }
 
-int launch_pyramid(const DevFrame& f, const int* modes, cudaStream_t s, long long* launches)
+cudaError_t launch_pyramid(const DevFrame& f, const int* modes, cudaStream_t s, long long* launches)
 {
-  if (f.n_levels <= 1) return 0;
+  if (f.n_levels <= 1) return cudaSuccess;
   if (fused_ok(f)) {
-    int mask = 0;
-    for (int l = 0; l + 1 < f.n_levels; ++l) if (modes[l] == SVOB200_ROUND_SSE2) mask |= 1 << l;
-    launch_fused<false>(f, mask, YuvPlanes{}, s);
     ++*launches;
-  } else {
-    for (int l = 0; l + 1 < f.n_levels; ++l) {
-      dim3 blk(32, 8), grid((f.w[l + 1] + 31) / 32, (f.h[l + 1] + 7) / 8, f.batch);
-      if (f.w[l + 1] == 0 || f.h[l + 1] == 0) break;
-      half_sample_generic_kernel<<<grid, blk, 0, s>>>(f.lvl[l], f.pitch[l], f.img_stride[l], f.w[l], f.h[l],
-                                                      f.lvl[l + 1], f.pitch[l + 1], f.img_stride[l + 1], modes[l]);
-      ++*launches;
-    }
+    return launch_fused<false>(f, modes, YuvPlanes{}, s);
   }
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+  for (int l = 0; l + 1 < f.n_levels; ++l) {
+    dim3 blk(32, 8), grid((f.w[l + 1] + 31) / 32, (f.h[l + 1] + 7) / 8, f.batch);
+    if (f.w[l + 1] == 0 || f.h[l + 1] == 0) break;
+    half_sample_generic_kernel<<<grid, blk, 0, s>>>(f.lvl[l], f.pitch[l], f.img_stride[l], f.w[l], f.h[l],
+                                                    f.lvl[l + 1], f.pitch[l + 1], f.img_stride[l + 1], modes[l]);
+    ++*launches;
+    if (cudaError_t e = cudaGetLastError()) return e;
+  }
+  return cudaSuccess;
 }
 
-int launch_half_sample_single(const uint8_t* in, int in_pitch, int w, int h, uint8_t* out, int out_pitch, int mode,
-                              cudaStream_t s, long long* launches)
+cudaError_t launch_half_sample_single(const uint8_t* in, int in_pitch, int w, int h, uint8_t* out, int out_pitch, int mode,
+                                      cudaStream_t s, long long* launches)
 {
-  if (w / 2 == 0 || h / 2 == 0) return 0;
+  if (w / 2 == 0 || h / 2 == 0) return cudaSuccess;
   dim3 blk(32, 8), grid((w / 2 + 31) / 32, (h / 2 + 7) / 8, 1);
   half_sample_generic_kernel<<<grid, blk, 0, s>>>(in, in_pitch, 0, w, h, out, out_pitch, 0, mode);
   ++*launches;
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+  return cudaGetLastError();
 }

@@ -757,15 +757,15 @@ __global__ void __launch_bounds__(BLOCK) chi2_chain_test_kernel(const float* res
 
 }  // namespace
 
-int launch_chi2_chain_test(int block, const float* d_res, const uint8_t* d_visible, const uint8_t* d_contrib, int n, float* d_sums, int* d_cnts,
-                           cudaStream_t s, long long* launches)
+cudaError_t launch_chi2_chain_test(int block, const float* d_res, const uint8_t* d_visible, const uint8_t* d_contrib, int n, float* d_sums, int* d_cnts,
+                                   cudaStream_t s, long long* launches)
 {
   if (block == 128) chi2_chain_test_kernel<128><<<1, 128, 0, s>>>(d_res, d_visible, d_contrib, n, d_sums, d_cnts);
   else if (block == 256) chi2_chain_test_kernel<256><<<1, 256, 0, s>>>(d_res, d_visible, d_contrib, n, d_sums, d_cnts);
   else if (block == 512) chi2_chain_test_kernel<512><<<1, 512, 0, s>>>(d_res, d_visible, d_contrib, n, d_sums, d_cnts);
-  else return -1;
+  else return cudaErrorInvalidValue;
   ++*launches;
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+  return cudaGetLastError();
 }
 
 // per feature: 16 floats x (ref_patch, gdx, gdy, res0, res1) + 15 doubles (a, b, patch gradient sums) + 3 flag bytes
@@ -775,10 +775,10 @@ size_t sparse_align_scratch_bytes(int total_features)
   return n * (16 * sizeof(float) * 5 + JAB * sizeof(double) + 3) + 4096;
 }
 
-int launch_sparse_align(const DevFrame& ref, const DevFrame& cur, const DevCam& cam, int batch, int total_features, int max_per_problem,
-                        const int* d_offsets, const double* d_px, const double* d_xyz, const uint8_t* d_has_point,
-                        const double* d_T_init, svob200_align_opts opts, svob200_align_result* d_results,
-                        void* d_scratch, cudaStream_t s, long long* launches, const double* d_T_ref_w, double* d_T_cur_w)
+cudaError_t launch_sparse_align(const DevFrame& ref, const DevFrame& cur, const DevCam& cam, int batch, int total_features, int max_per_problem,
+                                const int* d_offsets, const double* d_px, const double* d_xyz, const uint8_t* d_has_point,
+                                const double* d_T_init, svob200_align_opts opts, svob200_align_result* d_results,
+                                void* d_scratch, cudaStream_t s, long long* launches, const double* d_T_ref_w, double* d_T_cur_w)
 {
   AlignArgs A{};
   A.T_ref_w = d_T_ref_w; A.T_cur_w = d_T_cur_w;
@@ -817,7 +817,8 @@ int launch_sparse_align(const DevFrame& ref, const DevFrame& cur, const DevCam& 
     else if (cluster == 4) e = cudaLaunchKernelEx(&cfg, sparse_align_kernel<256, 4>, A);
     else e = cudaLaunchKernelEx(&cfg, sparse_align_kernel<256, 2>, A);
     ++*launches;
-    return e == cudaSuccess && cudaGetLastError() == cudaSuccess ? 0 : -1;
+    const cudaError_t last = cudaGetLastError();      // (also clears the error a failed launch leaves behind)
+    return e != cudaSuccess ? e : last;
   }
   if (max_per_problem > 512) sparse_align_kernel<512, 1><<<batch, 512, 0, s>>>(A);
   else if (max_per_problem > 128 || batch < 296) sparse_align_kernel<256, 1><<<batch, 256, 0, s>>>(A);
@@ -825,5 +826,5 @@ int launch_sparse_align(const DevFrame& ref, const DevFrame& cur, const DevCam& 
   // 0.176 against 0.143 ms per 512 — the pass is bound by its own dependent latency, not by how many problems share the SM)
   else sparse_align_kernel<128, 1><<<batch, 128, 0, s>>>(A);
   ++*launches;
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+  return cudaGetLastError();
 }

@@ -32,11 +32,11 @@ __global__ void synth_render_kernel(const uint8_t* tex, int size, double ppm, do
 }
 }  // namespace
 
-int launch_synth_render(const uint8_t* d_tex, int tex_size, double ppm, double plane_z, const DevCam& cam, int batch,
-                        const double* d_rc, uint8_t* d_out, cudaStream_t s, long long* launches)
+cudaError_t launch_synth_render(const uint8_t* d_tex, int tex_size, double ppm, double plane_z, const DevCam& cam, int batch,
+                                const double* d_rc, uint8_t* d_out, cudaStream_t s, long long* launches)
 {
   dim3 blk(32, 8), grid((cam.width + 31) / 32, (cam.height + 7) / 8, batch);
   synth_render_kernel<<<grid, blk, 0, s>>>(d_tex, tex_size, ppm, plane_z, cam, d_rc, d_out);
   ++*launches;
-  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+  return cudaGetLastError();
 }

@@ -394,7 +394,7 @@ __global__ void __launch_bounds__(256) kf_append_seeds_kernel(DevCam cam, const 
                                                               const float* depth_min, const int* seed_off, SeedRef* refs, svob200_seed* seeds,
                                                               const int* kf_new, const int* batch_counter, int* appended, int* dropped)
 {
-  __shared__ int s_slot_of_rank[8192];                // grids up to 8,192 cells (svob200_tracker_set_detector / _add_keyframe)
+  __shared__ int s_slot_of_rank[kMaxGridCells];
   const int b = blockIdx.x, tid = threadIdx.x;
   const int kf = kf_new[b], batch_id = batch_counter[b];
   if (kf < 0) { if (tid == 0) appended[b] = dropped[b] = kf == -2 ? -1 : 0; return; }   // refused (batch counter exhausted) / not selected
@@ -838,7 +838,6 @@ int svob200_tracker_set_keyframe(svob200_tracker* t, const uint8_t* imgs, int st
   const int i_so = st.add(seed_offsets, nullptr, sizeof(int) * (B + 1), 0), i_spx = st.add(seed_px, nullptr, sizeof(double) * 2 * S_in, 0);
   const int i_slv = st.add(seed_level, nullptr, sizeof(int) * S_in, 0);
   if (int e = st.layout()) return e;
-  st.upload();
   if (int e = st.push()) return e;
   if (N || S) {
     kf_init_slots_kernel<<<B, 128, 0, s>>>(to_cam(&t->cam), t->max_kfs, slot, t->d_T_kf, t->d_ftr_off, st.dev<int>(i_fo), st.dev<double>(i_px),
@@ -846,7 +845,7 @@ int svob200_tracker_set_keyframe(svob200_tracker* t, const uint8_t* imgs, int st
                                            st.dev<int>(i_slv), t->seed_init, t->d_ftr_image, t->d_has_point, t->d_sel, t->d_pt_world, t->d_ftrs,
                                            t->d_points, t->d_pobs, t->d_T_pobs, t->d_seed_refs, t->d_seeds);
     ++ctx->launches;
-    if (cudaGetLastError() != cudaSuccess) return fail(ctx, SVOB200_ERR_CUDA, "tracker_set_keyframe: launch error");
+    CU_AT("tracker_set_keyframe: kf_init_slots_kernel", cudaGetLastError());
   }
   return st.download();                                  // the caller's arrays are host memory
 }
@@ -880,8 +879,8 @@ int svob200_tracker_set_detector(svob200_tracker* t, int cell_size, int n_detect
   if (!t) return SVOB200_ERR_ARG;
   svob200_ctx* ctx = t->ctx;
   if (cell_size <= 0 || n_detect_levels < 1 || n_detect_levels > t->n_levels) return fail(ctx, SVOB200_ERR_ARG, "tracker_set_detector: bad arguments");
-  const int n_cells = ((t->cam.width + cell_size - 1) / cell_size) * ((t->cam.height + cell_size - 1) / cell_size);
-  if (n_cells > 8192) return fail(ctx, SVOB200_ERR_UNSUPPORTED, "tracker_set_detector: grid of %d cells exceeds the kernel's table (8192)", n_cells);
+  const long long n_cells = grid_cells(t->cam.width, t->cam.height, cell_size);
+  if (n_cells > kMaxGridCells) return fail(ctx, SVOB200_ERR_UNSUPPORTED, "tracker_set_detector: grid of %lld cells exceeds the limit of %d", n_cells, kMaxGridCells);
   t->det_cell = cell_size; t->det_levels = n_detect_levels; t->det_thr = detection_threshold;
   return SVOB200_OK;
 }
@@ -898,9 +897,9 @@ int svob200_tracker_add_keyframes(svob200_tracker* t, const uint8_t* which, cons
   if (!t->d_stats || t->steps_done == 0) return fail(ctx, SVOB200_ERR_ARG, "tracker_add_keyframes: needs a keyframe and at least one step");
   if (t->chain_cell > 0) return fail(ctx, SVOB200_ERR_UNSUPPORTED, "tracker_add_keyframes: not available in chain mode");
   const int B = t->batch, N = t->N, S = t->S;
-  const int gc = (t->cam.width + t->det_cell - 1) / t->det_cell, gr = (t->cam.height + t->det_cell - 1) / t->det_cell;
-  const int n_cells = gc * gr;
-  if (n_cells > 8192) return fail(ctx, SVOB200_ERR_UNSUPPORTED, "tracker_add_keyframes: grid of %d cells exceeds the kernel's table (8192)", n_cells);
+  const long long grid = grid_cells(t->cam.width, t->cam.height, t->det_cell);
+  if (grid > kMaxGridCells) return fail(ctx, SVOB200_ERR_UNSUPPORTED, "tracker_add_keyframes: grid of %lld cells exceeds the limit of %d", grid, kMaxGridCells);
+  const int gc = (t->cam.width + t->det_cell - 1) / t->det_cell, gr = (t->cam.height + t->det_cell - 1) / t->det_cell, n_cells = (int)grid;
   cudaStream_t s = ctx->stream;
   // the keyframe store (allocated here when set_seed_pool did not) and the detector scratch
   bool new_store = false;
@@ -929,45 +928,53 @@ int svob200_tracker_add_keyframes(svob200_tracker* t, const uint8_t* which, cons
   const bool may_evict = t->n_kfs == t->max_kfs;           // (no sequence holds more keyframes than n_kfs)
   kf_select_kernel<<<(B + 127) / 128, 128, 0, s>>>(B, t->max_kfs, d_which, t->d_kf_batch, t->d_batch_counter, t->d_kf_new, t->d_kf_old, t->d_T_cur, t->d_T_kf);
   ++ctx->launches;
+  CU_AT("tracker_add_keyframes: kf_select_kernel", cudaGetLastError());
   if (!may_evict) { t->n_kfs = std::min(t->max_kfs, t->n_kfs + 1); drop_graphs(t); }   // captured steps hold n_kfs
   if (may_evict) {
-    if (S) { kf_erase_seeds_kernel<<<(S + 255) / 256, 256, 0, s>>>(S, t->d_seed_refs, t->d_kf_old); ++ctx->launches; }
+    if (S) {
+      kf_erase_seeds_kernel<<<(S + 255) / 256, 256, 0, s>>>(S, t->d_seed_refs, t->d_kf_old); ++ctx->launches;
+      CU_AT("tracker_add_keyframes: kf_erase_seeds_kernel", cudaGetLastError());
+    }
     if (N) {                                                 // Map::safeDeleteFrame: the points forget the keyframe
       if (t->pt_capacity >= 0) {
         kf_drop_candidates_kernel<<<(N + 255) / 256, 256, 0, s>>>(N, t->d_points, t->d_pobs, t->d_match_ok, t->d_has_point, t->d_ftr_image, t->d_kf_old,
                                                                   t->d_kf_slot);
         ++ctx->launches;
+        CU_AT("tracker_add_keyframes: kf_drop_candidates_kernel", cudaGetLastError());
       }
       kf_drop_obs_kernel<<<(N + 255) / 256, 256, 0, s>>>(N, t->max_kfs, t->d_points, t->d_pobs, t->d_T_pobs, t->d_ftr_image, t->d_kf_old, t->d_kf_slot,
                                                          t->d_sel);
       ++ctx->launches;
+      CU_AT("tracker_add_keyframes: kf_drop_obs_kernel", cudaGetLastError());
     }
   }
   // 2. the frame: the last step's current frame (now `last`), every level, into the store
-  FrameRec* r = find_frame(ctx, t->fid_last);
-  if (!r) return fail(ctx, SVOB200_ERR_NOFRAME, "tracker_add_keyframes: last frame missing");
+  FrameRec* r = resident_frame(ctx, t->fid_last, "tracker_add_keyframes"); if (!r) return SVOB200_ERR_NOFRAME;
   kf_store_copy_kernel<<<dim3(16, B), 256, 0, s>>>(r->f, ctx->d_table, t->d_kf_slot, t->d_kf_new);
   ++ctx->launches;
+  CU_AT("tracker_add_keyframes: kf_store_copy_kernel", cudaGetLastError());
   // 3. occupancy from the frame's features (the map points matched in it), FAST + Shi-Tomasi + grid on the selected images,
   // one seed per new corner
   CU(cudaMemsetAsync(t->d_occ, 0, (size_t)B * n_cells, s));
   if (N) {
     kf_occupancy_kernel<<<(N + 255) / 256, 256, 0, s>>>(N, t->d_ftr_image, t->d_px_out, t->d_match_ok, t->d_kf_new, t->det_cell, gc, n_cells, t->d_occ);
     ++ctx->launches;
+    CU_AT("tracker_add_keyframes: kf_occupancy_kernel", cudaGetLastError());
   }
-  if (launch_fast_detect(r->f, t->det_levels, t->det_cell, gc, gr, t->det_thr, t->d_occ, t->d_det_keys, t->d_det_cells, t->d_det_counts, s, &ctx->launches,
-                         t->d_kf_new))
-    return fail(ctx, SVOB200_ERR_CUDA, "tracker_add_keyframes: detector launch failed");
+  CU_AT("tracker_add_keyframes: launch_fast_detect",
+        launch_fast_detect(r->f, t->det_levels, t->det_cell, gc, gr, t->det_thr, t->d_occ, t->d_det_keys, t->d_det_cells, t->d_det_counts, s, &ctx->launches,
+                           t->d_kf_new));
   kf_append_seeds_kernel<<<B, 256, 0, s>>>(to_cam(&t->cam), t->d_det_cells, n_cells, t->det_thr, d_dm, d_dn, t->d_seed_off, t->d_seed_refs,
                                            t->d_seeds, t->d_kf_new, t->d_batch_counter, t->d_kf_appended, t->d_kf_dropped);
   ++ctx->launches;
+  CU_AT("tracker_add_keyframes: kf_append_seeds_kernel", cudaGetLastError());
   // 4. the matched map points gain an observation in the new keyframe (frame_handler_mono.cpp:277-279)
   if (N) {
     kf_add_obs_kernel<<<(N + 255) / 256, 256, 0, s>>>(to_cam(&t->cam), N, t->max_kfs, t->d_points, t->d_pobs, t->d_T_pobs, t->d_ftr_image, t->d_match_ok, t->d_px_out,
                                                       t->d_match_level, t->d_kf_new, t->d_kf_slot, t->d_T_cur);
     ++ctx->launches;
+    CU_AT("tracker_add_keyframes: kf_add_obs_kernel", cudaGetLastError());
   }
-  if (cudaGetLastError() != cudaSuccess) return fail(ctx, SVOB200_ERR_CUDA, "tracker_add_keyframes: launch error");
   // the counts (unselected sequences: 0, refused ones: -1).  Without a seed pool n_dropped repeats n_new_seeds, and is 0 when
   // n_new_seeds is not asked for (as svob200_tracker_add_keyframe always reported it)
   const cudaMemcpyKind kind = mem == SVOB200_MEM_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
@@ -997,7 +1004,7 @@ int svob200_tracker_scene_depth(svob200_tracker* t, float* depth_mean, float* de
   scene_depth_kernel<<<B, 128, 0, s>>>(t->d_ftr_off, t->d_points, t->d_match_ok, t->d_T_cur, t->d_sd_z, dev ? depth_mean : t->d_depth_mean,
                                        dev ? depth_min : t->d_depth_min, dev ? n_points : t->d_sd_n);
   ++ctx->launches;
-  if (cudaGetLastError() != cudaSuccess) return fail(ctx, SVOB200_ERR_CUDA, "tracker_scene_depth: launch error");
+  CU_AT("tracker_scene_depth: scene_depth_kernel", cudaGetLastError());
   if (dev) return SVOB200_OK;
   std::vector<float> dm(B), dn(B);
   std::vector<int> n(B);
@@ -1070,8 +1077,8 @@ int svob200_tracker_set_chain(svob200_tracker* t, int cell_size, int max_fts, in
   drop_graphs(t);                                                  // captured steps belong to the other mode
   if (cell_size <= 0) { t->chain_cell = 0; return SVOB200_OK; }
   const int B = t->batch, N = t->N;
-  const int n_cells = ((t->cam.width + cell_size - 1) / cell_size) * ((t->cam.height + cell_size - 1) / cell_size);
-  if (n_cells > 8192) return fail(ctx, SVOB200_ERR_UNSUPPORTED, "tracker_set_chain: grid of %d cells exceeds the kernel's table (8192)", n_cells);
+  const long long n_cells = grid_cells(t->cam.width, t->cam.height, cell_size);
+  if (n_cells > kMaxGridCells) return fail(ctx, SVOB200_ERR_UNSUPPORTED, "tracker_set_chain: grid of %lld cells exceeds the limit of %d", n_cells, kMaxGridCells);
   if (!t->d_reproj || n_cells != t->chain_cells) {
     const size_t M = (size_t)B * n_cells;
     int err = 0;
@@ -1085,7 +1092,7 @@ int svob200_tracker_set_chain(svob200_tracker* t, int cell_size, int max_fts, in
   // d_obs / d_T_obs already hold them with their observation lists)
   CU(cudaMemsetAsync(t->d_pose, 0, sizeof(svob200_pose_opt_result) * (size_t)B, ctx->stream));
   CU(cudaStreamSynchronize(ctx->stream));
-  t->chain_cell = cell_size; t->chain_max_fts = max_fts; t->chain_pose_opt = pose_opt ? 1 : 0; t->chain_cells = n_cells;
+  t->chain_cell = cell_size; t->chain_max_fts = max_fts; t->chain_pose_opt = pose_opt ? 1 : 0; t->chain_cells = (int)n_cells;
   return SVOB200_OK;
 }
 
@@ -1118,10 +1125,10 @@ static int enqueue_seeds_update(svob200_tracker* t, int c0, int c1, const SeedPo
 {
   svob200_ctx* ctx = t->ctx;
   const int s0 = t->h_seed_off[c0], ns = t->h_seed_off[c1] - s0;
-  if (launch_seeds_update_compact(ctx->d_table, find_frame(ctx, t->fid_cur)->slot, to_cam(&t->cam), ns, t->d_seed_refs + s0, t->d_kf_slot, t->batch, table,
-                                  t->d_batch_counter, t->max_n_kfs, t->mopts, t->conv_thresh, t->d_seeds + s0, t->d_obs + s0, t->d_seed_scratch, t->S, s0,
-                                  st, &ctx->launches, marks))
-    return fail(ctx, SVOB200_ERR_CUDA, "tracker_step: seeds_update failed");
+  CU_AT("tracker_step: launch_seeds_update_compact",
+        launch_seeds_update_compact(ctx->d_table, find_frame(ctx, t->fid_cur)->slot, to_cam(&t->cam), ns, t->d_seed_refs + s0, t->d_kf_slot, t->batch, table,
+                                    t->d_batch_counter, t->max_n_kfs, t->mopts, t->conv_thresh, t->d_seeds + s0, t->d_obs + s0, t->d_seed_scratch, t->S, s0,
+                                    st, &ctx->launches, marks));
   return 0;
 }
 
@@ -1135,10 +1142,11 @@ static int enqueue_step_stats(svob200_tracker* t, int c0, int c1, int parts, svo
   kernel<<<cnt, 128, 0, st>>>(t->d_ftr_off + c0, t->d_seed_off + c0, t->d_align + c0, t->d_T_cur + 7 * (size_t)c0, t->d_match_ok, t->d_obs,
                               t->d_seeds, t->seed_init, t->reseed, d_stats + c0, parts, t->d_seed_refs, cand);
   ++ctx->launches;
+  CU_AT("tracker_step: step_stats_kernel", cudaGetLastError());
   if (t->chain_cell > 0) {
     chain_stats_kernel<<<(cnt + 127) / 128, 128, 0, st>>>(cnt, t->d_rstats + c0, t->d_pose + c0, t->chain_pose_opt, d_stats + c0); ++ctx->launches;
+    CU_AT("tracker_step: chain_stats_kernel", cudaGetLastError());
   }
-  if (cudaGetLastError() != cudaSuccess) return fail(ctx, SVOB200_ERR_CUDA, "tracker_step: launch error");
   return 0;
 }
 
@@ -1153,7 +1161,7 @@ static int enqueue_insert_candidates(svob200_tracker* t)
                                                         t->d_points, t->d_pt_world, t->d_pobs, t->d_T_pobs, t->d_sel, t->d_has_point, t->d_pt_rank,
                                                         t->d_pt_dropped);
   ++ctx->launches;
-  if (cudaGetLastError() != cudaSuccess) return fail(ctx, SVOB200_ERR_CUDA, "tracker_step: candidate insertion launch error");
+  CU_AT("tracker_step: cand_insert_kernel", cudaGetLastError());
   return 0;
 }
 
@@ -1182,20 +1190,22 @@ static int run_range(svob200_tracker* t, int c0, int c1, const double* d_T_last,
   {
     int modes[SVOB200_MAX_LEVELS];
     pyramid_round_modes(vcur, nullptr, modes);
-    if (launch_pyramid(vcur, modes, s, &ctx->launches)) return fail(ctx, SVOB200_ERR_CUDA, "tracker_step: pyramid launch failed");
+    CU_AT("tracker_step: launch_pyramid", launch_pyramid(vcur, modes, s, &ctx->launches));
   }
   MARK(1);
   // 2. Feature ctor / xyz_ref of the last frame's features, initial relative pose
-  if (launch_features_prepare(cam, nf, d_last_px + 2 * (size_t)f0, t->d_pt_world + 3 * (size_t)f0, t->d_ftr_image + f0, d_T_last, nullptr,
-                              t->d_xyz + 3 * (size_t)f0, s2, &ctx->launches)) return fail(ctx, SVOB200_ERR_CUDA, "tracker_step: features_prepare failed");
+  CU_AT("tracker_step: launch_features_prepare",
+        launch_features_prepare(cam, nf, d_last_px + 2 * (size_t)f0, t->d_pt_world + 3 * (size_t)f0, t->d_ftr_image + f0, d_T_last, nullptr,
+                                t->d_xyz + 3 * (size_t)f0, s2, &ctx->launches));
   init_pose_kernel<<<(cnt + 127) / 128, 128, 0, s2>>>(cnt, d_T_last + 7 * (size_t)c0, t->d_T_init + 7 * (size_t)c0); ++ctx->launches;
+  CU_AT("tracker_step: init_pose_kernel", cudaGetLastError());
   if (fork) { CU(cudaEventRecord(t->fork_ev[1], s2)); CU(cudaStreamWaitEvent(s, t->fork_ev[1], 0)); }
   MARK(2);
   // 3. SparseImgAlign::run(last, cur)
-  if (launch_sparse_align(vlast, vcur, cam, cnt, t->N, t->max_per, t->d_ftr_off + c0, d_last_px, t->d_xyz, t->d_has_point,
-                          t->d_T_init + 7 * (size_t)c0, t->aopts, t->d_align + c0, t->d_align_scratch, s, &ctx->launches,
-                          d_T_last + 7 * (size_t)c0, t->d_T_cur + 7 * (size_t)c0))
-    return fail(ctx, SVOB200_ERR_CUDA, "tracker_step: sparse_align failed");
+  CU_AT("tracker_step: launch_sparse_align",
+        launch_sparse_align(vlast, vcur, cam, cnt, t->N, t->max_per, t->d_ftr_off + c0, d_last_px, t->d_xyz, t->d_has_point,
+                            t->d_T_init + 7 * (size_t)c0, t->aopts, t->d_align + c0, t->d_align_scratch, s, &ctx->launches,
+                            d_T_last + 7 * (size_t)c0, t->d_T_cur + 7 * (size_t)c0));
   MARK(3);
   // 4. cur.T_f_w = T_cur_from_ref * last.T_f_w (written by the alignment kernel's epilogue) ; reprojection of the map points
   // chain mode: the depth filter waits for the pose optimiser's T_cur, so its branch cannot start here
@@ -1206,6 +1216,7 @@ static int run_range(svob200_tracker* t, int c0, int c1, const double* d_T_last,
     points_select_kernel<<<(nf + 127) / 128, 128, 0, s>>>(cam, nf, t->d_points + f0, t->d_pobs, t->d_T_pobs, t->d_ftr_image + f0, t->d_T_cur, t->d_ftrs + f0,
                                                           t->d_depth_ref + f0, t->d_px_in + 2 * (size_t)f0, t->d_active + f0, t->d_sel + f0);
     ++ctx->launches;
+    CU_AT("tracker_step: points_select_kernel", cudaGetLastError());
   }
   MARK(4);
   if (t->chain_cell > 0) {
@@ -1213,35 +1224,37 @@ static int run_range(svob200_tracker* t, int c0, int c1, const double* d_T_last,
     // maxFts) over the keyframe's map points, then pose_optimizer::optimizeGaussNewton on the frame's new features (in place
     // on T_cur, so the depth filter sees the optimised pose).
     const size_t cb = (size_t)c0 * t->chain_cells;
-    const int rc = launch_reproject_map(ctx->d_table, cur->slot, cam, cnt, t->d_T_cur + 7 * (size_t)c0, t->d_ftr_off + c0, t->N, t->d_points, t->d_pobs,
-                                        t->d_T_pobs, t->chain_cell, t->chain_max_fts, t->mopts, t->d_reproj, t->d_winner + cb, t->d_rstats + c0,
-                                        t->d_reproj_scratch, t->d_match_scratch, t->d_m_f + 3 * cb, t->d_m_level + cb, t->d_m_pos + 3 * cb,
-                                        t->d_m_point + cb, t->d_m_count + c0, s, &ctx->launches, c0, f0, nf);
-    if (rc) return fail(ctx, SVOB200_ERR_CUDA, "tracker_step: reproject_map failed (%d)", rc);
+    CU_AT("tracker_step: launch_reproject_map",
+          launch_reproject_map(ctx->d_table, cur->slot, cam, cnt, t->d_T_cur + 7 * (size_t)c0, t->d_ftr_off + c0, t->N, t->d_points, t->d_pobs,
+                               t->d_T_pobs, t->chain_cell, t->chain_max_fts, t->mopts, t->d_reproj, t->d_winner + cb, t->d_rstats + c0,
+                               t->d_reproj_scratch, t->d_match_scratch, t->d_m_f + 3 * cb, t->d_m_level + cb, t->d_m_pos + 3 * cb,
+                               t->d_m_point + cb, t->d_m_count + c0, s, &ctx->launches, c0, f0, nf));
     MARK(5); MARK(6);
     chain_export_kernel<<<(nf + 127) / 128, 128, 0, s>>>(nf, t->d_reproj + f0, t->d_px_out + 2 * (size_t)f0, t->d_match_ok + f0); ++ctx->launches;
+    CU_AT("tracker_step: chain_export_kernel", cudaGetLastError());
     if (t->chain_pose_opt) {
       chain_segments_kernel<<<(cnt + 127) / 128, 128, 0, s>>>(cnt, t->chain_cells, t->d_m_count + c0, t->d_seg_begin + c0, t->d_seg_end + c0); ++ctx->launches;
+      CU_AT("tracker_step: chain_segments_kernel", cudaGetLastError());
       // segments are relative to this range's slice of the compacted arrays
-      if (launch_pose_optimize(cam, cnt, t->d_seg_begin + c0, t->d_seg_end + c0, t->d_m_f + 3 * cb, t->d_m_level + cb, t->d_m_pos + 3 * cb, 2.0, 10,
-                               0.0000000001, 8.6851f, t->d_T_cur + 7 * (size_t)c0, t->d_pose + c0, t->d_outlier + cb, t->d_pose_work + cb, s, &ctx->launches))
-        return fail(ctx, SVOB200_ERR_CUDA, "tracker_step: pose_optimize failed");
+      CU_AT("tracker_step: launch_pose_optimize",
+            launch_pose_optimize(cam, cnt, t->d_seg_begin + c0, t->d_seg_end + c0, t->d_m_f + 3 * cb, t->d_m_level + cb, t->d_m_pos + 3 * cb, 2.0, 10,
+                                 0.0000000001, 8.6851f, t->d_T_cur + 7 * (size_t)c0, t->d_pose + c0, t->d_outlier + cb, t->d_pose_work + cb, s, &ctx->launches));
     }
     MARK(7);
   } else {
   // 5. Matcher::findMatchDirect per map point (keyframe patch -> current frame)
   // (item indices inside the call are relative to f0, so the output arrays are passed at f0 as well)
-  if (launch_match_direct(ctx->d_table, cur->slot, cam, nf, t->d_ftrs + f0, t->d_depth_ref + f0, t->d_px_in + 2 * (size_t)f0, t->mopts, nullptr,
-                          t->d_px_out + 2 * (size_t)f0, t->d_match_ok + f0, t->d_match_scratch, t->N, f0, s, &ctx->launches,
-                          (marks && t->profiling) ? &t->ev[5] : nullptr, t->d_active + f0, t->d_match_level + f0, t->d_match_A + 4 * (size_t)f0))
-    return fail(ctx, SVOB200_ERR_CUDA, "tracker_step: match_direct failed");
+  CU_AT("tracker_step: launch_match_direct",
+        launch_match_direct(ctx->d_table, cur->slot, cam, nf, t->d_ftrs + f0, t->d_depth_ref + f0, t->d_px_in + 2 * (size_t)f0, t->mopts, nullptr,
+                            t->d_px_out + 2 * (size_t)f0, t->d_match_ok + f0, t->d_match_scratch, t->N, f0, s, &ctx->launches,
+                            (marks && t->profiling) ? &t->ev[5] : nullptr, t->d_active + f0, t->d_match_level + f0, t->d_match_A + 4 * (size_t)f0));
   MARK(7);
   }
   if (out_px) CU(cudaMemcpyAsync(out_px + 2 * (size_t)f0, t->d_px_out + 2 * (size_t)f0, sizeof(double) * 2 * (size_t)nf, cudaMemcpyDeviceToDevice, s));
   if (out_ok) CU(cudaMemcpyAsync(out_ok + f0, t->d_match_ok + f0, sizeof(int) * (size_t)nf, cudaMemcpyDeviceToDevice, s));
   // 6. DepthFilter::updateSeeds(cur): this range's rows of the pose table (from the step's final T_cur), then the seeds
-  if (launch_seed_pose_table(cam, t->batch, t->n_kfs, c0, cnt, t->d_T_kf, t->d_T_cur, sh.pose_table, s_seeds, &ctx->launches))
-    return fail(ctx, SVOB200_ERR_CUDA, "tracker_step: seed pose table failed");
+  CU_AT("tracker_step: launch_seed_pose_table",
+        launch_seed_pose_table(cam, t->batch, t->n_kfs, c0, cnt, t->d_T_kf, t->d_T_cur, sh.pose_table, s_seeds, &ctx->launches));
   if (sh.defer_df) {
     // asynchronous depth filter (never forked: s_seeds == s): the df stream starts from the pose rows and writes its half of
     // the step records after the tracking half; the events tell it when

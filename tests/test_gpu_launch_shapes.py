@@ -76,7 +76,7 @@ def test_align_case_table_reaches_every_instance():
     """CPU: the case table reaches all six kernel instances of launch_sparse_align, places both sides of every branch,
     mixes small problems into every batch, and the restated rule still reads like the launcher."""
     src = open(os.path.join(ROOT, "android_svo_b200", "csrc", "sparse_align.cu")).read()
-    body = src[src.index("int launch_sparse_align("):]
+    body = src[src.index("cudaError_t launch_sparse_align("):]
     for line in ("if (batch <= 16 && max_per_problem >= 64) cluster = 8;",
                  "else if (batch <= 32 && max_per_problem >= 64) cluster = 4;",
                  "else if (batch <= 64 && max_per_problem >= 128) cluster = 2;",
@@ -317,8 +317,9 @@ def _oracle_reproject(om, oracle, sc, max_fts):
                             oracle.matcher_opts(cfg["n_pyr"]))
 
 
-def _gpu_reproject(ctx, scs, max_fts, cam=None, fid0=9200):
-    """one svob200_reproject_map call over images b = 0.. (scs[b] None: an image without points, frames of scs[0])"""
+def _gpu_reproject(ctx, scs, max_fts, cam=None, fid0=9200, launched=None):
+    """one svob200_reproject_map call over images b = 0.. (scs[b] None: an image without points, frames of scs[0]);
+    launched (a list) receives the kernel launches of that call alone"""
     real = [sc for sc in scs if sc is not None]
     cfg = real[0]["cfg"]
     n_kf = len(real[0]["kf_imgs"])
@@ -339,10 +340,13 @@ def _gpu_reproject(ctx, scs, max_fts, cam=None, fid0=9200):
         gp, go, To = to_gpu_records(sc["pts"], sc["obs_o"], sc["T_kf"], kf_fids, b, obs_base)
         gps.append(gp); gos.append(go); Tos.append(To)
         obs_base += len(go); off.append(off[-1] + len(gp))
+    n0 = ctx.launch_count()
     try:
         got = ctx.reproject_map(fid0, cam or _gcam(cfg), np.stack([sc["T_cur"] for sc in img_of]), off, np.concatenate(gps), np.concatenate(gos),
                                 np.concatenate(Tos), real[0]["cell"], max_fts, ctx.matcher_opts(cfg["n_pyr"]))
     finally:
+        if launched is not None:
+            launched.append(ctx.launch_count() - n0)
         for fid in kf_fids + [fid0]:
             ctx.frame_release(fid)
     return got, off, bases
@@ -387,7 +391,7 @@ def test_reprojector_1080p_grid(ctx, om, oracle, max_fts):
 @pytest.mark.gpu
 def test_reprojector_grid_limit(ctx, om, oracle):
     """A grid of exactly 8,192 cells (2048x1024 at cell 16) is accepted and matches the oracle; one grid row more is
-    refused with SVOB200_ERR_UNSUPPORTED."""
+    refused with SVOB200_ERR_UNSUPPORTED before anything is launched."""
     sc = _map_scene(oracle, WIDE, 7, 100, 16)
     assert -(-WIDE["w"] // 16) * -(-WIDE["h"] // 16) == 8192
     for max_fts in (120, 100000):
@@ -395,8 +399,10 @@ def test_reprojector_grid_limit(ctx, om, oracle):
         assert got[1].shape == (2, 8192)
         _check_images(om, oracle, [sc, None], max_fts, got, off, bases)
     over = capi.Camera.make(WIDE["w"], WIDE["h"] + 1, WIDE["fx"], WIDE["fy"], WIDE["cx"], WIDE["cy"])    # 128 x 65 = 8,320 cells
-    with pytest.raises(capi.Svob200Error, match=r"error -4\b"):
-        _gpu_reproject(ctx, [sc], 120, cam=over)
+    launched = []
+    with pytest.raises(capi.Svob200Error, match=r"error -4\b.*8320 cells exceeds the limit of 8192"):
+        _gpu_reproject(ctx, [sc], 120, cam=over, launched=launched)
+    assert launched == [0], "the refused call launched kernels"
 
 
 # ------------------------------------------------------------------ FAST detection on partial tiles
