@@ -87,6 +87,7 @@ def load_library():
     L.svob200_last_error.restype = C.c_char_p
     L.svob200_ctx_stream.restype = C.c_void_p
     L.svob200_ctx_launch_count.restype = C.c_longlong
+    L.svob200_tracker_device_bytes.restype = C.c_longlong
     V = C.c_void_p
     L.svob200_ctx_create.argtypes = [C.c_int, C.POINTER(V)]
     for name in ("svob200_ctx_destroy", "svob200_ctx_sync", "svob200_ctx_timer_start"):
@@ -131,6 +132,7 @@ def load_library():
     L.svob200_tracker_num_seed_slots.argtypes = [V]
     L.svob200_tracker_set_point_pool.argtypes = [V, C.c_int]
     L.svob200_tracker_num_point_slots.argtypes = [V]
+    L.svob200_tracker_device_bytes.argtypes = [V]
     L.svob200_tracker_get_points.argtypes = [V, V, V, V, V, V]
     L.svob200_tracker_step.argtypes = [V, V, C.c_int, V, V, V, V, V, C.c_int]
     L.svob200_tracker_get_seeds.argtypes = [V, V]
@@ -183,7 +185,7 @@ EXPORTED_SYMBOLS = [
     "svob200_points_optimize", "svob200_seeds_initialize", "svob200_tracker_debug_align", "svob200_tracker_set_chain",
     "svob200_tracker_set_seed_pool", "svob200_tracker_set_detector", "svob200_tracker_add_keyframe", "svob200_tracker_get_seed_refs",
     "svob200_tracker_num_seed_slots", "svob200_tracker_set_point_pool", "svob200_tracker_num_point_slots", "svob200_tracker_get_points",
-    "svob200_tracker_add_keyframes", "svob200_tracker_scene_depth",
+    "svob200_tracker_add_keyframes", "svob200_tracker_scene_depth", "svob200_tracker_device_bytes",
 ]
 
 
@@ -539,6 +541,10 @@ class Tracker:
         cr = np.zeros(self.batch, np.int32); dr = np.zeros(self.batch, np.int32)
         self.ctx._ck(self.L.svob200_tracker_get_points(self.h, _ptr(pos), _ptr(ty), _ptr(no), _ptr(cr), _ptr(dr)))
         return pos[:P], ty[:P], no[:P], cr, dr
+
+    def device_bytes(self):
+        """bytes of device memory the tracker's own arrays hold now (svob200_tracker_device_bytes; frames not included)"""
+        return int(self.L.svob200_tracker_device_bytes(self.h))
 
     def set_detector(self, cell, levels, thr):
         self.ctx._ck(self.L.svob200_tracker_set_detector(self.h, int(cell), int(levels), float(thr)))

@@ -514,6 +514,96 @@ static const char* const kStageNames[kNumStages] = {"frame+pyramid", "features_p
                                                     "match_geom", "match_prepare", "match_refine", "seeds_geom", "seeds_search",
                                                     "seeds_refine", "seeds_finish", "stats"};
 
+// The device arrays of one group, one cudaMalloc each, and their byte total; all are freed with the owner.  Move-only: a
+// move-assignment swaps, so the arrays it replaces are freed when the moved-from temporary goes.
+class DevArrays {
+ public:
+  DevArrays() = default;
+  DevArrays(const DevArrays&) = delete;
+  DevArrays& operator=(const DevArrays&) = delete;
+  DevArrays(DevArrays&& o) noexcept { swap(o); }
+  DevArrays& operator=(DevArrays&& o) noexcept { swap(o); return *this; }
+  ~DevArrays() { for (void* p : ptrs_) cudaFree(p); }
+  // p = an array of n elements (of one element when n == 0: an array that is present is never null); false if it failed
+  template <class T> bool alloc(T*& p, size_t n)
+  {
+    const size_t bytes = sizeof(T) * (n ? n : 1);
+    if (cudaMalloc((void**)&p, bytes) != cudaSuccess) { cudaGetLastError(); return false; }
+    ptrs_.push_back(p);
+    bytes_ += (long long)bytes;
+    return true;
+  }
+  bool empty() const { return ptrs_.empty(); }
+  long long bytes() const { return bytes_; }
+
+ private:
+  void swap(DevArrays& o) { std::swap(ptrs_, o.ptrs_); std::swap(bytes_, o.bytes_); }
+  std::vector<void*> ptrs_;
+  long long bytes_ = 0;
+};
+
+// The tracker's device arrays, grouped by the call that sizes them.  A sizing call builds a whole new group before it changes
+// the tracker and then moves it in, so a failed allocation leaves the tracker as it was.  A group exists once its call made it.
+// Slots (set_keyframe): the point and seed slots of every sequence, the keyframe tables, the step buffers and their scratch.
+struct Slots {
+  DevArrays mem;
+  int *ftr_off = nullptr, *seed_off = nullptr, *ftr_image = nullptr, *match_ok = nullptr;
+  uint8_t* has_point = nullptr;
+  svob200_feature_ref* ftrs = nullptr;            // the observation chosen for each map point in the current step
+  double* pt_world = nullptr;
+  svob200_map_point* points = nullptr;
+  // map points: K = max_kfs observation slots each (points / observations as svob200_reproject_map takes them)
+  svob200_feature_ref* pobs = nullptr; double* T_pobs = nullptr; uint8_t* active = nullptr;
+  int* match_level = nullptr; double* match_A = nullptr;
+  int* sel = nullptr;                    // observation slot currently copied into ftrs[i] (-1: none)
+  // point pool (present only with one): the candidates of the steps of each parity wait in cand[parity] (one entry per point
+  // slot) until two steps later
+  CandRec* cand[2] = {};
+  int* cand_n[2] = {};                   // candidates of the sequence in that step (the entries beyond its slots are dropped)
+  int *pt_created = nullptr, *pt_dropped = nullptr, *pt_rank = nullptr;
+  // keyframe rings: kf_batch[k][b] = Seed::batch_id of ring index k of sequence b (-1: free), batch_counter[b] =
+  // Seed::batch_counter (depth_filter.cpp:139)
+  int *kf_batch = nullptr, *batch_counter = nullptr;
+  int *kf_new = nullptr, *kf_old = nullptr;     // of the latest insertion: the ring index taken / left, per sequence (-1: none)
+  uint8_t* kf_which = nullptr;                  // host-memory insertion masks, staged
+  float *depth_mean = nullptr, *depth_min = nullptr;
+  double* sd_z = nullptr;                // svob200_tracker_scene_depth: the depths of the matched point slots
+  int* sd_n = nullptr;
+  // depth-filter seeds: 32-byte compact records + keyframe tables (pose per (keyframe, image), frame slot per keyframe)
+  SeedRef* seed_refs = nullptr;
+  double* T_kf = nullptr;                // [max_kfs][batch][7]
+  int* kf_slot = nullptr;                // [max_kfs]
+  SeedPoseRec *seed_poses = nullptr, *seed_poses2 = nullptr;   // [max_kfs][batch], refreshed every step (2: odd steps)
+  svob200_seed* seeds = nullptr;
+  double* step_in = nullptr;             // [T_last_w 7B | last_px 2N]
+  double *xyz = nullptr, *T_init = nullptr, *T_cur = nullptr, *depth_ref = nullptr, *px_in = nullptr, *px_out = nullptr;
+  svob200_align_result* align = nullptr;
+  svob200_seed_obs* obs = nullptr;
+  svob200_step_stats *stats = nullptr, *stats2 = nullptr;     // step records (2: odd steps)
+  uint8_t *align_scratch = nullptr, *seed_scratch = nullptr, *match_scratch = nullptr;
+};
+
+// Detector (the first add_keyframes after set_keyframe or after set_detector changed the grid): scratch of n_cells per image
+struct Detector {
+  DevArrays mem;
+  int n_cells = 0;
+  uint8_t* occ = nullptr; unsigned long long* keys = nullptr; svob200_corner* cells = nullptr;
+  int *counts = nullptr, *kf_appended = nullptr, *kf_dropped = nullptr;
+};
+
+// Chain (set_chain on a tracker without one, or with another grid): the reprojector's and the pose optimiser's arrays
+struct Chain {
+  DevArrays mem;
+  int n_cells = 0;
+  svob200_reproj_result* reproj = nullptr;
+  svob200_reproj_stats* rstats = nullptr;
+  svob200_pose_opt_result* pose = nullptr;
+  int *winner = nullptr, *m_level = nullptr, *m_point = nullptr, *m_count = nullptr, *seg_begin = nullptr, *seg_end = nullptr;
+  double *m_f = nullptr, *m_pos = nullptr, *pose_work = nullptr;
+  uint8_t* outlier = nullptr;
+  uint8_t* reproj_scratch = nullptr;
+};
+
 struct svob200_tracker {
   svob200_ctx* ctx = nullptr;
   svob200_camera cam{};
@@ -526,59 +616,25 @@ struct svob200_tracker {
   int64_t uid = 0;                     // frame ids of this tracker: -(uid << 8 | n), n = 1, 2, ... (new_frame)
   int64_t fid_last = 0, fid_cur = 0;
   // keyframes: every sequence has its own ring of max_kfs keyframes.  Ring index k of sequence b is image b of the keyframe
-  // store's frame fid_kfs[k] (frame slot d_kf_slot[k], pose d_T_kf[k][b]); the ring state lives on the device, per sequence:
-  // d_kf_batch[k][b] = Seed::batch_id of that keyframe (-1: free), d_batch_counter[b] = Seed::batch_counter (depth_filter.cpp:139)
+  // store's frame fid_kfs[k] (frame slot slots.kf_slot[k], pose slots.T_kf[k][b]); the ring state lives on the device
   static constexpr int MAX_KFS = 16;
   int64_t fid_kfs[MAX_KFS] = {};
   std::vector<int64_t> frame_pool;     // every frame this tracker created
   int64_t next_fid = 0;
-  int *d_kf_batch = nullptr, *d_batch_counter = nullptr;
-  int *d_kf_new = nullptr, *d_kf_old = nullptr;     // of the latest insertion: the ring index taken / left, per sequence (-1: none)
-  uint8_t* d_kf_which = nullptr;                    // host-memory insertion masks, staged
-  double* d_sd_z = nullptr;            // svob200_tracker_scene_depth: the depths of the matched point slots
-  int* d_sd_n = nullptr;
   int max_n_kfs = 3;                   // DepthFilter::Options::max_n_kfs (depth_filter.h:75)
   int seed_capacity = 0;               // slots per sequence of the seed pool (0: exactly the seeds of set_keyframe)
   int det_cell = 30, det_levels = 3;   // Config::gridSize / nPyrLevels, Config::triangMinCornerScore
   double det_thr = 20.0;
-  uint8_t* d_occ = nullptr; unsigned long long* d_det_keys = nullptr; svob200_corner* d_det_cells = nullptr;
-  int *d_det_counts = nullptr, *d_kf_appended = nullptr, *d_kf_dropped = nullptr;
-  float *d_depth_mean = nullptr, *d_depth_min = nullptr;
-  int det_cells_alloc = 0;
   long long steps_done = 0;
   int N = 0, S = 0, max_per = 0;
-  int *d_ftr_off = nullptr, *d_seed_off = nullptr, *d_ftr_image = nullptr, *d_match_ok = nullptr;
-  uint8_t* d_has_point = nullptr;
-  svob200_feature_ref* d_ftrs = nullptr;            // the observation chosen for each map point in the current step
-  double* d_pt_world = nullptr;
-  // map points: K = max_kfs observation slots each (points / observations as svob200_reproject_map takes them)
-  svob200_feature_ref* d_pobs = nullptr; double* d_T_pobs = nullptr; uint8_t* d_active = nullptr;
-  int* d_match_level = nullptr; double* d_match_A = nullptr;
-  int* d_sel = nullptr;                    // observation slot currently copied into d_ftrs[i] (-1: none)
-  // point pool (svob200_tracker_set_point_pool): every sequence owns max(its set_keyframe points, pt_capacity) point slots;
-  // the candidates of the steps of each parity wait in d_cand[parity] (one entry per point slot) until two steps later
-  int pt_capacity = -1;                    // -1: no pool
-  CandRec* d_cand[2] = {};
-  int* d_cand_n[2] = {};                   // candidates of the sequence in that step (the entries beyond its slots are dropped)
-  int *d_pt_created = nullptr, *d_pt_dropped = nullptr, *d_pt_rank = nullptr;
-  // depth-filter seeds: 32-byte compact records + keyframe tables (pose per (keyframe, image), frame slot per keyframe)
-  SeedRef* d_seed_refs = nullptr;
-  double* d_T_kf = nullptr;            // [max_kfs][batch][7]
-  int* d_kf_slot = nullptr;            // [max_kfs]
-  SeedPoseRec* d_seed_poses = nullptr; // [max_kfs][batch], refreshed every step
+  // point pool (svob200_tracker_set_point_pool): every sequence owns max(its set_keyframe points, pt_capacity) point slots
+  int pt_capacity = -1;                // -1: no pool
   int n_kfs = 1;                       // rows of the tables in use (no sequence has more keyframes: min(max_kfs, 1 + insertions))
   int max_kfs = 4;                     // keyframe ring (svob200_tracker_set_keyframe_ring)
-  svob200_seed* d_seeds = nullptr;
-  double *d_step_in = nullptr;      // [T_last_w 7B | last_px 2N]
-  double *d_xyz = nullptr, *d_T_init = nullptr, *d_T_cur = nullptr, *d_depth_ref = nullptr, *d_px_in = nullptr, *d_px_out = nullptr;
-  svob200_align_result* d_align = nullptr;
-  svob200_seed_obs* d_obs = nullptr;
-  svob200_step_stats* d_stats = nullptr;
-  uint8_t* d_align_scratch = nullptr;
-  uint8_t* d_seed_scratch = nullptr;
-  uint8_t* d_match_scratch = nullptr;
+  Slots slots;
+  Detector det;
+  Chain chain;
   uint8_t* h_pinned = nullptr; size_t h_cap = 0;
-  std::vector<void*> owned;
   std::vector<int> h_ftr_off, h_seed_off;
   static constexpr int CHUNK = 256;    // sequences per H2D/compute pipeline chunk (host mode)
   // Asynchronous depth filter (device-memory steps of big batches): like the reference, whose DepthFilter runs in its own
@@ -591,20 +647,10 @@ struct svob200_tracker {
   cudaEvent_t df_done[2] = {}, ev_pose = nullptr, ev_track = nullptr;
   bool df_pending[2] = {false, false};
   long long step_no = 0;
-  SeedPoseRec* d_seed_poses2 = nullptr;      // second pose table (odd steps)
-  svob200_step_stats* d_stats2 = nullptr;    // second step-record array (odd steps)
   cudaStream_t copy_stream = nullptr;
   std::vector<cudaEvent_t> chunk_ev;
   // chain mode (svob200_tracker_set_chain): reprojector grid rules + pose optimiser instead of refining every map point
-  int chain_cell = 0, chain_max_fts = 0, chain_pose_opt = 0, chain_cells = 0;
-  svob200_map_point* d_points = nullptr;
-  svob200_reproj_result* d_reproj = nullptr;
-  svob200_reproj_stats* d_rstats = nullptr;
-  svob200_pose_opt_result* d_pose = nullptr;
-  int *d_winner = nullptr, *d_m_level = nullptr, *d_m_point = nullptr, *d_m_count = nullptr, *d_seg_begin = nullptr, *d_seg_end = nullptr;
-  double *d_m_f = nullptr, *d_m_pos = nullptr, *d_pose_work = nullptr;
-  uint8_t* d_outlier = nullptr;
-  uint8_t* d_reproj_scratch = nullptr;
+  int chain_cell = 0, chain_max_fts = 0, chain_pose_opt = 0;
   // single-stream latency: in device mode with small batches the 14 launches of a step are replayed as ONE CUDA graph
   // (captured once per distinct set of buffer addresses: a camera ring buffer has only a few), which removes the
   // per-launch driver cost and most of the inter-kernel gaps
@@ -619,15 +665,6 @@ struct svob200_tracker {
   bool profiling = false;
   cudaEvent_t ev[kNumStages + 1] = {};
 };
-
-// a device buffer of n elements that the tracker owns (freed by svob200_tracker_destroy)
-template <class T> static int alloc_owned(svob200_tracker* t, T*& p, size_t n)
-{
-  p = nullptr;
-  if (cudaMalloc((void**)&p, sizeof(T) * (n ? n : 1)) != cudaSuccess) { cudaGetLastError(); return fail(t->ctx, SVOB200_ERR_NOMEM, "tracker: device alloc of %zu bytes failed", sizeof(T) * n); }
-  t->owned.push_back(p);
-  return 0;
-}
 
 // a new frame of the tracker's pool
 static int new_frame(svob200_tracker* t, int64_t* out_id)
@@ -694,13 +731,13 @@ static int graph_or_direct(svob200_tracker* t, bool use_graph, const std::vector
   return 0;
 }
 
-// the frame slot of every store frame that exists (d_kf_slot, constant once the store is complete)
+// the frame slot of every store frame that exists (slots.kf_slot, constant once the store is complete)
 static int upload_kf_slots(svob200_tracker* t)
 {
   svob200_ctx* ctx = t->ctx;
   int slots[svob200_tracker::MAX_KFS] = {};
   for (int k = 0; k < t->max_kfs; ++k) if (t->fid_kfs[k]) slots[k] = svob200_frame_slot(ctx, t->fid_kfs[k]);
-  CU(cudaMemcpyAsync(t->d_kf_slot, slots, sizeof(int) * t->max_kfs, cudaMemcpyHostToDevice, ctx->stream));
+  CU(cudaMemcpyAsync(t->slots.kf_slot, slots, sizeof(int) * t->max_kfs, cudaMemcpyHostToDevice, ctx->stream));
   return 0;
 }
 
@@ -740,7 +777,6 @@ void svob200_tracker_destroy(svob200_tracker* t)
   ctx_join_aux(ctx);
   cudaStreamSynchronize(ctx->stream);
   for (int64_t id : t->frame_pool) svob200_frame_release(ctx, id);
-  for (void* p : t->owned) cudaFree(p);
   if (t->h_pinned) cudaFreeHost(t->h_pinned);
   for (auto e : t->chunk_ev) cudaEventDestroy(e);
   drop_graphs(t);
@@ -763,7 +799,7 @@ int svob200_tracker_set_keyframe(svob200_tracker* t, const uint8_t* imgs, int st
 {
   if (!t || !imgs || !T_kf_w || !ftr_offsets || !seed_offsets) return SVOB200_ERR_ARG;
   svob200_ctx* ctx = t->ctx;
-  if (t->d_stats) return fail(ctx, SVOB200_ERR_UNSUPPORTED, "tracker_set_keyframe: keyframe already set (svob200_tracker_add_keyframe inserts further ones)");
+  if (!t->slots.mem.empty()) return fail(ctx, SVOB200_ERR_UNSUPPORTED, "tracker_set_keyframe: keyframe already set (svob200_tracker_add_keyframe inserts further ones)");
   const int B = t->batch;
   const int N_in = ftr_offsets[B];
   const int S_in = seed_offsets[B];
@@ -785,50 +821,48 @@ int svob200_tracker_set_keyframe(svob200_tracker* t, const uint8_t* imgs, int st
   };
   const std::vector<int> pt_off = slot_offsets(ftr_offsets, t->pt_capacity), pool_off = slot_offsets(seed_offsets, t->seed_capacity);
   const int N = pt_off[B], S = pool_off[B];
-  t->N = N; t->S = S;
+  int max_per = 0;
+  for (int b = 0; b < B; ++b) max_per = std::max(max_per, pt_off[b + 1] - pt_off[b]);
+  const int slot = svob200_frame_slot(ctx, t->fid_kfs[0]);
+  const size_t K = t->max_kfs;
+  Slots g;
+  DevArrays& m = g.mem;
+  bool ok = m.alloc(g.ftr_off, B + 1) && m.alloc(g.seed_off, B + 1) && m.alloc(g.ftr_image, N) && m.alloc(g.match_ok, N) && m.alloc(g.has_point, N) &&
+            m.alloc(g.ftrs, N) && m.alloc(g.seed_refs, S) && m.alloc(g.pt_world, 3 * (size_t)N) &&
+            m.alloc(g.pobs, N * K) && m.alloc(g.T_pobs, 7 * (size_t)N * K) && m.alloc(g.active, N) && m.alloc(g.match_level, N) && m.alloc(g.match_A, 4 * (size_t)N) &&
+            m.alloc(g.sel, N) && m.alloc(g.points, N) &&
+            m.alloc(g.T_kf, 7 * (size_t)B * K) && m.alloc(g.kf_slot, K) && m.alloc(g.seed_poses, B * K) && m.alloc(g.seed_poses2, B * K) &&
+            m.alloc(g.seeds, S) && m.alloc(g.step_in, 7 * (size_t)B + 2 * (size_t)N) && m.alloc(g.xyz, 3 * (size_t)N) && m.alloc(g.T_init, 7 * (size_t)B) &&
+            m.alloc(g.T_cur, 7 * (size_t)B) && m.alloc(g.depth_ref, N) && m.alloc(g.px_in, 2 * (size_t)N) && m.alloc(g.px_out, 2 * (size_t)N) &&
+            m.alloc(g.align, B) && m.alloc(g.obs, S) && m.alloc(g.stats, B) && m.alloc(g.stats2, B) &&
+            m.alloc(g.kf_batch, B * K) && m.alloc(g.batch_counter, B) && m.alloc(g.kf_new, B) && m.alloc(g.kf_old, B) && m.alloc(g.kf_which, B) &&
+            m.alloc(g.depth_mean, B) && m.alloc(g.depth_min, B) && m.alloc(g.sd_n, B) && m.alloc(g.sd_z, N) &&
+            m.alloc(g.align_scratch, sparse_align_scratch_bytes(N)) && m.alloc(g.seed_scratch, seeds_scratch_bytes(S)) &&
+            m.alloc(g.match_scratch, match_scratch_bytes(N));
+  if (ok && t->pt_capacity >= 0)
+    ok = m.alloc(g.cand[0], N) && m.alloc(g.cand_n[0], B) && m.alloc(g.cand[1], N) && m.alloc(g.cand_n[1], B) && m.alloc(g.pt_created, B) &&
+         m.alloc(g.pt_dropped, B) && m.alloc(g.pt_rank, N);
+  if (!ok) return fail(ctx, SVOB200_ERR_NOMEM, "tracker_set_keyframe: out of device memory for the slot arrays");
+  t->slots = std::move(g);
+  t->N = N; t->S = S; t->max_per = max_per;
   t->h_ftr_off = pt_off;
   t->h_seed_off = pool_off;
-  for (int b = 0; b < B; ++b) t->max_per = std::max(t->max_per, pt_off[b + 1] - pt_off[b]);
-  const int slot = svob200_frame_slot(ctx, t->fid_kfs[0]);
   t->n_kfs = 1;
-  int err = 0;
-  auto own = [&](auto*& p, size_t n) { if (!err) err = alloc_owned(t, p, n); };
-  own(t->d_ftr_off, B + 1); own(t->d_seed_off, B + 1); own(t->d_ftr_image, N); own(t->d_match_ok, N); own(t->d_has_point, N);
-  own(t->d_ftrs, N); own(t->d_seed_refs, S); own(t->d_pt_world, 3 * (size_t)N);
-  own(t->d_pobs, (size_t)N * t->max_kfs); own(t->d_T_pobs, 7 * (size_t)N * t->max_kfs); own(t->d_active, N); own(t->d_match_level, N); own(t->d_match_A, 4 * (size_t)N); own(t->d_sel, N);
-  own(t->d_points, N);
-  own(t->d_T_kf, 7 * (size_t)B * t->max_kfs); own(t->d_kf_slot, t->max_kfs); own(t->d_seed_poses, (size_t)B * t->max_kfs); own(t->d_seed_poses2, (size_t)B * t->max_kfs);
-  own(t->d_seeds, S); own(t->d_step_in, 7 * (size_t)B + 2 * (size_t)N); own(t->d_xyz, 3 * (size_t)N); own(t->d_T_init, 7 * (size_t)B);
-  own(t->d_T_cur, 7 * (size_t)B); own(t->d_depth_ref, N); own(t->d_px_in, 2 * (size_t)N); own(t->d_px_out, 2 * (size_t)N);
-  own(t->d_align, B); own(t->d_obs, S); own(t->d_stats, B); own(t->d_stats2, B);
-  own(t->d_kf_batch, (size_t)B * t->max_kfs); own(t->d_batch_counter, B); own(t->d_kf_new, B); own(t->d_kf_old, B); own(t->d_kf_which, B);
-  own(t->d_depth_mean, B); own(t->d_depth_min, B); own(t->d_sd_n, B); own(t->d_sd_z, N);
-  own(t->d_align_scratch, sparse_align_scratch_bytes(N)); own(t->d_seed_scratch, seeds_scratch_bytes(S)); own(t->d_match_scratch, match_scratch_bytes(N));
-  if (t->pt_capacity >= 0) {
-    for (int p = 0; p < 2; ++p) { own(t->d_cand[p], N); own(t->d_cand_n[p], B); }
-    own(t->d_pt_created, B); own(t->d_pt_dropped, B); own(t->d_pt_rank, N);
-  }
-  if (err) {                 // an allocation that failed leaves the tracker as it was before the call (it can be retried or destroyed)
-    for (void* q : t->owned) cudaFree(q);
-    t->owned.clear();
-    t->N = t->S = 0; t->max_per = 0; t->d_stats = nullptr; t->d_reproj = nullptr; t->det_cells_alloc = 0; t->d_det_counts = nullptr; t->d_kf_batch = nullptr;
-    return err;
-  }
   cudaStream_t s = ctx->stream;
-  CU(cudaMemcpyAsync(t->d_ftr_off, pt_off.data(), sizeof(int) * (B + 1), cudaMemcpyHostToDevice, s));
-  CU(cudaMemcpyAsync(t->d_seed_off, pool_off.data(), sizeof(int) * (B + 1), cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(t->slots.ftr_off, pt_off.data(), sizeof(int) * (B + 1), cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(t->slots.seed_off, pool_off.data(), sizeof(int) * (B + 1), cudaMemcpyHostToDevice, s));
   if (t->pt_capacity >= 0) {
-    for (int p = 0; p < 2; ++p) CU(cudaMemsetAsync(t->d_cand_n[p], 0, sizeof(int) * B, s));
-    CU(cudaMemsetAsync(t->d_pt_created, 0, sizeof(int) * B, s));
-    CU(cudaMemsetAsync(t->d_pt_dropped, 0, sizeof(int) * B, s));
+    for (int p = 0; p < 2; ++p) CU(cudaMemsetAsync(t->slots.cand_n[p], 0, sizeof(int) * B, s));
+    CU(cudaMemsetAsync(t->slots.pt_created, 0, sizeof(int) * B, s));
+    CU(cudaMemsetAsync(t->slots.pt_dropped, 0, sizeof(int) * B, s));
   }
   // every ring index starts with keyframe 0's pose: the pose table of a step covers rows whose index a sequence has not used yet
-  for (int k = 0; k < t->max_kfs; ++k) CU(cudaMemcpyAsync(t->d_T_kf + 7 * (size_t)B * k, T_kf_w, sizeof(double) * 7 * B, cudaMemcpyHostToDevice, s));
+  for (int k = 0; k < t->max_kfs; ++k) CU(cudaMemcpyAsync(t->slots.T_kf + 7 * (size_t)B * k, T_kf_w, sizeof(double) * 7 * B, cudaMemcpyHostToDevice, s));
   {                                                      // every sequence's ring holds keyframe 0 (batch id 0), nothing else
     std::vector<int> kb((size_t)B * t->max_kfs, -1);
     std::fill(kb.begin(), kb.begin() + B, 0);
-    CU(cudaMemcpyAsync(t->d_kf_batch, kb.data(), sizeof(int) * kb.size(), cudaMemcpyHostToDevice, s));
-    CU(cudaMemsetAsync(t->d_batch_counter, 0, sizeof(int) * B, s));
+    CU(cudaMemcpyAsync(t->slots.kf_batch, kb.data(), sizeof(int) * kb.size(), cudaMemcpyHostToDevice, s));
+    CU(cudaMemsetAsync(t->slots.batch_counter, 0, sizeof(int) * B, s));
   }
   if (int e = upload_kf_slots(t)) return e;
   // the caller's arrays in one copy; every point slot and seed slot is written on the device
@@ -840,10 +874,10 @@ int svob200_tracker_set_keyframe(svob200_tracker* t, const uint8_t* imgs, int st
   if (int e = st.layout()) return e;
   if (int e = st.push()) return e;
   if (N || S) {
-    kf_init_slots_kernel<<<B, 128, 0, s>>>(to_cam(&t->cam), t->max_kfs, slot, t->d_T_kf, t->d_ftr_off, st.dev<int>(i_fo), st.dev<double>(i_px),
-                                           st.dev<int>(i_lv), st.dev<double>(i_pt), t->d_seed_off, st.dev<int>(i_so), st.dev<double>(i_spx),
-                                           st.dev<int>(i_slv), t->seed_init, t->d_ftr_image, t->d_has_point, t->d_sel, t->d_pt_world, t->d_ftrs,
-                                           t->d_points, t->d_pobs, t->d_T_pobs, t->d_seed_refs, t->d_seeds);
+    kf_init_slots_kernel<<<B, 128, 0, s>>>(to_cam(&t->cam), t->max_kfs, slot, t->slots.T_kf, t->slots.ftr_off, st.dev<int>(i_fo), st.dev<double>(i_px),
+                                           st.dev<int>(i_lv), st.dev<double>(i_pt), t->slots.seed_off, st.dev<int>(i_so), st.dev<double>(i_spx),
+                                           st.dev<int>(i_slv), t->seed_init, t->slots.ftr_image, t->slots.has_point, t->slots.sel, t->slots.pt_world, t->slots.ftrs,
+                                           t->slots.points, t->slots.pobs, t->slots.T_pobs, t->slots.seed_refs, t->slots.seeds);
     ++ctx->launches;
     CU_AT("tracker_set_keyframe: kf_init_slots_kernel", cudaGetLastError());
   }
@@ -854,7 +888,7 @@ int svob200_tracker_set_seed_pool(svob200_tracker* t, int capacity_per_sequence,
 {
   if (!t) return SVOB200_ERR_ARG;
   svob200_ctx* ctx = t->ctx;
-  if (t->d_stats) return fail(ctx, SVOB200_ERR_ARG, "tracker_set_seed_pool: call before set_keyframe");
+  if (!t->slots.mem.empty()) return fail(ctx, SVOB200_ERR_ARG, "tracker_set_seed_pool: call before set_keyframe");
   if (capacity_per_sequence < 0 || max_keyframes < 1 || max_keyframes > svob200_tracker::MAX_KFS || max_n_kfs < 0 || reseed < 0 || reseed > 3)
     return fail(ctx, SVOB200_ERR_ARG, "tracker_set_seed_pool: bad arguments");
   t->seed_capacity = capacity_per_sequence; t->max_kfs = max_keyframes; t->max_n_kfs = max_n_kfs; t->reseed = reseed;
@@ -868,7 +902,7 @@ int svob200_tracker_set_point_pool(svob200_tracker* t, int capacity_per_sequence
 {
   if (!t) return SVOB200_ERR_ARG;
   svob200_ctx* ctx = t->ctx;
-  if (t->d_stats) return fail(ctx, SVOB200_ERR_ARG, "tracker_set_point_pool: call before set_keyframe");
+  if (!t->slots.mem.empty()) return fail(ctx, SVOB200_ERR_ARG, "tracker_set_point_pool: call before set_keyframe");
   if (capacity_per_sequence < 0) return fail(ctx, SVOB200_ERR_ARG, "tracker_set_point_pool: negative capacity %d", capacity_per_sequence);
   t->pt_capacity = capacity_per_sequence;
   return SVOB200_OK;
@@ -881,6 +915,12 @@ int svob200_tracker_set_detector(svob200_tracker* t, int cell_size, int n_detect
   if (cell_size <= 0 || n_detect_levels < 1 || n_detect_levels > t->n_levels) return fail(ctx, SVOB200_ERR_ARG, "tracker_set_detector: bad arguments");
   const long long n_cells = grid_cells(t->cam.width, t->cam.height, cell_size);
   if (n_cells > kMaxGridCells) return fail(ctx, SVOB200_ERR_UNSUPPORTED, "tracker_set_detector: grid of %lld cells exceeds the limit of %d", n_cells, kMaxGridCells);
+  // a grid of another size releases the detector scratch (the next insertion makes it anew) once no insertion reads it
+  if (!t->det.mem.empty() && t->det.n_cells != n_cells) {
+    if (int e = ctx_join_aux(ctx)) return e;
+    CU(cudaStreamSynchronize(ctx->stream));
+    t->det = Detector();
+  }
   t->det_cell = cell_size; t->det_levels = n_detect_levels; t->det_thr = detection_threshold;
   return SVOB200_OK;
 }
@@ -894,93 +934,96 @@ int svob200_tracker_add_keyframes(svob200_tracker* t, const uint8_t* which, cons
   if (!t || !depth_mean || !depth_min) return SVOB200_ERR_ARG;
   svob200_ctx* ctx = t->ctx;
   if (mem != SVOB200_MEM_HOST && mem != SVOB200_MEM_DEVICE) return fail(ctx, SVOB200_ERR_ARG, "tracker_add_keyframes: bad mem %d", mem);
-  if (!t->d_stats || t->steps_done == 0) return fail(ctx, SVOB200_ERR_ARG, "tracker_add_keyframes: needs a keyframe and at least one step");
+  if (t->slots.mem.empty() || t->steps_done == 0) return fail(ctx, SVOB200_ERR_ARG, "tracker_add_keyframes: needs a keyframe and at least one step");
   if (t->chain_cell > 0) return fail(ctx, SVOB200_ERR_UNSUPPORTED, "tracker_add_keyframes: not available in chain mode");
   const int B = t->batch, N = t->N, S = t->S;
   const long long grid = grid_cells(t->cam.width, t->cam.height, t->det_cell);
   if (grid > kMaxGridCells) return fail(ctx, SVOB200_ERR_UNSUPPORTED, "tracker_add_keyframes: grid of %lld cells exceeds the limit of %d", grid, kMaxGridCells);
   const int gc = (t->cam.width + t->det_cell - 1) / t->det_cell, gr = (t->cam.height + t->det_cell - 1) / t->det_cell, n_cells = (int)grid;
   cudaStream_t s = ctx->stream;
-  // the keyframe store (allocated here when set_seed_pool did not) and the detector scratch
+  // the detector scratch when the tracker has none (after set_keyframe, or after set_detector released it once no work in
+  // flight used it), then the keyframe store when set_seed_pool did not make it; the scratch goes in once both exist
+  Detector det;
+  if (t->det.mem.empty()) {
+    const size_t M = (size_t)B * n_cells;
+    DevArrays& m = det.mem;
+    if (!(m.alloc(det.occ, M) && m.alloc(det.keys, M) && m.alloc(det.cells, M) && m.alloc(det.counts, B) && m.alloc(det.kf_appended, B) &&
+          m.alloc(det.kf_dropped, B)))
+      return fail(ctx, SVOB200_ERR_NOMEM, "tracker_add_keyframes: out of device memory for the detector scratch");
+    det.n_cells = n_cells;
+  }
   bool new_store = false;
   for (int k = 1; k < t->max_kfs; ++k)
     if (!t->fid_kfs[k]) { if (int e = new_frame(t, &t->fid_kfs[k])) return e; new_store = true; }
   if (new_store) if (int e = upload_kf_slots(t)) return e;
-  if (t->det_cells_alloc < n_cells) {
-    const size_t M = (size_t)B * n_cells;
-    int err = 0;
-    auto own = [&](auto*& p, size_t n) { if (!err) err = alloc_owned(t, p, n); };
-    own(t->d_occ, M); own(t->d_det_keys, M); own(t->d_det_cells, M);
-    if (!t->d_det_counts) { own(t->d_det_counts, B); own(t->d_kf_appended, B); own(t->d_kf_dropped, B); }
-    if (err) return err;
-    t->det_cells_alloc = n_cells;
-  }
+  if (t->det.mem.empty()) t->det = std::move(det);
   if (int e = df_join(t)) return e;                        // the depth filter of the last step may still be running
   const float *d_dm = depth_mean, *d_dn = depth_min;
   const uint8_t* d_which = which;
   if (mem == SVOB200_MEM_HOST) {
-    CU(cudaMemcpyAsync(t->d_depth_mean, depth_mean, sizeof(float) * B, cudaMemcpyHostToDevice, s));
-    CU(cudaMemcpyAsync(t->d_depth_min, depth_min, sizeof(float) * B, cudaMemcpyHostToDevice, s));
-    if (which) CU(cudaMemcpyAsync(t->d_kf_which, which, (size_t)B, cudaMemcpyHostToDevice, s));
-    d_dm = t->d_depth_mean; d_dn = t->d_depth_min; d_which = which ? t->d_kf_which : nullptr;
+    CU(cudaMemcpyAsync(t->slots.depth_mean, depth_mean, sizeof(float) * B, cudaMemcpyHostToDevice, s));
+    CU(cudaMemcpyAsync(t->slots.depth_min, depth_min, sizeof(float) * B, cudaMemcpyHostToDevice, s));
+    if (which) CU(cudaMemcpyAsync(t->slots.kf_which, which, (size_t)B, cudaMemcpyHostToDevice, s));
+    d_dm = t->slots.depth_mean; d_dn = t->slots.depth_min; d_which = which ? t->slots.kf_which : nullptr;
   }
   // 1. every selected sequence's ring index: a free one, else its oldest keyframe leaves (its seeds with it: removeKeyframe)
   const bool may_evict = t->n_kfs == t->max_kfs;           // (no sequence holds more keyframes than n_kfs)
-  kf_select_kernel<<<(B + 127) / 128, 128, 0, s>>>(B, t->max_kfs, d_which, t->d_kf_batch, t->d_batch_counter, t->d_kf_new, t->d_kf_old, t->d_T_cur, t->d_T_kf);
+  kf_select_kernel<<<(B + 127) / 128, 128, 0, s>>>(B, t->max_kfs, d_which, t->slots.kf_batch, t->slots.batch_counter, t->slots.kf_new, t->slots.kf_old,
+                                                   t->slots.T_cur, t->slots.T_kf);
   ++ctx->launches;
   CU_AT("tracker_add_keyframes: kf_select_kernel", cudaGetLastError());
   if (!may_evict) { t->n_kfs = std::min(t->max_kfs, t->n_kfs + 1); drop_graphs(t); }   // captured steps hold n_kfs
   if (may_evict) {
     if (S) {
-      kf_erase_seeds_kernel<<<(S + 255) / 256, 256, 0, s>>>(S, t->d_seed_refs, t->d_kf_old); ++ctx->launches;
+      kf_erase_seeds_kernel<<<(S + 255) / 256, 256, 0, s>>>(S, t->slots.seed_refs, t->slots.kf_old); ++ctx->launches;
       CU_AT("tracker_add_keyframes: kf_erase_seeds_kernel", cudaGetLastError());
     }
     if (N) {                                                 // Map::safeDeleteFrame: the points forget the keyframe
       if (t->pt_capacity >= 0) {
-        kf_drop_candidates_kernel<<<(N + 255) / 256, 256, 0, s>>>(N, t->d_points, t->d_pobs, t->d_match_ok, t->d_has_point, t->d_ftr_image, t->d_kf_old,
-                                                                  t->d_kf_slot);
+        kf_drop_candidates_kernel<<<(N + 255) / 256, 256, 0, s>>>(N, t->slots.points, t->slots.pobs, t->slots.match_ok, t->slots.has_point, t->slots.ftr_image, t->slots.kf_old,
+                                                                  t->slots.kf_slot);
         ++ctx->launches;
         CU_AT("tracker_add_keyframes: kf_drop_candidates_kernel", cudaGetLastError());
       }
-      kf_drop_obs_kernel<<<(N + 255) / 256, 256, 0, s>>>(N, t->max_kfs, t->d_points, t->d_pobs, t->d_T_pobs, t->d_ftr_image, t->d_kf_old, t->d_kf_slot,
-                                                         t->d_sel);
+      kf_drop_obs_kernel<<<(N + 255) / 256, 256, 0, s>>>(N, t->max_kfs, t->slots.points, t->slots.pobs, t->slots.T_pobs, t->slots.ftr_image, t->slots.kf_old, t->slots.kf_slot,
+                                                         t->slots.sel);
       ++ctx->launches;
       CU_AT("tracker_add_keyframes: kf_drop_obs_kernel", cudaGetLastError());
     }
   }
   // 2. the frame: the last step's current frame (now `last`), every level, into the store
   FrameRec* r = resident_frame(ctx, t->fid_last, "tracker_add_keyframes"); if (!r) return SVOB200_ERR_NOFRAME;
-  kf_store_copy_kernel<<<dim3(16, B), 256, 0, s>>>(r->f, ctx->d_table, t->d_kf_slot, t->d_kf_new);
+  kf_store_copy_kernel<<<dim3(16, B), 256, 0, s>>>(r->f, ctx->d_table, t->slots.kf_slot, t->slots.kf_new);
   ++ctx->launches;
   CU_AT("tracker_add_keyframes: kf_store_copy_kernel", cudaGetLastError());
   // 3. occupancy from the frame's features (the map points matched in it), FAST + Shi-Tomasi + grid on the selected images,
   // one seed per new corner
-  CU(cudaMemsetAsync(t->d_occ, 0, (size_t)B * n_cells, s));
+  CU(cudaMemsetAsync(t->det.occ, 0, (size_t)B * n_cells, s));
   if (N) {
-    kf_occupancy_kernel<<<(N + 255) / 256, 256, 0, s>>>(N, t->d_ftr_image, t->d_px_out, t->d_match_ok, t->d_kf_new, t->det_cell, gc, n_cells, t->d_occ);
+    kf_occupancy_kernel<<<(N + 255) / 256, 256, 0, s>>>(N, t->slots.ftr_image, t->slots.px_out, t->slots.match_ok, t->slots.kf_new, t->det_cell, gc, n_cells, t->det.occ);
     ++ctx->launches;
     CU_AT("tracker_add_keyframes: kf_occupancy_kernel", cudaGetLastError());
   }
   CU_AT("tracker_add_keyframes: launch_fast_detect",
-        launch_fast_detect(r->f, t->det_levels, t->det_cell, gc, gr, t->det_thr, t->d_occ, t->d_det_keys, t->d_det_cells, t->d_det_counts, s, &ctx->launches,
-                           t->d_kf_new));
-  kf_append_seeds_kernel<<<B, 256, 0, s>>>(to_cam(&t->cam), t->d_det_cells, n_cells, t->det_thr, d_dm, d_dn, t->d_seed_off, t->d_seed_refs,
-                                           t->d_seeds, t->d_kf_new, t->d_batch_counter, t->d_kf_appended, t->d_kf_dropped);
+        launch_fast_detect(r->f, t->det_levels, t->det_cell, gc, gr, t->det_thr, t->det.occ, t->det.keys, t->det.cells, t->det.counts, s, &ctx->launches,
+                           t->slots.kf_new));
+  kf_append_seeds_kernel<<<B, 256, 0, s>>>(to_cam(&t->cam), t->det.cells, n_cells, t->det_thr, d_dm, d_dn, t->slots.seed_off, t->slots.seed_refs,
+                                           t->slots.seeds, t->slots.kf_new, t->slots.batch_counter, t->det.kf_appended, t->det.kf_dropped);
   ++ctx->launches;
   CU_AT("tracker_add_keyframes: kf_append_seeds_kernel", cudaGetLastError());
   // 4. the matched map points gain an observation in the new keyframe (frame_handler_mono.cpp:277-279)
   if (N) {
-    kf_add_obs_kernel<<<(N + 255) / 256, 256, 0, s>>>(to_cam(&t->cam), N, t->max_kfs, t->d_points, t->d_pobs, t->d_T_pobs, t->d_ftr_image, t->d_match_ok, t->d_px_out,
-                                                      t->d_match_level, t->d_kf_new, t->d_kf_slot, t->d_T_cur);
+    kf_add_obs_kernel<<<(N + 255) / 256, 256, 0, s>>>(to_cam(&t->cam), N, t->max_kfs, t->slots.points, t->slots.pobs, t->slots.T_pobs, t->slots.ftr_image,
+                                                      t->slots.match_ok, t->slots.px_out, t->slots.match_level, t->slots.kf_new, t->slots.kf_slot, t->slots.T_cur);
     ++ctx->launches;
     CU_AT("tracker_add_keyframes: kf_add_obs_kernel", cudaGetLastError());
   }
   // the counts (unselected sequences: 0, refused ones: -1).  Without a seed pool n_dropped repeats n_new_seeds, and is 0 when
   // n_new_seeds is not asked for (as svob200_tracker_add_keyframe always reported it)
   const cudaMemcpyKind kind = mem == SVOB200_MEM_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
-  if (n_new_seeds) CU(cudaMemcpyAsync(n_new_seeds, t->d_kf_appended, sizeof(int) * B, kind, s));
+  if (n_new_seeds) CU(cudaMemcpyAsync(n_new_seeds, t->det.kf_appended, sizeof(int) * B, kind, s));
   const bool zero_dropped = n_dropped && !S && !n_new_seeds;
-  if (n_dropped && !zero_dropped) CU(cudaMemcpyAsync(n_dropped, t->d_kf_dropped, sizeof(int) * B, kind, s));
+  if (n_dropped && !zero_dropped) CU(cudaMemcpyAsync(n_dropped, t->det.kf_dropped, sizeof(int) * B, kind, s));
   if (zero_dropped && mem == SVOB200_MEM_DEVICE) CU(cudaMemsetAsync(n_dropped, 0, sizeof(int) * B, s));
   if (mem == SVOB200_MEM_HOST) CU(cudaStreamSynchronize(s));   // depth_mean / depth_min / which are the caller's; the counts go back
   if (zero_dropped && mem == SVOB200_MEM_HOST) memset(n_dropped, 0, sizeof(int) * B);
@@ -997,20 +1040,20 @@ int svob200_tracker_scene_depth(svob200_tracker* t, float* depth_mean, float* de
   if (!t || !depth_mean || !depth_min) return SVOB200_ERR_ARG;
   svob200_ctx* ctx = t->ctx;
   if (mem != SVOB200_MEM_HOST && mem != SVOB200_MEM_DEVICE) return fail(ctx, SVOB200_ERR_ARG, "tracker_scene_depth: bad mem %d", mem);
-  if (!t->d_stats || t->steps_done == 0) return fail(ctx, SVOB200_ERR_ARG, "tracker_scene_depth: needs a keyframe and at least one step");
+  if (t->slots.mem.empty() || t->steps_done == 0) return fail(ctx, SVOB200_ERR_ARG, "tracker_scene_depth: needs a keyframe and at least one step");
   const int B = t->batch;
   cudaStream_t s = ctx->stream;
   const bool dev = mem == SVOB200_MEM_DEVICE;
-  scene_depth_kernel<<<B, 128, 0, s>>>(t->d_ftr_off, t->d_points, t->d_match_ok, t->d_T_cur, t->d_sd_z, dev ? depth_mean : t->d_depth_mean,
-                                       dev ? depth_min : t->d_depth_min, dev ? n_points : t->d_sd_n);
+  scene_depth_kernel<<<B, 128, 0, s>>>(t->slots.ftr_off, t->slots.points, t->slots.match_ok, t->slots.T_cur, t->slots.sd_z, dev ? depth_mean : t->slots.depth_mean,
+                                       dev ? depth_min : t->slots.depth_min, dev ? n_points : t->slots.sd_n);
   ++ctx->launches;
   CU_AT("tracker_scene_depth: scene_depth_kernel", cudaGetLastError());
   if (dev) return SVOB200_OK;
   std::vector<float> dm(B), dn(B);
   std::vector<int> n(B);
-  CU(cudaMemcpyAsync(dm.data(), t->d_depth_mean, sizeof(float) * B, cudaMemcpyDeviceToHost, s));
-  CU(cudaMemcpyAsync(dn.data(), t->d_depth_min, sizeof(float) * B, cudaMemcpyDeviceToHost, s));
-  CU(cudaMemcpyAsync(n.data(), t->d_sd_n, sizeof(int) * B, cudaMemcpyDeviceToHost, s));
+  CU(cudaMemcpyAsync(dm.data(), t->slots.depth_mean, sizeof(float) * B, cudaMemcpyDeviceToHost, s));
+  CU(cudaMemcpyAsync(dn.data(), t->slots.depth_min, sizeof(float) * B, cudaMemcpyDeviceToHost, s));
+  CU(cudaMemcpyAsync(n.data(), t->slots.sd_n, sizeof(int) * B, cudaMemcpyDeviceToHost, s));
   CU(cudaStreamSynchronize(s));
   for (int b = 0; b < B; ++b) {
     if (n[b] > 0) { depth_mean[b] = dm[b]; depth_min[b] = dn[b]; }
@@ -1026,7 +1069,7 @@ int svob200_tracker_get_seed_refs(svob200_tracker* t, double* px, int* level, in
   svob200_ctx* ctx = t->ctx;
   if (int e = ctx_join_aux(ctx)) return e;
   std::vector<SeedRef> refs((size_t)std::max(t->S, 1));
-  CU(cudaMemcpyAsync(refs.data(), t->d_seed_refs, sizeof(SeedRef) * (size_t)t->S, cudaMemcpyDeviceToHost, ctx->stream));
+  CU(cudaMemcpyAsync(refs.data(), t->slots.seed_refs, sizeof(SeedRef) * (size_t)t->S, cudaMemcpyDeviceToHost, ctx->stream));
   CU(cudaStreamSynchronize(ctx->stream));
   for (int i = 0; i < t->S; ++i) {
     if (px) { px[2 * i] = refs[i].px[0]; px[2 * i + 1] = refs[i].px[1]; }
@@ -1049,10 +1092,10 @@ int svob200_tracker_get_points(svob200_tracker* t, double* pos, int* type, int* 
   const int B = t->batch;
   std::vector<svob200_map_point> pts((size_t)std::max(t->N, 1));
   std::vector<int> cr(B, 0), dr(B, 0);
-  if (t->N) CU(cudaMemcpyAsync(pts.data(), t->d_points, sizeof(svob200_map_point) * (size_t)t->N, cudaMemcpyDeviceToHost, ctx->stream));
-  if (t->d_pt_created) {
-    CU(cudaMemcpyAsync(cr.data(), t->d_pt_created, sizeof(int) * B, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaMemcpyAsync(dr.data(), t->d_pt_dropped, sizeof(int) * B, cudaMemcpyDeviceToHost, ctx->stream));
+  if (t->N) CU(cudaMemcpyAsync(pts.data(), t->slots.points, sizeof(svob200_map_point) * (size_t)t->N, cudaMemcpyDeviceToHost, ctx->stream));
+  if (t->pt_capacity >= 0 && !t->slots.mem.empty()) {          // a point pool
+    CU(cudaMemcpyAsync(cr.data(), t->slots.pt_created, sizeof(int) * B, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaMemcpyAsync(dr.data(), t->slots.pt_dropped, sizeof(int) * B, cudaMemcpyDeviceToHost, ctx->stream));
   }
   CU(cudaStreamSynchronize(ctx->stream));
   for (int i = 0; i < t->N; ++i) {
@@ -1065,12 +1108,13 @@ int svob200_tracker_get_points(svob200_tracker* t, double* pos, int* type, int* 
   return SVOB200_OK;
 }
 int svob200_tracker_num_point_slots(svob200_tracker* t) { return t ? t->N : 0; }
+long long svob200_tracker_device_bytes(const svob200_tracker* t) { return t ? t->slots.mem.bytes() + t->det.mem.bytes() + t->chain.mem.bytes() : 0; }
 
 int svob200_tracker_set_chain(svob200_tracker* t, int cell_size, int max_fts, int pose_opt)
 {
   if (!t) return SVOB200_ERR_ARG;
   svob200_ctx* ctx = t->ctx;
-  if (!t->d_stats) return fail(ctx, SVOB200_ERR_ARG, "tracker_set_chain: set_keyframe first");
+  if (t->slots.mem.empty()) return fail(ctx, SVOB200_ERR_ARG, "tracker_set_chain: set_keyframe first");
   if (t->pt_capacity >= 0) return fail(ctx, SVOB200_ERR_UNSUPPORTED, "tracker_set_chain: not available with a point pool");
   if (int e = ctx_join_aux(ctx)) return e;
   CU(cudaStreamSynchronize(ctx->stream));
@@ -1079,20 +1123,22 @@ int svob200_tracker_set_chain(svob200_tracker* t, int cell_size, int max_fts, in
   const int B = t->batch, N = t->N;
   const long long n_cells = grid_cells(t->cam.width, t->cam.height, cell_size);
   if (n_cells > kMaxGridCells) return fail(ctx, SVOB200_ERR_UNSUPPORTED, "tracker_set_chain: grid of %lld cells exceeds the limit of %d", n_cells, kMaxGridCells);
-  if (!t->d_reproj || n_cells != t->chain_cells) {
+  if (t->chain.mem.empty() || n_cells != t->chain.n_cells) {
     const size_t M = (size_t)B * n_cells;
-    int err = 0;
-    auto own = [&](auto*& p, size_t n) { if (!err) err = alloc_owned(t, p, n); };
-    if (!t->d_reproj) { own(t->d_reproj, N); own(t->d_rstats, B); own(t->d_pose, B); own(t->d_m_count, B); own(t->d_seg_begin, B); own(t->d_seg_end, B);
-                        own(t->d_reproj_scratch, reproject_scratch_bytes(N)); }
-    own(t->d_winner, M); own(t->d_m_level, M); own(t->d_m_point, M); own(t->d_m_f, 3 * M); own(t->d_m_pos, 3 * M); own(t->d_pose_work, M); own(t->d_outlier, M);
-    if (err) return err;
+    Chain g;
+    DevArrays& m = g.mem;
+    if (!(m.alloc(g.reproj, N) && m.alloc(g.rstats, B) && m.alloc(g.pose, B) && m.alloc(g.m_count, B) && m.alloc(g.seg_begin, B) &&
+          m.alloc(g.seg_end, B) && m.alloc(g.reproj_scratch, reproject_scratch_bytes(N)) && m.alloc(g.winner, M) && m.alloc(g.m_level, M) &&
+          m.alloc(g.m_point, M) && m.alloc(g.m_f, 3 * M) && m.alloc(g.m_pos, 3 * M) && m.alloc(g.pose_work, M) && m.alloc(g.outlier, M)))
+      return fail(ctx, SVOB200_ERR_NOMEM, "tracker_set_chain: out of device memory for the chain arrays");
+    g.n_cells = (int)n_cells;
+    t->chain = std::move(g);
   }
-  // the map points as reprojector candidates: insertion order = the keyframe's fts_ order, every point TYPE_UNKNOWN (d_points /
-  // d_obs / d_T_obs already hold them with their observation lists)
-  CU(cudaMemsetAsync(t->d_pose, 0, sizeof(svob200_pose_opt_result) * (size_t)B, ctx->stream));
+  t->chain_cell = cell_size; t->chain_max_fts = max_fts; t->chain_pose_opt = pose_opt ? 1 : 0;
+  // the map points as reprojector candidates: insertion order = the keyframe's fts_ order, every point TYPE_UNKNOWN (slots.points
+  // / pobs / T_pobs already hold them with their observation lists)
+  CU(cudaMemsetAsync(t->chain.pose, 0, sizeof(svob200_pose_opt_result) * (size_t)B, ctx->stream));
   CU(cudaStreamSynchronize(ctx->stream));
-  t->chain_cell = cell_size; t->chain_max_fts = max_fts; t->chain_pose_opt = pose_opt ? 1 : 0; t->chain_cells = (int)n_cells;
   return SVOB200_OK;
 }
 
@@ -1126,8 +1172,8 @@ static int enqueue_seeds_update(svob200_tracker* t, int c0, int c1, const SeedPo
   svob200_ctx* ctx = t->ctx;
   const int s0 = t->h_seed_off[c0], ns = t->h_seed_off[c1] - s0;
   CU_AT("tracker_step: launch_seeds_update_compact",
-        launch_seeds_update_compact(ctx->d_table, find_frame(ctx, t->fid_cur)->slot, to_cam(&t->cam), ns, t->d_seed_refs + s0, t->d_kf_slot, t->batch, table,
-                                    t->d_batch_counter, t->max_n_kfs, t->mopts, t->conv_thresh, t->d_seeds + s0, t->d_obs + s0, t->d_seed_scratch, t->S, s0,
+        launch_seeds_update_compact(ctx->d_table, find_frame(ctx, t->fid_cur)->slot, to_cam(&t->cam), ns, t->slots.seed_refs + s0, t->slots.kf_slot, t->batch, table,
+                                    t->slots.batch_counter, t->max_n_kfs, t->mopts, t->conv_thresh, t->slots.seeds + s0, t->slots.obs + s0, t->slots.seed_scratch, t->S, s0,
                                     st, &ctx->launches, marks));
   return 0;
 }
@@ -1137,14 +1183,14 @@ static int enqueue_step_stats(svob200_tracker* t, int c0, int c1, int parts, svo
 {
   svob200_ctx* ctx = t->ctx;
   const int cnt = c1 - c0, par = (int)(t->step_no & 1);
-  const CandStage cand = {t->d_cand[par], t->d_cand_n[par], t->d_pt_created, t->d_ftr_off, t->d_T_kf, t->batch, c0};
+  const CandStage cand = {t->slots.cand[par], t->slots.cand_n[par], t->slots.pt_created, t->slots.ftr_off, t->slots.T_kf, t->batch, c0};
   auto kernel = cand.rec ? step_stats_kernel<true> : step_stats_kernel<false>;
-  kernel<<<cnt, 128, 0, st>>>(t->d_ftr_off + c0, t->d_seed_off + c0, t->d_align + c0, t->d_T_cur + 7 * (size_t)c0, t->d_match_ok, t->d_obs,
-                              t->d_seeds, t->seed_init, t->reseed, d_stats + c0, parts, t->d_seed_refs, cand);
+  kernel<<<cnt, 128, 0, st>>>(t->slots.ftr_off + c0, t->slots.seed_off + c0, t->slots.align + c0, t->slots.T_cur + 7 * (size_t)c0, t->slots.match_ok, t->slots.obs,
+                              t->slots.seeds, t->seed_init, t->reseed, d_stats + c0, parts, t->slots.seed_refs, cand);
   ++ctx->launches;
   CU_AT("tracker_step: step_stats_kernel", cudaGetLastError());
   if (t->chain_cell > 0) {
-    chain_stats_kernel<<<(cnt + 127) / 128, 128, 0, st>>>(cnt, t->d_rstats + c0, t->d_pose + c0, t->chain_pose_opt, d_stats + c0); ++ctx->launches;
+    chain_stats_kernel<<<(cnt + 127) / 128, 128, 0, st>>>(cnt, t->chain.rstats + c0, t->chain.pose + c0, t->chain_pose_opt, d_stats + c0); ++ctx->launches;
     CU_AT("tracker_step: chain_stats_kernel", cudaGetLastError());
   }
   return 0;
@@ -1157,9 +1203,9 @@ static int enqueue_insert_candidates(svob200_tracker* t)
   if (t->pt_capacity < 0) return 0;
   svob200_ctx* ctx = t->ctx;
   const int par = (int)(t->step_no & 1);
-  cand_insert_kernel<<<t->batch, 128, 0, ctx->stream>>>(t->max_kfs, t->batch, t->d_ftr_off, t->d_cand[par], t->d_cand_n[par], t->d_kf_batch, t->d_kf_slot, t->d_T_kf,
-                                                        t->d_points, t->d_pt_world, t->d_pobs, t->d_T_pobs, t->d_sel, t->d_has_point, t->d_pt_rank,
-                                                        t->d_pt_dropped);
+  cand_insert_kernel<<<t->batch, 128, 0, ctx->stream>>>(t->max_kfs, t->batch, t->slots.ftr_off, t->slots.cand[par], t->slots.cand_n[par], t->slots.kf_batch,
+                                                        t->slots.kf_slot, t->slots.T_kf, t->slots.points, t->slots.pt_world, t->slots.pobs, t->slots.T_pobs, t->slots.sel,
+                                                        t->slots.has_point, t->slots.pt_rank, t->slots.pt_dropped);
   ++ctx->launches;
   CU_AT("tracker_step: cand_insert_kernel", cudaGetLastError());
   return 0;
@@ -1195,17 +1241,17 @@ static int run_range(svob200_tracker* t, int c0, int c1, const double* d_T_last,
   MARK(1);
   // 2. Feature ctor / xyz_ref of the last frame's features, initial relative pose
   CU_AT("tracker_step: launch_features_prepare",
-        launch_features_prepare(cam, nf, d_last_px + 2 * (size_t)f0, t->d_pt_world + 3 * (size_t)f0, t->d_ftr_image + f0, d_T_last, nullptr,
-                                t->d_xyz + 3 * (size_t)f0, s2, &ctx->launches));
-  init_pose_kernel<<<(cnt + 127) / 128, 128, 0, s2>>>(cnt, d_T_last + 7 * (size_t)c0, t->d_T_init + 7 * (size_t)c0); ++ctx->launches;
+        launch_features_prepare(cam, nf, d_last_px + 2 * (size_t)f0, t->slots.pt_world + 3 * (size_t)f0, t->slots.ftr_image + f0, d_T_last, nullptr,
+                                t->slots.xyz + 3 * (size_t)f0, s2, &ctx->launches));
+  init_pose_kernel<<<(cnt + 127) / 128, 128, 0, s2>>>(cnt, d_T_last + 7 * (size_t)c0, t->slots.T_init + 7 * (size_t)c0); ++ctx->launches;
   CU_AT("tracker_step: init_pose_kernel", cudaGetLastError());
   if (fork) { CU(cudaEventRecord(t->fork_ev[1], s2)); CU(cudaStreamWaitEvent(s, t->fork_ev[1], 0)); }
   MARK(2);
   // 3. SparseImgAlign::run(last, cur)
   CU_AT("tracker_step: launch_sparse_align",
-        launch_sparse_align(vlast, vcur, cam, cnt, t->N, t->max_per, t->d_ftr_off + c0, d_last_px, t->d_xyz, t->d_has_point,
-                            t->d_T_init + 7 * (size_t)c0, t->aopts, t->d_align + c0, t->d_align_scratch, s, &ctx->launches,
-                            d_T_last + 7 * (size_t)c0, t->d_T_cur + 7 * (size_t)c0));
+        launch_sparse_align(vlast, vcur, cam, cnt, t->N, t->max_per, t->slots.ftr_off + c0, d_last_px, t->slots.xyz, t->slots.has_point,
+                            t->slots.T_init + 7 * (size_t)c0, t->aopts, t->slots.align + c0, t->slots.align_scratch, s, &ctx->launches,
+                            d_T_last + 7 * (size_t)c0, t->slots.T_cur + 7 * (size_t)c0));
   MARK(3);
   // 4. cur.T_f_w = T_cur_from_ref * last.T_f_w (written by the alignment kernel's epilogue) ; reprojection of the map points
   // chain mode: the depth filter waits for the pose optimiser's T_cur, so its branch cannot start here
@@ -1213,8 +1259,8 @@ static int run_range(svob200_tracker* t, int c0, int c1, const double* d_T_last,
   if (s_seeds != s) { CU(cudaEventRecord(t->fork_ev[2], s)); CU(cudaStreamWaitEvent(s_seeds, t->fork_ev[2], 0)); }
   if (t->chain_cell <= 0 && nf > 0) {
     // Point::getCloseViewObs per map point + px = cur.w2c(pos), depth_ref, T_cur_ref (the head of findMatchDirect)
-    points_select_kernel<<<(nf + 127) / 128, 128, 0, s>>>(cam, nf, t->d_points + f0, t->d_pobs, t->d_T_pobs, t->d_ftr_image + f0, t->d_T_cur, t->d_ftrs + f0,
-                                                          t->d_depth_ref + f0, t->d_px_in + 2 * (size_t)f0, t->d_active + f0, t->d_sel + f0);
+    points_select_kernel<<<(nf + 127) / 128, 128, 0, s>>>(cam, nf, t->slots.points + f0, t->slots.pobs, t->slots.T_pobs, t->slots.ftr_image + f0, t->slots.T_cur,
+                                                          t->slots.ftrs + f0, t->slots.depth_ref + f0, t->slots.px_in + 2 * (size_t)f0, t->slots.active + f0, t->slots.sel + f0);
     ++ctx->launches;
     CU_AT("tracker_step: points_select_kernel", cudaGetLastError());
   }
@@ -1223,38 +1269,38 @@ static int run_range(svob200_tracker* t, int c0, int c1, const double* d_T_last,
     // 4b-5. chain mode: Reprojector::reprojectMap (grid, every in-frame candidate matched in parallel, per-cell first success,
     // maxFts) over the keyframe's map points, then pose_optimizer::optimizeGaussNewton on the frame's new features (in place
     // on T_cur, so the depth filter sees the optimised pose).
-    const size_t cb = (size_t)c0 * t->chain_cells;
+    const size_t cb = (size_t)c0 * t->chain.n_cells;
     CU_AT("tracker_step: launch_reproject_map",
-          launch_reproject_map(ctx->d_table, cur->slot, cam, cnt, t->d_T_cur + 7 * (size_t)c0, t->d_ftr_off + c0, t->N, t->d_points, t->d_pobs,
-                               t->d_T_pobs, t->chain_cell, t->chain_max_fts, t->mopts, t->d_reproj, t->d_winner + cb, t->d_rstats + c0,
-                               t->d_reproj_scratch, t->d_match_scratch, t->d_m_f + 3 * cb, t->d_m_level + cb, t->d_m_pos + 3 * cb,
-                               t->d_m_point + cb, t->d_m_count + c0, s, &ctx->launches, c0, f0, nf));
+          launch_reproject_map(ctx->d_table, cur->slot, cam, cnt, t->slots.T_cur + 7 * (size_t)c0, t->slots.ftr_off + c0, t->N, t->slots.points, t->slots.pobs,
+                               t->slots.T_pobs, t->chain_cell, t->chain_max_fts, t->mopts, t->chain.reproj, t->chain.winner + cb, t->chain.rstats + c0,
+                               t->chain.reproj_scratch, t->slots.match_scratch, t->chain.m_f + 3 * cb, t->chain.m_level + cb, t->chain.m_pos + 3 * cb,
+                               t->chain.m_point + cb, t->chain.m_count + c0, s, &ctx->launches, c0, f0, nf));
     MARK(5); MARK(6);
-    chain_export_kernel<<<(nf + 127) / 128, 128, 0, s>>>(nf, t->d_reproj + f0, t->d_px_out + 2 * (size_t)f0, t->d_match_ok + f0); ++ctx->launches;
+    chain_export_kernel<<<(nf + 127) / 128, 128, 0, s>>>(nf, t->chain.reproj + f0, t->slots.px_out + 2 * (size_t)f0, t->slots.match_ok + f0); ++ctx->launches;
     CU_AT("tracker_step: chain_export_kernel", cudaGetLastError());
     if (t->chain_pose_opt) {
-      chain_segments_kernel<<<(cnt + 127) / 128, 128, 0, s>>>(cnt, t->chain_cells, t->d_m_count + c0, t->d_seg_begin + c0, t->d_seg_end + c0); ++ctx->launches;
+      chain_segments_kernel<<<(cnt + 127) / 128, 128, 0, s>>>(cnt, t->chain.n_cells, t->chain.m_count + c0, t->chain.seg_begin + c0, t->chain.seg_end + c0); ++ctx->launches;
       CU_AT("tracker_step: chain_segments_kernel", cudaGetLastError());
       // segments are relative to this range's slice of the compacted arrays
       CU_AT("tracker_step: launch_pose_optimize",
-            launch_pose_optimize(cam, cnt, t->d_seg_begin + c0, t->d_seg_end + c0, t->d_m_f + 3 * cb, t->d_m_level + cb, t->d_m_pos + 3 * cb, 2.0, 10,
-                                 0.0000000001, 8.6851f, t->d_T_cur + 7 * (size_t)c0, t->d_pose + c0, t->d_outlier + cb, t->d_pose_work + cb, s, &ctx->launches));
+            launch_pose_optimize(cam, cnt, t->chain.seg_begin + c0, t->chain.seg_end + c0, t->chain.m_f + 3 * cb, t->chain.m_level + cb, t->chain.m_pos + 3 * cb, 2.0, 10,
+                                 0.0000000001, 8.6851f, t->slots.T_cur + 7 * (size_t)c0, t->chain.pose + c0, t->chain.outlier + cb, t->chain.pose_work + cb, s, &ctx->launches));
     }
     MARK(7);
   } else {
   // 5. Matcher::findMatchDirect per map point (keyframe patch -> current frame)
   // (item indices inside the call are relative to f0, so the output arrays are passed at f0 as well)
   CU_AT("tracker_step: launch_match_direct",
-        launch_match_direct(ctx->d_table, cur->slot, cam, nf, t->d_ftrs + f0, t->d_depth_ref + f0, t->d_px_in + 2 * (size_t)f0, t->mopts, nullptr,
-                            t->d_px_out + 2 * (size_t)f0, t->d_match_ok + f0, t->d_match_scratch, t->N, f0, s, &ctx->launches,
-                            (marks && t->profiling) ? &t->ev[5] : nullptr, t->d_active + f0, t->d_match_level + f0, t->d_match_A + 4 * (size_t)f0));
+        launch_match_direct(ctx->d_table, cur->slot, cam, nf, t->slots.ftrs + f0, t->slots.depth_ref + f0, t->slots.px_in + 2 * (size_t)f0, t->mopts, nullptr,
+                            t->slots.px_out + 2 * (size_t)f0, t->slots.match_ok + f0, t->slots.match_scratch, t->N, f0, s, &ctx->launches,
+                            (marks && t->profiling) ? &t->ev[5] : nullptr, t->slots.active + f0, t->slots.match_level + f0, t->slots.match_A + 4 * (size_t)f0));
   MARK(7);
   }
-  if (out_px) CU(cudaMemcpyAsync(out_px + 2 * (size_t)f0, t->d_px_out + 2 * (size_t)f0, sizeof(double) * 2 * (size_t)nf, cudaMemcpyDeviceToDevice, s));
-  if (out_ok) CU(cudaMemcpyAsync(out_ok + f0, t->d_match_ok + f0, sizeof(int) * (size_t)nf, cudaMemcpyDeviceToDevice, s));
+  if (out_px) CU(cudaMemcpyAsync(out_px + 2 * (size_t)f0, t->slots.px_out + 2 * (size_t)f0, sizeof(double) * 2 * (size_t)nf, cudaMemcpyDeviceToDevice, s));
+  if (out_ok) CU(cudaMemcpyAsync(out_ok + f0, t->slots.match_ok + f0, sizeof(int) * (size_t)nf, cudaMemcpyDeviceToDevice, s));
   // 6. DepthFilter::updateSeeds(cur): this range's rows of the pose table (from the step's final T_cur), then the seeds
   CU_AT("tracker_step: launch_seed_pose_table",
-        launch_seed_pose_table(cam, t->batch, t->n_kfs, c0, cnt, t->d_T_kf, t->d_T_cur, sh.pose_table, s_seeds, &ctx->launches));
+        launch_seed_pose_table(cam, t->batch, t->n_kfs, c0, cnt, t->slots.T_kf, t->slots.T_cur, sh.pose_table, s_seeds, &ctx->launches));
   if (sh.defer_df) {
     // asynchronous depth filter (never forked: s_seeds == s): the df stream starts from the pose rows and writes its half of
     // the step records after the tracking half; the events tell it when
@@ -1278,7 +1324,7 @@ int svob200_tracker_step(svob200_tracker* t, const uint8_t* cur_imgs, int stride
 {
   if (!t || !cur_imgs || !T_last_w || !last_px) return SVOB200_ERR_ARG;
   svob200_ctx* ctx = t->ctx;
-  if (!t->d_stats) return fail(ctx, SVOB200_ERR_ARG, "tracker_step: set_keyframe first");
+  if (t->slots.mem.empty()) return fail(ctx, SVOB200_ERR_ARG, "tracker_step: set_keyframe first");
   const int B = t->batch, N = t->N;
   cudaStream_t s = ctx->stream;
   const size_t in_bytes = sizeof(double) * (7 * (size_t)B + 2 * (size_t)N);
@@ -1311,8 +1357,8 @@ int svob200_tracker_step(svob200_tracker* t, const uint8_t* cur_imgs, int stride
     if (int e = enqueue_insert_candidates(t)) return e;
     // graph + fork (only a capture runs the body then), asynchronous depth filter on this parity's pose table and step
     // records, or in place; with a point pool the captured step records its candidates into this parity's staging
-    const RangeShape shape = {use_graph ? t->fork_stream : s, df_on_stream, (df_on_stream && par) ? t->d_seed_poses2 : t->d_seed_poses,
-                              (df_on_stream && par) ? t->d_stats2 : t->d_stats};
+    const RangeShape shape = {use_graph ? t->fork_stream : s, df_on_stream, (df_on_stream && par) ? t->slots.seed_poses2 : t->slots.seed_poses,
+                              (df_on_stream && par) ? t->slots.stats2 : t->slots.stats};
     const int rc = graph_or_direct(t, use_graph, key, [&]() -> int {
       if (int e = run_range(t, 0, B, T_last_w, last_px, true, shape, px_refined, match_ok)) return e;
       if (!df_on_stream) {
@@ -1345,8 +1391,8 @@ int svob200_tracker_step(svob200_tracker* t, const uint8_t* cur_imgs, int stride
       CU(cudaMallocHost((void**)&t->h_pinned, in_bytes + out_bytes + 512));
       t->h_cap = in_bytes + out_bytes + 512;
     }
-    const double* d_T_last = t->d_step_in;
-    const double* d_last_px = t->d_step_in + 7 * (size_t)B;
+    const double* d_T_last = t->slots.step_in;
+    const double* d_last_px = t->slots.step_in + 7 * (size_t)B;
     // the per-step inputs (poses, last pixel positions: 16 B per feature) are queued BEFORE the frame chunks: H2D copies are
     // served in submission order whatever their stream, and the first chunk's kernels wait for these (queued after the
     // chunks they cost 24.1 -> 30.7 ms per step).  Page-locked caller buffers are read by the copy engine directly, pageable
@@ -1358,12 +1404,12 @@ int svob200_tracker_step(svob200_tracker* t, const uint8_t* cur_imgs, int stride
         return at.type == cudaMemoryTypeHost;
       };
       if (B >= 64 && is_pinned(T_last_w) && is_pinned(last_px)) {
-        CU(cudaMemcpyAsync(t->d_step_in, T_last_w, sizeof(double) * 7 * B, cudaMemcpyHostToDevice, s));
-        CU(cudaMemcpyAsync(t->d_step_in + 7 * (size_t)B, last_px, sizeof(double) * 2 * (size_t)N, cudaMemcpyHostToDevice, s));
+        CU(cudaMemcpyAsync(t->slots.step_in, T_last_w, sizeof(double) * 7 * B, cudaMemcpyHostToDevice, s));
+        CU(cudaMemcpyAsync(t->slots.step_in + 7 * (size_t)B, last_px, sizeof(double) * 2 * (size_t)N, cudaMemcpyHostToDevice, s));
       } else {
         memcpy(t->h_pinned, T_last_w, sizeof(double) * 7 * B);
         memcpy(t->h_pinned + sizeof(double) * 7 * B, last_px, sizeof(double) * 2 * (size_t)N);
-        CU(cudaMemcpyAsync(t->d_step_in, t->h_pinned, in_bytes, cudaMemcpyHostToDevice, s));
+        CU(cudaMemcpyAsync(t->slots.step_in, t->h_pinned, in_bytes, cudaMemcpyHostToDevice, s));
       }
     }
     if (int e = enqueue_insert_candidates(t)) return e;
@@ -1393,7 +1439,7 @@ int svob200_tracker_step(svob200_tracker* t, const uint8_t* cur_imgs, int stride
     // host mode: 0.202 -> 0.199 ms for C2.)
     const bool use_graph = !t->profiling && n_chunks == 1 && B <= svob200_tracker::GRAPH_MAX_BATCH;
     if (use_graph) if (int e = ensure_fork_stream(t)) return e;
-    const RangeShape shape = {use_graph ? t->fork_stream : s, false, t->d_seed_poses, t->d_stats};
+    const RangeShape shape = {use_graph ? t->fork_stream : s, false, t->slots.seed_poses, t->slots.stats};
     // each chunk's kernels wait for its own frame copy
     for (int c = 0; c < n_chunks; ++c) {
       const int c0 = c * chunk, c1 = std::min(B, c0 + chunk);
@@ -1408,9 +1454,9 @@ int svob200_tracker_step(svob200_tracker* t, const uint8_t* cur_imgs, int stride
     }
     uint8_t* ho = t->h_pinned + ((in_bytes + 255) & ~(size_t)255);
     uint8_t* h_stats = ho; uint8_t* h_px = h_stats + sizeof(svob200_step_stats) * B; uint8_t* h_ok = h_px + sizeof(double) * 2 * (size_t)N;
-    if (stats) CU(cudaMemcpyAsync(h_stats, t->d_stats, sizeof(svob200_step_stats) * B, cudaMemcpyDeviceToHost, s));
-    if (px_refined) CU(cudaMemcpyAsync(h_px, t->d_px_out, sizeof(double) * 2 * (size_t)N, cudaMemcpyDeviceToHost, s));
-    if (match_ok) CU(cudaMemcpyAsync(h_ok, t->d_match_ok, sizeof(int) * (size_t)N, cudaMemcpyDeviceToHost, s));
+    if (stats) CU(cudaMemcpyAsync(h_stats, t->slots.stats, sizeof(svob200_step_stats) * B, cudaMemcpyDeviceToHost, s));
+    if (px_refined) CU(cudaMemcpyAsync(h_px, t->slots.px_out, sizeof(double) * 2 * (size_t)N, cudaMemcpyDeviceToHost, s));
+    if (match_ok) CU(cudaMemcpyAsync(h_ok, t->slots.match_ok, sizeof(int) * (size_t)N, cudaMemcpyDeviceToHost, s));
     CU(cudaStreamSynchronize(s));
     if (stats) memcpy(stats, h_stats, sizeof(svob200_step_stats) * B);
     if (px_refined) memcpy(px_refined, h_px, sizeof(double) * 2 * (size_t)N);
@@ -1426,7 +1472,7 @@ int svob200_tracker_get_seeds(svob200_tracker* t, svob200_seed* out)
   if (!t || !out) return SVOB200_ERR_ARG;
   svob200_ctx* ctx = t->ctx;
   if (int e = ctx_join_aux(ctx)) return e;
-  CU(cudaMemcpyAsync(out, t->d_seeds, sizeof(svob200_seed) * (size_t)t->S, cudaMemcpyDeviceToHost, ctx->stream));
+  CU(cudaMemcpyAsync(out, t->slots.seeds, sizeof(svob200_seed) * (size_t)t->S, cudaMemcpyDeviceToHost, ctx->stream));
   CU(cudaStreamSynchronize(ctx->stream));
   return SVOB200_OK;
 }
@@ -1436,9 +1482,9 @@ int svob200_tracker_launches_per_step(void) { return 14; }
 // raw svob200_align_result records of the most recent step (diagnostics: tools/align_timing.py)
 int svob200_tracker_debug_align(svob200_tracker* t, svob200_align_result* out)
 {
-  if (!t || !out || !t->d_align) return SVOB200_ERR_ARG;
+  if (!t || !out || t->slots.mem.empty()) return SVOB200_ERR_ARG;
   svob200_ctx* ctx = t->ctx;
-  CU(cudaMemcpyAsync(out, t->d_align, sizeof(svob200_align_result) * (size_t)t->batch, cudaMemcpyDeviceToHost, ctx->stream));
+  CU(cudaMemcpyAsync(out, t->slots.align, sizeof(svob200_align_result) * (size_t)t->batch, cudaMemcpyDeviceToHost, ctx->stream));
   CU(cudaStreamSynchronize(ctx->stream));
   return SVOB200_OK;
 }
@@ -1471,7 +1517,7 @@ int svob200_tracker_get_seed_obs(svob200_tracker* t, svob200_seed_obs* out)
   if (!t || !out) return SVOB200_ERR_ARG;
   svob200_ctx* ctx = t->ctx;
   if (int e = ctx_join_aux(ctx)) return e;
-  CU(cudaMemcpyAsync(out, t->d_obs, sizeof(svob200_seed_obs) * (size_t)t->S, cudaMemcpyDeviceToHost, ctx->stream));
+  CU(cudaMemcpyAsync(out, t->slots.obs, sizeof(svob200_seed_obs) * (size_t)t->S, cudaMemcpyDeviceToHost, ctx->stream));
   CU(cudaStreamSynchronize(ctx->stream));
   return SVOB200_OK;
 }

@@ -281,7 +281,8 @@ int  svob200_tracker_create(svob200_ctx* ctx, const svob200_camera* cam, int bat
                             double seed_convergence_sigma2_thresh, float depth_mean, float depth_min, int reseed,
                             svob200_tracker** out);
 void svob200_tracker_destroy(svob200_tracker* t);
-/* all arguments in host memory; offsets are batch+1 prefix sums */
+/* all arguments in host memory; offsets are batch+1 prefix sums.
+ * Sizing calls (set_keyframe, set_detector, set_chain, add_keyframes): SVOB200_ERR_NOMEM leaves the tracker as it was. */
 int  svob200_tracker_set_keyframe(svob200_tracker* t, const uint8_t* imgs, int stride, const double* T_kf_w,
                                   const int* ftr_offsets, const double* kf_px, const int* kf_level,
                                   const double* pt_world, const int* seed_offsets, const double* seed_px,
@@ -295,7 +296,8 @@ int  svob200_tracker_set_last(svob200_tracker* t, const uint8_t* imgs, int strid
  *   older than `max_n_kfs` keyframe insertions are erased (DepthFilter::Options::max_n_kfs, default 3); reseed as in
  *   svob200_tracker_create, plus 3 = finished seeds (converged / NaN) leave the pool like they leave the reference's list.
  * svob200_tracker_set_detector: FastDetector(cell size = Config::gridSize, levels = Config::nPyrLevels) and the threshold
- *   DepthFilter::initializeSeeds passes (Config::triangMinCornerScore).
+ *   DepthFilter::initializeSeeds passes (Config::triangMinCornerScore).  A grid of another cell count releases the detector
+ *   scratch, after synchronising with the context's stream.
  * Every sequence has its own keyframe ring, as if it were its own FrameHandlerMono + DepthFilter: its own ring indices
  *   (a free one, else its oldest keyframe leaves), its own Seed::batch_counter and its own evictions.  The keyframe images live
  *   in a store of max_keyframes frame batches (ring index k of sequence b = image b of store frame k); an insertion copies the
@@ -317,7 +319,8 @@ int  svob200_tracker_set_last(svob200_tracker* t, const uint8_t* imgs, int strid
  *   takes at most 65,534 keyframes; a selected sequence past that is left untouched and reports -1 in both counts (the limit
  *   counts the sequence's own keyframes, not calls).  mem: where ALL
  *   the arrays live.  In SVOB200_MEM_DEVICE mode the call is ordered on the context's stream and does not synchronise with
- *   the host (the first insertion allocates the keyframe store when svob200_tracker_set_seed_pool did not).  Not available in
+ *   the host, except that the first insertion after set_keyframe or after set_detector changed the grid allocates the
+ *   detector scratch (and the keyframe store when svob200_tracker_set_seed_pool did not).  Not available in
  *   chain mode (SVOB200_ERR_UNSUPPORTED); SVOB200_ERR_ARG before set_keyframe, before the first step, or for a bad mem.
  * svob200_tracker_add_keyframe(t, dm, dn, nn, nd) = svob200_tracker_add_keyframes(t, NULL, dm, dn, nn, nd, SVOB200_MEM_HOST).
  * svob200_tracker_scene_depth: frame_utils::getSceneDepth of the most recent step's frame, per sequence, over the point slots
@@ -364,7 +367,7 @@ int  svob200_tracker_get_points(svob200_tracker* t, double* pos, int* type, int*
  * pose_opt != 0, pose_optimizer::optimizeGaussNewton on the matched features — FrameHandlerMono::processFrame's Step 2 and
  * Step 3 (frame_handler_mono.cpp:191-222) — instead of refining every map point; the depth filter then sees the optimised
  * pose.  Every point enters as TYPE_UNKNOWN each frame (the per-point reprojection counters are host-side map management).
- * cell_size <= 0 switches back. */
+ * cell_size <= 0 switches back (the chain arrays stay for the next switch). */
 int  svob200_tracker_set_chain(svob200_tracker* t, int cell_size, int max_fts, int pose_opt);
 /* cur_imgs: batch images; T_last_w: 7 doubles per sequence (pose of the last frame); last_px: 2 doubles
  * per map feature (its pixel in the last frame).  stats (batch), px_refined (2 per feature), match_ok
@@ -389,6 +392,8 @@ int  svob200_tracker_num_stages(void);
 const char* svob200_tracker_stage_name(int i);
 int  svob200_tracker_stage_ms(svob200_tracker* t, float* ms, int cap);
 int  svob200_tracker_get_seed_obs(svob200_tracker* t, svob200_seed_obs* out /*host*/);
+/* bytes of device memory the tracker's own arrays hold now (its frames, held by the context's frame store, not included) */
+long long svob200_tracker_device_bytes(const svob200_tracker* t);
 
 /* ================================================================ callers either side of the hot path
  * (SURVEY.md §8f "next" rows; same conventions: POD, mem = HOST | DEVICE, int status) */
